@@ -13,6 +13,8 @@ output exchange; NCCL over NVLink; weak scaling: per-GPU fragments fixed).  Its 
 of the SAME comparison grouped on one GPU (outside the timed region).  --multi independent: one independent
 sequence-pair comparison per GPU.
 `--impl reference` times the reference's own CPU code (oracle/_ref, built from /root/reference) on host cores.
+`--dump-outputs DIR` (one GPU) writes what the last timed step left in HBM, as DIR/<name>.npy, so that two builds can be
+compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -54,7 +56,14 @@ def parse():
     ap.add_argument("--multi", default="partitioned", choices=["partitioned", "independent"],
                     help="N > 1: one comparison range-partitioned over the GPUs (default) or one independent comparison per GPU")
     ap.add_argument("--profile-kernels", type=int, default=1, help="CUDA-event pairs around every kernel launch in the timed region")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output arrays of the last timed step to DIR/<name>.npy (float32/float64; our arm on one GPU only)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the output of our arm; the reference arm writes none")
+    return args
 
 
 def workload(args, rank=0):
@@ -255,6 +264,41 @@ ALG_BYTES_PER_UNIT = {
 }
 
 
+DUMP_MAX_LINES = 1 << 20   # --dump-outputs: larger outputs are sampled at this many seeded line positions (32 MB in all)
+
+
+class _DeviceArray:
+    """A 1-D array in the library's device memory, as torch.as_tensor sees it (no copy)."""
+
+    def __init__(self, ptr, n, typestr):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (ptr, False), "version": 2}
+
+
+def dump_outputs(out_dir, res, device):
+    """The arrays a caller of rk_group receives (order, gid, repval, identity; the last step's device buffers), plus n_kept
+    and n_groups, as DIR/<name>.npy.  Integers become float64 (exact), repval and identity float32.  Outputs of more than
+    DUMP_MAX_LINES lines are sampled at sorted line positions drawn with a fixed seed from n_kept alone, so two builds that
+    agree on n_kept sample the same lines; `line` holds the positions."""
+    import numpy as np
+    import torch
+    m = res.n_kept
+    line = np.arange(m, dtype=np.int64)
+    if m > DUMP_MAX_LINES:
+        line = np.sort(np.random.default_rng(0).choice(m, DUMP_MAX_LINES, replace=False))
+    out = {"n_kept": np.array([m], np.float64), "n_groups": np.array([res.n_groups], np.float64), "line": line.astype(np.float64)}
+    idx = torch.from_numpy(line).to(device)
+    for name, typestr, dt, ft in (("order", "<i4", np.uint32, np.float64), ("gid", "<i4", np.uint32, np.float64),
+                                  ("repval", "|u1", np.uint8, np.float32), ("identity", "<f4", np.float32, np.float32)):
+        v = np.zeros(0, dt)
+        if m:
+            t = torch.as_tensor(_DeviceArray(res.d_ptrs[name], m, typestr), device=device)
+            v = t[idx].cpu().numpy().view(dt)
+        out[name] = v.astype(ft)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+
+
 def ours(args):
     import numpy as np
     import torch
@@ -264,6 +308,8 @@ def ours(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the output of one process: run it with one GPU")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the product path has no CPU fallback")
     torch.cuda.set_device(local)
@@ -380,6 +426,8 @@ def ours(args):
         prof = ctx.profile_read(reset=True)
         ctx.profile_enable(False)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:   # before the e2e and checksum calls below overwrite the result buffers
+        dump_outputs(args.dump_outputs, last[1], device)
 
     if do_e2e:
         with torch.cuda.stream(stream):

@@ -64,7 +64,8 @@ def test_decomposition_invariants(medium_cases):
     assert int(roots.sum()) == g.n_groups
 
 
-@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref not built (no /root/reference on this box)")
+@pytest.mark.skipif(not O.have_ref(), reason="needs the compiled original repkiller in oracle/_ref; its output on this "
+                                                "workload is not stored in tests/golden")
 def test_oracle_vs_live_reference(tmp_path):
     """When the compiled reference is present, run it live on a fresh workload the fixtures do not hold."""
     from dataclasses import replace
