@@ -179,6 +179,44 @@ def std_sort_by_key(idx: np.ndarray, h: np.ndarray) -> np.ndarray:
     return out
 
 
+class Sol:
+    """One SequenceOcupationList of the restatement (rko_sol_*): the checker of repkiller_b200.capi.Sol"""
+
+    def __init__(self, len_ratio: float, pos_ratio: float, seq_size: int):
+        L = lib()
+        L.rko_sol_create.argtypes = [C.c_double, C.c_double, C.c_uint64]
+        L.rko_sol_create.restype = C.c_void_p
+        L.rko_sol_insert.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64]
+        L.rko_sol_get.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(C.c_uint64)]
+        L.rko_sol_destroy.argtypes = [C.c_void_p]
+        self._L = L
+        self._h = L.rko_sol_create(len_ratio, pos_ratio, seq_size)
+        if not self._h:
+            raise MemoryError("rko_sol_create")
+
+    def insert(self, center: int, length: int, tag: int) -> None:
+        rc = self._L.rko_sol_insert(self._h, center, length, tag)
+        if rc == -1:
+            raise IndexError(f"center {center} lies beyond the lists")
+        if rc:
+            raise MemoryError("rko_sol_insert")
+
+    def get(self, center: int, length: int) -> int:
+        """tag of the entry get_associated_group returns, 0 for none"""
+        t = C.c_uint64()
+        if self._L.rko_sol_get(self._h, center, length, C.byref(t)):
+            raise IndexError(f"a probe of center {center} reads beyond the lists")
+        return t.value
+
+    def close(self):
+        if self._h:
+            self._L.rko_sol_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        self.close()
+
+
 def have_ref() -> bool:
     return os.path.exists(REF_BIN) and os.access(REF_BIN, os.X_OK)
 

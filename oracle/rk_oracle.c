@@ -225,6 +225,52 @@ static int sol_insert(sol_t *s, pool_t *p, uint64_t center, uint64_t length, uin
   return 0;
 }
 
+/* the lists above behind an exported handle (rk_oracle.h); the entry's `rank` field is unused, its tag is tag[entry] */
+struct rko_sol {
+  sol_t s;
+  pool_t p;
+  uint64_t *tag;
+  size_t tag_cap;
+};
+
+rko_sol *rko_sol_create(double len_ratio, double pos_ratio, uint64_t seq_size) {
+  rko_sol *h = (rko_sol *)calloc(1, sizeof *h);
+  if (!h) return NULL;
+  if (sol_init(&h->s, len_ratio, pos_ratio, seq_size)) { free(h); return NULL; }
+  return h;
+}
+
+int rko_sol_insert(rko_sol *h, uint64_t center, uint64_t length, uint64_t tag) {
+  if (sol_insert(&h->s, &h->p, center, length, 0, 0)) return -1;
+  if (h->p.n > h->tag_cap) {
+    uint64_t *t = (uint64_t *)realloc(h->tag, h->p.cap * sizeof(uint64_t));
+    if (!t) { /* take the entry just pushed back: the list stays as it was */
+      const ocupation *o = &h->p.e[--h->p.n];
+      h->s.head[o->center / 100] = o->next;
+      return -2;
+    }
+    h->tag = t;
+    h->tag_cap = h->p.cap;
+  }
+  h->tag[h->p.n - 1] = tag;
+  return 0;
+}
+
+int rko_sol_get(const rko_sol *h, uint64_t center, uint64_t length, uint64_t *tag) {
+  const int64_t e = sol_get(&h->s, &h->p, center, length);
+  if (e == -2) return -2;
+  *tag = e >= 0 ? h->tag[e] : 0;
+  return 0;
+}
+
+void rko_sol_destroy(rko_sol *h) {
+  if (!h) return;
+  free(h->s.head);
+  free(h->p.e);
+  free(h->tag);
+  free(h);
+}
+
 /* ------------------------------------------------------------------------------------------------
  * std::sort as libstdc++ implements it (bits/stl_algo.h: __sort, __introsort_loop,
  * __unguarded_partition_pivot, __move_median_to_first, __final_insertion_sort; bits/stl_heap.h) —

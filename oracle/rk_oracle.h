@@ -85,6 +85,16 @@ typedef struct {
 } rko_group_stats;
 int rko_group_statistics(const rko_frag *recs, const rko_result *r, rko_group_stats *out /* r->n_groups entries */);
 
+/* One SequenceOcupationList (SequenceOcupationList.cpp:3-96) with a 64-bit tag per entry in place of the FragsGroup
+ * pointer: the checker of rk_sol_*.  insert returns -1 when center/100 lies beyond the lists, -2 when memory runs out
+ * (nothing inserted); get stores the tag of the winner (0: none) and returns -2 when a probe would read beyond the
+ * lists (the reference reads out of bounds). */
+typedef struct rko_sol rko_sol;
+rko_sol *rko_sol_create(double len_ratio, double pos_ratio, uint64_t seq_size);
+int rko_sol_insert(rko_sol *s, uint64_t center, uint64_t length, uint64_t tag);
+int rko_sol_get(const rko_sol *s, uint64_t center, uint64_t length, uint64_t *tag);
+void rko_sol_destroy(rko_sol *s);
+
 void rko_free(void *p);
 
 #ifdef __cplusplus

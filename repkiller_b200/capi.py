@@ -118,6 +118,13 @@ def load_library():
     L.rk_multi_load_aos.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint, C.POINTER(_LoadStats)]
     L.rk_multi_group.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_uint, C.POINTER(_Result)]
     L.rk_multi_info.argtypes = [C.c_void_p, C.c_int, C.POINTER(_DistInfo)]
+    L.rk_sol_create.argtypes = [C.c_int, C.c_double, C.c_double, C.c_uint64]
+    L.rk_sol_create.restype = C.c_void_p
+    L.rk_sol_destroy.argtypes = [C.c_void_p]
+    L.rk_sol_insert.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64]
+    L.rk_sol_get_associated.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(C.c_uint64)]
+    L.rk_sol_last_error.argtypes = [C.c_void_p]
+    L.rk_sol_last_error.restype = C.c_char_p
     _lib = L
     return L
 
@@ -379,6 +386,46 @@ def pack_records(rec: np.ndarray):
                       rec["similarity"].view(np.uint32)], axis=1)
     strand = rec["strand"].view(np.uint8).copy()
     return np.ascontiguousarray(key4), strand, np.ascontiguousarray(rest4)
+
+
+class Sol:
+    """One device-resident SequenceOcupationList (rk_sol_*): inserts are queued and applied in order before the next
+    query; a query returns the tag of the entry get_associated_group picks, 0 for none.  Tags must be non-zero."""
+
+    def __init__(self, device: int, len_ratio: float, pos_ratio: float, seq_size: int):
+        self._L = load_library()
+        self._h = self._L.rk_sol_create(device, len_ratio, pos_ratio, seq_size)
+        if not self._h:
+            raise RkError(-1, f"rk_sol_create({device}, {len_ratio}, {pos_ratio}, {seq_size}) failed")
+
+    def _check(self, rc: int):
+        if rc != 0:
+            raise RkError(rc, self._L.rk_sol_last_error(self._h).decode())
+
+    def insert(self, center: int, length: int, tag: int):
+        self._check(self._L.rk_sol_insert(self._h, center, length, tag))
+
+    def get_associated(self, center: int, length: int) -> int:
+        t = C.c_uint64()
+        self._check(self._L.rk_sol_get_associated(self._h, center, length, C.byref(t)))
+        return t.value
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._L.rk_sol_destroy(self._h)
+            self._h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def dist_unique_id() -> bytes:
