@@ -244,8 +244,9 @@ int rk_dist_load_aos(rk_ctx *ctx, const void *frags, uint64_t n_local, uint64_t 
 int rk_dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flags, rk_result *out, rk_dist_info *info);
 
 typedef struct rk_multi rk_multi;
-/* One context per listed device.  Distinct devices talk over NCCL; a device listed twice (tests on a one-GPU box) makes
- * the ranks exchange through device copies.  NULL on failure (rk_create_error). */
+/* One context per listed device.  The ranks push their rows into each other's device memory.  Distinct devices exchange
+ * the small tables and meet at barriers over NCCL; a device listed twice (tests on a one-GPU box), or NCCL failing to
+ * start, makes the ranks do that through host memory.  NULL on failure (rk_create_error). */
 rk_multi *rk_create_multi(const int *devices, int ndev);
 void rk_destroy_multi(rk_multi *m);
 const char *rk_multi_last_error(const rk_multi *m);

@@ -17,10 +17,12 @@
 //
 // Every rank's partition arena is carved identically and mapped into every peer (cudaIpc handles between processes, raw
 // pointers + cudaDeviceEnablePeerAccess inside one), so a local buffer address translates to the same buffer on any rank;
-// kernels store rows straight into it (k7_dist.cu: k_push_rows, scatter_store), copy engines push the Y rows.
-// NCCL (dlopen'ed: the process may already hold torch's libnccl.so.2) carries the small tables (ncclAllGather of counts,
-// histograms, link maps) and is the barrier behind every push.  Ranks that are threads of one process, possibly on the same
-// device (tests on a one-GPU box), exchange the small tables through host memory between host barriers instead.
+// kernels store rows straight into it (k7_dist.cu: k_push_rows, scatter_store), copy engines push the X halo and Y rows
+// (Transport::exchange_rows).  Rows travel this one way under both transports; they differ only in the small tables and
+// the barrier.  NCCL (dlopen'ed: the process may already hold torch's libnccl.so.2) carries the small tables
+// (ncclAllGather of counts, histograms, link maps) and is the barrier behind every push.  Ranks that are threads of one
+// process, possibly on the same device (tests on a one-GPU box), exchange the small tables through host memory between
+// host barriers instead, and their barrier is a stream synchronisation followed by a host barrier.
 #include <dlfcn.h>
 #include <nccl.h>
 #include <unistd.h>
@@ -48,11 +50,7 @@ struct NcclApi {
   decltype(&ncclCommInitRank) CommInitRank = nullptr;
   decltype(&ncclCommInitAll) CommInitAll = nullptr;
   decltype(&ncclCommDestroy) CommDestroy = nullptr;
-  decltype(&ncclSend) Send = nullptr;
-  decltype(&ncclRecv) Recv = nullptr;
   decltype(&ncclAllGather) AllGather = nullptr;
-  decltype(&ncclGroupStart) GroupStart = nullptr;
-  decltype(&ncclGroupEnd) GroupEnd = nullptr;
   decltype(&ncclGetErrorString) GetErrorString = nullptr;
   bool ok() const { return lib != nullptr && err.empty(); }
 };
@@ -74,11 +72,7 @@ static NcclApi &nccl_api() {
     RK_NCCL_SYM(CommInitRank, "ncclCommInitRank")
     RK_NCCL_SYM(CommInitAll, "ncclCommInitAll")
     RK_NCCL_SYM(CommDestroy, "ncclCommDestroy")
-    RK_NCCL_SYM(Send, "ncclSend")
-    RK_NCCL_SYM(Recv, "ncclRecv")
     RK_NCCL_SYM(AllGather, "ncclAllGather")
-    RK_NCCL_SYM(GroupStart, "ncclGroupStart")
-    RK_NCCL_SYM(GroupEnd, "ncclGroupEnd")
     RK_NCCL_SYM(GetErrorString, "ncclGetErrorString")
 #undef RK_NCCL_SYM
   });
@@ -98,44 +92,143 @@ constexpr int W_X2 = 43;         // forest: fragments of the rank whose chain is
 constexpr int W_CUTSX = 64;      // [2][nr] the first X super-bucket key every rank owns, per strand class
 constexpr int W_CUTS = 44;       // [nr+1] the cuts of the exchange (identical on every rank; the host sizes the local sort keys from them)
 
+struct Exchange {  // counts of one variable all-to-all, as this rank sees it (elements)
+  u64 soff[DIST_MAX_RANKS], scnt[DIST_MAX_RANKS], roff[DIST_MAX_RANKS], rcnt[DIST_MAX_RANKS];
+  u64 poff[DIST_MAX_RANKS];   // forward: start of my block in rank p's receive buffer (= p's roff[me])
+  u64 rpoff[DIST_MAX_RANKS];  // the way back: start of my block in rank p's send-order buffer (= p's soff[me])
+  u64 n_send = 0, n_recv = 0;
+  // from the gathered count matrix: row s = what rank s sends to every destination
+  void from_matrix(const u32 *h_all, int word0, int nr, int me) {
+    n_send = n_recv = 0;
+    for (int d = 0; d < nr; ++d) {
+      soff[d] = n_send;
+      scnt[d] = h_all[(size_t)me * SMALL_WORDS + word0 + d];
+      n_send += scnt[d];
+    }
+    for (int s = 0; s < nr; ++s) {
+      roff[s] = n_recv;
+      rcnt[s] = h_all[(size_t)s * SMALL_WORDS + word0 + me];
+      n_recv += rcnt[s];
+    }
+    for (int p = 0; p < nr; ++p) {
+      u64 f = 0, r = 0;
+      for (int s = 0; s < me; ++s) f += h_all[(size_t)s * SMALL_WORDS + word0 + p];
+      for (int d = 0; d < me; ++d) r += h_all[(size_t)p * SMALL_WORDS + word0 + d];
+      poff[p] = f, rpoff[p] = r;
+    }
+  }
+};
+
+// column `word` of the gathered count matrix summed over the ranks (word = W_CNT_A + d: the rows rank d receives)
+static u64 column_sum(const u32 *h_all, int word, int nr) {
+  u64 s = 0;
+  for (int r = 0; r < nr; ++r) s += h_all[(size_t)r * SMALL_WORDS + word];
+  return s;
+}
+
 struct Transport {
   int rank = 0, world = 1;
   std::string err;
   u64 bytes_sent = 0;  // payload this rank handed to other ranks
-  virtual ~Transport() {}
-  // every rank contributes SMALL_WORDS u32 from device memory; all rows land in h_all[world][SMALL_WORDS] (pinned).
-  // Synchronises the stream.
-  virtual int gather_small(const u32 *d_row, u32 *d_all, u32 *h_all, cudaStream_t st) = 0;
-  // The same in two halves: begin() leaves all rows in DEVICE memory d_all (stream-ordered: kernels queued behind it may
-  // read the other ranks' counts), end() brings them to the host and synchronises.
+  virtual ~Transport() {
+    if (ev_a) cudaEventDestroy(ev_a);
+    if (ev_b) cudaEventDestroy(ev_b);
+    for (auto &a : aux) if (a) cudaStreamDestroy(a);
+    for (auto &e : aux_ev) if (e) cudaEventDestroy(e);
+  }
+  // every rank contributes SMALL_WORDS u32 from device memory.  begin() leaves all rows in DEVICE memory d_all
+  // (stream-ordered: kernels queued behind it may read the other ranks' counts), end() brings them to the host
+  // h_all[world][SMALL_WORDS] (pinned) and synchronises the stream.
   virtual int gather_small_begin(const u32 *d_row, u32 *d_all, u32 *h_all, cudaStream_t st) = 0;
   virtual int gather_small_end(const u32 *d_all, u32 *h_all, cudaStream_t st) = 0;
   // all ranks' streams meet: work queued behind it starts after every rank's work queued before it is complete
   virtual int barrier(cudaStream_t st) = 0;
   // recv[world][bytes] <- every rank's send[bytes]; stream-ordered; doubles as a barrier between the ranks' streams
   virtual int all_gather(const void *send, void *recv, size_t bytes, cudaStream_t st) = 0;
-  // variable all-to-all; offsets and counts in elements of `elem` bytes.  poff[p] = where this rank's block starts in
-  // rank p's receive buffer (used by the transports that write into the peer's memory).
-  virtual int all_to_all(const void *send, const u64 *soff, const u64 *scnt, void *recv, const u64 *roff, const u64 *rcnt,
-                         const u64 *poff, size_t elem, cudaStream_t st) = 0;
-  // The same in two halves, so that rows can travel while kernels run: begin() enqueues the transfers on `side`, ordered
-  // after everything queued on st so far; end() makes st wait for them and for every other rank's.  (Default: all in begin.)
-  virtual int a2a_begin(const void *send, const u64 *soff, const u64 *scnt, void *recv, const u64 *roff, const u64 *rcnt,
-                        const u64 *poff, size_t elem, cudaStream_t st, cudaStream_t) {
-    return all_to_all(send, soff, scnt, recv, roff, rcnt, poff, elem, st);
-  }
-  virtual int a2a_end(cudaStream_t) { return RK_OK; }
   // peer memory: every rank's partition arena has the same layout, so a local pointer translates to any peer's copy
   const u8 *my_base = nullptr;
   u8 *peer_base[DIST_MAX_RANKS] = {nullptr};
-  bool peers_mapped = false;
   template <class T>
   T *on_peer(int p, T *local) const { return (T *)(peer_base[p] + ((const u8 *)local - my_base)); }
+
+  // The rows of a variable all-to-all (counts of `ex` in elements of `elem` bytes).  Every rank PUSHES its blocks into
+  // the peers' receive buffers with copy-engine copies (peer copies over NVLink between GPUs), then enters barrier().
+  // A rank's stream holds its pushes when it enters the barrier, so after the barrier every block addressed to this rank
+  // has landed.  The caller makes sure that no rank still reads its receive buffer when the pushes start.
+  int exchange_rows(const void *send, const Exchange &ex, void *recv, size_t elem, cudaStream_t st) {
+    const int rc = push_blocks(send, ex, recv, elem, st);
+    return rc ? rc : barrier(st);
+  }
+  // The same in two halves, so that rows can travel while kernels run: begin() enqueues the pushes on `side`, ordered
+  // after everything queued on st so far; end() makes st wait for them, then enters the barrier.
+  int exchange_rows_begin(const void *send, const Exchange &ex, void *recv, size_t elem, cudaStream_t st, cudaStream_t side) {
+    if (!ev_a && (cudaEventCreateWithFlags(&ev_a, cudaEventDisableTiming) != cudaSuccess ||
+                  cudaEventCreateWithFlags(&ev_b, cudaEventDisableTiming) != cudaSuccess)) {
+      err = "row exchange: cudaEventCreate failed";
+      return RK_ERR_CUDA;
+    }
+    cudaEventRecord(ev_a, st);
+    cudaStreamWaitEvent(side, ev_a, 0);
+    const int rc = push_blocks(send, ex, recv, elem, side);
+    if (rc) return rc;
+    cudaEventRecord(ev_b, side);
+    split_pending = true;
+    return RK_OK;
+  }
+  int exchange_rows_end(cudaStream_t st) {
+    if (!split_pending) return RK_OK;
+    split_pending = false;
+    cudaStreamWaitEvent(st, ev_b, 0);
+    return barrier(st);
+  }
+  cudaEvent_t ev_a = nullptr, ev_b = nullptr;
+  bool split_pending = false;
+  // This rank's blocks into the peers' receive buffers, peers in staggered order so that no receiver is hit by everybody
+  // at once.  Large exchanges are spread over a few copy streams (one copy engine each), forked from st and joined into
+  // it again: a single peer copy does not fill the links of a GPU (measured 550 GB/s for one copy at a time).
+  static constexpr int NAUX = 3;
+  cudaStream_t aux[NAUX] = {nullptr, nullptr, nullptr};
+  cudaEvent_t aux_ev[NAUX + 1] = {nullptr, nullptr, nullptr, nullptr};
+  int push_blocks(const void *send, const Exchange &ex, void *recv, size_t elem, cudaStream_t st) {
+    u64 total = 0;
+    int peers = 0;
+    for (int p = 0; p < world; ++p)
+      if (p != rank && ex.scnt[p]) total += ex.scnt[p] * elem, ++peers;
+    const bool spread = peers > 1 && total >= (8u << 20);
+    if (spread && !aux[0]) {
+      for (int a = 0; a < NAUX; ++a) cudaStreamCreateWithFlags(&aux[a], cudaStreamNonBlocking);
+      for (int a = 0; a <= NAUX; ++a) cudaEventCreateWithFlags(&aux_ev[a], cudaEventDisableTiming);
+    }
+    if (spread) {
+      cudaEventRecord(aux_ev[NAUX], st);
+      for (int a = 0; a < NAUX; ++a) cudaStreamWaitEvent(aux[a], aux_ev[NAUX], 0);
+    }
+    int turn = 0;
+    for (int k = 0; k < world; ++k) {
+      const int p = (rank + k) % world;
+      if (!ex.scnt[p]) continue;
+      u8 *dst = (p == rank ? (u8 *)recv : on_peer(p, (u8 *)recv)) + ex.poff[p] * elem;
+      cudaStream_t cs = st;
+      if (spread && p != rank) cs = (turn % (NAUX + 1)) == NAUX ? st : aux[turn % (NAUX + 1)], ++turn;
+      if (cudaMemcpyAsync(dst, (const u8 *)send + ex.soff[p] * elem, ex.scnt[p] * elem, cudaMemcpyDeviceToDevice, cs) != cudaSuccess) {
+        err = std::string("row exchange: peer copy failed: ") + cudaGetErrorString(cudaGetLastError());
+        return RK_ERR_CUDA;
+      }
+      if (p != rank) bytes_sent += ex.scnt[p] * elem;
+    }
+    if (spread)
+      for (int a = 0; a < NAUX; ++a) {
+        cudaEventRecord(aux_ev[a], aux[a]);
+        cudaStreamWaitEvent(st, aux_ev[a], 0);
+      }
+    return RK_OK;
+  }
 };
 
 struct NcclTransport : Transport {
   ncclComm_t comm = nullptr;
   bool own_comm = true;
+  u32 *d_flag = nullptr, *d_flag_all = nullptr;  // barrier payload (set by the owner of the transport)
   int check(ncclResult_t r, const char *what) {
     if (r == ncclSuccess) return RK_OK;
     err = std::string(what) + ": " + nccl_api().GetErrorString(r);
@@ -143,21 +236,6 @@ struct NcclTransport : Transport {
   }
   ~NcclTransport() override {
     if (comm && own_comm) nccl_api().CommDestroy(comm);
-    if (ev_a) cudaEventDestroy(ev_a);
-    if (ev_b) cudaEventDestroy(ev_b);
-    for (auto &a : aux) if (a) cudaStreamDestroy(a);
-    for (auto &e : aux_ev) if (e) cudaEventDestroy(e);
-  }
-  int gather_small(const u32 *d_row, u32 *d_all, u32 *h_all, cudaStream_t st) override {
-    int rc = check(nccl_api().AllGather(d_row, d_all, SMALL_WORDS * sizeof(u32), ncclUint8, comm, st), "ncclAllGather");
-    if (rc) return rc;
-    cudaError_t e = cudaMemcpyAsync(h_all, d_all, (size_t)world * SMALL_WORDS * sizeof(u32), cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) {
-      err = std::string("count exchange: ") + cudaGetErrorString(e);
-      return RK_ERR_CUDA;
-    }
-    return RK_OK;
   }
   int gather_small_begin(const u32 *d_row, u32 *d_all, u32 *, cudaStream_t st) override {
     return check(nccl_api().AllGather(d_row, d_all, SMALL_WORDS * sizeof(u32), ncclUint8, comm, st), "ncclAllGather");
@@ -171,115 +249,16 @@ struct NcclTransport : Transport {
     }
     return RK_OK;
   }
+  // a 4-byte all-gather: it completes on a rank only after every rank's stream has reached it
   int barrier(cudaStream_t st) override { return check(nccl_api().AllGather(d_flag, d_flag_all, 4, ncclUint8, comm, st), "ncclAllGather (barrier)"); }
   int all_gather(const void *send, void *recv, size_t bytes, cudaStream_t st) override {
     bytes_sent += bytes * (u64)(world - 1);
     return check(nccl_api().AllGather(send, recv, bytes, ncclUint8, comm, st), "ncclAllGather");
   }
-  // Bulk rows do not go through NCCL's send/recv kernels: every rank PUSHES its blocks into the peers' receive buffers
-  // with copy-engine peer copies over NVLink (the arenas are mapped into each other: cudaIpc between processes), peers
-  // in staggered order so that no receiver is hit by everybody at once; a 4-byte ncclAllGather behind the copies is the
-  // barrier that tells a rank that all blocks addressed to it have landed.
-  int all_to_all(const void *send, const u64 *soff, const u64 *scnt, void *recv, const u64 *roff, const u64 *rcnt,
-                 const u64 *poff, size_t elem, cudaStream_t st) override {
-    const NcclApi &N = nccl_api();
-    if (peers_mapped && !getenv_nccl_rows()) {
-      const int rc = push_blocks(send, soff, scnt, recv, poff, elem, st, st);
-      if (rc) return rc;
-      return check(N.AllGather(d_flag, d_flag_all, 4, ncclUint8, comm, st), "ncclAllGather (barrier)");
-    }
-    if (scnt[rank]) {
-      if (cudaMemcpyAsync((u8 *)recv + roff[rank] * elem, (const u8 *)send + soff[rank] * elem, scnt[rank] * elem,
-                          cudaMemcpyDeviceToDevice, st) != cudaSuccess) {
-        err = "all_to_all: local copy failed";
-        return RK_ERR_CUDA;
-      }
-    }
-    int rc = check(N.GroupStart(), "ncclGroupStart");
-    for (int p = 0; p < world && !rc; ++p) {
-      if (p == rank) continue;
-      if (scnt[p]) {
-        rc = check(N.Send((const u8 *)send + soff[p] * elem, scnt[p] * elem, ncclUint8, p, comm, st), "ncclSend");
-        bytes_sent += scnt[p] * elem;
-      }
-      if (rcnt[p] && !rc) rc = check(N.Recv((u8 *)recv + roff[p] * elem, rcnt[p] * elem, ncclUint8, p, comm, st), "ncclRecv");
-    }
-    const int rc2 = check(N.GroupEnd(), "ncclGroupEnd");
-    return rc ? rc : rc2;
-  }
-  int a2a_begin(const void *send, const u64 *soff, const u64 *scnt, void *recv, const u64 *roff, const u64 *rcnt, const u64 *poff,
-                size_t elem, cudaStream_t st, cudaStream_t side) override {
-    if (!(peers_mapped && !getenv_nccl_rows())) return all_to_all(send, soff, scnt, recv, roff, rcnt, poff, elem, st);
-    if (!ev_a && (cudaEventCreateWithFlags(&ev_a, cudaEventDisableTiming) != cudaSuccess ||
-                  cudaEventCreateWithFlags(&ev_b, cudaEventDisableTiming) != cudaSuccess)) {
-      err = "a2a_begin: cudaEventCreate failed";
-      return RK_ERR_CUDA;
-    }
-    cudaEventRecord(ev_a, st);
-    cudaStreamWaitEvent(side, ev_a, 0);
-    const int rc = push_blocks(send, soff, scnt, recv, poff, elem, side, side);
-    if (rc) return rc;
-    cudaEventRecord(ev_b, side);
-    split_pending = true;
-    return RK_OK;
-  }
-  int a2a_end(cudaStream_t st) override {
-    if (!split_pending) return RK_OK;
-    split_pending = false;
-    cudaStreamWaitEvent(st, ev_b, 0);
-    return check(nccl_api().AllGather(d_flag, d_flag_all, 4, ncclUint8, comm, st), "ncclAllGather (barrier)");
-  }
-  // This rank's blocks into the peers' receive buffers, peers in staggered order.  Large exchanges are spread over a few
-  // copy streams (one copy engine each), forked from `from` and joined into `into`: a single peer copy does not fill the
-  // links of a GPU (measured 550 GB/s for one copy at a time).
-  static constexpr int NAUX = 3;
-  cudaStream_t aux[NAUX] = {nullptr, nullptr, nullptr};
-  cudaEvent_t aux_ev[NAUX + 1] = {nullptr, nullptr, nullptr, nullptr};
-  int push_blocks(const void *send, const u64 *soff, const u64 *scnt, void *recv, const u64 *poff, size_t elem, cudaStream_t from,
-                  cudaStream_t into) {
-    u64 total = 0;
-    int peers = 0;
-    for (int p = 0; p < world; ++p)
-      if (p != rank && scnt[p]) total += scnt[p] * elem, ++peers;
-    const bool spread = peers > 1 && total >= (8u << 20);
-    if (spread && !aux[0]) {
-      for (int a = 0; a < NAUX; ++a) cudaStreamCreateWithFlags(&aux[a], cudaStreamNonBlocking);
-      for (int a = 0; a <= NAUX; ++a) cudaEventCreateWithFlags(&aux_ev[a], cudaEventDisableTiming);
-    }
-    if (spread) {
-      cudaEventRecord(aux_ev[NAUX], from);
-      for (int a = 0; a < NAUX; ++a) cudaStreamWaitEvent(aux[a], aux_ev[NAUX], 0);
-    }
-    int turn = 0;
-    for (int k = 0; k < world; ++k) {
-      const int p = (rank + k) % world;
-      if (!scnt[p]) continue;
-      u8 *dst = (p == rank ? (u8 *)recv : on_peer(p, (u8 *)recv)) + poff[p] * elem;
-      cudaStream_t cs = from;
-      if (spread && p != rank) cs = (turn % (NAUX + 1)) == NAUX ? from : aux[turn % (NAUX + 1)], ++turn;
-      if (cudaMemcpyAsync(dst, (const u8 *)send + soff[p] * elem, scnt[p] * elem, cudaMemcpyDeviceToDevice, cs) != cudaSuccess) {
-        err = std::string("all_to_all: peer copy failed: ") + cudaGetErrorString(cudaGetLastError());
-        return RK_ERR_CUDA;
-      }
-      if (p != rank) bytes_sent += scnt[p] * elem;
-    }
-    if (spread)
-      for (int a = 0; a < NAUX; ++a) {
-        cudaEventRecord(aux_ev[a], aux[a]);
-        cudaStreamWaitEvent(into, aux_ev[a], 0);
-      }
-    return RK_OK;
-  }
-  cudaEvent_t ev_a = nullptr, ev_b = nullptr;
-  bool split_pending = false;
-  u32 *d_flag = nullptr, *d_flag_all = nullptr;  // barrier payload (set by the owner of the transport)
-  static bool getenv_nccl_rows() {  // RK_DIST_NCCL_ROWS=1: rows through ncclSend/ncclRecv (tuning reference)
-    static const bool v = getenv("RK_DIST_NCCL_ROWS") != nullptr;
-    return v;
-  }
 };
 
-// ranks = threads of one process (any devices, also the same one): device copies between host barriers
+// ranks = threads of one process (any devices, also the same one): the small tables meet in host memory between host
+// barriers
 struct LocalGroup {
   int n = 0;
   std::mutex mu;
@@ -287,8 +266,6 @@ struct LocalGroup {
   int waiting = 0;
   u64 generation = 0;
   const void *ptr[DIST_MAX_RANKS] = {nullptr};
-  u64 soff[DIST_MAX_RANKS][DIST_MAX_RANKS] = {{0}};
-  u64 scnt[DIST_MAX_RANKS][DIST_MAX_RANKS] = {{0}};
   u32 small[DIST_MAX_RANKS][SMALL_WORDS] = {{0}};
   void barrier() {
     std::unique_lock<std::mutex> lk(mu);
@@ -310,17 +287,15 @@ struct LocalTransport : Transport {
     err = std::string(what) + ": " + cudaGetErrorString(e);
     return RK_ERR_CUDA;
   }
-  int gather_small(const u32 *d_row, u32 *, u32 *h_all, cudaStream_t st) override {
+  // the host exchange, then the matrix goes back to the device
+  int gather_small_begin(const u32 *d_row, u32 *d_all, u32 *h_all, cudaStream_t st) override {
     cudaError_t e = cudaMemcpyAsync(h_all + (size_t)rank * SMALL_WORDS, d_row, SMALL_WORDS * sizeof(u32), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e == cudaSuccess) memcpy(g->small[rank], h_all + (size_t)rank * SMALL_WORDS, SMALL_WORDS * sizeof(u32));
     g->barrier();
     for (int r = 0; r < world; ++r) memcpy(h_all + (size_t)r * SMALL_WORDS, g->small[r], SMALL_WORDS * sizeof(u32));
     g->barrier();
-    return cuda(e, "count exchange");
-  }
-  int gather_small_begin(const u32 *d_row, u32 *d_all, u32 *h_all, cudaStream_t st) override {
-    const int rc = gather_small(d_row, d_all, h_all, st);  // the host exchange, then the matrix goes back to the device
+    const int rc = cuda(e, "count exchange");
     if (rc) return rc;
     return cuda(cudaMemcpyAsync(d_all, h_all, (size_t)world * SMALL_WORDS * sizeof(u32), cudaMemcpyHostToDevice, st), "count upload");
   }
@@ -340,28 +315,6 @@ struct LocalTransport : Transport {
     g->barrier();
     bytes_sent += bytes * (u64)(world - 1);
     return cuda(e, "all_gather");
-  }
-  int all_to_all(const void *send, const u64 *soff, const u64 *scnt, void *recv, const u64 *roff, const u64 *rcnt, const u64 *,
-                 size_t elem, cudaStream_t st) override {
-    cudaError_t e = cudaStreamSynchronize(st);
-    g->ptr[rank] = send;
-    for (int p = 0; p < world; ++p) g->soff[rank][p] = soff[p], g->scnt[rank][p] = scnt[p];
-    g->barrier();
-    bool mismatch = false;
-    for (int r = 0; r < world && e == cudaSuccess; ++r) {
-      const u64 cnt = g->scnt[r][rank];
-      if (cnt != rcnt[r]) mismatch = true;
-      if (cnt && !mismatch)
-        e = cudaMemcpyAsync((u8 *)recv + roff[r] * elem, (const u8 *)g->ptr[r] + g->soff[r][rank] * elem, cnt * elem, cudaMemcpyDefault, st);
-      if (r != rank) bytes_sent += scnt[r] * elem;
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    g->barrier();
-    if (mismatch) {
-      err = "all_to_all: send and receive counts disagree";
-      return RK_ERR_INTERNAL;
-    }
-    return cuda(e, "all_to_all");
   }
 };
 
@@ -397,7 +350,7 @@ struct Trace {
     for (auto &r : recs) {
       float ms = 0.f;
       if (cudaEventElapsedTime(&ms, r.a, r.b) != cudaSuccess) cudaGetLastError();
-      // label: the transport function and its first argument, e.g. all_to_all(D.send_rows
+      // label: the transport function and its first argument, e.g. exchange_rows(D.halo_send
       std::string w(r.what);
       const size_t p0 = w.find("->"), p1 = w.find(',');
       w = w.substr(p0 == std::string::npos ? 0 : p0 + 2, p1 == std::string::npos ? std::string::npos : p1 - (p0 == std::string::npos ? 0 : p0 + 2));
@@ -410,33 +363,6 @@ struct Trace {
     }
     recs.clear();
     fprintf(stderr, "%s | comm total %.3f ms\n", line.c_str(), total);
-  }
-};
-
-struct Exchange {  // counts of one variable all-to-all, as this rank sees it (elements)
-  u64 soff[DIST_MAX_RANKS], scnt[DIST_MAX_RANKS], roff[DIST_MAX_RANKS], rcnt[DIST_MAX_RANKS];
-  u64 poff[DIST_MAX_RANKS];   // forward: start of my block in rank p's receive buffer (= p's roff[me])
-  u64 rpoff[DIST_MAX_RANKS];  // the way back: start of my block in rank p's send-order buffer (= p's soff[me])
-  u64 n_send = 0, n_recv = 0;
-  // from the gathered count matrix: row s = what rank s sends to every destination
-  void from_matrix(const u32 *h_all, int word0, int nr, int me) {
-    n_send = n_recv = 0;
-    for (int d = 0; d < nr; ++d) {
-      soff[d] = n_send;
-      scnt[d] = h_all[(size_t)me * SMALL_WORDS + word0 + d];
-      n_send += scnt[d];
-    }
-    for (int s = 0; s < nr; ++s) {
-      roff[s] = n_recv;
-      rcnt[s] = h_all[(size_t)s * SMALL_WORDS + word0 + me];
-      n_recv += rcnt[s];
-    }
-    for (int p = 0; p < nr; ++p) {
-      u64 f = 0, r = 0;
-      for (int s = 0; s < me; ++s) f += h_all[(size_t)s * SMALL_WORDS + word0 + p];
-      for (int d = 0; d < me; ++d) r += h_all[(size_t)p * SMALL_WORDS + word0 + d];
-      poff[p] = f, rpoff[p] = r;
-    }
   }
 };
 
@@ -606,7 +532,6 @@ static void dist_release_buffers(Dist &D) {
   D.peers_ready = false;
   if (D.arena) cudaFree(D.arena);
   D.arena = nullptr;
-  if (D.tr) D.tr->peers_mapped = false;
   D.cap = D.hcap = 0;
   D.loaded = false;
 }
@@ -698,7 +623,6 @@ static int dist_import(rk_ctx *ctx, const u8 *blobs, size_t stride) {
     D.pt.res[r] = (const u64 *)(base + ((const u8 *)D.res - (const u8 *)D.arena));
   }
   D.tr->my_base = (const u8 *)D.arena;
-  D.tr->peers_mapped = true;
   if (NcclTransport *nt = dynamic_cast<NcclTransport *>(D.tr)) nt->d_flag = D.flag, nt->d_flag_all = D.flag_all;
   D.pt.nr = D.world, D.pt.me = D.rank;
   D.peers_ready = true;
@@ -706,7 +630,7 @@ static int dist_import(rk_ctx *ctx, const u8 *blobs, size_t stride) {
 }
 
 // the count exchange with the matrix left on the device as well (d_small_all) and on the host (h_small); synchronises
-static int dist_gather_counts_dev(rk_ctx *ctx) {
+static int dist_gather_counts(rk_ctx *ctx) {
   Dist &D = *ctx->dist;
   CK(cudaMemcpyAsync(D.d_small + W_ERR, &D.cnt->err, sizeof(u32), cudaMemcpyDeviceToDevice, ctx->stream));
   TR(D.tr->gather_small_begin(D.d_small, D.d_small_all, D.h_small, ctx->stream));
@@ -742,13 +666,6 @@ static ScatterTable scatter_table(const Dist &D, const Exchange &ex, bool back, 
   }
   t.start[D.world] = (u32)run;
   return t;
-}
-
-static int dist_gather_counts(rk_ctx *ctx) {
-  Dist &D = *ctx->dist;
-  CK(cudaMemcpyAsync(D.d_small + W_ERR, &D.cnt->err, sizeof(u32), cudaMemcpyDeviceToDevice, ctx->stream));
-  TR(D.tr->gather_small(D.d_small, D.d_small_all, D.h_small, ctx->stream));
-  return RK_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -857,21 +774,18 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   }
   D.ex1.from_matrix(D.h_small, W_CNT_A, nr, me);
   D.tr->bytes_sent += (D.ex1.n_send - D.ex1.scnt[me]) * 24;  // (the rows this rank's kernels stored into peer memory)
-  u64 m_total = 0, loaded_total = 0;
-  u64 m_of[DIST_MAX_RANKS] = {0};
-  for (int s = 0; s < nr; ++s) {
-    for (int d = 0; d < nr; ++d) m_of[d] += D.h_small[(size_t)s * SMALL_WORDS + W_CNT_A + d];
-    for (int d = 0; d <= nr; ++d) loaded_total += D.h_small[(size_t)s * SMALL_WORDS + W_CNT_A + d];
-  }
+  u64 loaded_total = 0, m_of[DIST_MAX_RANKS] = {0};
+  for (int d = 0; d <= nr; ++d) loaded_total += column_sum(D.h_small, W_CNT_A + d, nr);
   u64 off = 0;
   for (int d = 0; d < nr; ++d) {
+    m_of[d] = column_sum(D.h_small, W_CNT_A + d, nr);
     D.pt.roff[d] = (u32)off;
     if (d == me) D.rank_off = (u32)off;
     off += m_of[d];
     if (m_of[d] > D.cap) return fail(ctx, RK_ERR_NOMEM, "rank %d would own %llu fragments, capacity is %llu rows per rank", d,
                                      (unsigned long long)m_of[d], (unsigned long long)D.cap);
   }
-  m_total = off;
+  const u64 m_total = off;
   D.pt.roff[nr] = (u32)m_total;
   for (int d = nr + 1; d <= DIST_MAX_RANKS; ++d) D.pt.roff[d] = 0xFFFFFFFFu;
   CK(cudaMemcpyAsync(D.roff_dev, D.pt.roff, (nr + 1) * sizeof(u32), cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
@@ -915,11 +829,8 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   D.exh.from_matrix(D.h_small, W_CNT_A, nr, me);
   D.exy.from_matrix(D.h_small, W_CNT_B, nr, me);
   for (int d = 0; d < nr; ++d) {
-    u64 halo_in = 0, halo_out = 0, y_in = 0;
-    for (int s = 0; s < nr; ++s) {
-      halo_in += D.h_small[(size_t)s * SMALL_WORDS + W_CNT_A + d];
-      y_in += D.h_small[(size_t)s * SMALL_WORDS + W_CNT_B + d];
-    }
+    const u64 halo_in = column_sum(D.h_small, W_CNT_A + d, nr), y_in = column_sum(D.h_small, W_CNT_B + d, nr);
+    u64 halo_out = 0;
     for (int t = 0; t < nr; ++t) halo_out += D.h_small[(size_t)d * SMALL_WORDS + W_CNT_A + t];
     if (halo_in > D.hcap || halo_out > D.hcap)
       return fail(ctx, RK_ERR_NOMEM, "rank %d: %llu halo fragments in / %llu out, the halo capacity is %llu", d,
@@ -934,9 +845,11 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   const u64 ky_end = (me + 1 < nr && cutsy_h[me + 1] < 2ull * g.nby) ? cutsy_h[me + 1] : 2ull * g.nby;
   const int bits_y_l = ceil_log2(ky_end > ky_base ? ky_end - ky_base : 1) < 1 ? 1 : ceil_log2(ky_end - ky_base);
 
-  TR(D.tr->all_to_all(D.halo_send, D.exh.soff, D.exh.scnt, D.halo_recv, D.exh.roff, D.exh.rcnt, D.exh.poff, 16, st));
+  // Both row exchanges come right after host sync 2: every rank's work queued before it is complete, so no rank still
+  // reads its halo_recv / recv_rows (last read by the previous load and group) when the peers' pushes start.
+  TR(D.tr->exchange_rows(D.halo_send, D.exh, D.halo_recv, 16, st));
   // the Y rows travel (copy engines, NVLink) while this GPU unpacks its halo and sorts its X buckets
-  TR(D.tr->a2a_begin(D.send_rows, D.exy.soff, D.exy.scnt, D.recv_rows, D.exy.roff, D.exy.rcnt, D.exy.poff, 16, st, D.side));
+  TR(D.tr->exchange_rows_begin(D.send_rows, D.exy, D.recv_rows, 16, st, D.side));
   // X sort keys relative to the first super-bucket of the rank's range (per strand class)
   const u32 *cutsx_h = D.h_small + (size_t)me * SMALL_WORDS + W_CUTSX;
   u32 x_base[2], x_range[2];
@@ -953,7 +866,7 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   launches += launch_sort_pairs(D.kx2, nullptr, D.skx, D.rx, D.tmp_k, D.tmp_v, (u64)m + D.n_halo, bits_x_l, D.sort_work, st, &D.cnt->err,
                                 (m + D.n_halo) ? D.prehist + 1024 : nullptr);
   CK(cudaEventRecord(ev[6], st));
-  TR(D.tr->a2a_end(st));
+  TR(D.tr->exchange_rows_end(st));
   launches += dist_unpack_axis_rows(D.recv_rows, D.m_y, ky_base, D.ky_a, D.yl_a, D.grank_a, hist_of(2, bits_y_l), st);
   launches += launch_sort_pairs(D.ky_a, nullptr, D.sky_a, D.ry_a, D.tmp_k, D.tmp_v, D.m_y, bits_y_l, D.sort_work, st, &D.cnt->err,
                                 D.m_y ? D.prehist + 2048 : nullptr);
@@ -1031,7 +944,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   launches += dist_chase_local(D.parent, D.gidscan, m, D.rank_off, D.lroot, D.res, D.pend_idx[0], D.pend_key[0], D.n_pend, st);
   CK(cudaMemcpyAsync(D.d_small + W_X2, D.n_pend, sizeof(u32), cudaMemcpyDeviceToDevice, st));
   {
-    const int rc = dist_gather_counts_dev(ctx);  // host sync: roots and pending chains of every rank (also: every rank's res[] is final)
+    const int rc = dist_gather_counts(ctx);  // host sync: roots and pending chains of every rank (also: every rank's res[] is final)
     if (rc) return rc;
   }
   // the root counts stay on the device as a column of the gathered matrix, in a copy that later gathers do not overwrite
@@ -1058,8 +971,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
     Exchange exq;
     exq.from_matrix(D.h_small, W_CNT_A, nr, me);
     for (int d = 0; d < nr; ++d) {
-      u64 in = 0;
-      for (int sr = 0; sr < nr; ++sr) in += D.h_small[(size_t)sr * SMALL_WORDS + W_CNT_A + d];
+      const u64 in = column_sum(D.h_small, W_CNT_A + d, nr);
       if (in > D.cap) return fail(ctx, RK_ERR_NOMEM, "rank %d is asked about %llu chain ends, capacity is %llu rows per rank", d,
                                   (unsigned long long)in, (unsigned long long)D.cap);
     }
@@ -1073,7 +985,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
     CK(cudaMemcpyAsync(D.n_pend, D.n_pend + 1, sizeof(u32), cudaMemcpyDeviceToDevice, st));
     cur ^= 1;
     CK(cudaMemcpyAsync(D.d_small + W_X2, D.n_pend, sizeof(u32), cudaMemcpyDeviceToDevice, st));
-    const int rc = dist_gather_counts_dev(ctx);  // how many chains are still open, everywhere
+    const int rc = dist_gather_counts(ctx);  // how many chains are still open, everywhere
     if (rc) return rc;
   }
   launches += dist_chase_finish(D.pt, nroots, SMALL_WORDS, m, D.res, D.lroot, D.pend_idx[cur], D.pend_key[cur], D.n_pend, D.gid_l, D.gid_rank, st);
@@ -1110,8 +1022,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   const u64 total_groups = D.h_small[(size_t)me * SMALL_WORDS + W_X1];
   u64 line_off = 0;
   for (int d = 0; d < nr; ++d) {
-    u64 in = 0;
-    for (int s = 0; s < nr; ++s) in += D.h_small[(size_t)s * SMALL_WORDS + W_CNT_A + d];
+    const u64 in = column_sum(D.h_small, W_CNT_A + d, nr);
     if (in > D.cap) return fail(ctx, RK_ERR_NOMEM, "rank %d would own %llu output lines, capacity is %llu rows per rank", d,
                                 (unsigned long long)in, (unsigned long long)D.cap);
     if (d < me) line_off += in;
@@ -1367,8 +1278,7 @@ rk_multi *rk_create_multi(const int *devices, int ndev) {
   bool distinct = true;
   for (int i = 0; i < ndev; ++i)
     for (int j = 0; j < i; ++j) distinct = distinct && devices[i] != devices[j];
-  const char *force = getenv("RK_MULTI_TRANSPORT");  // "local" or "nccl"
-  mg->use_nccl = distinct && ndev > 1 && !(force && !strcmp(force, "local"));
+  mg->use_nccl = distinct && ndev > 1;
   for (int r = 0; r < ndev; ++r) {
     rk_ctx *c = rk_create(devices[r]);
     if (!c) {
@@ -1383,7 +1293,7 @@ rk_multi *rk_create_multi(const int *devices, int ndev) {
     mg->comms.resize(ndev);
     if (!N.ok() || N.CommInitAll(mg->comms.data(), ndev, devices) != ncclSuccess) {
       mg->comms.clear();
-      mg->use_nccl = false;  // ranks are threads of this process: the copy transport always works
+      mg->use_nccl = false;  // ranks are threads of this process: the local transport always works
     }
   }
   return mg;

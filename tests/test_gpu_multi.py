@@ -1,7 +1,8 @@
 """One comparison partitioned over several ranks (csrc/multi.cu) against the oracle, bit for bit:
-  * rk_create_multi with the same device listed several times — ranks are threads of one process that exchange through
-    device copies — so the whole partitioned path (cuts, halo, Y exchange, forest over peer pointers, output exchange) is
-    checked on a one-GPU box for 1, 2, 3, 5 and 8 ranks;
+  * rk_create_multi with the same device listed several times — ranks are threads of one process that exchange the small
+    tables through host memory and push their rows into each other's buffers as the NCCL transport does — so the whole
+    partitioned path (cuts, halo and Y row exchanges, forest over peer pointers, output exchange) is checked on a one-GPU
+    box for 1, 2, 3, 5 and 8 ranks;
   * rk_dist_* with one process per GPU over NCCL where the box has the GPUs (2, 4, 8)."""
 import os
 import socket
@@ -24,6 +25,8 @@ def _workload(name):
         return replace(gen.WORKLOADS["c1"], n=3_000, lx=30_000, ly=25_000, families=12, p_rep=0.6, seed=21)
     if name == "c3":
         return gen.scaled(gen.WORKLOADS["c3"], 200_000)
+    if name == "c2_6m":    # large enough that the row exchanges spread their copies over several streams
+        return gen.scaled(gen.WORKLOADS["c2"], 6_000_000)
     return gen.scaled(gen.WORKLOADS["c2"], 300_000)
 
 
@@ -71,10 +74,13 @@ def test_forest_bulk_rounds_match_oracle(monkeypatch, world, wl):
         _assert_same(m.group(0.5, 0.5), O.group(rec, w.lx + 1, w.ly + 1, 0.5, 0.5))
 
 
-@pytest.mark.parametrize("world,wl", [(8, "c2"), (3, "dense"), (5, "c2"), (2, "tiny")])
+@pytest.mark.parametrize("world,wl", [(8, "c2"), (3, "dense"), (5, "c2"), (2, "tiny"), (3, "c2_6m")])
 def test_output_ranges_respect_the_row_capacity(monkeypatch, world, wl):
     """the output ranges are cut by estimated sort_groups work, which gives the ranks with small groups more lines; no rank
-    may get more lines than it has rows for (RK_DIST_LINE_CAP stands in for a tight capacity)"""
+    may get more lines than it has rows for (RK_DIST_LINE_CAP stands in for a tight capacity).
+    (3, c2_6m) also takes the row exchange's spread over several copy streams, which needs at least 2 destination peers
+    and 8 MiB per exchange: each of the 3 ranks holds about 2M fragments and sends about 2/3 of its Y rows, 16 B each, to
+    the other two: about 21 MB, more than twice the threshold."""
     w = _workload(wl)
     rec = gen.generate(w)
     g = O.group(rec, w.lx + 1, w.ly + 1, w.len_ratio, w.pos_ratio)
