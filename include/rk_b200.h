@@ -35,6 +35,8 @@ typedef enum {
 #define RK_F_HOST_RESULT 1u /* copy order/gid/repval/identity to library-owned pinned host arrays */
 #define RK_F_NO_SORT 2u     /* stop after generate_fragment_groups: members stay in push_back (rank) order */
 #define RK_F_TIMING 4u      /* record per-stage CUDA-event times into rk_result / rk_load_stats */
+#define RK_F_LINE_RECORDS 8u /* rk_dist_group / rk_multi_group: also bring every output line's record to the rank that holds
+                                the line, for rk_dist_format_lines / rk_dist_group_statistics (rk_group ignores it) */
 
 enum { /* stage indices of ms_stage[] */
   RK_ST_H2D = 0,     /* host -> device copy of the records (0 when the input was a device pointer) */
@@ -242,6 +244,17 @@ int rk_dist_load_aos(rk_ctx *ctx, const void *frags, uint64_t n_local, uint64_t 
 /* out: THIS RANK's range of output lines (order = file indices of the whole file, gid = global group ids); n_groups is
  * the global count.  info may be NULL. */
 int rk_dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flags, rk_result *out, rk_dist_info *info);
+/* After an rk_dist_group with RK_F_LINE_RECORDS: the output of THIS rank, with no collective step (the group call brought
+ * the record of every line to the rank that holds the line).  Both return RK_ERR_STATE after a group without the flag.
+ * The records must still be where rk_dist_load_aos found them when they were given as a DEVICE pointer.  rk_dist_group refuses
+ * RK_F_LINE_RECORDS with RK_ERR_ARG (on every rank) when the ranks' slices, by their file_offset, overlap or are out of rank order.
+ * rk_dist_format_lines: the text of local lines first_line .. first_line+n_lines-1 (0 .. rk_dist_info.n_lines), byte for byte
+ *   what rk_format_lines writes for the same lines on one GPU; the same limits and the same two alternating buffers.
+ * rk_dist_group_statistics: rk_group_statistics of the groups of this rank, first_gid .. first_gid+n_groups-1 (a group is
+ *   never split over ranks; first_line is the global line index). */
+int rk_dist_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_text *out);
+int rk_dist_group_statistics(rk_ctx *ctx, unsigned flags, const rk_group_stats **stats, const rk_group_stats **d_stats,
+                             uint64_t *first_gid, uint64_t *n_groups);
 
 typedef struct rk_multi rk_multi;
 /* One context per listed device.  The ranks push their rows into each other's device memory.  Distinct devices exchange
@@ -259,6 +272,12 @@ int rk_multi_load_aos(rk_multi *m, const void *frags, uint64_t n, uint64_t seqx_
 /* out: the whole result in pinned host memory owned by m (device pointers are NULL), valid until the next call. */
 int rk_multi_group(rk_multi *m, double len_ratio, double pos_ratio, unsigned flags, rk_result *out);
 int rk_multi_info(const rk_multi *m, int rank, rk_dist_info *info);
+/* After an rk_multi_group with RK_F_LINE_RECORDS, as rk_format_lines / rk_group_statistics on one GPU:
+ * rk_multi_format_lines: GLOBAL lines first_line .. first_line+n_lines-1; every rank formats its part on its GPU, the parts
+ *   land in one pinned buffer owned by m in rank order (two buffers alternate, as in rk_format_lines).
+ * rk_multi_group_statistics: all groups in gid order, in host memory owned by m (valid until the next call). */
+int rk_multi_format_lines(rk_multi *m, uint64_t first_line, uint64_t n_lines, rk_text *out);
+int rk_multi_group_statistics(rk_multi *m, const rk_group_stats **stats, uint64_t *n_groups);
 
 /* Tooling: records start .. start+count of the synthetic workload of repkiller_b200/gen.py, generated on the device
  * (lx, ly are the header values, i.e. loaded length - 1). */

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "librk_b200%s.so" % os.environ.get("RK_LIB_SUFFIX", ""))  # suffix: tuning variants only
 
 RK_NONE = 0xFFFFFFFF
-F_HOST_RESULT, F_NO_SORT, F_TIMING = 1, 2, 4
+F_HOST_RESULT, F_NO_SORT, F_TIMING, F_LINE_RECORDS = 1, 2, 4, 8
 STAGES = ["h2d", "decode", "ranksort", "keys", "xsort", "ysort", "xmatch", "ymatch", "forest", "hkey", "gsort",
           "final", "d2h"]
 NSTAGES = len(STAGES)
@@ -26,8 +26,9 @@ SYMBOLS = ["rk_create", "rk_create_error", "rk_destroy", "rk_last_error", "rk_se
            "rk_gen_workload", "rk_sort_members", "rk_group_statistics", "rk_sol_create", "rk_sol_destroy", "rk_sol_insert", "rk_sol_get_associated", "rk_sol_last_error",
            # one comparison over several GPUs
            "rk_dist_unique_id", "rk_dist_init", "rk_dist_export", "rk_dist_import", "rk_dist_load_aos", "rk_dist_group",
+           "rk_dist_format_lines", "rk_dist_group_statistics",
            "rk_create_multi", "rk_destroy_multi", "rk_multi_last_error", "rk_multi_ranks", "rk_multi_ctx", "rk_multi_transport",
-           "rk_multi_load_aos", "rk_multi_group", "rk_multi_info"]
+           "rk_multi_load_aos", "rk_multi_group", "rk_multi_info", "rk_multi_format_lines", "rk_multi_group_statistics"]
 DIST_ID_BYTES, DIST_BLOB_BYTES = 128, 128
 GROUP_STATS_DTYPE = np.dtype([("count", "<u4"), ("x_lo", "<u4"), ("x_hi", "<u4"), ("y_lo", "<u4"), ("y_hi", "<u4"), ("first_line", "<u4"),
                               ("mean_identity", "<f8"), ("multiplicity", "<f8")])
@@ -105,6 +106,9 @@ def load_library():
     L.rk_dist_import.argtypes = [C.c_void_p, C.c_void_p]
     L.rk_dist_load_aos.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint, C.POINTER(_LoadStats)]
     L.rk_dist_group.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_uint, C.POINTER(_Result), C.POINTER(_DistInfo)]
+    L.rk_dist_format_lines.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(_Text)]
+    L.rk_dist_group_statistics.argtypes = [C.c_void_p, C.c_uint, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_uint64),
+                                           C.POINTER(C.c_uint64)]
     L.rk_create_multi.argtypes = [C.POINTER(C.c_int), C.c_int]
     L.rk_create_multi.restype = C.c_void_p
     L.rk_destroy_multi.argtypes = [C.c_void_p]
@@ -118,6 +122,8 @@ def load_library():
     L.rk_multi_load_aos.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint, C.POINTER(_LoadStats)]
     L.rk_multi_group.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_uint, C.POINTER(_Result)]
     L.rk_multi_info.argtypes = [C.c_void_p, C.c_int, C.POINTER(_DistInfo)]
+    L.rk_multi_format_lines.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(_Text)]
+    L.rk_multi_group_statistics.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]
     L.rk_sol_create.argtypes = [C.c_int, C.c_double, C.c_double, C.c_uint64]
     L.rk_sol_create.restype = C.c_void_p
     L.rk_sol_destroy.argtypes = [C.c_void_p]
@@ -256,19 +262,9 @@ class Context:
     def format_lines(self, first_line: int = 0, n_lines: int | None = None) -> bytes:
         """Text of the output lines of the last group() (commonFunctions.cpp:101-115), formatted on the device; the
         16 header lines are the caller's.  Chunks of FORMAT_MAX_LINES lines are concatenated."""
-        out, self.ms_format = [], 0.0
-        total = self._last_m if n_lines is None else n_lines
-        done = 0
-        while done < total or (total == 0 and not out):
-            cnt = min(FORMAT_MAX_LINES, total - done)
-            t = _Text()
-            self._check(self._L.rk_format_lines(self._h, first_line + done, cnt, C.byref(t)))
-            out.append(C.string_at(t.text, t.n_bytes) if t.n_bytes else b"")
-            self.ms_format += t.ms_device
-            done += cnt
-            if total == 0:
-                break
-        return b"".join(out)
+        text, self.ms_format = _format_chunks(lambda a, k, t: self._check(self._L.rk_format_lines(self._h, a, k, t)), first_line,
+                                              self._last_m if n_lines is None else n_lines)
+        return text
 
     def generate_device(self, w, start: int, count: int, out_ptr: int):
         """Records start..start+count of workload `w` (repkiller_b200.gen.Workload) written to device memory at out_ptr
@@ -317,9 +313,7 @@ class Context:
         """per-group statistics of the last group() as a structured array (GROUP_STATS_DTYPE), one row per group id"""
         hp, dp, ng = C.c_void_p(), C.c_void_p(), C.c_uint64()
         self._check(self._L.rk_group_statistics(self._h, F_HOST_RESULT, C.byref(hp), C.byref(dp), C.byref(ng)))
-        if ng.value == 0:
-            return np.zeros(0, dtype=GROUP_STATS_DTYPE)
-        return np.frombuffer(C.string_at(hp.value, ng.value * GROUP_STATS_DTYPE.itemsize), dtype=GROUP_STATS_DTYPE).copy()
+        return _stats_array(hp.value, ng.value)
 
     def sort_members(self, gid: np.ndarray, y: np.ndarray, d: np.ndarray) -> np.ndarray:
         """sort_groups as a pure function: perm[j] = index of the member std::sort leaves at position j (members given
@@ -352,12 +346,48 @@ class Context:
                          st.n_launches)
 
     def dist_group(self, len_ratio: float, pos_ratio: float, host_result: bool = True, sort: bool = True, timing: bool = False,
-                   copy: bool = True):
-        """(Groups of THIS rank's range of output lines, info dict)"""
-        flags = (F_HOST_RESULT if host_result else 0) | (0 if sort else F_NO_SORT) | (F_TIMING if timing else 0)
+                   copy: bool = True, line_records: bool = False):
+        """(Groups of THIS rank's range of output lines, info dict); line_records: for dist_format_lines /
+        dist_group_statistics"""
+        flags = ((F_HOST_RESULT if host_result else 0) | (0 if sort else F_NO_SORT) | (F_TIMING if timing else 0)
+                 | (F_LINE_RECORDS if line_records else 0))
         r, info = _Result(), _DistInfo()
         self._check(self._L.rk_dist_group(self._h, len_ratio, pos_ratio, flags, C.byref(r), C.byref(info)))
+        self._dist_lines = info.n_lines
         return _groups_of(r, host_result, copy), _info_dict(info)
+
+    def dist_format_lines(self, first_line: int = 0, n_lines: int | None = None) -> bytes:
+        """text of THIS rank's lines first_line .. (local indices) after dist_group(..., line_records=True)"""
+        text, self.ms_format = _format_chunks(lambda a, k, t: self._check(self._L.rk_dist_format_lines(self._h, a, k, t)), first_line,
+                                              self._dist_lines if n_lines is None else n_lines)
+        return text
+
+    def dist_group_statistics(self):
+        """(first gid, statistics of THIS rank's groups) after dist_group(..., line_records=True)"""
+        hp, dp, fg, ng = C.c_void_p(), C.c_void_p(), C.c_uint64(), C.c_uint64()
+        self._check(self._L.rk_dist_group_statistics(self._h, F_HOST_RESULT, C.byref(hp), C.byref(dp), C.byref(fg), C.byref(ng)))
+        return fg.value, _stats_array(hp.value, ng.value)
+
+
+def _format_chunks(call, first_line: int, n_lines: int):
+    """(text, device ms) of lines first_line .. first_line + n_lines in calls of at most FORMAT_MAX_LINES lines;
+    call(first, count, byref(_Text)) formats one chunk"""
+    out, ms, done = [], 0.0, 0
+    while True:
+        cnt = min(FORMAT_MAX_LINES, n_lines - done)
+        t = _Text()
+        call(first_line + done, cnt, C.byref(t))
+        out.append(C.string_at(t.text, t.n_bytes) if t.n_bytes else b"")
+        ms += t.ms_device
+        done += cnt
+        if done >= n_lines:
+            return b"".join(out), ms
+
+
+def _stats_array(ptr, n: int) -> np.ndarray:
+    if n == 0:
+        return np.zeros(0, dtype=GROUP_STATS_DTYPE)
+    return np.frombuffer(C.string_at(ptr, n * GROUP_STATS_DTYPE.itemsize), dtype=GROUP_STATS_DTYPE).copy()
 
 
 def _groups_of(r: "_Result", host_result: bool, copy: bool) -> Groups:
@@ -481,10 +511,25 @@ class Multi:
         self._check(self._L.rk_multi_load_aos(self._h, C.c_void_p(rec.ctypes.data), rec.nbytes // 109, seqx_len, seqy_len, 0, C.byref(st)))
         return LoadStats(st.n_loaded, st.n_kept, st.vsize, {}, st.ms_device, st.n_launches)
 
-    def group(self, len_ratio: float, pos_ratio: float, sort: bool = True) -> Groups:
+    def group(self, len_ratio: float, pos_ratio: float, sort: bool = True, line_records: bool = False) -> Groups:
+        """line_records: every rank also gets the records of its output lines, for format_lines / group_statistics"""
         r = _Result()
-        self._check(self._L.rk_multi_group(self._h, len_ratio, pos_ratio, 0 if sort else F_NO_SORT, C.byref(r)))
+        flags = (0 if sort else F_NO_SORT) | (F_LINE_RECORDS if line_records else 0)
+        self._check(self._L.rk_multi_group(self._h, len_ratio, pos_ratio, flags, C.byref(r)))
+        self._last_m = r.n_kept
         return _groups_of(r, True, True)
+
+    def format_lines(self, first_line: int = 0, n_lines: int | None = None) -> bytes:
+        """Context.format_lines over the whole comparison (global line indices), after group(..., line_records=True)"""
+        text, self.ms_format = _format_chunks(lambda a, k, t: self._check(self._L.rk_multi_format_lines(self._h, a, k, t)), first_line,
+                                              self._last_m if n_lines is None else n_lines)
+        return text
+
+    def group_statistics(self) -> np.ndarray:
+        """Context.group_statistics over the whole comparison (all groups in gid order), after group(..., line_records=True)"""
+        hp, ng = C.c_void_p(), C.c_uint64()
+        self._check(self._L.rk_multi_group_statistics(self._h, C.byref(hp), C.byref(ng)))
+        return _stats_array(hp.value, ng.value)
 
     def info(self, rank: int) -> dict:
         i = _DistInfo()

@@ -518,14 +518,14 @@ int rk_sort_groups(rk_ctx *ctx, unsigned flags, rk_result *out) {
   return finish_group(ctx, flags, out, launches);
 }
 
-int rk_group_statistics(rk_ctx *ctx, unsigned flags, const rk_group_stats **stats, const rk_group_stats **d_stats, uint64_t *n_groups) {
-  static_assert(sizeof(rk_group_stats) == sizeof(rk_group_stats_dev) && sizeof(rk_group_stats) == 40, "stats layout");
-  if (!ctx) return RK_ERR_ARG;
-  if (!ctx->loaded || !ctx->have_group) return fail(ctx, RK_ERR_STATE, "rk_group_statistics before rk_group");
+}  // extern "C"
+
+// (shared with multi.cu, rk_ctx.cuh)
+namespace rk {
+int group_stats_run(rk_ctx *ctx, unsigned flags, const u32 *order, const u32 *gid, const float *identity, const uint4 *rec4,
+                    const LineRow *rows, u32 m, u64 ng, u32 gid_base, u32 line_off) {
   CK(cudaSetDevice(ctx->device));
-  ProfGuard pg(ctx);
   cudaStream_t st = ctx->stream;
-  const u64 ng = ctx->n_groups_last;
   if (ng > ctx->stats_cap) {
     CK(cudaStreamSynchronize(st));
     if (ctx->d_stats) cudaFree(ctx->d_stats);
@@ -538,7 +538,7 @@ int rk_group_statistics(rk_ctx *ctx, unsigned flags, const rk_group_stats **stat
     }
     ctx->stats_cap = cap;
   }
-  launch_group_stats(ctx->out_order, ctx->out_gid, ctx->out_identity, ctx->rec4, ctx->m, (u32)ng, (rk_group_stats_dev *)ctx->d_stats, st);
+  launch_group_stats(order, gid, identity, rec4, rows, m, (u32)ng, gid_base, line_off, (rk_group_stats_dev *)ctx->d_stats, st);
   if ((flags & RK_F_HOST_RESULT) && ng) {
     if (ng > ctx->h_stats_cap) {
       CK(cudaStreamSynchronize(st));
@@ -552,6 +552,21 @@ int rk_group_statistics(rk_ctx *ctx, unsigned flags, const rk_group_stats **stat
   }
   CK(cudaStreamSynchronize(st));
   CK(cudaGetLastError());
+  return RK_OK;
+}
+}  // namespace rk
+
+extern "C" {
+
+int rk_group_statistics(rk_ctx *ctx, unsigned flags, const rk_group_stats **stats, const rk_group_stats **d_stats, uint64_t *n_groups) {
+  static_assert(sizeof(rk_group_stats) == sizeof(rk_group_stats_dev) && sizeof(rk_group_stats) == 40, "stats layout");
+  if (!ctx) return RK_ERR_ARG;
+  if (!ctx->loaded || !ctx->have_group) return fail(ctx, RK_ERR_STATE, "rk_group_statistics before rk_group");
+  CK(cudaSetDevice(ctx->device));
+  ProfGuard pg(ctx);
+  const u64 ng = ctx->n_groups_last;
+  const int rc = group_stats_run(ctx, flags, ctx->out_order, ctx->out_gid, ctx->out_identity, ctx->rec4, nullptr, ctx->m, ng, 0, 0);
+  if (rc) return rc;
   if (stats) *stats = ((flags & RK_F_HOST_RESULT) && ng) ? (const rk_group_stats *)ctx->h_stats : nullptr;
   if (d_stats) *d_stats = (const rk_group_stats *)ctx->d_stats;
   if (n_groups) *n_groups = ng;
@@ -574,17 +589,14 @@ int rk_diagonal_func(rk_ctx *ctx, uint64_t *diag_func) {
   return RK_OK;
 }
 
-int rk_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_text *out) {
-  if (!ctx || !out) return RK_ERR_ARG;
-  if (!ctx->loaded || !ctx->have_group) return fail(ctx, RK_ERR_STATE, "rk_format_lines before rk_group");
-  if (!ctx->aos_dev && !ctx->pk_rest)
-    return fail(ctx, RK_ERR_STATE, "the database was loaded with rk_load_packed without the xEnd/yEnd/score/similarity array");
-  if (first_line > ctx->m || n_lines > ctx->m - first_line) return fail(ctx, RK_ERR_ARG, "line range beyond the %u output lines", ctx->m);
-  if (n_lines > RK_FORMAT_MAX_LINES) return fail(ctx, RK_ERR_ARG, "at most %llu lines per call", (unsigned long long)RK_FORMAT_MAX_LINES);
+}  // extern "C"
+
+// (shared with multi.cu, rk_ctx.cuh)
+namespace rk {
+int format_on_device(rk_ctx *ctx, FormatArgs fa, u64 *nbytes) {
   CK(cudaSetDevice(ctx->device));
-  ProfGuard pg(ctx);
-  memset(out, 0, sizeof *out);
   cudaStream_t st = ctx->stream;
+  const u64 n_lines = fa.n_lines;
   const u64 text_cap = align_up(n_lines * RK_FORMAT_MAX_LINE + 16, 256);
   const u64 need = text_cap + format_work_bytes((u32)n_lines);
   if (need > ctx->d_text_bytes) {
@@ -598,10 +610,6 @@ int rk_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_text 
     }
     ctx->d_text_bytes = need;
   }
-  FormatArgs fa{};
-  fa.aos = ctx->aos_dev, fa.pk_key = ctx->pk_key, fa.pk_rest = ctx->pk_rest, fa.pk_strand = ctx->pk_strand;
-  fa.order = ctx->out_order, fa.gid = ctx->out_gid, fa.repval = ctx->out_repval, fa.identity = ctx->out_identity;
-  fa.first_line = (u32)first_line, fa.n_lines = (u32)n_lines;
   fa.text = (char *)ctx->d_text;
   u32 *work = (u32 *)((u8 *)ctx->d_text + text_cap);
   fa.total_bytes = work;  // first word of the work area; launch_format carves the rest after it
@@ -610,7 +618,11 @@ int rk_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_text 
   CK(cudaMemcpyAsync(&ctx->h_cnt->pad, fa.total_bytes, sizeof(u32), cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
   CK(cudaGetLastError());
-  const u64 nbytes = ctx->h_cnt->pad;
+  *nbytes = ctx->h_cnt->pad;
+  return RK_OK;
+}
+
+int format_text_buffer(rk_ctx *ctx, u64 nbytes, char **buf) {
   const int hb = ctx->h_text_next;
   ctx->h_text_next ^= 1;
   if (nbytes + 1 > ctx->h_text_bytes[hb]) {
@@ -620,12 +632,45 @@ int rk_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_text 
     CK(cudaHostAlloc((void **)&ctx->h_text[hb], cap, cudaHostAllocDefault));
     ctx->h_text_bytes[hb] = cap;
   }
-  if (nbytes) CK(cudaMemcpyAsync(ctx->h_text[hb], ctx->d_text, nbytes, cudaMemcpyDeviceToHost, st));
+  *buf = ctx->h_text[hb];
+  return RK_OK;
+}
+
+int format_to_host(rk_ctx *ctx, u64 nbytes, char *dst, float *ms_device) {
+  CK(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  if (nbytes) CK(cudaMemcpyAsync(dst, ctx->d_text, nbytes, cudaMemcpyDeviceToHost, st));
   CK(cudaEventRecord(ctx->ev[1], st));
   CK(cudaStreamSynchronize(st));
-  out->text = ctx->h_text[hb];
+  *ms_device = ev_ms(ctx->ev[0], ctx->ev[1]);
+  return RK_OK;
+}
+}  // namespace rk
+
+extern "C" {
+
+int rk_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_text *out) {
+  if (!ctx || !out) return RK_ERR_ARG;
+  if (!ctx->loaded || !ctx->have_group) return fail(ctx, RK_ERR_STATE, "rk_format_lines before rk_group");
+  if (!ctx->aos_dev && !ctx->pk_rest)
+    return fail(ctx, RK_ERR_STATE, "the database was loaded with rk_load_packed without the xEnd/yEnd/score/similarity array");
+  if (first_line > ctx->m || n_lines > ctx->m - first_line) return fail(ctx, RK_ERR_ARG, "line range beyond the %u output lines", ctx->m);
+  if (n_lines > RK_FORMAT_MAX_LINES) return fail(ctx, RK_ERR_ARG, "at most %llu lines per call", (unsigned long long)RK_FORMAT_MAX_LINES);
+  CK(cudaSetDevice(ctx->device));
+  ProfGuard pg(ctx);
+  memset(out, 0, sizeof *out);
+  FormatArgs fa{};
+  fa.aos = ctx->aos_dev, fa.pk_key = ctx->pk_key, fa.pk_rest = ctx->pk_rest, fa.pk_strand = ctx->pk_strand;
+  fa.order = ctx->out_order, fa.gid = ctx->out_gid, fa.repval = ctx->out_repval, fa.identity = ctx->out_identity;
+  fa.first_line = (u32)first_line, fa.n_lines = (u32)n_lines;
+  u64 nbytes = 0;
+  char *buf = nullptr;
+  int rc = format_on_device(ctx, fa, &nbytes);
+  if (!rc) rc = format_text_buffer(ctx, nbytes, &buf);
+  if (!rc) rc = format_to_host(ctx, nbytes, buf, &out->ms_device);
+  if (rc) return rc;
+  out->text = buf;
   out->n_bytes = nbytes;
-  out->ms_device = ev_ms(ctx->ev[0], ctx->ev[1]);
   return RK_OK;
 }
 

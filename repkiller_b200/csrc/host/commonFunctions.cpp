@@ -54,7 +54,7 @@ void build_groups(const FragmentsDatabase &db, const rk_result &r, FGList &out) 
 }
 
 [[noreturn]] void device_error(const FragmentsDatabase &db) {
-  throw std::runtime_error(std::string("repkiller-b200: ") + rk_last_error(db.ctx()));
+  throw std::runtime_error(std::string("repkiller-b200: ") + (db.multi() ? rk_multi_last_error(db.multi()) : rk_last_error(db.ctx())));
 }
 
 }  // namespace
@@ -189,7 +189,8 @@ void save_frag_pair(std::ostream &out_file, uint64_t, uint64_t, const sequence_m
 }
 
 // The same file as save_all_frag_pairs, without the detour over an FGList: the lines of the last rk_group on this
-// database are formatted on the device (rk_format_lines, K6) and written chunk by chunk.
+// database are formatted on the device (rk_format_lines, K6; over several GPUs rk_multi_format_lines, every GPU its own
+// lines) and written chunk by chunk.
 void save_device_text(const std::string &out_file_base_path, const sequence_manager &seq_manager, const FragmentsDatabase &db,
                       float *ms_format) {
   std::ofstream out_file(out_file_base_path, std::ofstream::out | std::ofstream::binary);
@@ -205,7 +206,7 @@ void save_device_text(const std::string &out_file_base_path, const sequence_mana
   while (done < kept) {
     const uint64_t cnt = kept - done < kChunk ? kept - done : kChunk;
     rk_text t;
-    const int rc = rk_format_lines(db.ctx(), done, cnt, &t);
+    const int rc = db.multi() ? rk_multi_format_lines(db.multi(), done, cnt, &t) : rk_format_lines(db.ctx(), done, cnt, &t);
     if (writer.joinable()) writer.join();  // chunk k-1 is on its way to the file before chunk k+1 may reuse its buffer
     if (rc != RK_OK) device_error(db);
     writer = std::thread([&out_file, t] { out_file.write(t.text, (std::streamsize)t.n_bytes); });

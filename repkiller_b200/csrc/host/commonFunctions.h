@@ -34,7 +34,8 @@ void save_frag_pair(std::ostream &out_file, uint64_t seq1_label, uint64_t seq2_l
                     const FGList &fgl);
 void save_all_frag_pairs(const std::string &out_file_base_path, const sequence_manager &seq_manager, const FGList &fgl);
 // The same file for the result of the last rk_group on frags_db, its lines formatted on the device (K6, rk_format_lines):
-// no FGList, no per-line host formatting.  Throws std::runtime_error when the path cannot be opened (like the above).
+// no FGList, no per-line host formatting.  Over several GPUs (frags_db.multi()) the last rk_multi_group must have had
+// RK_F_LINE_RECORDS; every GPU formats its own lines (rk_multi_format_lines).  Throws std::runtime_error when the path cannot be opened (like the above).
 void save_device_text(const std::string &out_file_base_path, const sequence_manager &seq_manager, const FragmentsDatabase &frags_db,
                       float *ms_format = nullptr);
 void free_groups(FGList *fgl);

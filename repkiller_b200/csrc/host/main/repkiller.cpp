@@ -4,9 +4,11 @@
 // Parameter pairs are processed in argv order on one device context while the writer thread saves the previous
 // result; every pair writes the same path (as in the reference, repkiller.cpp:95-96), so the last pair's file
 // remains ([survey choice]: the reference's 3-thread pool makes the survivor timing dependent).
-// RK_TIMING=1 prints per-stage device times on stderr; RK_DEVICE selects the GPU; RK_LEGACY_WRITER=1 formats the output on
-// the host through FGList + SaverQueue instead of on the device (K6).  RK_DEVICES=0,1,... partitions the comparison over
-// several GPUs (rk_create_multi; NCCL between distinct devices); its lines are written by the host writer.
+// RK_TIMING=1 prints per-stage device times on stderr (writer=device|host: which writer made the file); RK_DEVICE selects
+// the GPU; RK_LEGACY_WRITER=1 formats the output on the host through FGList + SaverQueue instead of on the device (K6).
+// RK_DEVICES=0,1,... partitions the comparison over several GPUs (rk_create_multi; NCCL between distinct devices); every
+// GPU formats its own range of output lines (RK_F_LINE_RECORDS, rk_multi_format_lines), or the host writer does it
+// under RK_LEGACY_WRITER=1.
 #include <chrono>
 #include <cstdlib>
 #include <fstream>
@@ -31,13 +33,18 @@ static void execWithParams(const FragmentsDatabase &frag_db, const sequence_mana
     FGList *groups = group_and_sort(frag_db, param.first, param.second, &st);  // repkiller.cpp:83-91 in one device pass
     if (timing)
       std::cerr << "[rk] len_ratio=" << param.first << " pos_ratio=" << param.second << " groups=" << st.n_groups
-                << " device_ms=" << st.ms_device << " launches=" << st.n_launches << "\n";
+                << " device_ms=" << st.ms_device << " launches=" << st.n_launches << " writer=host\n";
     sq.addRequest(out_path, groups);  // repkiller.cpp:95-96
     return;
   }
-  // grouping (K3-K5) and the text of the output file (K6) on the device; the host only writes bytes
-  if (rk_group(frag_db.ctx(), param.first, param.second, RK_F_TIMING, &st) != RK_OK)
+  // grouping (K3-K5) and the text of the output file (K6) on the device; the host only writes bytes.  Over several GPUs
+  // every line's record is first brought to the GPU that holds the line.
+  if (frag_db.multi()) {
+    if (rk_multi_group(frag_db.multi(), param.first, param.second, RK_F_LINE_RECORDS | RK_F_TIMING, &st) != RK_OK)
+      throw std::runtime_error(std::string("repkiller-b200: ") + rk_multi_last_error(frag_db.multi()));
+  } else if (rk_group(frag_db.ctx(), param.first, param.second, RK_F_TIMING, &st) != RK_OK) {
     throw std::runtime_error(std::string("repkiller-b200: ") + rk_last_error(frag_db.ctx()));
+  }
   float ms_format = 0.f;
   const auto tw0 = std::chrono::steady_clock::now();
   try {
@@ -50,7 +57,7 @@ static void execWithParams(const FragmentsDatabase &frag_db, const sequence_mana
   if (timing)
     std::cerr << "[rk] len_ratio=" << param.first << " pos_ratio=" << param.second << " groups=" << st.n_groups
               << " device_ms=" << st.ms_device << " launches=" << st.n_launches << " format_ms=" << ms_format << " write_call_ms="
-              << std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tw0).count() << "\n";
+              << std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tw0).count() << " writer=device\n";
 }
 
 int main(int argc, char *argv[]) {
@@ -71,7 +78,6 @@ int main(int argc, char *argv[]) {
                "\n"
             << std::flush;
   const bool timing = getenv("RK_TIMING") != nullptr;
-  const bool legacy_env = getenv("RK_LEGACY_WRITER") != nullptr;
   std::vector<int> devices;
   if (const char *list = getenv("RK_DEVICES")) {
     for (const char *p = list; *p;) {
@@ -81,7 +87,7 @@ int main(int argc, char *argv[]) {
     }
   }
   if (devices.empty()) devices.push_back(getenv("RK_DEVICE") ? atoi(getenv("RK_DEVICE")) : 0);
-  const bool legacy_writer = legacy_env || devices.size() > 1;
+  const bool legacy_writer = getenv("RK_LEGACY_WRITER") != nullptr;
 
   sequence_manager seq_manager;
   // (beside the reference's CSV: GECKO's binary .frags container, see FragmentsDatabase.h)

@@ -8,55 +8,38 @@
 // Two passes over a range of output lines: (1) the length of every line (the same formatter with a counting sink),
 // an exclusive scan gives the byte offset of every line; (2) a CTA formats its 128 lines into shared memory and copies
 // the block out with coalesced stores.  The "%g" digits are exact (rk_fmt.cuh: integer arithmetic on the binary value).
+// A line's fields come from its record (order[j] into the loaded records) or, on a rank of a partitioned comparison, from
+// the line row that rk_dist_group brought to the rank (RK_F_LINE_RECORDS): the same fields, so the same bytes.
 #include "rk_common.cuh"
 #include "rk_fmt.cuh"
 #include "rk_scan.cuh"
 
 namespace rk {
 
-constexpr int OFF_XEND = 24, OFF_YEND = 32, OFF_SCORE = 56, OFF_SIMILARITY = 64;
 constexpr int FMT_THREADS = 128;
 constexpr int FMT_MAX_LINE = RK_FORMAT_MAX_LINE;  // 5 + 8 x 20 digits + 10 (gid) + 1 + 2 x 13 ("%g") + 2 + 13 commas + newline, rounded up
 
-__device__ __forceinline__ u64 ldg_u64_unaligned(const u8 *p) {  // records are 109 bytes apart: no alignment to rely on
-  u64 v = 0;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) v |= (u64)p[i] << (8 * i);
-  return v;
-}
-
-struct LineFields {  // what one output line prints of its record
-  u64 xs, ys, xe, ye, len, score, ident;
-  u32 sim_bits;
-  char strand;
-};
-__device__ __forceinline__ LineFields load_fields(const FormatArgs &a, u32 fidx) {
-  LineFields f;
-  if (a.aos) {
-    const u8 *rec = a.aos + (u64)fidx * FRAG_BYTES;
-    f.xs = ldg_u64_unaligned(rec + OFF_XSTART), f.ys = ldg_u64_unaligned(rec + OFF_YSTART);
-    f.xe = ldg_u64_unaligned(rec + OFF_XEND), f.ye = ldg_u64_unaligned(rec + OFF_YEND);
-    f.len = ldg_u64_unaligned(rec + OFF_LENGTH), f.score = ldg_u64_unaligned(rec + OFF_SCORE), f.ident = ldg_u64_unaligned(rec + OFF_IDENT);
-    f.sim_bits = (u32)rec[OFF_SIMILARITY] | ((u32)rec[OFF_SIMILARITY + 1] << 8) | ((u32)rec[OFF_SIMILARITY + 2] << 16) |
-                 ((u32)rec[OFF_SIMILARITY + 3] << 24);
-    f.strand = (char)rec[OFF_STRAND];
-  } else {  // compact ingest: two 16-byte words and a byte
-    const uint4 k = a.pk_key[fidx], r = a.pk_rest[fidx];
-    f.xs = k.x, f.ys = k.y, f.len = k.z, f.ident = k.w;
-    f.xe = r.x, f.ye = r.y, f.score = r.z, f.sim_bits = r.w;
-    f.strand = (char)a.pk_strand[fidx];
-  }
+// what output line j prints of its record: its line row, or the record order[j] (109-byte records or the compact arrays)
+__device__ __forceinline__ LineRow load_fields(const FormatArgs &a, u32 j) {
+  if (a.rows) return a.rows[j];
+  const u32 fidx = a.order[j];
+  if (a.aos) return line_row_of_record(a.aos + (u64)fidx * FRAG_BYTES);
+  LineRow f;  // compact ingest: two 16-byte words and a byte
+  const uint4 k = a.pk_key[fidx], r = a.pk_rest[fidx];
+  f.xs = k.x, f.ys = k.y, f.len = k.z, f.ident = k.w;
+  f.xe = r.x, f.ye = r.y, f.score = r.z, f.sim_bits = r.w;
+  f.strand = a.pk_strand[fidx];
   return f;
 }
 
 template <class Sink>
-__device__ __forceinline__ void format_line(Sink &s, const LineFields &f, u32 gid, u32 identity_bits, u32 repval) {
+__device__ __forceinline__ void format_line(Sink &s, const LineRow &f, u32 gid, u32 identity_bits, u32 repval) {
   s.put('F'), s.put('r'), s.put('a'), s.put('g'), s.put(',');
   rkfmt::put_u64(s, f.xs), s.put(',');
   rkfmt::put_u64(s, f.ys), s.put(',');
   rkfmt::put_u64(s, f.xe), s.put(',');
   rkfmt::put_u64(s, f.ye), s.put(',');
-  s.put(f.strand), s.put(',');
+  s.put((char)f.strand), s.put(',');
   rkfmt::put_u64(s, gid), s.put(',');
   rkfmt::put_u64(s, f.len), s.put(',');
   rkfmt::put_u64(s, f.score), s.put(',');
@@ -72,7 +55,7 @@ __global__ void __launch_bounds__(FMT_THREADS) k_format_len(FormatArgs a) {
   if (i >= a.n_lines) return;
   const u32 j = a.first_line + i;
   rkfmt::CountSink s;
-  format_line(s, load_fields(a, a.order[j]), a.gid[j], __float_as_uint(a.identity[j]), a.repval[j]);
+  format_line(s, load_fields(a, j), a.gid[j], __float_as_uint(a.identity[j]), a.repval[j]);
   a.line_len[i] = s.n;
 }
 
@@ -85,7 +68,7 @@ __global__ void __launch_bounds__(FMT_THREADS) k_format_write(FormatArgs a) {
   if (i < a.n_lines) {
     const u32 j = a.first_line + i;
     rkfmt::BufSink s(s_text + (a.line_off[i] - base));
-    format_line(s, load_fields(a, a.order[j]), a.gid[j], __float_as_uint(a.identity[j]), a.repval[j]);
+    format_line(s, load_fields(a, j), a.gid[j], __float_as_uint(a.identity[j]), a.repval[j]);
   }
   __syncthreads();
   char *out = a.text + base;

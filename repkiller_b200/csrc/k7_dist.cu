@@ -318,6 +318,14 @@ struct PayQuery {  // forest: "what is behind global rank keys[i]?" asked of the
   __device__ __forceinline__ void load(u32 i, uint4 *v) const { v[0] = make_uint4(keys[i], 0u, 0u, 0u); }
 };
 
+struct PayLineReq {  // line records: "send me the record of file index keys[i] for my line i", asked of the rank that loaded it
+  typedef uint4 Word;
+  static constexpr int WPR = 1;
+  const u32 *keys;
+  RowOuts out;
+  __device__ __forceinline__ void load(u32 i, uint4 *v) const { v[0] = make_uint4(keys[i], i, 0u, 0u); }
+};
+
 template <int MODE, class Pay>
 __global__ void __launch_bounds__(256) k_split_pack(RouteArgs a, const u32 *__restrict__ tile_off, Pay pay, u32 *__restrict__ perm) {
   __shared__ u32 s_cuts[2 * DIST_MAX_RANKS + 2];
@@ -760,6 +768,23 @@ __global__ void __launch_bounds__(256) k_chase_map(const u64 *__restrict__ res, 
   gid_rank[i] = (w & RES_ROOT) ? s_base + (u32)w : gid_l[lroot[i]];
 }
 
+// ---- line records ----------------------------------------------------------------------------------------------------
+// The rank that loaded a record answers every request for it with the line row, stored straight into the asking rank's
+// rows[line] (requests arrive in blocks by source rank: the block gives the asking rank, the request its line).
+__global__ void __launch_bounds__(256) k_line_answer(const uint4 *__restrict__ requests, u32 n, const u8 *__restrict__ aos, u32 file_lo,
+                                                     ScatterTable back) {
+  const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const uint4 q = requests[t];
+  int s = 0;
+  for (int r = 1; r < back.nr; ++r) s = back.start[r] <= t ? r : s;
+  const LineRow row = line_row_of_record(aos + (u64)(q.x - file_lo) * FRAG_BYTES);
+  uint4 *dst = reinterpret_cast<uint4 *>(reinterpret_cast<LineRow *>(back.out[s]) + q.y);
+  const uint4 *src = reinterpret_cast<const uint4 *>(&row);
+#pragma unroll
+  for (int k = 0; k < 4; ++k) dst[k] = src[k];
+}
+
 // ---- small helpers ---------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_or_rows(const u32 *__restrict__ all, u64 row_stride, int nr, u64 words, u32 *__restrict__ out) {
   const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
@@ -840,6 +865,8 @@ cudaError_t dist_init_device() {  // dynamic shared memory opt-in of the push ke
   e = cudaFuncSetAttribute(k_push_rows<PayRec24>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PushSmem<uint2, 3>));
   if (e != cudaSuccess) return e;
   e = cudaFuncSetAttribute(k_push_rows<PayQuery>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PushSmem<uint4, 1>));
+  if (e != cudaSuccess) return e;
+  e = cudaFuncSetAttribute(k_push_rows<PayLineReq>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PushSmem<uint4, 1>));
   if (e != cudaSuccess) return e;
   return cudaFuncSetAttribute(k_push_rows<PayGidRow>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PushSmem<uint4, 1>));
 }
@@ -1001,6 +1028,17 @@ int dist_chase_finish(const PeerTable &pt, const u32 *nroots, u32 stride, u32 m,
   KScope ks(KID_CHASE, st, m);
   k_chase_map<<<blocks_for(m), 256, 0, st>>>(res, lroot, gid_l, nroots, stride, pt.me, m, gid_rank);
   return 2;
+}
+int dist_line_ask_push(const u32 *order, u32 n, const u32 *file_cuts, int nr, uint4 *const *outs, u32 out_cap, u32 *tile_cnt,
+                       const u32 *counts_all, u32 row_stride, int me, cudaStream_t st) {
+  return push_rows(RouteArgs{order, n, file_cuts, nr, me, 0xFFFFFFFFu, 0, out_cap, nullptr}, tile_cnt, counts_all, row_stride, me,
+                   PayLineReq{order, row_outs<uint4>(outs, nr)}, st);
+}
+int dist_line_answer(const uint4 *requests, u32 n, const u8 *aos, u32 file_lo, const ScatterTable &back, cudaStream_t st) {
+  if (n == 0) return 0;
+  KScope ks(KID_DIST_ROWS, st, n);
+  k_line_answer<<<blocks_for(n), 256, 0, st>>>(requests, n, aos, file_lo, back);
+  return 1;
 }
 int dist_or_rows(const u32 *all, u64 row_stride, int nr, u64 words, u32 *out, cudaStream_t st) {
   if (words == 0) return 0;

@@ -26,7 +26,8 @@ __global__ void __launch_bounds__(256) k_stats_init(rk_group_stats_dev *__restri
 }
 
 __global__ void __launch_bounds__(256) k_group_stats(const u32 *__restrict__ out_order, const u32 *__restrict__ out_gid,
-                                                     const float *__restrict__ out_identity, const uint4 *__restrict__ rec4, u32 m,
+                                                     const float *__restrict__ out_identity, const uint4 *__restrict__ rec4,
+                                                     const LineRow *__restrict__ rows, u32 m, u32 gid_base, u32 line_off,
                                                      rk_group_stats_dev *__restrict__ st) {
   const u32 j = blockIdx.x * blockDim.x + threadIdx.x;
   const u32 lane = threadIdx.x & 31;
@@ -35,9 +36,15 @@ __global__ void __launch_bounds__(256) k_group_stats(const u32 *__restrict__ out
   double slen = 0.0, sid = 0.0;
   if (valid) {
     gid = out_gid[j];
-    const uint4 r = rec4[2 * (u64)out_order[j]];  // {xStart, yStart, length, flags}
-    cnt = 1, xlo = r.x, xhi = r.x + r.z, ylo = r.y, yhi = r.y + r.z, first = j;
-    slen = (double)r.z;
+    u32 xs, ys, len;
+    if (rows) {
+      xs = (u32)rows[j].xs, ys = (u32)rows[j].ys, len = (u32)rows[j].len;  // K1 refused anything wider
+    } else {
+      const uint4 r = rec4[2 * (u64)out_order[j]];  // {xStart, yStart, length, flags}
+      xs = r.x, ys = r.y, len = r.z;
+    }
+    cnt = 1, xlo = xs, xhi = xs + len, ylo = ys, yhi = ys + len, first = line_off + j;
+    slen = (double)len;
     sid = (double)out_identity[j];
   }
   // segmented inclusive scan inside the warp: lane l accumulates the lanes of its run at or before it
@@ -59,7 +66,7 @@ __global__ void __launch_bounds__(256) k_group_stats(const u32 *__restrict__ out
   const u32 gnext = __shfl_down_sync(0xFFFFFFFFu, gid, 1);
   const bool run_end = valid && (lane == 31 || gnext != gid);
   if (run_end) {
-    rk_group_stats_dev *s = st + gid;
+    rk_group_stats_dev *s = st + (gid - gid_base);
     atomicAdd(&s->count, cnt);
     atomicMin(&s->x_lo, xlo);
     atomicMax(&s->x_hi, xhi);
@@ -81,12 +88,12 @@ __global__ void __launch_bounds__(256) k_stats_final(rk_group_stats_dev *__restr
   st[g] = s;
 }
 
-int launch_group_stats(const u32 *out_order, const u32 *out_gid, const float *out_identity, const uint4 *rec4, u32 m, u32 n_groups,
-                       rk_group_stats_dev *st, cudaStream_t stream) {
+int launch_group_stats(const u32 *out_order, const u32 *out_gid, const float *out_identity, const uint4 *rec4, const LineRow *rows,
+                       u32 m, u32 n_groups, u32 gid_base, u32 line_off, rk_group_stats_dev *st, cudaStream_t stream) {
   if (n_groups == 0) return 0;
   KScope ks(KID_STATS, stream, m);
   k_stats_init<<<(n_groups + 255) / 256, 256, 0, stream>>>(st, n_groups);
-  k_group_stats<<<(m + 255) / 256, 256, 0, stream>>>(out_order, out_gid, out_identity, rec4, m, st);
+  k_group_stats<<<(m + 255) / 256, 256, 0, stream>>>(out_order, out_gid, out_identity, rec4, rows, m, gid_base, line_off, st);
   k_stats_final<<<(n_groups + 255) / 256, 256, 0, stream>>>(st, n_groups);
   return 3;
 }

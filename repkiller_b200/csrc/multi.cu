@@ -14,6 +14,8 @@
 //          -> Y pass (K3) -> the Y owners stored at the home ranks -> root scan; local chains; chains that leave the GPU in
 //          bulk ask/answer rounds (many) or by walking the peers' res[] (few) (K4) -> output rows (16 B) stored at the
 //          owner of their group-id range -> K5b/c                                                [2 host syncs: counts]
+//          (RK_F_LINE_RECORDS) -> every line asks the rank that loaded its record; that rank stores the 64-byte line row
+//          at the asker's line_rows[line], for K6 / K8 on the rank that holds the line            [1 host sync: counts]
 //
 // Every rank's partition arena is carved identically and mapped into every peer (cudaIpc handles between processes, raw
 // pointers + cudaDeviceEnablePeerAccess inside one), so a local buffer address translates to the same buffer on any rank;
@@ -91,6 +93,7 @@ constexpr int W_X1 = 42;         // total groups
 constexpr int W_X2 = 43;         // forest: fragments of the rank whose chain is still waiting for an answer from another rank
 constexpr int W_CUTSX = 64;      // [2][nr] the first X super-bucket key every rank owns, per strand class
 constexpr int W_CUTS = 44;       // [nr+1] the cuts of the exchange (identical on every rank; the host sizes the local sort keys from them)
+constexpr int W_FOFF = 61;       // exchange 1: the file index of the rank's first record (rk_dist_load_aos's file_offset)
 
 struct Exchange {  // counts of one variable all-to-all, as this rank sees it (elements)
   u64 soff[DIST_MAX_RANKS], scnt[DIST_MAX_RANKS], roff[DIST_MAX_RANKS], rcnt[DIST_MAX_RANKS];
@@ -399,6 +402,14 @@ struct Dist {
   u32 m_loc = 0, rank_off = 0, n_halo = 0, n_away = 0, m_y = 0;
   u64 m_total = 0, n_total_loaded = 0;
   Exchange ex1, exh, exy;
+  const u8 *aos_src = nullptr;          // this rank's slice of the records on the device (aos_buf or the caller's pointer)
+  u32 file_off[DIST_MAX_RANKS] = {0};  // first file index of every rank's slice
+  bool slices_in_order = false;         // every slice ends at or before the next rank's starts: file_off[] routes a file index
+
+  // state of the last group: this rank's output lines and groups; line rows (RK_F_LINE_RECORDS) valid
+  bool have_rows = false;
+  u32 n_lines = 0, gid_base = 0, n_groups_rank = 0;
+  u64 line_off = 0;
 
   // carved device pointers
   Counters *cnt = nullptr;
@@ -407,6 +418,7 @@ struct Dist {
   u32 *hist = nullptr, *hist_all = nullptr, *cuts0 = nullptr, *cuts_y = nullptr, *cuts_x = nullptr, *cuts_g = nullptr;
   uint4 *rec4_loc = nullptr, *send_rows = nullptr, *recv_rows = nullptr;
   uint2 *rec6_arr = nullptr;  // the records this rank owns, in arrival order: 24-byte rows stored by the peers' push kernels
+  LineRow *line_rows = nullptr;  // RK_F_LINE_RECORDS: one row per output line, over rec4_loc ++ send_rows ++ rec6_arr
   u32 *key0_loc = nullptr, *tile_cnt = nullptr, *perm_x = nullptr, *perm_y = nullptr;
   u32 *key0a = nullptr, *k0_r = nullptr, *aidx_r = nullptr, *tmp_k = nullptr, *tmp_v = nullptr;
   void *sort_work = nullptr;
@@ -458,6 +470,10 @@ static u64 dist_carve(Dist &D, u8 *base) {
   D.rec4_loc = (uint4 *)take(M * 32);
   D.send_rows = (uint4 *)take(M * 16);
   D.rec6_arr = (uint2 *)take(M * 24);
+  // Only the load reads or writes the three regions above, so after it they hold the line rows of rk_dist_group with
+  // RK_F_LINE_RECORDS: 72 B per row of capacity, back to back, for 64 B per line (a rank never holds more lines than rows).
+  D.line_rows = (LineRow *)D.rec4_loc;
+  static_assert(sizeof(LineRow) <= 32 + 16 + 24, "line rows fit in the load-time regions");
   D.recv_rows = (uint4 *)take(M * 16);
   D.key0_loc = (u32 *)take(M * 4);
   D.tile_cnt = (u32 *)take(dist_split_work_bytes(M));
@@ -683,6 +699,7 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   ProfGuard pg(ctx);
   cudaStream_t st = ctx->stream;
   D.loaded = false;
+  D.have_rows = false;
   ctx->have_group = false;
   // NOTE: argument errors that only ONE rank can see (n_loc > cap) are turned into an error word all ranks receive with
   // the first count exchange, so that no rank is left waiting in a collective.
@@ -729,6 +746,7 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
     CK(cudaMemcpyAsync(D.aos_buf, frags, n_use * RK_FRAG_BYTES, cudaMemcpyHostToDevice, st));
     aos = D.aos_buf;
   }
+  D.aos_src = aos;
   CK(cudaEventRecord(ev[1], st));
   u64 launches = 0;
 
@@ -760,6 +778,8 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   launches += dist_count_plain(D.key0_loc, (u32)n_use, D.cuts0, nr, g.vsize - 1, D.tile_cnt, D.d_small + W_CNT_A, st);
   CK(cudaMemcpyAsync(D.d_small + W_ERR, &D.cnt->err, sizeof(u32), cudaMemcpyDeviceToDevice, st));
   CK(cudaMemcpyAsync(D.d_small + W_CUTS, D.cuts0, (nr + 1) * sizeof(u32), cudaMemcpyDeviceToDevice, st));
+  const u32 foff32 = (u32)file_off;
+  CK(cudaMemcpyAsync(D.d_small + W_FOFF, &foff32, sizeof(u32), cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
   TR(D.tr->gather_small_begin(D.d_small, D.d_small_all, D.h_small, st));
   launches += dist_push_records(D.key0_loc, (u32)n_use, D.cuts0, nr, g.vsize - 1, D.rec4_loc, outs, (u32)D.cap, D.tile_cnt, D.d_small_all,
                                 SMALL_WORDS, me, st);
@@ -773,6 +793,16 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
     return dist_check_small(ctx, true);
   }
   D.ex1.from_matrix(D.h_small, W_CNT_A, nr, me);
+  // where every rank's slice starts (as its caller said) and, from the row sums of the count matrix (the dropped column
+  // included), how long it is: the line records of RK_F_LINE_RECORDS find the rank that loaded a record by these starts,
+  // which needs the slices in rank order without overlap.  Every rank sees the same matrix, so all agree on the verdict.
+  D.slices_in_order = true;
+  for (int s = 0; s < nr; ++s) {
+    u64 n_s = 0;
+    for (int d = 0; d <= nr; ++d) n_s += D.h_small[(size_t)s * SMALL_WORDS + W_CNT_A + d];
+    D.file_off[s] = D.h_small[(size_t)s * SMALL_WORDS + W_FOFF];
+    if (s + 1 < nr && D.file_off[s] + n_s > D.h_small[(size_t)(s + 1) * SMALL_WORDS + W_FOFF]) D.slices_in_order = false;
+  }
   D.tr->bytes_sent += (D.ex1.n_send - D.ex1.scnt[me]) * 24;  // (the rows this rank's kernels stored into peer memory)
   u64 loaded_total = 0, m_of[DIST_MAX_RANKS] = {0};
   for (int d = 0; d <= nr; ++d) loaded_total += column_sum(D.h_small, W_CNT_A + d, nr);
@@ -902,6 +932,8 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   if (!D.loaded) return fail(ctx, RK_ERR_STATE, "rk_dist_group before a successful rk_dist_load_aos");
   if (!(len_ratio > 0)) return fail(ctx, RK_ERR_ARG, "Ratio between length and position must be greater than zero");
   if (!(pos_ratio > 0)) return fail(ctx, RK_ERR_ARG, "Position proximity must be greater than zero");
+  if ((flags & RK_F_LINE_RECORDS) && !D.slices_in_order)
+    return fail(ctx, RK_ERR_ARG, "RK_F_LINE_RECORDS needs the ranks' slices of the file in rank order (file_offset of rk_dist_load_aos)");
   CK(cudaSetDevice(ctx->device));
   ProfGuard pg(ctx);
   memset(out, 0, sizeof *out);
@@ -910,6 +942,8 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   const u32 m = D.m_loc, nh = D.n_halo, mc = m + nh;
   u64 launches = 0;
   const u64 sent0 = D.tr->bytes_sent;
+  const bool line_records = (flags & RK_F_LINE_RECORDS) != 0;
+  D.have_rows = false;
   CK(cudaMemsetAsync(D.d_small, 0, SMALL_WORDS * 4, st));
 
   CK(cudaEventRecord(ev[0], st));
@@ -1048,6 +1082,34 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   oa.err = &D.cnt->err;
   launches += launch_order(oa, st);
   CK(cudaEventRecord(ev[5], st));
+  // line records: every line asks the rank that loaded its record for what the line prints, and that rank stores the
+  // 64-byte row straight into line_rows[line] here.  A bulk round of the forest in form: a count exchange, the requests
+  // pushed into the owners' `queries` (free again: the forest is done), the answers stored back by the owners' kernel,
+  // a barrier.  The gid cuts are spent, so cuts_g carries the slice starts.
+  if (line_records) {
+    CK(cudaMemcpyAsync(D.cuts_g, D.file_off, nr * sizeof(u32), cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
+    uint4 *qouts[DIST_MAX_RANKS];
+    peer_rows(D, D.queries, qouts);
+    launches += dist_count_plain(D.out_order, mg, D.cuts_g, nr, 0xFFFFFFFFu, D.tile_cnt, D.d_small + W_CNT_A, st);
+    CK(cudaMemcpyAsync(D.d_small + W_ERR, &D.cnt->err, sizeof(u32), cudaMemcpyDeviceToDevice, st));
+    TR(D.tr->gather_small_begin(D.d_small, D.d_small_all, D.h_small, st));
+    launches += dist_line_ask_push(D.out_order, mg, D.cuts_g, nr, qouts, (u32)D.cap, D.tile_cnt, D.d_small_all, SMALL_WORDS, me, st);
+    TR(D.tr->barrier(st));
+    TR(D.tr->gather_small_end(D.d_small_all, D.h_small, st));  // host sync 4
+    const int rc2 = dist_check_small(ctx, false);
+    if (rc2) return rc2;
+    for (int d = 0; d < nr; ++d) {  // (a rank is asked only about the records of its slice, which fits its rows)
+      const u64 in = column_sum(D.h_small, W_CNT_A + d, nr);
+      if (in > D.cap) return fail(ctx, RK_ERR_NOMEM, "rank %d is asked for %llu line records, capacity is %llu rows per rank", d,
+                                  (unsigned long long)in, (unsigned long long)D.cap);
+    }
+    Exchange exl;
+    exl.from_matrix(D.h_small, W_CNT_A, nr, me);
+    D.tr->bytes_sent += (exl.n_send - exl.scnt[me]) * 16 + (exl.n_recv - exl.rcnt[me]) * sizeof(LineRow);
+    launches += dist_line_answer(D.queries, (u32)exl.n_recv, D.aos_src, D.file_off[me], scatter_table(D, exl, true, D.line_rows), st);
+    TR(D.tr->barrier(st));
+    CK(cudaEventRecord(ev[8], st));
+  }
 
   u32 *h_order = nullptr, *h_gid = nullptr;
   float *h_ident = nullptr;
@@ -1078,12 +1140,20 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   CK(cudaGetLastError());
   if (ctx->h_cnt->err) return fail(ctx, RK_ERR_INTERNAL, "%s", err_bits_text(ctx->h_cnt->err));
   if (D.trace.on) {
-    char cb[200];
+    char cb[240];
     snprintf(cb, sizeof cb, "ranked=%u halo_in=%u halo_out=%u y=%u lines=%u groups=%llu stages x=%.3f y=%.3f forest=%.3f exch=%.3f order=%.3f |", m, nh,
              D.n_away, D.m_y, mg, (unsigned long long)total_groups, ev_ms(ev[0], ev[1]), ev_ms(ev[1], ev[2]), ev_ms(ev[2], ev[3]),
              ev_ms(ev[3], ev[4]), ev_ms(ev[4], ev[5]));
+    if (line_records) {
+      const size_t k = strlen(cb) - 2;  // before the closing " |"
+      snprintf(cb + k, sizeof cb - k, " rows=%.3f |", ev_ms(ev[5], ev[8]));
+    }
     D.trace.dump(me, cb);
   }
+  D.n_lines = mg, D.line_off = line_off;
+  D.gid_base = (u32)std::min<u64>(gid_base, total_groups);
+  D.n_groups_rank = (u32)(gid_end > D.gid_base ? gid_end - D.gid_base : 0);
+  D.have_rows = line_records;
 
   out->n_kept = mg;
   out->n_groups = total_groups;
@@ -1097,7 +1167,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
     out->ms_stage[RK_ST_HKEY] = ev_ms(ev[3], ev[4]);   // output exchange
     out->ms_stage[RK_ST_GSORT] = ev_ms(ev[4], ev[5]);
     if (h_order) out->ms_stage[RK_ST_D2H] = ev_ms(ev[6], ev[7]);
-    out->ms_device = ev_ms(ev[0], ev[5]);
+    out->ms_device = ev_ms(ev[0], line_records ? ev[8] : ev[5]);
   }
   if (info) {
     memset(info, 0, sizeof *info);
@@ -1119,6 +1189,38 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
 
 static void peer_rows(const Dist &D, uint4 *local, uint4 **outs) {
   for (int d = 0; d < D.world; ++d) outs[d] = d == D.rank ? local : D.tr->on_peer(d, local);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// output of a rank from its line rows: K6 and K8 as on one GPU (no collective step)
+// ---------------------------------------------------------------------------------------------------------------------
+static int dist_rows_ready(rk_ctx *ctx, const char *what) {
+  if (!ctx->dist) return fail(ctx, RK_ERR_STATE, "%s before rk_dist_init", what);
+  if (!ctx->dist->have_rows) return fail(ctx, RK_ERR_STATE, "%s needs the last rk_dist_group to have RK_F_LINE_RECORDS", what);
+  return RK_OK;
+}
+
+// K6 over local lines first_line .. first_line+n_lines of the last grouping, into the context's device text buffer
+static int dist_format_device(rk_ctx *ctx, u64 first_line, u64 n_lines, u64 *nbytes) {
+  const int rc = dist_rows_ready(ctx, "rk_dist_format_lines");
+  if (rc) return rc;
+  const Dist &D = *ctx->dist;
+  if (first_line > D.n_lines || n_lines > D.n_lines - first_line)
+    return fail(ctx, RK_ERR_ARG, "line range beyond the %u output lines of rank %d", D.n_lines, D.rank);
+  if (n_lines > RK_FORMAT_MAX_LINES) return fail(ctx, RK_ERR_ARG, "at most %llu lines per call", (unsigned long long)RK_FORMAT_MAX_LINES);
+  FormatArgs fa{};
+  fa.rows = D.line_rows;
+  fa.order = D.out_order, fa.gid = D.out_gid, fa.repval = D.out_repval, fa.identity = D.out_identity;
+  fa.first_line = (u32)first_line, fa.n_lines = (u32)n_lines;
+  return format_on_device(ctx, fa, nbytes);
+}
+
+static int dist_group_stats(rk_ctx *ctx, unsigned flags) {
+  const int rc = dist_rows_ready(ctx, "rk_dist_group_statistics");
+  if (rc) return rc;
+  const Dist &D = *ctx->dist;
+  return group_stats_run(ctx, flags, D.out_order, D.out_gid, D.out_identity, nullptr, D.line_rows, D.n_lines, D.n_groups_rank, D.gid_base,
+                         (u32)D.line_off);
 }
 
 void dist_destroy(rk_ctx *c) {
@@ -1199,6 +1301,38 @@ int rk_dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flag
   return dist_group(ctx, len_ratio, pos_ratio, flags, out, info);
 }
 
+int rk_dist_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_text *out) {
+  if (!ctx || !out) return RK_ERR_ARG;
+  memset(out, 0, sizeof *out);
+  CK(cudaSetDevice(ctx->device));
+  ProfGuard pg(ctx);
+  u64 nbytes = 0;
+  char *buf = nullptr;
+  int rc = dist_format_device(ctx, first_line, n_lines, &nbytes);
+  if (!rc) rc = format_text_buffer(ctx, nbytes, &buf);
+  if (!rc) rc = format_to_host(ctx, nbytes, buf, &out->ms_device);
+  if (rc) return rc;
+  out->text = buf;
+  out->n_bytes = nbytes;
+  return RK_OK;
+}
+
+int rk_dist_group_statistics(rk_ctx *ctx, unsigned flags, const rk_group_stats **stats, const rk_group_stats **d_stats,
+                             uint64_t *first_gid, uint64_t *n_groups) {
+  if (!ctx) return RK_ERR_ARG;
+  CK(cudaSetDevice(ctx->device));
+  ProfGuard pg(ctx);
+  const int rc = dist_group_stats(ctx, flags);
+  if (rc) return rc;
+  const Dist &D = *ctx->dist;
+  const u64 ng = D.n_groups_rank;
+  if (stats) *stats = ((flags & RK_F_HOST_RESULT) && ng) ? (const rk_group_stats *)ctx->h_stats : nullptr;
+  if (d_stats) *d_stats = (const rk_group_stats *)ctx->d_stats;
+  if (first_gid) *first_gid = D.gid_base;
+  if (n_groups) *n_groups = ng;
+  return RK_OK;
+}
+
 }  // extern "C"
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -1218,6 +1352,12 @@ struct rk_multi {
   void *h_res = nullptr;
   u64 h_res_cap = 0;
   std::vector<rk_dist_info> infos;
+  // rk_multi_format_lines: two alternating pinned text buffers; rk_multi_group_statistics: all groups (pinned)
+  char *h_text[2] = {nullptr, nullptr};
+  u64 h_text_bytes[2] = {0, 0};
+  int h_text_next = 0;
+  void *h_stats = nullptr;
+  u64 h_stats_cap = 0;
 };
 
 namespace {
@@ -1304,6 +1444,8 @@ void rk_destroy_multi(rk_multi *mg) {
   for (rk_ctx *c : mg->ctx) rk_destroy(c);
   for (ncclComm_t c : mg->comms) nccl_api().CommDestroy(c);
   if (mg->h_res) cudaFreeHost(mg->h_res);
+  for (char *t : mg->h_text) if (t) cudaFreeHost(t);
+  if (mg->h_stats) cudaFreeHost(mg->h_stats);
   delete mg;
 }
 
@@ -1397,6 +1539,102 @@ int rk_multi_group(rk_multi *mg, double len_ratio, double pos_ratio, unsigned fl
 int rk_multi_info(const rk_multi *mg, int rank, rk_dist_info *info) {
   if (!mg || !info || rank < 0 || rank >= (int)mg->infos.size()) return RK_ERR_ARG;
   *info = mg->infos[rank];
+  return RK_OK;
+}
+
+int rk_multi_format_lines(rk_multi *mg, uint64_t first_line, uint64_t n_lines, rk_text *out) {
+  if (!mg || !out) return RK_ERR_ARG;
+  memset(out, 0, sizeof *out);
+  if ((int)mg->infos.size() != mg->n) {
+    mg->err = "rk_multi_format_lines before a successful rk_multi_group";
+    return RK_ERR_STATE;
+  }
+  u64 total = 0;
+  for (const rk_dist_info &i : mg->infos) total += i.n_lines;
+  if (first_line > total || n_lines > total - first_line) {
+    mg->err = "line range beyond the " + std::to_string(total) + " output lines";
+    return RK_ERR_ARG;
+  }
+  if (n_lines > RK_FORMAT_MAX_LINES) {
+    mg->err = "at most " + std::to_string(RK_FORMAT_MAX_LINES) + " lines per call";
+    return RK_ERR_ARG;
+  }
+  // every rank formats its part of the range on its GPU (an empty part too: every rank checks its state) ...
+  std::vector<u64> nb(mg->n, 0), pos(mg->n + 1, 0);
+  std::vector<float> ms(mg->n, 0.f);
+  int rc = run_ranks(mg, [&](int r) -> int {
+    rk_ctx *ctx = mg->ctx[r];
+    const u64 lo = mg->infos[r].line_offset, hi = lo + mg->infos[r].n_lines;
+    const u64 a = std::max<u64>(first_line, lo), b = std::min<u64>(first_line + n_lines, hi);
+    CK(cudaSetDevice(ctx->device));
+    ProfGuard pg(ctx);
+    return dist_format_device(ctx, b > a ? a - lo : 0, b > a ? b - a : 0, &nb[r]);
+  });
+  if (rc) return rc;
+  // ... and copies it to its place in one buffer: the parts in rank order are the lines in order
+  for (int r = 0; r < mg->n; ++r) pos[r + 1] = pos[r] + nb[r];
+  const u64 nbytes = pos[mg->n];
+  const int hb = mg->h_text_next;
+  mg->h_text_next ^= 1;
+  if (nbytes + 1 > mg->h_text_bytes[hb]) {
+    if (mg->h_text[hb]) cudaFreeHost(mg->h_text[hb]);
+    mg->h_text[hb] = nullptr, mg->h_text_bytes[hb] = 0;
+    const u64 cap = align_up(nbytes + nbytes / 8 + 4096, 4096);
+    if (cudaHostAlloc((void **)&mg->h_text[hb], cap, cudaHostAllocPortable) != cudaSuccess) {  // (copied into by every GPU)
+      cudaGetLastError();
+      mg->err = "cudaHostAlloc for the text failed";
+      return RK_ERR_NOMEM;
+    }
+    mg->h_text_bytes[hb] = cap;
+  }
+  char *buf = mg->h_text[hb];
+  rc = run_ranks(mg, [&](int r) { return format_to_host(mg->ctx[r], nb[r], buf + pos[r], &ms[r]); });
+  if (rc) return rc;
+  out->text = buf;
+  out->n_bytes = nbytes;
+  out->ms_device = *std::max_element(ms.begin(), ms.end());
+  return RK_OK;
+}
+
+int rk_multi_group_statistics(rk_multi *mg, const rk_group_stats **stats, uint64_t *n_groups) {
+  if (!mg) return RK_ERR_ARG;
+  if ((int)mg->infos.size() != mg->n) {
+    mg->err = "rk_multi_group_statistics before a successful rk_multi_group";
+    return RK_ERR_STATE;
+  }
+  const u64 total = mg->infos[0].total_groups;
+  const u64 need = total * sizeof(rk_group_stats);
+  if (need > mg->h_stats_cap) {
+    if (mg->h_stats) cudaFreeHost(mg->h_stats);
+    mg->h_stats = nullptr, mg->h_stats_cap = 0;
+    if (cudaHostAlloc(&mg->h_stats, need + need / 8 + 4096, cudaHostAllocPortable) != cudaSuccess) {
+      cudaGetLastError();
+      mg->err = "cudaHostAlloc for the group statistics failed";
+      return RK_ERR_NOMEM;
+    }
+    mg->h_stats_cap = need + need / 8 + 4096;
+  }
+  rk_group_stats *h = (rk_group_stats *)mg->h_stats;
+  // every rank reduces its own groups (a group is never split) and copies them to their place in gid order
+  const int rc = run_ranks(mg, [&](int r) -> int {
+    rk_ctx *ctx = mg->ctx[r];
+    CK(cudaSetDevice(ctx->device));
+    ProfGuard pg(ctx);
+    const int rc2 = dist_group_stats(ctx, 0);
+    if (rc2) return rc2;
+    const Dist &D = *ctx->dist;
+    if ((u64)D.gid_base + D.n_groups_rank > total)
+      return fail(ctx, RK_ERR_INTERNAL, "groups %u .. %u of rank %d beyond the %llu groups", D.gid_base, D.gid_base + D.n_groups_rank, r,
+                  (unsigned long long)total);
+    if (D.n_groups_rank) {
+      CK(cudaMemcpyAsync(h + D.gid_base, ctx->d_stats, (u64)D.n_groups_rank * sizeof(rk_group_stats), cudaMemcpyDeviceToHost, ctx->stream));
+      CK(cudaStreamSynchronize(ctx->stream));
+    }
+    return RK_OK;
+  });
+  if (rc) return rc;
+  if (stats) *stats = total ? h : nullptr;
+  if (n_groups) *n_groups = total;
   return RK_OK;
 }
 

@@ -19,6 +19,7 @@ constexpr int OFF_YSTART = 16;
 constexpr int OFF_LENGTH = 40;
 constexpr int OFF_IDENT = 48;
 constexpr int OFF_STRAND = 92;
+constexpr int OFF_XEND = 24, OFF_YEND = 32, OFF_SCORE = 56, OFF_SIMILARITY = 64;  // printed only (K6)
 
 // constants of the reference
 constexpr u32 XBUCKET = 10;   // FragmentsDatabase.cpp:84,96 ; commonFunctions.cpp:152,154
@@ -244,9 +245,33 @@ struct OrderArgs {
   float *out_identity;
   u32 *err;
 };
+// What one output line prints of its record, in line order: a partitioned comparison brings it to the rank that holds the
+// line (RK_F_LINE_RECORDS), since the record itself sits on the rank that loaded it.  The integers stay 64-bit as in the file.
+struct __align__(16) LineRow {
+  u64 xs, ys, len, xe, ye, score, ident;
+  u32 sim_bits, strand;
+};
+static_assert(sizeof(LineRow) == 64, "line row size");
+__device__ __forceinline__ u64 ldg_u64_unaligned(const u8 *p) {  // records are 109 bytes apart: no alignment to rely on
+  u64 v = 0;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) v |= (u64)p[i] << (8 * i);
+  return v;
+}
+__device__ __forceinline__ LineRow line_row_of_record(const u8 *rec) {
+  LineRow f;
+  f.xs = ldg_u64_unaligned(rec + OFF_XSTART), f.ys = ldg_u64_unaligned(rec + OFF_YSTART);
+  f.xe = ldg_u64_unaligned(rec + OFF_XEND), f.ye = ldg_u64_unaligned(rec + OFF_YEND);
+  f.len = ldg_u64_unaligned(rec + OFF_LENGTH), f.score = ldg_u64_unaligned(rec + OFF_SCORE), f.ident = ldg_u64_unaligned(rec + OFF_IDENT);
+  f.sim_bits = (u32)rec[OFF_SIMILARITY] | ((u32)rec[OFF_SIMILARITY + 1] << 8) | ((u32)rec[OFF_SIMILARITY + 2] << 16) |
+               ((u32)rec[OFF_SIMILARITY + 3] << 24);
+  f.strand = rec[OFF_STRAND];
+  return f;
+}
 // K6: the text of output lines first_line .. first_line+n_lines (commonFunctions.cpp:101-115) from the loaded records and
 // the result arrays of the last grouping.
 struct FormatArgs {
+  const LineRow *rows;     // the line rows, indexed by line (partitioned comparisons) — or, indexed by order[line]:
   const u8 *aos;           // the loaded records, file order, 109 bytes each — or, after rk_load_packed (aos == nullptr):
   const uint4 *pk_key;     //   {xStart, yStart, length, ident}
   const uint4 *pk_rest;    //   {xEnd, yEnd, score, similarity bits}
@@ -319,6 +344,11 @@ int dist_chase_apply(const PeerTable &pt, const u32 *nroots, u32 stride, u32 bou
 int dist_chase_finish(const PeerTable &pt, const u32 *nroots, u32 stride, u32 m, const u64 *res, const u32 *lroot, const u32 *pend_idx,
                       const u32 *pend_key, const u32 *n_pend, u32 *gid_l, u32 *gid_rank, cudaStream_t st);
 int dist_or_rows(const u32 *all, u64 row_stride, int nr, u64 words, u32 *out, cudaStream_t st);
+// line records: every line asks the rank that loaded its record ({file index, line} to the owner of the file range,
+// cuts = the ranks' first file indices); the owner answers with the line row, stored at the asking rank's rows[line]
+int dist_line_ask_push(const u32 *order, u32 n, const u32 *file_cuts, int nr, uint4 *const *outs, u32 out_cap, u32 *tile_cnt,
+                       const u32 *counts_all, u32 row_stride, int me, cudaStream_t st);
+int dist_line_answer(const uint4 *requests, u32 n, const u8 *aos, u32 file_lo, const ScatterTable &back, cudaStream_t st);
 
 // sort_groups as a function of (groups, diag_func): h = |y - d| per member, member index, zero identity (sol.cu)
 int launch_member_keys(const u64 *y, const u64 *d, u32 m, u32 *h, u32 *idx, float *zero, u32 *err, cudaStream_t st);
@@ -328,8 +358,10 @@ struct rk_group_stats_dev {
   u32 count, x_lo, x_hi, y_lo, y_hi, first_line;
   double mean_identity, multiplicity;
 };
-int launch_group_stats(const u32 *out_order, const u32 *out_gid, const float *out_identity, const uint4 *rec4, u32 m, u32 n_groups,
-                       rk_group_stats_dev *st, cudaStream_t stream);
+// The span fields come from rec4[2 * order[j]] (one GPU) or from rows[j] (rows != nullptr: a rank of a partitioned
+// comparison, whose groups gid_base .. gid_base+n_groups-1 are all on the rank and whose line j is line line_off + j).
+int launch_group_stats(const u32 *out_order, const u32 *out_gid, const float *out_identity, const uint4 *rec4, const LineRow *rows,
+                       u32 m, u32 n_groups, u32 gid_base, u32 line_off, rk_group_stats_dev *st, cudaStream_t stream);
 
 u64 order_scratch_bytes(u64 m);
 void order_carve(OrderArgs &a, void *scratch, u64 m);  // sets packed .. worklist, work_cap

@@ -175,4 +175,15 @@ const char *err_bits_text(u32 e);
 float ev_ms(cudaEvent_t a, cudaEvent_t b);
 void dist_destroy(rk_ctx *c);  // multi.cu: releases c->dist (called by rk_destroy)
 
+// capi.cu: the work behind rk_format_lines / rk_group_statistics, shared with their partitioned forms (multi.cu).
+// K6 into the context's device text buffer (records ev[0]); *nbytes = the bytes formatted.  Synchronises.
+int format_on_device(rk_ctx *ctx, FormatArgs fa, u64 *nbytes);
+// the next of the context's two alternating pinned text buffers, grown to hold nbytes
+int format_text_buffer(rk_ctx *ctx, u64 nbytes, char **buf);
+// the formatted text to dst (pinned host memory); *ms_device = ev[0] .. the end of the copy.  Synchronises.
+int format_to_host(rk_ctx *ctx, u64 nbytes, char *dst, float *ms_device);
+// K8 into ctx->d_stats (and ctx->h_stats with RK_F_HOST_RESULT); see launch_group_stats.  Synchronises.
+int group_stats_run(rk_ctx *ctx, unsigned flags, const u32 *order, const u32 *gid, const float *identity, const uint4 *rec4,
+                    const LineRow *rows, u32 m, u64 ng, u32 gid_base, u32 line_off);
+
 }  // namespace rk
