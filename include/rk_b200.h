@@ -87,12 +87,33 @@ typedef struct {
 } rk_result;
 
 /* One context per GPU and per concurrent grouping (mirrors one FragmentsDatabase + the per-call
- * SequenceOcupationLists, src/repkiller.cpp:52, src/commonFunctions.cpp:45-48).  Returns NULL on failure;
- * rk_create_error() then has the reason. */
+ * SequenceOcupationLists, src/repkiller.cpp:52, src/commonFunctions.cpp:45-48); concurrent groupings of one loaded
+ * database share the load through views (rk_create_view).  Returns NULL on failure; rk_create_error() then has the
+ * reason. */
 rk_ctx *rk_create(int device);
 const char *rk_create_error(void);
+/* Releases the context's own stream, workspace and buffers.  Its database goes with the last context that uses it: a
+ * base destroyed while views of it are live leaves the load to them. */
 void rk_destroy(rk_ctx *ctx);
 const char *rk_last_error(const rk_ctx *ctx);
+
+/* A second grouping context over the database loaded into `base`: same device, its own stream, events, counters, grouping
+ * workspace and result/text/statistics buffers; the loaded records, processing order, bucket sorts and h are shared
+ * read-only.  rk_group / rk_sort_groups / rk_format_lines / rk_group_statistics / rk_diagonal_func / rk_debug_fetch /
+ * rk_set_stream / rk_profile_* work on it as on base, and give bit-identical results for the same ratio pair.  Calls on
+ * different contexts that share a database may run concurrently from different host threads (calls on ONE context are
+ * still serialised by the caller).  NULL on failure (rk_create_error).
+ *  - base must hold a successful single-GPU load (rk_load_aos / rk_load_packed); a view of a view shares the same
+ *    database.  Contexts of a partitioned comparison (rk_dist_init, rk_multi_ctx) are refused.
+ *  - rk_create_view only reads the load of base, so it may run while another thread groups on base; not while base
+ *    loads or is destroyed.
+ *  - The database is reference-counted: it is freed with the last of base and its views.
+ *  - rk_load_* on a view, rk_load_* on a context with live views (the message names how many; nothing changes) and
+ *    rk_dist_init on either return RK_ERR_STATE.
+ *  - The grouping workspace and the pinned result arrays of a view are allocated here, sized from the load; later calls
+ *    allocate only the grow-only text, statistics and diagonal-table buffers on first use.
+ *  - After rk_load_packed with rest4, every context's first grouping waits for the side copy of that array. */
+rk_ctx *rk_create_view(rk_ctx *base);
 
 /* Use `cuda_stream` (a cudaStream_t) for all work of this context instead of its own stream. */
 int rk_set_stream(rk_ctx *ctx, void *cuda_stream);

@@ -21,7 +21,7 @@ STAGES = ["h2d", "decode", "ranksort", "keys", "xsort", "ysort", "xmatch", "ymat
 NSTAGES = len(STAGES)
 
 # every symbol include/rk_b200.h declares
-SYMBOLS = ["rk_create", "rk_create_error", "rk_destroy", "rk_last_error", "rk_set_stream", "rk_load_aos", "rk_load_packed", "rk_group", "rk_sort_groups", "rk_host_alloc", "rk_host_free",
+SYMBOLS = ["rk_create", "rk_create_view", "rk_create_error", "rk_destroy", "rk_last_error", "rk_set_stream", "rk_load_aos", "rk_load_packed", "rk_group", "rk_sort_groups", "rk_host_alloc", "rk_host_free",
            "rk_diagonal_func", "rk_format_lines", "rk_debug_fetch", "rk_profile_enable", "rk_profile_read", "rk_sort_pairs_work_bytes", "rk_sort_pairs", "rk_version",
            "rk_gen_workload", "rk_sort_members", "rk_group_statistics", "rk_sol_create", "rk_sol_destroy", "rk_sol_insert", "rk_sol_get_associated", "rk_sol_last_error",
            # one comparison over several GPUs
@@ -80,6 +80,8 @@ def load_library():
     L = C.CDLL(LIB_PATH)
     L.rk_create.argtypes = [C.c_int]
     L.rk_create.restype = C.c_void_p
+    L.rk_create_view.argtypes = [C.c_void_p]
+    L.rk_create_view.restype = C.c_void_p
     L.rk_create_error.restype = C.c_char_p
     L.rk_destroy.argtypes = [C.c_void_p]
     L.rk_last_error.argtypes = [C.c_void_p]
@@ -176,6 +178,23 @@ class Context:
         if not self._h:
             raise RkError(-1, self._L.rk_create_error().decode())
         self.device = device
+
+    @classmethod
+    def _wrap(cls, handle: int, device: int) -> "Context":
+        c = cls.__new__(cls)
+        c._L, c._h, c.device = load_library(), handle, device
+        return c
+
+    def view(self) -> "Context":
+        """A second grouping context over this context's loaded database (rk_create_view): its own stream and workspace,
+        the load shared.  Different contexts may group concurrently from different threads; close() releases the view,
+        and the database lives until the last context that shares it is closed."""
+        h = self._L.rk_create_view(self._h)
+        if not h:
+            raise RkError(-1, self._L.rk_create_error().decode())
+        v = Context._wrap(h, self.device)
+        v._keep = getattr(self, "_keep", None)  # records the load reads in place stay alive while the view uses them
+        return v
 
     def close(self):
         if getattr(self, "_h", None):

@@ -32,16 +32,20 @@ thread_local Profiler *tl_prof = nullptr;
 
 namespace {
 
-// carve the workspace for n records; returns bytes needed.  With base == nullptr only sizes are computed.
-u64 carve(rk_ctx *c, u8 *base, u64 n, u64 stage_bytes, u64 lxw, u64 lyw) {
-  u64 off = 0;
-  auto take = [&](u64 bytes) -> u8 * {
+auto taker(u8 *base, u64 &off) {
+  return [base, &off](u64 bytes) -> u8 * {
     u8 *p = base ? base + off : nullptr;
     off += align_up(bytes ? bytes : 16, 256);
     return p;
   };
+}
+
+// The database part for n records (Database::arena): what the load writes and every grouping only reads.  Returns the
+// bytes needed; with base == nullptr only sizes are computed.
+u64 carve_load(rk_ctx *c, u8 *base, u64 n, u64 stage_bytes, u64 lxw, u64 lyw) {
+  u64 off = 0;
+  auto take = taker(base, off);
   const u64 n1 = n ? n : 1;
-  c->d_cnt = (Counters *)take(sizeof(Counters));
   c->d_aos = stage_bytes ? take(stage_bytes) : nullptr;  // host records staged on the device (109 B or 33 B each)
   c->rec4 = (uint4 *)take(n1 * 32);
   c->key0 = (u32 *)take(n1 * 4);
@@ -51,8 +55,6 @@ u64 carve(rk_ctx *c, u8 *base, u64 n, u64 stage_bytes, u64 lxw, u64 lyw) {
   c->link_y = (u32 *)take(lyw * 4);
   c->k0_r = (u32 *)take(n1 * 4);
   c->fidx_r = (u32 *)take(n1 * 4);
-  c->tmp_k = (u32 *)take(n1 * 4);
-  c->tmp_v = (u32 *)take(n1 * 4);
   c->xl_r = (uint2 *)take(n1 * 8);
   c->yl_r = (uint2 *)take(n1 * 8);
   c->ys_r = (u32 *)take(n1 * 4);
@@ -62,12 +64,24 @@ u64 carve(rk_ctx *c, u8 *base, u64 n, u64 stage_bytes, u64 lxw, u64 lyw) {
   c->rx = (u32 *)take(n1 * 4);
   c->sky = (u32 *)take(n1 * 4);
   c->ry = (u32 *)take(n1 * 4);
+  c->h = (u32 *)take(n1 * 4);
+  return off;
+}
+
+// The grouping workspace for n loaded records (rk_ctx::arena): everything rk_group and the calls after it write, plus
+// the sort scratch and counters the load borrows from the loading context.  Every context has its own.
+u64 carve_work(rk_ctx *c, u8 *base, u64 n) {
+  u64 off = 0;
+  auto take = taker(base, off);
+  const u64 n1 = n ? n : 1;
+  c->d_cnt = (Counters *)take(sizeof(Counters));
+  c->tmp_k = (u32 *)take(n1 * 4);
+  c->tmp_v = (u32 *)take(n1 * 4);
   c->sort_work = take(sort_work_bytes(n1));
   c->prehist = (u32 *)take(4 * 4 * 256 * 4);
   c->parent = (u32 *)take(n1 * 4);
   c->xm_bits = (u32 *)take((n1 + 31) / 32 * 4);
   c->gid_rank = (u32 *)take(n1 * 4);
-  c->h = (u32 *)take(n1 * 4);
   c->sgid = (u32 *)take(n1 * 4);
   c->srank = (u32 *)take(n1 * 4);
   c->forest_work = take(forest_work_bytes((u32)n1));
@@ -82,6 +96,43 @@ u64 carve(rk_ctx *c, u8 *base, u64 n, u64 stage_bytes, u64 lxw, u64 lyw) {
   c->out_repval = take(n1);
   c->out_identity = (float *)take(n1 * 4);
   return off;
+}
+
+// (re)allocates a grow-only device buffer of at least `need` bytes; the stream is drained before the old one is freed
+int grow_device(rk_ctx *ctx, void **buf, u64 *cap, u64 need) {
+  if (need <= *cap) return RK_OK;
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (*buf) cudaFree(*buf);
+  *buf = nullptr;
+  *cap = 0;
+  cudaError_t e = cudaMalloc(buf, need);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail(ctx, RK_ERR_NOMEM, "cudaMalloc(%llu bytes): %s", (unsigned long long)need, cudaGetErrorString(e));
+  }
+  *cap = need;
+  return RK_OK;
+}
+
+// the pinned host arrays of RK_F_HOST_RESULT for m kept records (grow-only)
+int grow_host_result(rk_ctx *ctx, u32 m) {
+  const u64 need = 3 * align_up((u64)m * 4, 256) + align_up((u64)m, 256);
+  if (need <= ctx->h_res_cap) return RK_OK;
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (ctx->h_res) cudaFreeHost(ctx->h_res);
+  ctx->h_res = nullptr;
+  ctx->h_res_cap = 0;
+  CK(cudaHostAlloc(&ctx->h_res, need, cudaHostAllocDefault));
+  ctx->h_res_cap = need;
+  return RK_OK;
+}
+
+void release_database(Database *db) {
+  if (!db || --db->refs > 0) return;
+  if (db->copy_stream) cudaStreamSynchronize(db->copy_stream), cudaStreamDestroy(db->copy_stream);
+  if (db->copy_done) cudaEventDestroy(db->copy_done);
+  if (db->arena) cudaFree(db->arena);
+  delete db;
 }
 
 }  // namespace
@@ -150,15 +201,8 @@ int finish_group(rk_ctx *ctx, unsigned flags, rk_result *out, u64 launches) {
   cudaStream_t st = ctx->stream;
   cudaEvent_t *ev = ctx->ev;
   if ((flags & RK_F_HOST_RESULT) && m) {
-    const u64 need = 3 * align_up((u64)m * 4, 256) + align_up((u64)m, 256);
-    if (need > ctx->h_res_cap) {
-      CK(cudaStreamSynchronize(st));
-      if (ctx->h_res) cudaFreeHost(ctx->h_res);
-      ctx->h_res = nullptr;
-      ctx->h_res_cap = 0;
-      CK(cudaHostAlloc(&ctx->h_res, need, cudaHostAllocDefault));
-      ctx->h_res_cap = need;
-    }
+    const int rc = grow_host_result(ctx, m);
+    if (rc) return rc;
   }
   CK(cudaEventRecord(ev[6], st));
   u8 *hb = (u8 *)ctx->h_res;
@@ -178,7 +222,7 @@ int finish_group(rk_ctx *ctx, unsigned flags, rk_result *out, u64 launches) {
   CK(cudaEventRecord(ev[7], st));
   CK(cudaMemcpyAsync(ctx->h_cnt, ctx->d_cnt, sizeof(Counters), cudaMemcpyDeviceToHost, st));
   if (ctx->copy_pending) {  // the formatter-only part of a compact load: done by the time a grouping is handed back
-    CK(cudaStreamWaitEvent(st, ctx->copy_done, 0));
+    CK(cudaStreamWaitEvent(st, ctx->db->copy_done, 0));
     ctx->copy_pending = false;
   }
   CK(cudaStreamSynchronize(st));
@@ -243,8 +287,9 @@ rk_ctx *rk_create(int device) {
   c->own_stream = true;
   if (const char *gr = getenv("RK_L2_GRAN")) cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)atoi(gr));  // tuning switch
   for (auto &ev : c->ev) cudaEventCreate(&ev);
-  cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking);
-  cudaEventCreateWithFlags(&c->copy_done, cudaEventDisableTiming);
+  c->db = new Database;
+  cudaStreamCreateWithFlags(&c->db->copy_stream, cudaStreamNonBlocking);
+  cudaEventCreateWithFlags(&c->db->copy_done, cudaEventDisableTiming);
   if (cudaMalloc((void **)&c->st_cnt, sizeof(Counters)) != cudaSuccess) c->st_cnt = nullptr;
   // function attributes are per device: every context sets them for its own device (a process-wide flag would leave
   // the second device of a process without the shared-memory opt-in)
@@ -271,11 +316,73 @@ void rk_destroy(rk_ctx *c) {
   for (char *t : c->h_text) if (t) cudaFreeHost(t);
   if (c->h_res) cudaFreeHost(c->h_res);
   if (c->h_cnt) cudaFreeHost(c->h_cnt);
+  if (c->d_diag) cudaFree(c->d_diag);
   for (auto &ev : c->ev) cudaEventDestroy(ev);
-  if (c->copy_stream) cudaStreamSynchronize(c->copy_stream), cudaStreamDestroy(c->copy_stream);
-  if (c->copy_done) cudaEventDestroy(c->copy_done);
+  release_database(c->db);  // the load itself stays while views of it are live
   if (c->own_stream) cudaStreamDestroy(c->stream);
   delete c;
+}
+
+rk_ctx *rk_create_view(rk_ctx *base) {
+  if (!base) {
+    set_create_error("rk_create_view: null context");
+    return nullptr;
+  }
+  if (base->dist) {
+    set_create_error("rk_create_view: the context is part of a comparison partitioned over several GPUs (rk_dist_init / rk_multi), "
+                     "which has no views");
+    return nullptr;
+  }
+  if (!base->loaded || !base->db) {
+    set_create_error("rk_create_view: the context holds no database (it needs a successful rk_load_aos or rk_load_packed)");
+    return nullptr;
+  }
+  cudaError_t e;
+  rk_ctx *c = new rk_ctx;
+  c->device = base->device;
+  if ((e = cudaSetDevice(c->device)) != cudaSuccess || (e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking)) != cudaSuccess ||
+      (e = cudaHostAlloc((void **)&c->h_cnt, sizeof(Counters), cudaHostAllocDefault)) != cudaSuccess) {
+    set_create_error(std::string("rk_create_view: ") + cudaGetErrorString(e));
+    cudaGetLastError();
+    if (c->stream) cudaStreamDestroy(c->stream);
+    delete c;
+    return nullptr;
+  }
+  c->own_stream = true;
+  for (auto &ev : c->ev) cudaEventCreate(&ev);
+  if (cudaMalloc((void **)&c->st_cnt, sizeof(Counters)) != cudaSuccess) c->st_cnt = nullptr;
+  ++base->db->refs;
+  c->db = base->db;
+  c->is_view = true;
+  // the load's pointers and sizes (the database never changes while a view is live: loading is refused then)
+  c->d_aos = base->d_aos, c->rec4 = base->rec4, c->key0 = base->key0, c->identity_r = base->identity_r, c->hfi_r = base->hfi_r;
+  c->link_x = base->link_x, c->link_y = base->link_y, c->link_x_words = base->link_x_words, c->link_y_words = base->link_y_words;
+  c->k0_r = base->k0_r, c->fidx_r = base->fidx_r, c->xl_r = base->xl_r, c->yl_r = base->yl_r, c->ys_r = base->ys_r;
+  c->kx = base->kx, c->ky = base->ky, c->skx = base->skx, c->rx = base->rx, c->sky = base->sky, c->ry = base->ry, c->h = base->h;
+  c->aos_dev = base->aos_dev, c->pk_key = base->pk_key, c->pk_rest = base->pk_rest, c->pk_strand = base->pk_strand;
+  c->n = base->n, c->m = base->m, c->g = base->g;
+  c->bits_rank = base->bits_rank, c->bits_x = base->bits_x, c->bits_y = base->bits_y;
+  c->copy_pending = c->db->side_copy;  // its first grouping waits for the side copy, like the base's
+  // all of the grouping workspace now: its size is known from the load, and no later call of a view allocates it
+  const u64 need = carve_work(c, nullptr, c->n);
+  if ((e = cudaMalloc(&c->arena, need)) != cudaSuccess) {
+    cudaGetLastError();
+    c->arena = nullptr;
+    set_create_error(std::string("rk_create_view: cudaMalloc of the grouping workspace: ") + cudaGetErrorString(e));
+    rk_destroy(c);
+    return nullptr;
+  }
+  c->arena_bytes = need;
+  carve_work(c, (u8 *)c->arena, c->n);
+  if (grow_host_result(c, c->m) != RK_OK || (e = cudaMemsetAsync(c->d_cnt, 0, sizeof(Counters), c->stream)) != cudaSuccess ||
+      (e = cudaStreamSynchronize(c->stream)) != cudaSuccess) {
+    set_create_error("rk_create_view: " + (c->err.empty() ? std::string(cudaGetErrorString(e)) : c->err));
+    cudaGetLastError();
+    rk_destroy(c);
+    return nullptr;
+  }
+  c->loaded = true;
+  return c;
 }
 
 const char *rk_last_error(const rk_ctx *c) { return c ? c->err.c_str() : rk_create_error(); }
@@ -313,10 +420,17 @@ int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_le
   if (n >= 0xFFFFFFF0ull) return fail(ctx, RK_ERR_ARG, "more than 2^32-16 records per context; partition the input");
   if (seqx_len >= (1ull << 32) || seqy_len >= (1ull << 32))
     return fail(ctx, RK_ERR_RANGE, "sequence length does not fit in 32 bits");
+  if (ctx->is_view) return fail(ctx, RK_ERR_STATE, "a view groups the database of the context it was made from; load that context instead");
+  if (!ctx->db) return fail(ctx, RK_ERR_STATE, "this context has no database");
+  if (const int views = ctx->db->refs - 1)
+    return fail(ctx, RK_ERR_STATE, "%d view%s of this context %s live: destroy %s before loading another database", views,
+                views == 1 ? "" : "s", views == 1 ? "is" : "are", views == 1 ? "it" : "them");
   CK(cudaSetDevice(ctx->device));
   ProfGuard pg(ctx);
   ctx->loaded = false;
   ctx->have_group = false;
+  Database *db = ctx->db;
+  db->side_copy = false;
 
   const void *first = src.packed() ? src.key4 : src.aos;
   const bool on_device = n ? is_device_pointer(first) : false;
@@ -328,23 +442,14 @@ int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_le
   const Geometry g = make_geometry(seqx_len, seqy_len);
   const u64 lxw = (2ull * g.nbx + 31) / 32 + 1, lyw = (2ull * g.nby + 31) / 32 + 1;
 
-  // (re)carve the workspace; the staging area holds the host records on the device: 109 B or 33 B per record
+  // (re)carve the database and the workspace; the staging area holds the host records on the device: 109 B or 33 B per record
   const u64 stage_bytes = on_device ? 0 : (src.packed() ? align_up(n * 16, 256) + align_up(n, 256) + (src.rest4 ? align_up(n * 16, 256) : 0)
                                                         : align_up(n * RK_FRAG_BYTES, 16) + 16);
-  const u64 need = carve(ctx, nullptr, n, stage_bytes, lxw, lyw);
-  if (need > ctx->arena_bytes) {
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (ctx->arena) cudaFree(ctx->arena);
-    ctx->arena = nullptr;
-    ctx->arena_bytes = 0;
-    cudaError_t e = cudaMalloc(&ctx->arena, need);
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      return fail(ctx, RK_ERR_NOMEM, "cudaMalloc(%llu bytes): %s", (unsigned long long)need, cudaGetErrorString(e));
-    }
-    ctx->arena_bytes = need;
-  }
-  carve(ctx, (u8 *)ctx->arena, n, stage_bytes, lxw, lyw);
+  int rc = grow_device(ctx, &db->arena, &db->arena_bytes, carve_load(ctx, nullptr, n, stage_bytes, lxw, lyw));
+  if (!rc) rc = grow_device(ctx, &ctx->arena, &ctx->arena_bytes, carve_work(ctx, nullptr, n));
+  if (rc) return rc;
+  carve_load(ctx, (u8 *)db->arena, n, stage_bytes, lxw, lyw);
+  carve_work(ctx, (u8 *)ctx->arena, n);
   ctx->link_x_words = lxw;
   ctx->link_y_words = lyw;
   ctx->n = n;
@@ -367,11 +472,12 @@ int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_le
       CK(cudaMemcpyAsync(p, src.strand, n, cudaMemcpyHostToDevice, st));
       strand = p, p += align_up(n, 256);
       if (src.rest4) {  // only rk_format_lines reads these: the copy runs on its own stream while the kernels work
-        CK(cudaStreamSynchronize(ctx->copy_stream));           // (an earlier load's copy into the old arena)
-        CK(cudaEventRecord(ctx->copy_done, st));               // not before the work queued on st is done with the arena
-        CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_done, 0));
-        CK(cudaMemcpyAsync(p, src.rest4, n * 16, cudaMemcpyHostToDevice, ctx->copy_stream));
-        CK(cudaEventRecord(ctx->copy_done, ctx->copy_stream));
+        CK(cudaStreamSynchronize(db->copy_stream));           // (an earlier load's copy into the old arena)
+        CK(cudaEventRecord(db->copy_done, st));               // not before the work queued on st is done with the arena
+        CK(cudaStreamWaitEvent(db->copy_stream, db->copy_done, 0));
+        CK(cudaMemcpyAsync(p, src.rest4, n * 16, cudaMemcpyHostToDevice, db->copy_stream));
+        CK(cudaEventRecord(db->copy_done, db->copy_stream));
+        db->side_copy = true;
         ctx->copy_pending = true;
         rest4 = (const uint4 *)p;
       }
@@ -579,12 +685,12 @@ int rk_diagonal_func(rk_ctx *ctx, uint64_t *diag_func) {
   CK(cudaSetDevice(ctx->device));
   const u32 nb = ctx->g.vsize - 1;
   if (nb == 0) return RK_OK;
-  u64 *d = nullptr;
-  CK(cudaMalloc(&d, (u64)nb * 8));
-  launch_diag_table(ctx->k0_r, ctx->ys_r, ctx->m, ctx->g.vsize, d, nullptr, ctx->stream);
-  cudaError_t e = cudaMemcpyAsync(diag_func, d, (u64)nb * 8, cudaMemcpyDeviceToHost, ctx->stream);
+  // a grow-only table of the context: a cudaFree per call would synchronise the device, i.e. every other context on it
+  const int rc = grow_device(ctx, (void **)&ctx->d_diag, &ctx->d_diag_bytes, (u64)nb * 8);
+  if (rc) return rc;
+  launch_diag_table(ctx->k0_r, ctx->ys_r, ctx->m, ctx->g.vsize, ctx->d_diag, nullptr, ctx->stream);
+  cudaError_t e = cudaMemcpyAsync(diag_func, ctx->d_diag, (u64)nb * 8, cudaMemcpyDeviceToHost, ctx->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-  cudaFree(d);
   if (e != cudaSuccess) return fail(ctx, RK_ERR_CUDA, "rk_diagonal_func: %s", cudaGetErrorString(e));
   return RK_OK;
 }

@@ -54,6 +54,23 @@ class FragmentsDatabase {
   void build_buckets() const;
 
  public:
+  // The grouping contexts of the facades (generate_fragment_groups, generate_diagonal_func, group_and_sort), so that they
+  // may run on several threads at once like the reference's: a call checks out ctx() when it is free, else an idle view
+  // of it (rk_create_view, made by commonFunctions.cpp when every pooled context is busy), and checks it back in.  Over
+  // several GPUs the calls take multi_mu instead, one comparison at a time.
+  struct ContextPool {
+    std::mutex mu;
+    bool base_busy = false;              // ctx() is checked out
+    std::vector<rk_ctx *> views;         // every view made for the pool; destroyed with the database
+    std::vector<rk_ctx *> idle_views;    // the ones not checked out
+    std::mutex multi_mu;
+  };
+  ContextPool &pool() const { return pool_; }
+
+ private:
+  mutable ContextPool pool_;
+
+ public:
   // Parses the GECKO CSV exactly like the reference (16 header lines, Frag rows, readFragment's accept/pad
   // rules), fills seq_manager, then hands the records to the GPU.  Throws std::runtime_error like the
   // reference on "Unexpected number of fragments"; also on device errors (message from rk_last_error).

@@ -56,21 +56,59 @@ void build_groups(const FragmentsDatabase &db, const rk_result &r, FGList &out) 
 [[noreturn]] void device_error(const FragmentsDatabase &db) {
   throw std::runtime_error(std::string("repkiller-b200: ") + (db.multi() ? rk_multi_last_error(db.multi()) : rk_last_error(db.ctx())));
 }
+[[noreturn]] void device_error(rk_ctx *ctx) { throw std::runtime_error(std::string("repkiller-b200: ") + rk_last_error(ctx)); }
+
+// One grouping context of the database's pool (FragmentsDatabase::ContextPool) for the duration of one facade call:
+// ctx() when it is free, so that one thread makes exactly the calls it always made; else an idle view, or a new one.
+class PooledContext {
+  const FragmentsDatabase &db_;
+  rk_ctx *ctx_ = nullptr;
+
+ public:
+  explicit PooledContext(const FragmentsDatabase &db) : db_(db) {
+    if (!db.ctx()) return;  // several GPUs: no single-GPU context (the calls below then report the error)
+    FragmentsDatabase::ContextPool &p = db.pool();
+    std::lock_guard<std::mutex> lk(p.mu);
+    if (!p.base_busy) {
+      p.base_busy = true;
+      ctx_ = db.ctx();
+    } else if (!p.idle_views.empty()) {
+      ctx_ = p.idle_views.back();
+      p.idle_views.pop_back();
+    } else {  // reads only the load of ctx(), which may be grouping on another thread meanwhile
+      ctx_ = rk_create_view(db.ctx());
+      if (!ctx_) throw std::runtime_error(std::string("repkiller-b200: ") + rk_create_error());
+      p.views.push_back(ctx_);
+    }
+  }
+  ~PooledContext() {
+    if (!ctx_) return;
+    FragmentsDatabase::ContextPool &p = db_.pool();
+    std::lock_guard<std::mutex> lk(p.mu);
+    if (ctx_ == db_.ctx()) p.base_busy = false;
+    else p.idle_views.push_back(ctx_);
+  }
+  PooledContext(const PooledContext &) = delete;
+  PooledContext &operator=(const PooledContext &) = delete;
+  rk_ctx *get() const { return ctx_; }
+};
 
 }  // namespace
 
 size_t generate_fragment_groups(const FragmentsDatabase &frags_db, FGList &efrags_groups, const sequence_manager &,
                                 double lensim, double possim) {
   rk_result r;
-  if (rk_group(frags_db.ctx(), lensim, possim, RK_F_HOST_RESULT | RK_F_NO_SORT, &r) != RK_OK) device_error(frags_db);
-  build_groups(frags_db, r, efrags_groups);
+  PooledContext pc(frags_db);
+  if (rk_group(pc.get(), lensim, possim, RK_F_HOST_RESULT | RK_F_NO_SORT, &r) != RK_OK) device_error(pc.get());
+  build_groups(frags_db, r, efrags_groups);  // (before the context goes back: r's host arrays are the context's)
   std::cout << std::flush;  // reference: commonFunctions.cpp:78
   return efrags_groups.size();
 }
 
 void generate_diagonal_func(const FragmentsDatabase &fdb, size_t *diag_func) {
   static_assert(sizeof(size_t) == sizeof(uint64_t), "64-bit host");
-  if (rk_diagonal_func(fdb.ctx(), reinterpret_cast<uint64_t *>(diag_func)) != RK_OK) device_error(fdb);
+  PooledContext pc(fdb);
+  if (rk_diagonal_func(pc.get(), reinterpret_cast<uint64_t *>(diag_func)) != RK_OK) device_error(pc.get());
 }
 
 namespace {
@@ -122,15 +160,23 @@ void sort_groups(FGList &fgl, const size_t *diag_func) {
 
 FGList *group_and_sort(const FragmentsDatabase &frags_db, double len_ratio, double pos_ratio, rk_result *stats) {
   rk_result r;
-  if (frags_db.multi()) {  // one comparison over several GPUs: the ranks' ranges of lines come back concatenated
-    if (rk_multi_group(frags_db.multi(), len_ratio, pos_ratio, RK_F_TIMING, &r) != RK_OK)
-      throw std::runtime_error(std::string("repkiller-b200: ") + rk_multi_last_error(frags_db.multi()));
-  } else if (rk_group(frags_db.ctx(), len_ratio, pos_ratio, RK_F_HOST_RESULT | RK_F_TIMING, &r) != RK_OK) {
-    device_error(frags_db);
-  }
   FGList *fgl = new FGList;
-  build_groups(frags_db, r, *fgl);
-  if (stats) *stats = r;
+  if (frags_db.multi()) {  // one comparison over several GPUs: the ranks' ranges of lines come back concatenated
+    std::lock_guard<std::mutex> lk(frags_db.pool().multi_mu);
+    if (rk_multi_group(frags_db.multi(), len_ratio, pos_ratio, RK_F_TIMING, &r) != RK_OK) {
+      delete fgl;
+      throw std::runtime_error(std::string("repkiller-b200: ") + rk_multi_last_error(frags_db.multi()));
+    }
+    build_groups(frags_db, r, *fgl);
+  } else {
+    PooledContext pc(frags_db);
+    if (rk_group(pc.get(), len_ratio, pos_ratio, RK_F_HOST_RESULT | RK_F_TIMING, &r) != RK_OK) {
+      delete fgl;
+      device_error(pc.get());
+    }
+    build_groups(frags_db, r, *fgl);
+  }
+  if (stats) *stats = r;  // (its host arrays are the context's, valid until its next grouping)
   return fgl;
 }
 

@@ -9,6 +9,11 @@
 //                                             the reference's call sequence (repkiller.cpp:83-96):
 //                                             generate_fragment_groups -> generate_diagonal_func -> sort_groups ->
 //                                             save_all_frag_pairs, each through its own facade (GPU)
+//   rk_hostcheck pool <in.csv> <out_prefix> <threads> <len_ratio> <pos_ratio> [<len_ratio> <pos_ratio>]...
+//                                             the body of the reference's execWithParams (the four calls of steps) for
+//                                             every pair, run by <threads> threads that share one FragmentsDatabase, as
+//                                             the reference's thread pool does (repkiller.cpp:60-72); pair k writes
+//                                             <out_prefix>-<k>.csv.  Prints how many grouping contexts the facades used (GPU)
 //   rk_hostcheck steps_pure <in.csv> <out.csv> <len_ratio> <pos_ratio> <len_ratio2> <pos_ratio2>
 //                                             sort_groups is a pure function: a second grouping with other ratios is
 //                                             made BEFORE the first list is sorted; the output is the first one's (GPU)
@@ -25,6 +30,7 @@
 //                                             read_frags_head, read_frags_records) on a CSV or a .frags file: records,
 //                                             header text; prints "<seqX len> <seqY len> <stated records> <binary>" (no GPU)
 // Every mode that builds a FragmentsDatabase takes a CSV or a .frags file (detect_frags_input).
+#include <atomic>
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -33,7 +39,9 @@
 #include <fstream>
 #include <iostream>
 #include <iterator>
+#include <mutex>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "../FragmentsDatabase.h"
@@ -202,6 +210,43 @@ int main(int argc, char **argv) {
     generate_diagonal_func(db, diag.data());
     sort_groups(groups, diag.data());
     save_all_frag_pairs(argv[3], sm, groups);
+    return 0;
+  }
+  if (mode == "pool" && argc >= 7) {
+    std::ifstream in(argv[2], std::ifstream::in | std::ifstream::binary);
+    sequence_manager sm;
+    FragmentsDatabase db(in, sm, 0, detect_frags_input(argv[2], in));
+    const std::string prefix = argv[3];
+    const int nthreads = std::max(1, atoi(argv[4]));
+    std::vector<std::pair<double, double>> pairs;
+    for (int i = 5; i + 1 < argc; i += 2) pairs.emplace_back(std::stod(argv[i]), std::stod(argv[i + 1]));
+    std::atomic<size_t> next{0};
+    std::mutex err_mu;
+    std::string err;
+    auto worker = [&] {
+      for (size_t k; (k = next++) < pairs.size();) {
+        try {
+          FGList groups;
+          generate_fragment_groups(db, groups, sm, pairs[k].first, pairs[k].second);
+          std::vector<size_t> diag(db.getA());
+          generate_diagonal_func(db, diag.data());
+          sort_groups(groups, diag.data());
+          save_all_frag_pairs(prefix + "-" + std::to_string(k) + ".csv", sm, groups);
+          for (FragsGroup *g : groups) delete g;
+        } catch (const std::exception &e) {
+          std::lock_guard<std::mutex> lk(err_mu);
+          err = e.what();
+        }
+      }
+    };
+    std::vector<std::thread> pool;
+    for (int t = 0; t < nthreads; ++t) pool.emplace_back(worker);
+    for (auto &th : pool) th.join();
+    if (!err.empty()) {
+      fprintf(stderr, "%s\n", err.c_str());
+      return 4;
+    }
+    printf("%zu pairs on %d threads, %zu grouping contexts\n", pairs.size(), nthreads, 1 + db.pool().views.size());
     return 0;
   }
   if (mode == "steps_pure" && argc >= 8) {

@@ -588,6 +588,11 @@ static int dist_init_common(rk_ctx *ctx, int rank, int world, Transport *tr, u64
     delete tr;
     return fail(ctx, RK_ERR_ARG, "rank %d of %d: at most %d ranks", rank, world, DIST_MAX_RANKS);
   }
+  if (ctx->is_view || (ctx->db && ctx->db->refs > 1)) {  // partitioned comparisons have no views (rk_create_view)
+    delete tr;
+    return fail(ctx, RK_ERR_STATE, "%s", ctx->is_view ? "a view cannot take part in a partitioned comparison"
+                                                      : "views of this context are live: destroy them before rk_dist_init");
+  }
   dist_destroy(ctx);
   Dist *D = new Dist;
   D->rank = rank, D->world = world, D->tr = tr;

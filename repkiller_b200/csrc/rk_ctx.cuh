@@ -2,6 +2,7 @@
 // several GPUs): device workspace, pinned result buffers, per-kernel event profiler, error plumbing.
 #pragma once
 
+#include <atomic>
 #include <cstdarg>
 #include <cstdio>
 #include <string>
@@ -59,21 +60,33 @@ struct Counters {  // small device block, mirrored in pinned host memory
 
 struct Dist;  // multi.cu: this context's part in a comparison partitioned over several GPUs
 
+// What a load writes and a grouping only reads: the records (staged, or the caller's device pointer), the processing
+// order, the bucket sorts of both axes and h (carve_load), plus the side copy of a compact load.  A context owns one; its
+// views (rk_create_view) share it, and the last of them to be destroyed frees it.  The context fields that point into it
+// (rec4 .. h, aos_dev, pk_*) and the load's sizes are copied into every view.
+struct Database {
+  std::atomic<int> refs{1};  // the contexts that read it: the one that loaded it and its views
+  void *arena = nullptr;
+  u64 arena_bytes = 0;
+  cudaStream_t copy_stream = nullptr;  // H2D of data only the output formatter reads (rk_load_packed's rest4), beside the kernels
+  cudaEvent_t copy_done = nullptr;
+  bool side_copy = false;  // the last load queued such a copy; copy_done marks its end
+};
+
 }  // namespace rk
 
 struct rk_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
   bool own_stream = false;
-  cudaStream_t copy_stream = nullptr;  // H2D of data only the output formatter reads (rk_load_packed's rest4), beside the kernels
-  cudaEvent_t copy_done = nullptr;
-  bool copy_pending = false;
+  bool copy_pending = false;  // the database's side copy (Database::copy_done) is not yet waited for on this context's stream
   std::string err;
 
-  // device workspace (one allocation, carved by carve())
+  // the loaded database (shared with the views) and this context's grouping workspace (one allocation, carve_work())
+  rk::Database *db = nullptr;
+  bool is_view = false;  // made by rk_create_view: groups on another context's load, never loads
   void *arena = nullptr;
   rk::u64 arena_bytes = 0;
-  rk::u64 cap_n = 0;  // records the workspace was carved for
 
   // pinned host result buffers
   void *h_res = nullptr;
@@ -103,6 +116,10 @@ struct rk_ctx {
   rk::u64 stats_cap = 0, h_stats_cap = 0;
   rk::u64 n_groups_last = 0;
 
+  // rk_diagonal_func's table (grow-only)
+  rk::u64 *d_diag = nullptr;
+  rk::u64 d_diag_bytes = 0;
+
   bool loaded = false;
   rk::u64 n = 0;
   rk::u32 m = 0;
@@ -112,7 +129,8 @@ struct rk_ctx {
 
   rk::Dist *dist = nullptr;  // set by rk_dist_init (multi.cu)
 
-  // carved pointers
+  // carved pointers.  Database (carve_load, written by the load only): d_aos .. h below, except the workspace ones marked W.
+  // Workspace (carve_work, written by a grouping; the load uses the loading context's scratch and counters too): W.
   rk::u8 *d_aos = nullptr;
   uint4 *rec4 = nullptr;  // file order, two words per record: {xStart, yStart, length, flags} {identity bits, file index, 0, 0}
   float *identity_r = nullptr;  // rank order
@@ -120,16 +138,18 @@ struct rk_ctx {
   rk::u32 *key0 = nullptr;
   rk::u32 *link_x = nullptr, *link_y = nullptr;
   rk::u64 link_x_words = 0, link_y_words = 0;
-  rk::Counters *d_cnt = nullptr;
+  rk::Counters *d_cnt = nullptr;  // W
   rk::u32 *k0_r = nullptr, *fidx_r = nullptr;
-  rk::u32 *tmp_k = nullptr, *tmp_v = nullptr;
+  rk::u32 *tmp_k = nullptr, *tmp_v = nullptr;  // W
   uint2 *xl_r = nullptr, *yl_r = nullptr;  // rank order {center, length} per axis
   rk::u32 *ys_r = nullptr, *kx = nullptr, *ky = nullptr;
   rk::u32 *skx = nullptr, *rx = nullptr, *sky = nullptr, *ry = nullptr;
+  rk::u32 *h = nullptr;
+  // W from here on
   void *sort_work = nullptr;
   rk::u32 *prehist = nullptr;  // 4 x [4][256]: digit counts of key0, kx, ky, gid gathered by the kernels that produce them
   rk::u32 *xm_bits = nullptr;
-  rk::u32 *parent = nullptr, *gid_rank = nullptr, *h = nullptr, *sgid = nullptr, *srank = nullptr;
+  rk::u32 *parent = nullptr, *gid_rank = nullptr, *sgid = nullptr, *srank = nullptr;
   void *forest_work = nullptr;
   void *order_scratch = nullptr;
   rk::u32 *worklist = nullptr;
