@@ -27,7 +27,9 @@ typedef enum {
                            src/FragmentsDatabase.cpp:96-97), a center outside the occupation lists
                            (src/SequenceOcupationList.cpp:16-18), or a coordinate >= 2^31 */
   RK_ERR_STATE = -4,    /* call order: rk_group before rk_load_aos, ... */
-  RK_ERR_NOMEM = -5,
+  RK_ERR_NOMEM = -5,    /* a device or pinned host allocation failed: the last-error text names the call and the byte
+                           count, and the CUDA error is cleared, so the object stays usable; or a rank of a partitioned
+                           comparison is asked for more records than its capacity */
   RK_ERR_INTERNAL = -6  /* an internal invariant failed (bounded spin expired, worklist overflow) */
 } rk_status;
 

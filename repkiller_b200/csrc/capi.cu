@@ -42,29 +42,29 @@ auto taker(u8 *base, u64 &off) {
 
 // The database part for n records (Database::arena): what the load writes and every grouping only reads.  Returns the
 // bytes needed; with base == nullptr only sizes are computed.
-u64 carve_load(rk_ctx *c, u8 *base, u64 n, u64 stage_bytes, u64 lxw, u64 lyw) {
+u64 carve_load(Database &db, u8 *base, u64 n, u64 stage_bytes, LinkWords lw) {
   u64 off = 0;
   auto take = taker(base, off);
   const u64 n1 = n ? n : 1;
-  c->d_aos = stage_bytes ? take(stage_bytes) : nullptr;  // host records staged on the device (109 B or 33 B each)
-  c->rec4 = (uint4 *)take(n1 * 32);
-  c->key0 = (u32 *)take(n1 * 4);
-  c->identity_r = (float *)take(n1 * 4);
-  c->hfi_r = (uint4 *)take(n1 * 16);
-  c->link_x = (u32 *)take(lxw * 4);
-  c->link_y = (u32 *)take(lyw * 4);
-  c->k0_r = (u32 *)take(n1 * 4);
-  c->fidx_r = (u32 *)take(n1 * 4);
-  c->xl_r = (uint2 *)take(n1 * 8);
-  c->yl_r = (uint2 *)take(n1 * 8);
-  c->ys_r = (u32 *)take(n1 * 4);
-  c->kx = (u32 *)take(n1 * 4);
-  c->ky = (u32 *)take(n1 * 4);
-  c->skx = (u32 *)take(n1 * 4);
-  c->rx = (u32 *)take(n1 * 4);
-  c->sky = (u32 *)take(n1 * 4);
-  c->ry = (u32 *)take(n1 * 4);
-  c->h = (u32 *)take(n1 * 4);
+  db.d_aos = stage_bytes ? take(stage_bytes) : nullptr;  // host records staged on the device (109 B or 33 B each)
+  db.rec4 = (uint4 *)take(n1 * 32);
+  db.key0 = (u32 *)take(n1 * 4);
+  db.identity_r = (float *)take(n1 * 4);
+  db.hfi_r = (uint4 *)take(n1 * 16);
+  db.link_x = (u32 *)take(lw.x * 4);
+  db.link_y = (u32 *)take(lw.y * 4);
+  db.k0_r = (u32 *)take(n1 * 4);
+  db.fidx_r = (u32 *)take(n1 * 4);
+  db.xl_r = (uint2 *)take(n1 * 8);
+  db.yl_r = (uint2 *)take(n1 * 8);
+  db.ys_r = (u32 *)take(n1 * 4);
+  db.kx = (u32 *)take(n1 * 4);
+  db.ky = (u32 *)take(n1 * 4);
+  db.skx = (u32 *)take(n1 * 4);
+  db.rx = (u32 *)take(n1 * 4);
+  db.sky = (u32 *)take(n1 * 4);
+  db.ry = (u32 *)take(n1 * 4);
+  db.h = (u32 *)take(n1 * 4);
   return off;
 }
 
@@ -96,43 +96,6 @@ u64 carve_work(rk_ctx *c, u8 *base, u64 n) {
   c->out_repval = take(n1);
   c->out_identity = (float *)take(n1 * 4);
   return off;
-}
-
-// (re)allocates a grow-only device buffer of at least `need` bytes; the stream is drained before the old one is freed
-int grow_device(rk_ctx *ctx, void **buf, u64 *cap, u64 need) {
-  if (need <= *cap) return RK_OK;
-  CK(cudaStreamSynchronize(ctx->stream));
-  if (*buf) cudaFree(*buf);
-  *buf = nullptr;
-  *cap = 0;
-  cudaError_t e = cudaMalloc(buf, need);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    return fail(ctx, RK_ERR_NOMEM, "cudaMalloc(%llu bytes): %s", (unsigned long long)need, cudaGetErrorString(e));
-  }
-  *cap = need;
-  return RK_OK;
-}
-
-// the pinned host arrays of RK_F_HOST_RESULT for m kept records (grow-only)
-int grow_host_result(rk_ctx *ctx, u32 m) {
-  const u64 need = 3 * align_up((u64)m * 4, 256) + align_up((u64)m, 256);
-  if (need <= ctx->h_res_cap) return RK_OK;
-  CK(cudaStreamSynchronize(ctx->stream));
-  if (ctx->h_res) cudaFreeHost(ctx->h_res);
-  ctx->h_res = nullptr;
-  ctx->h_res_cap = 0;
-  CK(cudaHostAlloc(&ctx->h_res, need, cudaHostAllocDefault));
-  ctx->h_res_cap = need;
-  return RK_OK;
-}
-
-void release_database(Database *db) {
-  if (!db || --db->refs > 0) return;
-  if (db->copy_stream) cudaStreamSynchronize(db->copy_stream), cudaStreamDestroy(db->copy_stream);
-  if (db->copy_done) cudaEventDestroy(db->copy_done);
-  if (db->arena) cudaFree(db->arena);
-  delete db;
 }
 
 }  // namespace
@@ -186,9 +149,9 @@ namespace {
 // K5b tail + K5c on the state the last rk_group left on the device
 u64 run_order(rk_ctx *ctx, unsigned flags) {
   OrderArgs oa{};
-  oa.sgid = ctx->sgid, oa.srank = ctx->srank, oa.hfi_r = ctx->hfi_r;
-  oa.m = ctx->m, oa.do_sort = (flags & RK_F_NO_SORT) ? 0 : 1;
-  order_carve(oa, ctx->order_scratch, ctx->n);
+  oa.sgid = ctx->sgid, oa.srank = ctx->srank, oa.hfi_r = ctx->db->hfi_r;
+  oa.m = ctx->db->m, oa.do_sort = (flags & RK_F_NO_SORT) ? 0 : 1;
+  order_carve(oa, ctx->order_scratch, ctx->db->n);
   oa.work_count = ctx->d_cnt->work_g;
   oa.out_order = ctx->out_order, oa.out_gid = ctx->out_gid, oa.out_repval = ctx->out_repval, oa.out_identity = ctx->out_identity;
   oa.err = &ctx->d_cnt->err;
@@ -197,27 +160,19 @@ u64 run_order(rk_ctx *ctx, unsigned flags) {
 
 // optional D2H of the four output arrays, final synchronisation, error word, result struct (events 0..5 recorded)
 int finish_group(rk_ctx *ctx, unsigned flags, rk_result *out, u64 launches) {
-  const u32 m = ctx->m;
+  const u32 m = ctx->db->m;
   cudaStream_t st = ctx->stream;
   cudaEvent_t *ev = ctx->ev;
-  if ((flags & RK_F_HOST_RESULT) && m) {
-    const int rc = grow_host_result(ctx, m);
+  const bool host = (flags & RK_F_HOST_RESULT) && m;
+  if (host) {
+    const int rc = ctx->h_res.reserve(HostResult::bytes(m), st, ctx->err);
     if (rc) return rc;
   }
   CK(cudaEventRecord(ev[6], st));
-  u8 *hb = (u8 *)ctx->h_res;
-  u32 *h_order = nullptr, *h_gid = nullptr;
-  float *h_ident = nullptr;
-  u8 *h_rep = nullptr;
-  if ((flags & RK_F_HOST_RESULT) && m) {
-    h_order = (u32 *)hb;
-    h_gid = (u32 *)(hb + align_up((u64)m * 4, 256));
-    h_ident = (float *)(hb + 2 * align_up((u64)m * 4, 256));
-    h_rep = hb + 3 * align_up((u64)m * 4, 256);
-    CK(cudaMemcpyAsync(h_order, ctx->out_order, (u64)m * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(h_gid, ctx->out_gid, (u64)m * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(h_ident, ctx->out_identity, (u64)m * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(h_rep, ctx->out_repval, (u64)m, cudaMemcpyDeviceToHost, st));
+  HostResult hr;
+  if (host) {
+    hr = HostResult(ctx->h_res.ptr(), m);
+    CK(hr.fetch(ctx->out_order, ctx->out_gid, ctx->out_identity, ctx->out_repval, m, st));
   }
   CK(cudaEventRecord(ev[7], st));
   CK(cudaMemcpyAsync(ctx->h_cnt, ctx->d_cnt, sizeof(Counters), cudaMemcpyDeviceToHost, st));
@@ -233,10 +188,7 @@ int finish_group(rk_ctx *ctx, unsigned flags, rk_result *out, u64 launches) {
 
   out->n_kept = m;
   out->n_groups = ctx->h_cnt->n_groups;
-  out->order = h_order;
-  out->gid = h_gid;
-  out->repval = h_rep;
-  out->identity = h_ident;
+  hr.publish(out);
   out->d_order = ctx->out_order;
   out->d_gid = ctx->out_gid;
   out->d_repval = ctx->out_repval;
@@ -307,20 +259,12 @@ void rk_destroy(rk_ctx *c) {
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->stream);
   dist_destroy(c);
-  if (c->arena) cudaFree(c->arena);
   if (c->st_cnt) cudaFree(c->st_cnt);
-  if (c->st_scratch) cudaFree(c->st_scratch);
-  if (c->d_text) cudaFree(c->d_text);
-  if (c->d_stats) cudaFree(c->d_stats);
-  if (c->h_stats) cudaFreeHost(c->h_stats);
-  for (char *t : c->h_text) if (t) cudaFreeHost(t);
-  if (c->h_res) cudaFreeHost(c->h_res);
   if (c->h_cnt) cudaFreeHost(c->h_cnt);
-  if (c->d_diag) cudaFree(c->d_diag);
   for (auto &ev : c->ev) cudaEventDestroy(ev);
-  release_database(c->db);  // the load itself stays while views of it are live
+  if (c->db && --c->db->refs == 0) delete c->db;  // the load itself stays while views of it are live
   if (c->own_stream) cudaStreamDestroy(c->stream);
-  delete c;
+  delete c;  // frees the grow-only buffers: the device is current and the stream drained
 }
 
 rk_ctx *rk_create_view(rk_ctx *base) {
@@ -354,28 +298,12 @@ rk_ctx *rk_create_view(rk_ctx *base) {
   ++base->db->refs;
   c->db = base->db;
   c->is_view = true;
-  // the load's pointers and sizes (the database never changes while a view is live: loading is refused then)
-  c->d_aos = base->d_aos, c->rec4 = base->rec4, c->key0 = base->key0, c->identity_r = base->identity_r, c->hfi_r = base->hfi_r;
-  c->link_x = base->link_x, c->link_y = base->link_y, c->link_x_words = base->link_x_words, c->link_y_words = base->link_y_words;
-  c->k0_r = base->k0_r, c->fidx_r = base->fidx_r, c->xl_r = base->xl_r, c->yl_r = base->yl_r, c->ys_r = base->ys_r;
-  c->kx = base->kx, c->ky = base->ky, c->skx = base->skx, c->rx = base->rx, c->sky = base->sky, c->ry = base->ry, c->h = base->h;
-  c->aos_dev = base->aos_dev, c->pk_key = base->pk_key, c->pk_rest = base->pk_rest, c->pk_strand = base->pk_strand;
-  c->n = base->n, c->m = base->m, c->g = base->g;
-  c->bits_rank = base->bits_rank, c->bits_x = base->bits_x, c->bits_y = base->bits_y;
   c->copy_pending = c->db->side_copy;  // its first grouping waits for the side copy, like the base's
   // all of the grouping workspace now: its size is known from the load, and no later call of a view allocates it
-  const u64 need = carve_work(c, nullptr, c->n);
-  if ((e = cudaMalloc(&c->arena, need)) != cudaSuccess) {
-    cudaGetLastError();
-    c->arena = nullptr;
-    set_create_error(std::string("rk_create_view: cudaMalloc of the grouping workspace: ") + cudaGetErrorString(e));
-    rk_destroy(c);
-    return nullptr;
-  }
-  c->arena_bytes = need;
-  carve_work(c, (u8 *)c->arena, c->n);
-  if (grow_host_result(c, c->m) != RK_OK || (e = cudaMemsetAsync(c->d_cnt, 0, sizeof(Counters), c->stream)) != cudaSuccess ||
-      (e = cudaStreamSynchronize(c->stream)) != cudaSuccess) {
+  const int rc = c->arena.reserve(carve_work(c, nullptr, c->db->n), nullptr, c->err);
+  if (rc == RK_OK) carve_work(c, (u8 *)c->arena.ptr(), c->db->n);
+  if (rc != RK_OK || c->h_res.reserve(HostResult::bytes(c->db->m), c->stream, c->err) != RK_OK ||
+      (e = cudaMemsetAsync(c->d_cnt, 0, sizeof(Counters), c->stream)) != cudaSuccess || (e = cudaStreamSynchronize(c->stream)) != cudaSuccess) {
     set_create_error("rk_create_view: " + (c->err.empty() ? std::string(cudaGetErrorString(e)) : c->err));
     cudaGetLastError();
     rk_destroy(c);
@@ -400,13 +328,6 @@ int rk_set_stream(rk_ctx *ctx, void *cuda_stream) {
 
 namespace {
 
-bool is_device_pointer(const void *p) {
-  cudaPointerAttributes pa;
-  if (cudaPointerGetAttributes(&pa, p) == cudaSuccess) return pa.type == cudaMemoryTypeDevice;
-  cudaGetLastError();
-  return false;
-}
-
 // The two ingest forms: 109-byte records (rk_load_aos) or the compact arrays of rk_load_packed.
 struct LoadSource {
   const void *aos = nullptr;
@@ -429,8 +350,8 @@ int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_le
   ProfGuard pg(ctx);
   ctx->loaded = false;
   ctx->have_group = false;
-  Database *db = ctx->db;
-  db->side_copy = false;
+  Database &db = *ctx->db;
+  db.side_copy = false;
 
   const void *first = src.packed() ? src.key4 : src.aos;
   const bool on_device = n ? is_device_pointer(first) : false;
@@ -440,23 +361,19 @@ int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_le
     return fail(ctx, RK_ERR_ARG, "the arrays of rk_load_packed must all be host or all be device memory");
 
   const Geometry g = make_geometry(seqx_len, seqy_len);
-  const u64 lxw = (2ull * g.nbx + 31) / 32 + 1, lyw = (2ull * g.nby + 31) / 32 + 1;
+  const LinkWords lw = link_map_words(g);
 
   // (re)carve the database and the workspace; the staging area holds the host records on the device: 109 B or 33 B per record
   const u64 stage_bytes = on_device ? 0 : (src.packed() ? align_up(n * 16, 256) + align_up(n, 256) + (src.rest4 ? align_up(n * 16, 256) : 0)
                                                         : align_up(n * RK_FRAG_BYTES, 16) + 16);
-  int rc = grow_device(ctx, &db->arena, &db->arena_bytes, carve_load(ctx, nullptr, n, stage_bytes, lxw, lyw));
-  if (!rc) rc = grow_device(ctx, &ctx->arena, &ctx->arena_bytes, carve_work(ctx, nullptr, n));
+  int rc = db.arena.reserve(carve_load(db, nullptr, n, stage_bytes, lw), ctx->stream, ctx->err);
+  if (!rc) rc = ctx->arena.reserve(carve_work(ctx, nullptr, n), ctx->stream, ctx->err);
   if (rc) return rc;
-  carve_load(ctx, (u8 *)db->arena, n, stage_bytes, lxw, lyw);
-  carve_work(ctx, (u8 *)ctx->arena, n);
-  ctx->link_x_words = lxw;
-  ctx->link_y_words = lyw;
-  ctx->n = n;
-  ctx->g = g;
-  ctx->bits_rank = ceil_log2(g.vsize) < 1 ? 1 : ceil_log2(g.vsize);  // (the sort clamps to >= 1 bit as well)
-  ctx->bits_x = ceil_log2(2ull * g.nbx);                             // >= 2: nbx >= 2
-  ctx->bits_y = ceil_log2(2ull * g.nby);
+  carve_load(db, (u8 *)db.arena.ptr(), n, stage_bytes, lw);
+  carve_work(ctx, (u8 *)ctx->arena.ptr(), n);
+  db.n = n;
+  db.g = g;
+  const SortBits bits = sort_key_bits(g);
 
   cudaStream_t st = ctx->stream;
   cudaEvent_t *ev = ctx->ev;
@@ -466,44 +383,44 @@ int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_le
   const u8 *strand = (const u8 *)src.strand;
   if (!on_device && n) {
     if (src.packed()) {
-      u8 *p = ctx->d_aos;
+      u8 *p = db.d_aos;
       CK(cudaMemcpyAsync(p, src.key4, n * 16, cudaMemcpyHostToDevice, st));
       key4 = (const uint4 *)p, p += align_up(n * 16, 256);
       CK(cudaMemcpyAsync(p, src.strand, n, cudaMemcpyHostToDevice, st));
       strand = p, p += align_up(n, 256);
       if (src.rest4) {  // only rk_format_lines reads these: the copy runs on its own stream while the kernels work
-        CK(cudaStreamSynchronize(db->copy_stream));           // (an earlier load's copy into the old arena)
-        CK(cudaEventRecord(db->copy_done, st));               // not before the work queued on st is done with the arena
-        CK(cudaStreamWaitEvent(db->copy_stream, db->copy_done, 0));
-        CK(cudaMemcpyAsync(p, src.rest4, n * 16, cudaMemcpyHostToDevice, db->copy_stream));
-        CK(cudaEventRecord(db->copy_done, db->copy_stream));
-        db->side_copy = true;
+        CK(cudaStreamSynchronize(db.copy_stream));           // (an earlier load's copy into the old arena)
+        CK(cudaEventRecord(db.copy_done, st));               // not before the work queued on st is done with the arena
+        CK(cudaStreamWaitEvent(db.copy_stream, db.copy_done, 0));
+        CK(cudaMemcpyAsync(p, src.rest4, n * 16, cudaMemcpyHostToDevice, db.copy_stream));
+        CK(cudaEventRecord(db.copy_done, db.copy_stream));
+        db.side_copy = true;
         ctx->copy_pending = true;
         rest4 = (const uint4 *)p;
       }
     } else {
-      CK(cudaMemcpyAsync(ctx->d_aos, src.aos, n * RK_FRAG_BYTES, cudaMemcpyHostToDevice, st));
-      aos = ctx->d_aos;
+      CK(cudaMemcpyAsync(db.d_aos, src.aos, n * RK_FRAG_BYTES, cudaMemcpyHostToDevice, st));
+      aos = db.d_aos;
     }
   }
-  ctx->aos_dev = aos;
-  ctx->pk_key = key4, ctx->pk_rest = rest4, ctx->pk_strand = strand;
+  db.aos_dev = aos;
+  db.pk_key = key4, db.pk_rest = rest4, db.pk_strand = strand;
   CK(cudaEventRecord(ev[1], st));
   CK(cudaMemsetAsync(ctx->d_cnt, 0, sizeof(Counters), st));
-  CK(cudaMemsetAsync(ctx->link_x, 0, lxw * 4, st));
-  CK(cudaMemsetAsync(ctx->link_y, 0, lyw * 4, st));
+  CK(cudaMemsetAsync(db.link_x, 0, lw.x * 4, st));
+  CK(cudaMemsetAsync(db.link_y, 0, lw.y * 4, st));
   u64 launches = 0;
   CK(cudaMemsetAsync(ctx->prehist, 0, 3 * 4 * 256 * 4, st));
   auto hist_of = [&](int which, int bits) { return HistOut{ctx->prehist + which * 1024, (bits + 7) / 8, bits}; };
   if (src.packed())
-    launches += launch_decode_packed(key4, strand, n, g, ctx->key0, ctx->link_x, ctx->link_y, &ctx->d_cnt->n_dropped, &ctx->d_cnt->err, st,
-                                     ctx->rec4, hist_of(0, ctx->bits_rank));
+    launches += launch_decode_packed(key4, strand, n, g, db.key0, db.link_x, db.link_y, &ctx->d_cnt->n_dropped, &ctx->d_cnt->err, st,
+                                     db.rec4, hist_of(0, bits.rank));
   else
-    launches += launch_decode(aos, n, g, nullptr, nullptr, nullptr, nullptr, nullptr, ctx->key0, ctx->link_x, ctx->link_y,
-                              &ctx->d_cnt->n_dropped, &ctx->d_cnt->err, st, ctx->rec4, hist_of(0, ctx->bits_rank));
+    launches += launch_decode(aos, n, g, nullptr, nullptr, nullptr, nullptr, nullptr, db.key0, db.link_x, db.link_y,
+                              &ctx->d_cnt->n_dropped, &ctx->d_cnt->err, st, db.rec4, hist_of(0, bits.rank));
   CK(cudaEventRecord(ev[2], st));
   // the rank sort does not depend on the number of dropped records: they carry the largest key and sort last
-  launches += launch_sort_pairs(ctx->key0, nullptr, ctx->k0_r, ctx->fidx_r, ctx->tmp_k, ctx->tmp_v, n, ctx->bits_rank, ctx->sort_work, st, &ctx->d_cnt->err,
+  launches += launch_sort_pairs(db.key0, nullptr, db.k0_r, db.fidx_r, ctx->tmp_k, ctx->tmp_v, n, bits.rank, ctx->sort_work, st, &ctx->d_cnt->err,
                                 ctx->prehist);
   CK(cudaEventRecord(ev[3], st));
   CK(cudaMemcpyAsync(ctx->h_cnt, ctx->d_cnt, sizeof(Counters), cudaMemcpyDeviceToHost, st));
@@ -512,18 +429,18 @@ int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_le
   if (ctx->h_cnt->err) return fail(ctx, (ctx->h_cnt->err & (ERR_WORKLIST | ERR_SPIN)) ? RK_ERR_INTERNAL : RK_ERR_RANGE, "%s",
                                    err_bits_text(ctx->h_cnt->err));
   const u32 m = (u32)(n - ctx->h_cnt->n_dropped);
-  ctx->m = m;
+  db.m = m;
 
   CK(cudaEventRecord(ev[4], st));
-  launches += launch_keys(ctx->fidx_r, m, g, ctx->rec4, ctx->link_x, ctx->link_y, ctx->xl_r, ctx->yl_r, ctx->ys_r, ctx->kx, ctx->ky,
-                          ctx->identity_r, st, hist_of(1, ctx->bits_x), hist_of(2, ctx->bits_y));
+  launches += launch_keys(db.fidx_r, m, g, db.rec4, db.link_x, db.link_y, db.xl_r, db.yl_r, db.ys_r, db.kx, db.ky,
+                          db.identity_r, st, hist_of(1, bits.x), hist_of(2, bits.y));
   // generate_diagonal_func does not depend on the ratios: h and the per-rank output record are load-time work
-  launches += launch_hkey(ctx->k0_r, ctx->ys_r, m, ctx->h, st, ctx->fidx_r, ctx->identity_r, ctx->hfi_r);
+  launches += launch_hkey(db.k0_r, db.ys_r, m, db.h, st, db.fidx_r, db.identity_r, db.hfi_r);
   CK(cudaEventRecord(ev[5], st));
-  launches += launch_sort_pairs(ctx->kx, nullptr, ctx->skx, ctx->rx, ctx->tmp_k, ctx->tmp_v, m, ctx->bits_x, ctx->sort_work, st, &ctx->d_cnt->err,
+  launches += launch_sort_pairs(db.kx, nullptr, db.skx, db.rx, ctx->tmp_k, ctx->tmp_v, m, bits.x, ctx->sort_work, st, &ctx->d_cnt->err,
                                 ctx->prehist + 1024);
   CK(cudaEventRecord(ev[6], st));
-  launches += launch_sort_pairs(ctx->ky, nullptr, ctx->sky, ctx->ry, ctx->tmp_k, ctx->tmp_v, m, ctx->bits_y, ctx->sort_work, st, &ctx->d_cnt->err,
+  launches += launch_sort_pairs(db.ky, nullptr, db.sky, db.ry, ctx->tmp_k, ctx->tmp_v, m, bits.y, ctx->sort_work, st, &ctx->d_cnt->err,
                                 ctx->prehist + 2048);
   CK(cudaEventRecord(ev[7], st));
   CK(cudaStreamSynchronize(st));
@@ -579,21 +496,22 @@ int rk_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flags, rk
   CK(cudaSetDevice(ctx->device));
   ProfGuard pg(ctx);
   memset(out, 0, sizeof *out);
-  const u32 m = ctx->m;
+  const Database &db = *ctx->db;
+  const u32 m = db.m;
   cudaStream_t st = ctx->stream;
   cudaEvent_t *ev = ctx->ev;
   u64 launches = 0;
 
   CK(cudaEventRecord(ev[0], st));
   MatchArgs mx{};
-  mx.skey = ctx->skx, mx.srank = ctx->rx, mx.cl_r = ctx->xl_r, mx.parent = ctx->parent, mx.xm_bits = ctx->xm_bits;
-  mx.m = m, mx.max_index = ctx->g.mx, mx.len_ratio = len_ratio, mx.pos_ratio = pos_ratio, mx.is_y = 0;
+  mx.skey = db.skx, mx.srank = db.rx, mx.cl_r = db.xl_r, mx.parent = ctx->parent, mx.xm_bits = ctx->xm_bits;
+  mx.m = m, mx.max_index = db.g.mx, mx.len_ratio = len_ratio, mx.pos_ratio = pos_ratio, mx.is_y = 0;
   mx.worklist = ctx->worklist, mx.work_count = ctx->d_cnt->work_x, mx.work_cap = ctx->work_cap;
   mx.ent_rank = ctx->ent_rank, mx.ent_c = ctx->ent_c, mx.ent_len = ctx->ent_len, mx.err = &ctx->d_cnt->err;
   launches += launch_match(mx, st);
   CK(cudaEventRecord(ev[1], st));
   MatchArgs my = mx;
-  my.skey = ctx->sky, my.srank = ctx->ry, my.cl_r = ctx->yl_r, my.max_index = ctx->g.my, my.is_y = 1;
+  my.skey = db.sky, my.srank = db.ry, my.cl_r = db.yl_r, my.max_index = db.g.my, my.is_y = 1;
   my.work_count = ctx->d_cnt->work_y;
   launches += launch_match(my, st);
   CK(cudaEventRecord(ev[2], st));
@@ -632,29 +550,14 @@ int group_stats_run(rk_ctx *ctx, unsigned flags, const u32 *order, const u32 *gi
                     const LineRow *rows, u32 m, u64 ng, u32 gid_base, u32 line_off) {
   CK(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  if (ng > ctx->stats_cap) {
-    CK(cudaStreamSynchronize(st));
-    if (ctx->d_stats) cudaFree(ctx->d_stats);
-    ctx->d_stats = nullptr, ctx->stats_cap = 0;
-    const u64 cap = ng + ng / 8 + 1024;
-    cudaError_t e = cudaMalloc(&ctx->d_stats, cap * sizeof(rk_group_stats));
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      return fail(ctx, RK_ERR_NOMEM, "cudaMalloc(%llu bytes): %s", (unsigned long long)(cap * sizeof(rk_group_stats)), cudaGetErrorString(e));
-    }
-    ctx->stats_cap = cap;
-  }
-  launch_group_stats(order, gid, identity, rec4, rows, m, (u32)ng, gid_base, line_off, (rk_group_stats_dev *)ctx->d_stats, st);
+  const u64 need = ng * sizeof(rk_group_stats), grown = (ng + ng / 8 + 1024) * sizeof(rk_group_stats);
+  int rc = ctx->d_stats.reserve(need > ctx->d_stats.cap() ? grown : need, st, ctx->err);
+  if (rc) return rc;
+  launch_group_stats(order, gid, identity, rec4, rows, m, (u32)ng, gid_base, line_off, (rk_group_stats_dev *)ctx->d_stats.ptr(), st);
   if ((flags & RK_F_HOST_RESULT) && ng) {
-    if (ng > ctx->h_stats_cap) {
-      CK(cudaStreamSynchronize(st));
-      if (ctx->h_stats) cudaFreeHost(ctx->h_stats);
-      ctx->h_stats = nullptr, ctx->h_stats_cap = 0;
-      const u64 cap = ng + ng / 8 + 1024;
-      CK(cudaHostAlloc(&ctx->h_stats, cap * sizeof(rk_group_stats), cudaHostAllocDefault));
-      ctx->h_stats_cap = cap;
-    }
-    CK(cudaMemcpyAsync(ctx->h_stats, ctx->d_stats, ng * sizeof(rk_group_stats), cudaMemcpyDeviceToHost, st));
+    rc = ctx->h_stats.reserve(need > ctx->h_stats.cap() ? grown : need, st, ctx->err);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(ctx->h_stats.ptr(), ctx->d_stats.ptr(), need, cudaMemcpyDeviceToHost, st));
   }
   CK(cudaStreamSynchronize(st));
   CK(cudaGetLastError());
@@ -671,10 +574,10 @@ int rk_group_statistics(rk_ctx *ctx, unsigned flags, const rk_group_stats **stat
   CK(cudaSetDevice(ctx->device));
   ProfGuard pg(ctx);
   const u64 ng = ctx->n_groups_last;
-  const int rc = group_stats_run(ctx, flags, ctx->out_order, ctx->out_gid, ctx->out_identity, ctx->rec4, nullptr, ctx->m, ng, 0, 0);
+  const int rc = group_stats_run(ctx, flags, ctx->out_order, ctx->out_gid, ctx->out_identity, ctx->db->rec4, nullptr, ctx->db->m, ng, 0, 0);
   if (rc) return rc;
-  if (stats) *stats = ((flags & RK_F_HOST_RESULT) && ng) ? (const rk_group_stats *)ctx->h_stats : nullptr;
-  if (d_stats) *d_stats = (const rk_group_stats *)ctx->d_stats;
+  if (stats) *stats = ((flags & RK_F_HOST_RESULT) && ng) ? (const rk_group_stats *)ctx->h_stats.ptr() : nullptr;
+  if (d_stats) *d_stats = (const rk_group_stats *)ctx->d_stats.ptr();
   if (n_groups) *n_groups = ng;
   return RK_OK;
 }
@@ -683,13 +586,15 @@ int rk_diagonal_func(rk_ctx *ctx, uint64_t *diag_func) {
   if (!ctx || !diag_func) return RK_ERR_ARG;
   if (!ctx->loaded) return fail(ctx, RK_ERR_STATE, "rk_diagonal_func before rk_load_aos");
   CK(cudaSetDevice(ctx->device));
-  const u32 nb = ctx->g.vsize - 1;
+  const Database &db = *ctx->db;
+  const u32 nb = db.g.vsize - 1;
   if (nb == 0) return RK_OK;
   // a grow-only table of the context: a cudaFree per call would synchronise the device, i.e. every other context on it
-  const int rc = grow_device(ctx, (void **)&ctx->d_diag, &ctx->d_diag_bytes, (u64)nb * 8);
+  const int rc = ctx->d_diag.reserve((u64)nb * 8, ctx->stream, ctx->err);
   if (rc) return rc;
-  launch_diag_table(ctx->k0_r, ctx->ys_r, ctx->m, ctx->g.vsize, ctx->d_diag, nullptr, ctx->stream);
-  cudaError_t e = cudaMemcpyAsync(diag_func, ctx->d_diag, (u64)nb * 8, cudaMemcpyDeviceToHost, ctx->stream);
+  u64 *d_diag = (u64 *)ctx->d_diag.ptr();
+  launch_diag_table(db.k0_r, db.ys_r, db.m, db.g.vsize, d_diag, nullptr, ctx->stream);
+  cudaError_t e = cudaMemcpyAsync(diag_func, d_diag, (u64)nb * 8, cudaMemcpyDeviceToHost, ctx->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
   if (e != cudaSuccess) return fail(ctx, RK_ERR_CUDA, "rk_diagonal_func: %s", cudaGetErrorString(e));
   return RK_OK;
@@ -705,19 +610,10 @@ int format_on_device(rk_ctx *ctx, FormatArgs fa, u64 *nbytes) {
   const u64 n_lines = fa.n_lines;
   const u64 text_cap = align_up(n_lines * RK_FORMAT_MAX_LINE + 16, 256);
   const u64 need = text_cap + format_work_bytes((u32)n_lines);
-  if (need > ctx->d_text_bytes) {
-    CK(cudaStreamSynchronize(st));
-    if (ctx->d_text) cudaFree(ctx->d_text);
-    ctx->d_text = nullptr, ctx->d_text_bytes = 0;
-    cudaError_t e = cudaMalloc(&ctx->d_text, need);
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      return fail(ctx, RK_ERR_NOMEM, "cudaMalloc(%llu bytes): %s", (unsigned long long)need, cudaGetErrorString(e));
-    }
-    ctx->d_text_bytes = need;
-  }
-  fa.text = (char *)ctx->d_text;
-  u32 *work = (u32 *)((u8 *)ctx->d_text + text_cap);
+  const int rc = ctx->d_text.reserve(need, st, ctx->err);
+  if (rc) return rc;
+  fa.text = (char *)ctx->d_text.ptr();
+  u32 *work = (u32 *)(fa.text + text_cap);
   fa.total_bytes = work;  // first word of the work area; launch_format carves the rest after it
   CK(cudaEventRecord(ctx->ev[0], st));
   launch_format(fa, work + 8, st);
@@ -729,23 +625,17 @@ int format_on_device(rk_ctx *ctx, FormatArgs fa, u64 *nbytes) {
 }
 
 int format_text_buffer(rk_ctx *ctx, u64 nbytes, char **buf) {
-  const int hb = ctx->h_text_next;
+  GrowBuffer &b = ctx->h_text[ctx->h_text_next];
   ctx->h_text_next ^= 1;
-  if (nbytes + 1 > ctx->h_text_bytes[hb]) {
-    if (ctx->h_text[hb]) cudaFreeHost(ctx->h_text[hb]);
-    ctx->h_text[hb] = nullptr, ctx->h_text_bytes[hb] = 0;
-    const u64 cap = align_up(nbytes + nbytes / 8 + 4096, 4096);
-    CK(cudaHostAlloc((void **)&ctx->h_text[hb], cap, cudaHostAllocDefault));
-    ctx->h_text_bytes[hb] = cap;
-  }
-  *buf = ctx->h_text[hb];
-  return RK_OK;
+  const int rc = b.reserve(nbytes + 1 > b.cap() ? align_up(nbytes + nbytes / 8 + 4096, 4096) : nbytes + 1, nullptr, ctx->err);
+  *buf = (char *)b.ptr();
+  return rc;
 }
 
 int format_to_host(rk_ctx *ctx, u64 nbytes, char *dst, float *ms_device) {
   CK(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  if (nbytes) CK(cudaMemcpyAsync(dst, ctx->d_text, nbytes, cudaMemcpyDeviceToHost, st));
+  if (nbytes) CK(cudaMemcpyAsync(dst, ctx->d_text.ptr(), nbytes, cudaMemcpyDeviceToHost, st));
   CK(cudaEventRecord(ctx->ev[1], st));
   CK(cudaStreamSynchronize(st));
   *ms_device = ev_ms(ctx->ev[0], ctx->ev[1]);
@@ -758,15 +648,16 @@ extern "C" {
 int rk_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_text *out) {
   if (!ctx || !out) return RK_ERR_ARG;
   if (!ctx->loaded || !ctx->have_group) return fail(ctx, RK_ERR_STATE, "rk_format_lines before rk_group");
-  if (!ctx->aos_dev && !ctx->pk_rest)
+  const Database &db = *ctx->db;
+  if (!db.aos_dev && !db.pk_rest)
     return fail(ctx, RK_ERR_STATE, "the database was loaded with rk_load_packed without the xEnd/yEnd/score/similarity array");
-  if (first_line > ctx->m || n_lines > ctx->m - first_line) return fail(ctx, RK_ERR_ARG, "line range beyond the %u output lines", ctx->m);
+  if (first_line > db.m || n_lines > db.m - first_line) return fail(ctx, RK_ERR_ARG, "line range beyond the %u output lines", db.m);
   if (n_lines > RK_FORMAT_MAX_LINES) return fail(ctx, RK_ERR_ARG, "at most %llu lines per call", (unsigned long long)RK_FORMAT_MAX_LINES);
   CK(cudaSetDevice(ctx->device));
   ProfGuard pg(ctx);
   memset(out, 0, sizeof *out);
   FormatArgs fa{};
-  fa.aos = ctx->aos_dev, fa.pk_key = ctx->pk_key, fa.pk_rest = ctx->pk_rest, fa.pk_strand = ctx->pk_strand;
+  fa.aos = db.aos_dev, fa.pk_key = db.pk_key, fa.pk_rest = db.pk_rest, fa.pk_strand = db.pk_strand;
   fa.order = ctx->out_order, fa.gid = ctx->out_gid, fa.repval = ctx->out_repval, fa.identity = ctx->out_identity;
   fa.first_line = (u32)first_line, fa.n_lines = (u32)n_lines;
   u64 nbytes = 0;
@@ -783,17 +674,18 @@ int rk_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_text 
 int64_t rk_debug_fetch(rk_ctx *ctx, const char *name, void *host, uint64_t bytes) {
   if (!ctx || !name) return RK_ERR_ARG;
   if (!ctx->loaded) return fail(ctx, RK_ERR_STATE, "nothing loaded");
+  const Database &db = *ctx->db;
   const void *src = nullptr;
-  u64 sz = (u64)ctx->m * 4;
-  if (!strcmp(name, "rank_fidx")) src = ctx->fidx_r;
-  else if (!strcmp(name, "k0_r")) src = ctx->k0_r;
-  else if (!strcmp(name, "skx")) src = ctx->skx;
-  else if (!strcmp(name, "rx")) src = ctx->rx;
-  else if (!strcmp(name, "sky")) src = ctx->sky;
-  else if (!strcmp(name, "ry")) src = ctx->ry;
+  u64 sz = (u64)db.m * 4;
+  if (!strcmp(name, "rank_fidx")) src = db.fidx_r;
+  else if (!strcmp(name, "k0_r")) src = db.k0_r;
+  else if (!strcmp(name, "skx")) src = db.skx;
+  else if (!strcmp(name, "rx")) src = db.rx;
+  else if (!strcmp(name, "sky")) src = db.sky;
+  else if (!strcmp(name, "ry")) src = db.ry;
   else if (!strcmp(name, "parent")) src = ctx->parent;
   else if (!strcmp(name, "gid_rank")) src = ctx->gid_rank;
-  else if (!strcmp(name, "hkey")) src = ctx->h;
+  else if (!strcmp(name, "hkey")) src = db.h;
   else return fail(ctx, RK_ERR_ARG, "unknown array %s", name);
   if ((!strcmp(name, "parent") || !strcmp(name, "gid_rank")) && !ctx->have_group)
     return fail(ctx, RK_ERR_STATE, "no rk_group result yet");
@@ -853,24 +745,7 @@ int rk_sort_pairs(rk_ctx *ctx, const uint32_t *keys_in, const uint32_t *values_i
   return RK_OK;
 }
 
-// ---- scratch and error word of the calls that work on caller data (rk_sort_members) --------------------------
-
-static int st_scratch(rk_ctx *ctx, u64 bytes, void **out) {
-  if (bytes > ctx->st_scratch_bytes) {
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (ctx->st_scratch) cudaFree(ctx->st_scratch);
-    ctx->st_scratch = nullptr;
-    ctx->st_scratch_bytes = 0;
-    cudaError_t e = cudaMalloc(&ctx->st_scratch, bytes);
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      return fail(ctx, RK_ERR_NOMEM, "cudaMalloc(%llu bytes): %s", (unsigned long long)bytes, cudaGetErrorString(e));
-    }
-    ctx->st_scratch_bytes = bytes;
-  }
-  *out = ctx->st_scratch;
-  return RK_OK;
-}
+// ---- error word of the calls that work on caller data (rk_sort_members) ----------------------------------------
 
 static int st_check_errors(rk_ctx *ctx, bool range_errors) {
   CK(cudaMemcpyAsync(ctx->h_cnt, ctx->st_cnt, sizeof(Counters), cudaMemcpyDeviceToHost, ctx->stream));
@@ -895,10 +770,9 @@ int rk_sort_members(rk_ctx *ctx, uint64_t m, const uint32_t *gid, const uint64_t
   ProfGuard pg(ctx);
   cudaStream_t st = ctx->stream;
   const u64 a4 = align_up(m * 4, 256), a8 = align_up(m * 8, 256);
-  void *scr = nullptr;
-  const int rc = st_scratch(ctx, 2 * a8 + 7 * a4 + align_up(m, 256) + align_up(order_scratch_bytes(m), 256) + 256, &scr);
+  const int rc = ctx->st_scratch.reserve(2 * a8 + 7 * a4 + align_up(m, 256) + align_up(order_scratch_bytes(m), 256) + 256, st, ctx->err);
   if (rc != RK_OK) return rc;
-  u8 *p = (u8 *)scr;
+  u8 *p = (u8 *)ctx->st_scratch.ptr();
   u64 *d_y = (u64 *)p; p += a8;
   u64 *d_d = (u64 *)p; p += a8;
   u32 *d_gid = (u32 *)p; p += a4;

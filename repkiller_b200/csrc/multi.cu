@@ -388,12 +388,9 @@ struct Dist {
   Trace trace;
   cudaStream_t side = nullptr;  // rows that travel while kernels run (the Y exchange beside the X sort)
   // grow-only side buffers whose size depends on the input, not on cap
-  u8 *aos_buf = nullptr;
-  u64 aos_bytes = 0;
-  u32 *link_buf = nullptr;  // [hist0][linkx_loc][linky_loc] (one all-gather) [linkx][linky][gather: world * the first three]
-  u64 link_words = 0;
-  void *h_res = nullptr;
-  u64 h_res_cap = 0;
+  GrowBuffer aos_buf;
+  GrowBuffer link_buf;  // u32 [hist0][linkx_loc][linky_loc] (one all-gather) [linkx][linky][gather: world * the first three]
+  GrowBuffer h_res{cudaHostAllocDefault};
 
   // state of the last load
   bool loaded = false;
@@ -713,43 +710,27 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
 
   const Geometry g = make_geometry(seqx_len, seqy_len);
   D.g = g;
-  D.bits_rank = ceil_log2(g.vsize) < 1 ? 1 : ceil_log2(g.vsize);
-  D.bits_y = ceil_log2(2ull * g.nby);
-  const u64 lxw = (2ull * g.nbx + 31) / 32 + 1, lyw = (2ull * g.nby + 31) / 32 + 1, lmax = lxw > lyw ? lxw : lyw;
+  const SortBits bits = sort_key_bits(g);
+  D.bits_rank = bits.rank, D.bits_y = bits.y;
+  const LinkWords lw = link_map_words(g);
+  const u64 lxw = lw.x, lyw = lw.y;
   const u64 pub_words = DIST_BINS + lxw + lyw;  // what a rank publishes after K1: its xStart/10 histogram and its link maps
   const u64 link_need = pub_words + lxw + lyw + (u64)nr * pub_words + 64;
-  (void)lmax;
-  if (link_need > D.link_words) {
-    CK(cudaStreamSynchronize(st));
-    if (D.link_buf) cudaFree(D.link_buf);
-    D.link_buf = nullptr, D.link_words = 0;
-    CK(cudaMalloc((void **)&D.link_buf, link_need * 4));
-    D.link_words = link_need;
-  }
-  u32 *hist0 = D.link_buf, *linkx_loc = hist0 + DIST_BINS, *linky_loc = linkx_loc + lxw, *linkx = linky_loc + lyw, *linky = linkx + lxw,
+  const int rc = D.link_buf.reserve(link_need * 4, st, ctx->err);
+  if (rc) return rc;
+  u32 *hist0 = (u32 *)D.link_buf.ptr(), *linkx_loc = hist0 + DIST_BINS, *linky_loc = linkx_loc + lxw, *linkx = linky_loc + lyw, *linky = linkx + lxw,
       *pub_all = linky + lyw;
 
-  bool on_device = false;
-  if (n_use) {
-    cudaPointerAttributes pa;
-    if (cudaPointerGetAttributes(&pa, frags) == cudaSuccess) on_device = pa.type == cudaMemoryTypeDevice;
-    else cudaGetLastError();
-  }
+  const bool on_device = n_use && is_device_pointer(frags);
   if (on_device && ((uintptr_t)frags & 15)) return fail(ctx, RK_ERR_ARG, "device record pointer must be 16-byte aligned");
   const u8 *aos = (const u8 *)frags;
   cudaEvent_t *ev = ctx->ev;
   CK(cudaEventRecord(ev[0], st));
   if (!on_device && n_use) {
-    const u64 need = align_up(n_use * RK_FRAG_BYTES, 16) + 16;
-    if (need > D.aos_bytes) {
-      CK(cudaStreamSynchronize(st));
-      if (D.aos_buf) cudaFree(D.aos_buf);
-      D.aos_buf = nullptr, D.aos_bytes = 0;
-      CK(cudaMalloc((void **)&D.aos_buf, need));
-      D.aos_bytes = need;
-    }
-    CK(cudaMemcpyAsync(D.aos_buf, frags, n_use * RK_FRAG_BYTES, cudaMemcpyHostToDevice, st));
-    aos = D.aos_buf;
+    const int rc2 = D.aos_buf.reserve(align_up(n_use * RK_FRAG_BYTES, 16) + 16, st, ctx->err);
+    if (rc2) return rc2;
+    CK(cudaMemcpyAsync(D.aos_buf.ptr(), frags, n_use * RK_FRAG_BYTES, cudaMemcpyHostToDevice, st));
+    aos = (const u8 *)D.aos_buf.ptr();
   }
   D.aos_src = aos;
   CK(cudaEventRecord(ev[1], st));
@@ -1116,28 +1097,14 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
     CK(cudaEventRecord(ev[8], st));
   }
 
-  u32 *h_order = nullptr, *h_gid = nullptr;
-  float *h_ident = nullptr;
-  u8 *h_rep = nullptr;
+  HostResult hr;
   if ((flags & RK_F_HOST_RESULT) && mg) {
-    const u64 need = 3 * align_up((u64)mg * 4, 256) + align_up((u64)mg, 256);
-    if (need > D.h_res_cap) {
-      CK(cudaStreamSynchronize(st));
-      if (D.h_res) cudaFreeHost(D.h_res);
-      D.h_res = nullptr, D.h_res_cap = 0;
-      CK(cudaHostAlloc(&D.h_res, need + need / 4, cudaHostAllocDefault));
-      D.h_res_cap = need + need / 4;
-    }
-    u8 *hb = (u8 *)D.h_res;
-    h_order = (u32 *)hb;
-    h_gid = (u32 *)(hb + align_up((u64)mg * 4, 256));
-    h_ident = (float *)(hb + 2 * align_up((u64)mg * 4, 256));
-    h_rep = hb + 3 * align_up((u64)mg * 4, 256);
+    const u64 need = HostResult::bytes(mg);
+    const int rc2 = D.h_res.reserve(need > D.h_res.cap() ? need + need / 4 : need, st, ctx->err);
+    if (rc2) return rc2;
+    hr = HostResult(D.h_res.ptr(), mg);
     CK(cudaEventRecord(ev[6], st));
-    CK(cudaMemcpyAsync(h_order, D.out_order, (u64)mg * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(h_gid, D.out_gid, (u64)mg * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(h_ident, D.out_identity, (u64)mg * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(h_rep, D.out_repval, (u64)mg, cudaMemcpyDeviceToHost, st));
+    CK(hr.fetch(D.out_order, D.out_gid, D.out_identity, D.out_repval, mg, st));
     CK(cudaEventRecord(ev[7], st));
   }
   CK(cudaMemcpyAsync(ctx->h_cnt, D.cnt, sizeof(Counters), cudaMemcpyDeviceToHost, st));
@@ -1162,7 +1129,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
 
   out->n_kept = mg;
   out->n_groups = total_groups;
-  out->order = h_order, out->gid = h_gid, out->repval = h_rep, out->identity = h_ident;
+  hr.publish(out);
   out->d_order = D.out_order, out->d_gid = D.out_gid, out->d_repval = D.out_repval, out->d_identity = D.out_identity;
   out->n_launches = launches;
   if (flags & RK_F_TIMING) {
@@ -1171,7 +1138,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
     out->ms_stage[RK_ST_FOREST] = ev_ms(ev[2], ev[3]);
     out->ms_stage[RK_ST_HKEY] = ev_ms(ev[3], ev[4]);   // output exchange
     out->ms_stage[RK_ST_GSORT] = ev_ms(ev[4], ev[5]);
-    if (h_order) out->ms_stage[RK_ST_D2H] = ev_ms(ev[6], ev[7]);
+    if (hr.order) out->ms_stage[RK_ST_D2H] = ev_ms(ev[6], ev[7]);
     out->ms_device = ev_ms(ev[0], line_records ? ev[8] : ev[5]);
   }
   if (info) {
@@ -1234,9 +1201,6 @@ void dist_destroy(rk_ctx *c) {
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->stream);
   dist_release_buffers(*D);
-  if (D->aos_buf) cudaFree(D->aos_buf);
-  if (D->link_buf) cudaFree(D->link_buf);
-  if (D->h_res) cudaFreeHost(D->h_res);
   if (D->h_small) cudaFreeHost(D->h_small);
   if (D->side) cudaStreamSynchronize(D->side), cudaStreamDestroy(D->side);
   delete D->tr;
@@ -1331,8 +1295,8 @@ int rk_dist_group_statistics(rk_ctx *ctx, unsigned flags, const rk_group_stats *
   if (rc) return rc;
   const Dist &D = *ctx->dist;
   const u64 ng = D.n_groups_rank;
-  if (stats) *stats = ((flags & RK_F_HOST_RESULT) && ng) ? (const rk_group_stats *)ctx->h_stats : nullptr;
-  if (d_stats) *d_stats = (const rk_group_stats *)ctx->d_stats;
+  if (stats) *stats = ((flags & RK_F_HOST_RESULT) && ng) ? (const rk_group_stats *)ctx->h_stats.ptr() : nullptr;
+  if (d_stats) *d_stats = (const rk_group_stats *)ctx->d_stats.ptr();
   if (first_gid) *first_gid = D.gid_base;
   if (n_groups) *n_groups = ng;
   return RK_OK;
@@ -1354,15 +1318,13 @@ struct rk_multi {
   u64 cap = 0;
   bool have_load = false;
   // merged host result of the last rk_multi_group
-  void *h_res = nullptr;
-  u64 h_res_cap = 0;
+  GrowBuffer h_res{cudaHostAllocDefault};
   std::vector<rk_dist_info> infos;
-  // rk_multi_format_lines: two alternating pinned text buffers; rk_multi_group_statistics: all groups (pinned)
-  char *h_text[2] = {nullptr, nullptr};
-  u64 h_text_bytes[2] = {0, 0};
+  // rk_multi_format_lines: two alternating pinned text buffers; rk_multi_group_statistics: all groups (pinned, portable:
+  // copied into by every GPU)
+  GrowBuffer h_text[2] = {GrowBuffer(cudaHostAllocPortable), GrowBuffer(cudaHostAllocPortable)};
   int h_text_next = 0;
-  void *h_stats = nullptr;
-  u64 h_stats_cap = 0;
+  GrowBuffer h_stats{cudaHostAllocPortable};
 };
 
 namespace {
@@ -1448,9 +1410,6 @@ void rk_destroy_multi(rk_multi *mg) {
   if (!mg) return;
   for (rk_ctx *c : mg->ctx) rk_destroy(c);
   for (ncclComm_t c : mg->comms) nccl_api().CommDestroy(c);
-  if (mg->h_res) cudaFreeHost(mg->h_res);
-  for (char *t : mg->h_text) if (t) cudaFreeHost(t);
-  if (mg->h_stats) cudaFreeHost(mg->h_stats);
   delete mg;
 }
 
@@ -1503,36 +1462,24 @@ int rk_multi_group(rk_multi *mg, double len_ratio, double pos_ratio, unsigned fl
   // the ranks hold consecutive ranges of output lines: concatenate them
   u64 total = 0;
   for (int r = 0; r < mg->n; ++r) total += res[r].n_kept;
-  const u64 need = 3 * align_up(total * 4, 256) + align_up(total, 256) + 256;
-  if (need > mg->h_res_cap) {
-    if (mg->h_res) cudaFreeHost(mg->h_res);
-    mg->h_res = nullptr, mg->h_res_cap = 0;
-    if (cudaHostAlloc(&mg->h_res, need, cudaHostAllocDefault) != cudaSuccess) {
-      cudaGetLastError();
-      mg->err = "cudaHostAlloc for the merged result failed";
-      return RK_ERR_NOMEM;
-    }
-    mg->h_res_cap = need;
-  }
-  u8 *hb = (u8 *)mg->h_res;
-  u32 *h_order = (u32 *)hb, *h_gid = (u32 *)(hb + align_up(total * 4, 256));
-  float *h_ident = (float *)(hb + 2 * align_up(total * 4, 256));
-  u8 *h_rep = hb + 3 * align_up(total * 4, 256);
+  const int rc2 = mg->h_res.reserve(HostResult::bytes(total), nullptr, mg->err);
+  if (rc2) return rc2;
+  const HostResult hr(mg->h_res.ptr(), total);
   std::vector<std::thread> th;
   for (int r = 0; r < mg->n; ++r)
     th.emplace_back([&, r] {
       const u64 off = mg->infos[r].line_offset, k = res[r].n_kept;
       if (!k) return;
-      memcpy(h_order + off, res[r].order, k * 4);
-      memcpy(h_gid + off, res[r].gid, k * 4);
-      memcpy(h_ident + off, res[r].identity, k * 4);
-      memcpy(h_rep + off, res[r].repval, k);
+      memcpy(hr.order + off, res[r].order, k * 4);
+      memcpy(hr.gid + off, res[r].gid, k * 4);
+      memcpy(hr.identity + off, res[r].identity, k * 4);
+      memcpy(hr.repval + off, res[r].repval, k);
     });
   for (auto &t : th) t.join();
   memset(out, 0, sizeof *out);
   out->n_kept = total;
   out->n_groups = res[0].n_groups;
-  out->order = h_order, out->gid = h_gid, out->repval = h_rep, out->identity = h_ident;
+  hr.publish(out);
   for (int r = 0; r < mg->n; ++r) {
     out->n_launches += res[r].n_launches;
     out->ms_device = std::max(out->ms_device, res[r].ms_device);
@@ -1579,20 +1526,11 @@ int rk_multi_format_lines(rk_multi *mg, uint64_t first_line, uint64_t n_lines, r
   // ... and copies it to its place in one buffer: the parts in rank order are the lines in order
   for (int r = 0; r < mg->n; ++r) pos[r + 1] = pos[r] + nb[r];
   const u64 nbytes = pos[mg->n];
-  const int hb = mg->h_text_next;
+  GrowBuffer &hb = mg->h_text[mg->h_text_next];
   mg->h_text_next ^= 1;
-  if (nbytes + 1 > mg->h_text_bytes[hb]) {
-    if (mg->h_text[hb]) cudaFreeHost(mg->h_text[hb]);
-    mg->h_text[hb] = nullptr, mg->h_text_bytes[hb] = 0;
-    const u64 cap = align_up(nbytes + nbytes / 8 + 4096, 4096);
-    if (cudaHostAlloc((void **)&mg->h_text[hb], cap, cudaHostAllocPortable) != cudaSuccess) {  // (copied into by every GPU)
-      cudaGetLastError();
-      mg->err = "cudaHostAlloc for the text failed";
-      return RK_ERR_NOMEM;
-    }
-    mg->h_text_bytes[hb] = cap;
-  }
-  char *buf = mg->h_text[hb];
+  rc = hb.reserve(nbytes + 1 > hb.cap() ? align_up(nbytes + nbytes / 8 + 4096, 4096) : nbytes + 1, nullptr, mg->err);
+  if (rc) return rc;
+  char *buf = (char *)hb.ptr();
   rc = run_ranks(mg, [&](int r) { return format_to_host(mg->ctx[r], nb[r], buf + pos[r], &ms[r]); });
   if (rc) return rc;
   out->text = buf;
@@ -1609,17 +1547,9 @@ int rk_multi_group_statistics(rk_multi *mg, const rk_group_stats **stats, uint64
   }
   const u64 total = mg->infos[0].total_groups;
   const u64 need = total * sizeof(rk_group_stats);
-  if (need > mg->h_stats_cap) {
-    if (mg->h_stats) cudaFreeHost(mg->h_stats);
-    mg->h_stats = nullptr, mg->h_stats_cap = 0;
-    if (cudaHostAlloc(&mg->h_stats, need + need / 8 + 4096, cudaHostAllocPortable) != cudaSuccess) {
-      cudaGetLastError();
-      mg->err = "cudaHostAlloc for the group statistics failed";
-      return RK_ERR_NOMEM;
-    }
-    mg->h_stats_cap = need + need / 8 + 4096;
-  }
-  rk_group_stats *h = (rk_group_stats *)mg->h_stats;
+  const int rc2 = mg->h_stats.reserve(need > mg->h_stats.cap() ? need + need / 8 + 4096 : need, nullptr, mg->err);
+  if (rc2) return rc2;
+  rk_group_stats *h = (rk_group_stats *)mg->h_stats.ptr();
   // every rank reduces its own groups (a group is never split) and copies them to their place in gid order
   const int rc = run_ranks(mg, [&](int r) -> int {
     rk_ctx *ctx = mg->ctx[r];
@@ -1632,7 +1562,7 @@ int rk_multi_group_statistics(rk_multi *mg, const rk_group_stats **stats, uint64
       return fail(ctx, RK_ERR_INTERNAL, "groups %u .. %u of rank %d beyond the %llu groups", D.gid_base, D.gid_base + D.n_groups_rank, r,
                   (unsigned long long)total);
     if (D.n_groups_rank) {
-      CK(cudaMemcpyAsync(h + D.gid_base, ctx->d_stats, (u64)D.n_groups_rank * sizeof(rk_group_stats), cudaMemcpyDeviceToHost, ctx->stream));
+      CK(cudaMemcpyAsync(h + D.gid_base, ctx->d_stats.ptr(), (u64)D.n_groups_rank * sizeof(rk_group_stats), cudaMemcpyDeviceToHost, ctx->stream));
       CK(cudaStreamSynchronize(ctx->stream));
     }
     return RK_OK;

@@ -1,11 +1,13 @@
 // The context behind the C ABI (include/rk_b200.h), shared by capi.cu (single GPU) and multi.cu (one comparison over
-// several GPUs): device workspace, pinned result buffers, per-kernel event profiler, error plumbing.
+// several GPUs): the loaded database, device workspace, grow-only buffers, pinned result buffers, per-kernel event
+// profiler, error plumbing.
 #pragma once
 
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/rk_b200.h"
@@ -58,19 +60,138 @@ struct Counters {  // small device block, mirrored in pinned host memory
   u32 work_g[8];
 };
 
+// A grow-only buffer in device memory (cudaMalloc) or pinned host memory (cudaHostAlloc with the owner's flags).
+// reserve(bytes, drain, err) keeps it when it holds `bytes`; otherwise it drains `drain` when one is given (work queued
+// there may still use the old buffer), frees it and allocates exactly `bytes`; the contents are not kept.  A caller that
+// wants headroom asks for more only when what it needs exceeds cap().  A failed allocation clears the CUDA error, leaves
+// the buffer empty and returns RK_ERR_NOMEM; a failed drain returns RK_ERR_CUDA and keeps the buffer.  Either way `err`
+// names the call.  The destructor frees the buffer: the owner's device must be current then, with no work queued that
+// uses it.
+class GrowBuffer {
+ public:
+  GrowBuffer() = default;                                                          // device memory
+  explicit GrowBuffer(unsigned host_flags) : pinned_(true), flags_(host_flags) {}  // pinned host memory
+  GrowBuffer(const GrowBuffer &) = delete;
+  GrowBuffer &operator=(const GrowBuffer &) = delete;
+  GrowBuffer(GrowBuffer &&o) noexcept : p_(o.p_), cap_(o.cap_), pinned_(o.pinned_), flags_(o.flags_) { o.p_ = nullptr, o.cap_ = 0; }
+  GrowBuffer &operator=(GrowBuffer &&o) noexcept {
+    std::swap(p_, o.p_), std::swap(cap_, o.cap_), std::swap(pinned_, o.pinned_), std::swap(flags_, o.flags_);
+    return *this;
+  }
+  ~GrowBuffer() { release(); }
+
+  int reserve(u64 bytes, cudaStream_t drain, std::string &err) {
+    if (bytes <= cap_) return RK_OK;
+    cudaError_t e = drain ? cudaStreamSynchronize(drain) : cudaSuccess;
+    if (e != cudaSuccess) {
+      err = std::string("cudaStreamSynchronize: ") + cudaGetErrorString(e);
+      return RK_ERR_CUDA;
+    }
+    release();
+    e = pinned_ ? cudaHostAlloc(&p_, bytes, flags_) : cudaMalloc(&p_, bytes);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      p_ = nullptr;
+      err = std::string(pinned_ ? "cudaHostAlloc(" : "cudaMalloc(") + std::to_string(bytes) + " bytes): " + cudaGetErrorString(e);
+      return RK_ERR_NOMEM;
+    }
+    cap_ = bytes;
+    return RK_OK;
+  }
+  void *ptr() const { return p_; }
+  u64 cap() const { return cap_; }
+
+ private:
+  void release() {
+    if (p_) pinned_ ? cudaFreeHost(p_) : cudaFree(p_);
+    p_ = nullptr, cap_ = 0;
+  }
+  void *p_ = nullptr;
+  u64 cap_ = 0;
+  bool pinned_ = false;
+  unsigned flags_ = 0;
+};
+
+// The pinned host arrays of RK_F_HOST_RESULT for m lines, carved from one buffer of bytes(m) at 256-byte boundaries
+struct HostResult {
+  static u64 bytes(u64 m) { return 3 * align_up(m * 4, 256) + align_up(m, 256); }
+  u32 *order = nullptr, *gid = nullptr;
+  float *identity = nullptr;
+  u8 *repval = nullptr;
+  HostResult() = default;
+  HostResult(void *buf, u64 m) {
+    u8 *p = (u8 *)buf;
+    order = (u32 *)p, gid = (u32 *)(p + align_up(m * 4, 256)), identity = (float *)(p + 2 * align_up(m * 4, 256));
+    repval = p + 3 * align_up(m * 4, 256);
+  }
+  // queues the copies of a result's four device arrays into these
+  cudaError_t fetch(const u32 *d_order, const u32 *d_gid, const float *d_identity, const u8 *d_repval, u64 m, cudaStream_t st) const {
+    cudaError_t e = cudaMemcpyAsync(order, d_order, m * 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(gid, d_gid, m * 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(identity, d_identity, m * 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(repval, d_repval, m, cudaMemcpyDeviceToHost, st);
+    return e;
+  }
+  void publish(rk_result *out) const { out->order = order, out->gid = gid, out->identity = identity, out->repval = repval; }
+};
+
+Geometry make_geometry(u64 seqx_len, u64 seqy_len);
+// the word counts of a load's two link maps, and the bit widths of its rank, X and Y sort keys (host side: Geometry is a
+// kernel argument, and its parameter block stays as it is)
+struct LinkWords { u64 x, y; };
+inline LinkWords link_map_words(const Geometry &g) { return {(2ull * g.nbx + 31) / 32 + 1, (2ull * g.nby + 31) / 32 + 1}; }
+struct SortBits { int rank, x, y; };
+inline SortBits sort_key_bits(const Geometry &g) {
+  return {ceil_log2(g.vsize) < 1 ? 1 : ceil_log2(g.vsize),  // (the sort clamps to >= 1 bit as well)
+          ceil_log2(2ull * g.nbx),                          // >= 2: nbx >= 2
+          ceil_log2(2ull * g.nby)};
+}
+
+inline bool is_device_pointer(const void *p) {
+  cudaPointerAttributes pa;
+  if (cudaPointerGetAttributes(&pa, p) == cudaSuccess) return pa.type == cudaMemoryTypeDevice;
+  cudaGetLastError();
+  return false;
+}
+
 struct Dist;  // multi.cu: this context's part in a comparison partitioned over several GPUs
 
-// What a load writes and a grouping only reads: the records (staged, or the caller's device pointer), the processing
-// order, the bucket sorts of both axes and h (carve_load), plus the side copy of a compact load.  A context owns one; its
-// views (rk_create_view) share it, and the last of them to be destroyed frees it.  The context fields that point into it
-// (rec4 .. h, aos_dev, pk_*) and the load's sizes are copied into every view.
+// What a load writes and a grouping only reads: the load's sizes, the records (staged, or the caller's device pointer),
+// the processing order, the bucket sorts of both axes and h (carve_load), plus the side copy of a compact load.  A
+// context owns one; its views (rk_create_view) hold a reference to it instead of a copy, and the last context to be
+// destroyed frees it.  It does not change while views are live: loading is refused then.
 struct Database {
   std::atomic<int> refs{1};  // the contexts that read it: the one that loaded it and its views
-  void *arena = nullptr;
-  u64 arena_bytes = 0;
+  GrowBuffer arena;
   cudaStream_t copy_stream = nullptr;  // H2D of data only the output formatter reads (rk_load_packed's rest4), beside the kernels
   cudaEvent_t copy_done = nullptr;
   bool side_copy = false;  // the last load queued such a copy; copy_done marks its end
+
+  u64 n = 0;  // records loaded
+  u32 m = 0;  // records kept
+  Geometry g{};
+
+  const u8 *aos_dev = nullptr;  // the loaded records on the device (own copy, or the caller's device pointer)
+  const uint4 *pk_key = nullptr, *pk_rest = nullptr;  // ... or the compact arrays of rk_load_packed (aos_dev == nullptr)
+  const u8 *pk_strand = nullptr;
+
+  // carved by carve_load
+  u8 *d_aos = nullptr;  // the host records staged on the device
+  uint4 *rec4 = nullptr;  // file order, two words per record: {xStart, yStart, length, flags} {identity bits, file index, 0, 0}
+  float *identity_r = nullptr;  // rank order
+  uint4 *hfi_r = nullptr;       // rank order {h, file index, identity bits, 0}
+  u32 *key0 = nullptr;
+  u32 *link_x = nullptr, *link_y = nullptr;
+  u32 *k0_r = nullptr, *fidx_r = nullptr;
+  uint2 *xl_r = nullptr, *yl_r = nullptr;  // rank order {center, length} per axis
+  u32 *ys_r = nullptr, *kx = nullptr, *ky = nullptr;
+  u32 *skx = nullptr, *rx = nullptr, *sky = nullptr, *ry = nullptr;
+  u32 *h = nullptr;
+
+  ~Database() {
+    if (copy_stream) cudaStreamSynchronize(copy_stream), cudaStreamDestroy(copy_stream);
+    if (copy_done) cudaEventDestroy(copy_done);
+  }
 };
 
 }  // namespace rk
@@ -82,15 +203,13 @@ struct rk_ctx {
   bool copy_pending = false;  // the database's side copy (Database::copy_done) is not yet waited for on this context's stream
   std::string err;
 
-  // the loaded database (shared with the views) and this context's grouping workspace (one allocation, carve_work())
+  // the loaded database (shared with the views) and this context's grouping workspace (carve_work)
   rk::Database *db = nullptr;
   bool is_view = false;  // made by rk_create_view: groups on another context's load, never loads
-  void *arena = nullptr;
-  rk::u64 arena_bytes = 0;
+  rk::GrowBuffer arena;
 
   // pinned host result buffers
-  void *h_res = nullptr;
-  rk::u64 h_res_cap = 0;
+  rk::GrowBuffer h_res{cudaHostAllocDefault};
   rk::Counters *h_cnt = nullptr;
 
   cudaEvent_t ev[RK_NSTAGES + 2];
@@ -98,54 +217,28 @@ struct rk_ctx {
 
   // calls on caller data (rk_sort_members): own counters and a grow-only scratch area
   rk::Counters *st_cnt = nullptr;
-  void *st_scratch = nullptr;
-  rk::u64 st_scratch_bytes = 0;
+  rk::GrowBuffer st_scratch;
 
-  // K6 text output: device text + work area (grow-only), pinned host mirror
-  const rk::u8 *aos_dev = nullptr;  // the loaded records on the device (own copy, or the caller's device pointer)
-  const uint4 *pk_key = nullptr, *pk_rest = nullptr;  // ... or the compact arrays of rk_load_packed (aos_dev == nullptr)
-  const rk::u8 *pk_strand = nullptr;
-  void *d_text = nullptr;
-  rk::u64 d_text_bytes = 0;
-  char *h_text[2] = {nullptr, nullptr};  // alternating: a chunk stays valid while the next one is produced
-  rk::u64 h_text_bytes[2] = {0, 0};
+  // K6 text output: device text + work area, pinned host mirror
+  rk::GrowBuffer d_text;
+  // alternating: a chunk stays valid while the next one is produced
+  rk::GrowBuffer h_text[2] = {rk::GrowBuffer(cudaHostAllocDefault), rk::GrowBuffer(cudaHostAllocDefault)};
   int h_text_next = 0;
 
-  // K8 per-group statistics: device array + pinned host mirror (grow-only)
-  void *d_stats = nullptr, *h_stats = nullptr;
-  rk::u64 stats_cap = 0, h_stats_cap = 0;
+  // K8 per-group statistics: device array + pinned host mirror
+  rk::GrowBuffer d_stats, h_stats{cudaHostAllocDefault};
   rk::u64 n_groups_last = 0;
 
-  // rk_diagonal_func's table (grow-only)
-  rk::u64 *d_diag = nullptr;
-  rk::u64 d_diag_bytes = 0;
+  rk::GrowBuffer d_diag;  // rk_diagonal_func's table
 
   bool loaded = false;
-  rk::u64 n = 0;
-  rk::u32 m = 0;
-  rk::Geometry g{};
-  int bits_rank = 1, bits_x = 1, bits_y = 1;
   bool have_group = false;
 
   rk::Dist *dist = nullptr;  // set by rk_dist_init (multi.cu)
 
-  // carved pointers.  Database (carve_load, written by the load only): d_aos .. h below, except the workspace ones marked W.
-  // Workspace (carve_work, written by a grouping; the load uses the loading context's scratch and counters too): W.
-  rk::u8 *d_aos = nullptr;
-  uint4 *rec4 = nullptr;  // file order, two words per record: {xStart, yStart, length, flags} {identity bits, file index, 0, 0}
-  float *identity_r = nullptr;  // rank order
-  uint4 *hfi_r = nullptr;       // rank order {h, file index, identity bits, 0}
-  rk::u32 *key0 = nullptr;
-  rk::u32 *link_x = nullptr, *link_y = nullptr;
-  rk::u64 link_x_words = 0, link_y_words = 0;
-  rk::Counters *d_cnt = nullptr;  // W
-  rk::u32 *k0_r = nullptr, *fidx_r = nullptr;
-  rk::u32 *tmp_k = nullptr, *tmp_v = nullptr;  // W
-  uint2 *xl_r = nullptr, *yl_r = nullptr;  // rank order {center, length} per axis
-  rk::u32 *ys_r = nullptr, *kx = nullptr, *ky = nullptr;
-  rk::u32 *skx = nullptr, *rx = nullptr, *sky = nullptr, *ry = nullptr;
-  rk::u32 *h = nullptr;
-  // W from here on
+  // the workspace, carved by carve_work: written by a grouping; the load uses the loading context's scratch and counters too
+  rk::Counters *d_cnt = nullptr;
+  rk::u32 *tmp_k = nullptr, *tmp_v = nullptr;
   void *sort_work = nullptr;
   rk::u32 *prehist = nullptr;  // 4 x [4][256]: digit counts of key0, kx, ky, gid gathered by the kernels that produce them
   rk::u32 *xm_bits = nullptr;
@@ -190,7 +283,6 @@ struct ProfGuard {  // routes the launchers' KScope events to this context for t
   }
 };
 
-Geometry make_geometry(u64 seqx_len, u64 seqy_len);
 const char *err_bits_text(u32 e);
 float ev_ms(cudaEvent_t a, cudaEvent_t b);
 void dist_destroy(rk_ctx *c);  // multi.cu: releases c->dist (called by rk_destroy)

@@ -14,8 +14,7 @@
 #include <string>
 #include <vector>
 
-#include "../../include/rk_b200.h"
-#include "rk_common.cuh"
+#include "rk_ctx.cuh"
 
 using namespace rk;
 
@@ -108,8 +107,7 @@ struct rk_sol {
   u32 *head = nullptr;
   SolEntry *pool = nullptr;
   u64 pool_cap = 0, n_entries = 0;
-  SolInsert *d_ins = nullptr, *h_ins = nullptr;  // staging of the queued inserts (device, pinned host)
-  u64 ins_cap = 0;
+  GrowBuffer d_ins, h_ins{cudaHostAllocDefault};  // staging of the queued inserts (device, pinned host)
   std::vector<SolInsert> pending;
   u64 *h_result = nullptr, *d_result = nullptr;
   std::string err;
@@ -141,20 +139,15 @@ int sol_flush(rk_sol *s) {
     if (s->pool) cudaFree(s->pool);
     s->pool = np, s->pool_cap = cap;
   }
-  if (n > s->ins_cap) {
-    u64 cap = s->ins_cap ? s->ins_cap : 256;
-    while (cap < n) cap *= 2;
-    SK(cudaStreamSynchronize(s->stream));
-    if (s->d_ins) cudaFree(s->d_ins);
-    if (s->h_ins) cudaFreeHost(s->h_ins);
-    s->d_ins = nullptr, s->h_ins = nullptr, s->ins_cap = 0;
-    SK(cudaMalloc((void **)&s->d_ins, cap * sizeof(SolInsert)));
-    SK(cudaHostAlloc((void **)&s->h_ins, cap * sizeof(SolInsert), cudaHostAllocDefault));
-    s->ins_cap = cap;
-  }
-  memcpy(s->h_ins, s->pending.data(), n * sizeof(SolInsert));
-  SK(cudaMemcpyAsync(s->d_ins, s->h_ins, n * sizeof(SolInsert), cudaMemcpyHostToDevice, s->stream));
-  k_sol_apply<<<1, 32, 0, s->stream>>>(s->d_ins, (u32)n, s->pool, (u32)s->n_entries, s->head);
+  u64 cap = s->h_ins.cap() ? s->h_ins.cap() / sizeof(SolInsert) : 256;
+  while (cap < n) cap *= 2;
+  int rc = s->d_ins.reserve(cap * sizeof(SolInsert), s->stream, s->err);
+  if (!rc) rc = s->h_ins.reserve(cap * sizeof(SolInsert), s->stream, s->err);
+  if (rc) return rc;
+  SolInsert *d_ins = (SolInsert *)s->d_ins.ptr(), *h_ins = (SolInsert *)s->h_ins.ptr();
+  memcpy(h_ins, s->pending.data(), n * sizeof(SolInsert));
+  SK(cudaMemcpyAsync(d_ins, h_ins, n * sizeof(SolInsert), cudaMemcpyHostToDevice, s->stream));
+  k_sol_apply<<<1, 32, 0, s->stream>>>(d_ins, (u32)n, s->pool, (u32)s->n_entries, s->head);
   SK(cudaStreamSynchronize(s->stream));  // the pinned staging buffer is reused by the next flush
   s->n_entries += n;
   s->pending.clear();
@@ -194,12 +187,10 @@ void rk_sol_destroy(rk_sol *s) {
   if (s->stream) cudaStreamSynchronize(s->stream);
   if (s->head) cudaFree(s->head);
   if (s->pool) cudaFree(s->pool);
-  if (s->d_ins) cudaFree(s->d_ins);
-  if (s->h_ins) cudaFreeHost(s->h_ins);
   if (s->d_result) cudaFree(s->d_result);
   if (s->h_result) cudaFreeHost(s->h_result);
   if (s->stream) cudaStreamDestroy(s->stream);
-  delete s;
+  delete s;  // frees the insert staging: the device is current and the stream drained
 }
 
 const char *rk_sol_last_error(const rk_sol *s) { return s ? s->err.c_str() : "null rk_sol"; }
