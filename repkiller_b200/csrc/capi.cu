@@ -134,7 +134,7 @@ const char *err_bits_text(u32 e) {
 void prof_route(Profiler *p) { tl_prof = p; }
 void prof_begin(int kid, cudaStream_t st, unsigned long long units) {
   if (!tl_prof) return;
-  Profiler::Rec r{kid, tl_prof->get(), tl_prof->get(), (u64)units};
+  Profiler::Rec r{kid, tl_prof->pool.get(), tl_prof->pool.get(), (u64)units};
   cudaEventRecord(r.a, st);
   tl_prof->open_recs.push_back(r);
 }
@@ -515,7 +515,7 @@ int rk_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flags, rk
   my.work_count = ctx->d_cnt->work_y;
   launches += launch_match(my, st);
   CK(cudaEventRecord(ev[2], st));
-  const int bits_g = ceil_log2(m) < 1 ? 1 : ceil_log2(m);
+  const int bits_g = key_bits(m);
   CK(cudaMemsetAsync(ctx->prehist + 3072, 0, 4 * 256 * 4, st));
   launches += launch_forest(ctx->parent, m, ctx->gid_rank, &ctx->d_cnt->n_groups, ctx->forest_work, st, 0, 0xFFFFFFFFu,
                             HistOut{ctx->prehist + 3072, (bits_g + 7) / 8, bits_g});
@@ -624,14 +624,6 @@ int format_on_device(rk_ctx *ctx, FormatArgs fa, u64 *nbytes) {
   return RK_OK;
 }
 
-int format_text_buffer(rk_ctx *ctx, u64 nbytes, char **buf) {
-  GrowBuffer &b = ctx->h_text[ctx->h_text_next];
-  ctx->h_text_next ^= 1;
-  const int rc = b.reserve(nbytes + 1 > b.cap() ? align_up(nbytes + nbytes / 8 + 4096, 4096) : nbytes + 1, nullptr, ctx->err);
-  *buf = (char *)b.ptr();
-  return rc;
-}
-
 int format_to_host(rk_ctx *ctx, u64 nbytes, char *dst, float *ms_device) {
   CK(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
@@ -663,7 +655,7 @@ int rk_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_text 
   u64 nbytes = 0;
   char *buf = nullptr;
   int rc = format_on_device(ctx, fa, &nbytes);
-  if (!rc) rc = format_text_buffer(ctx, nbytes, &buf);
+  if (!rc) rc = ctx->h_text.next(nbytes, &buf, ctx->err);
   if (!rc) rc = format_to_host(ctx, nbytes, buf, &out->ms_device);
   if (rc) return rc;
   out->text = buf;

@@ -33,6 +33,7 @@
 #include <condition_variable>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <mutex>
 #include <thread>
 
@@ -153,6 +154,11 @@ struct Transport {
   u8 *peer_base[DIST_MAX_RANKS] = {nullptr};
   template <class T>
   T *on_peer(int p, T *local) const { return (T *)(peer_base[p] + ((const u8 *)local - my_base)); }
+  // out[d] = the buffer `local` on rank d, for every rank (kernels store rows straight into it)
+  template <class T, class U>
+  void peer_table(T *local, U **out) const {
+    for (int d = 0; d < world; ++d) out[d] = d == rank ? local : on_peer(d, local);
+  }
 
   // The rows of a variable all-to-all (counts of `ex` in elements of `elem` bytes).  Every rank PUSHES its blocks into
   // the peers' receive buffers with copy-engine copies (peer copies over NVLink between GPUs), then enters barrier().
@@ -330,16 +336,10 @@ struct Trace {
   bool on = false;
   struct Rec { const char *what; cudaEvent_t a, b; };
   std::vector<Rec> recs;
-  std::vector<cudaEvent_t> pool;
-  cudaEvent_t get() {
-    if (!pool.empty()) { cudaEvent_t e = pool.back(); pool.pop_back(); return e; }
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    return e;
-  }
+  EventPool pool;
   void begin(const char *what, cudaStream_t st) {
     if (!on) return;
-    Rec r{what, get(), get()};
+    Rec r{what, pool.get(), pool.get()};
     cudaEventRecord(r.a, st);
     recs.push_back(r);
   }
@@ -361,8 +361,8 @@ struct Trace {
       snprintf(buf, sizeof buf, " %s)=%.3f", w.c_str(), ms);
       line += buf;
       total += ms;
-      pool.push_back(r.a);
-      pool.push_back(r.b);
+      pool.put(r.a);
+      pool.put(r.b);
     }
     recs.clear();
     fprintf(stderr, "%s | comm total %.3f ms\n", line.c_str(), total);
@@ -380,10 +380,11 @@ struct Dist {
   int rank = 0, world = 1;
   Transport *tr = nullptr;
   u64 cap = 0, hcap = 0;
-  void *arena = nullptr;
+  GrowBuffer arena;  // carved by dist_carve for cap rows per rank; grows only (rk_dist_init makes a new Dist)
   void *peer_open[DIST_MAX_RANKS] = {nullptr};
   bool peers_ready = false;
-  u32 *h_small = nullptr;  // pinned [world][SMALL_WORDS]
+  GrowBuffer small_host{cudaHostAllocDefault};
+  u32 *h_small = nullptr;  // [world][SMALL_WORDS] in small_host
   PeerTable pt{};
   Trace trace;
   cudaStream_t side = nullptr;  // rows that travel while kernels run (the Y exchange beside the X sort)
@@ -543,13 +544,11 @@ static void dist_release_buffers(Dist &D) {
     D.peer_open[r] = nullptr;
   }
   D.peers_ready = false;
-  if (D.arena) cudaFree(D.arena);
-  D.arena = nullptr;
   D.cap = D.hcap = 0;
   D.loaded = false;
 }
 
-// (re)allocates the partition buffers for cap rows per rank; the peers must import again afterwards
+// grows the partition buffers to cap rows per rank; the peers must import again afterwards
 static int dist_allocate(rk_ctx *ctx, u64 cap) {
   Dist &D = *ctx->dist;
   CK(cudaSetDevice(ctx->device));
@@ -559,15 +558,13 @@ static int dist_allocate(rk_ctx *ctx, u64 cap) {
   if (cap >= 0xFFFFFF00ull) return fail(ctx, RK_ERR_ARG, "capacity per rank must stay below 2^32");
   D.cap = cap;
   D.hcap = cap / 8 + 65536;
-  const u64 need = dist_carve(D, nullptr);
-  cudaError_t e = cudaMalloc(&D.arena, need);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
+  std::string err;
+  const int rc = D.arena.reserve(dist_carve(D, nullptr), nullptr, err);
+  if (rc) {
     dist_release_buffers(D);
-    return fail(ctx, RK_ERR_NOMEM, "cudaMalloc(%llu bytes for %llu rows per rank): %s", (unsigned long long)need,
-                (unsigned long long)cap, cudaGetErrorString(e));
+    return fail(ctx, rc, "%llu rows per rank: %s", (unsigned long long)cap, err.c_str());
   }
-  dist_carve(D, (u8 *)D.arena);
+  dist_carve(D, (u8 *)D.arena.ptr());
   return RK_OK;
 }
 
@@ -597,7 +594,9 @@ static int dist_init_common(rk_ctx *ctx, int rank, int world, Transport *tr, u64
   ctx->dist = D;
   D->trace.on = getenv("RK_DIST_TRACE") != nullptr;
   CK(cudaSetDevice(ctx->device));
-  CK(cudaHostAlloc((void **)&D->h_small, (size_t)world * SMALL_WORDS * sizeof(u32), cudaHostAllocDefault));
+  const int rc = D->small_host.reserve((u64)world * SMALL_WORDS * sizeof(u32), nullptr, ctx->err);
+  if (rc) return rc;
+  D->h_small = (u32 *)D->small_host.ptr();
   CK(cudaStreamCreateWithFlags(&D->side, cudaStreamNonBlocking));
   return dist_allocate(ctx, cap);
 }
@@ -605,9 +604,9 @@ static int dist_init_common(rk_ctx *ctx, int rank, int world, Transport *tr, u64
 static int dist_export(rk_ctx *ctx, DistBlob *b) {
   Dist &D = *ctx->dist;
   memset(b, 0, sizeof *b);
-  b->pid = (u64)getpid(), b->ptr = (u64)(uintptr_t)D.arena, b->cap = D.cap, b->device = ctx->device;
+  b->pid = (u64)getpid(), b->ptr = (u64)(uintptr_t)D.arena.ptr(), b->cap = D.cap, b->device = ctx->device;
   CK(cudaSetDevice(ctx->device));
-  CK(cudaIpcGetMemHandle(&b->handle, D.arena));
+  CK(cudaIpcGetMemHandle(&b->handle, D.arena.ptr()));
   return RK_OK;
 }
 
@@ -621,7 +620,7 @@ static int dist_import(rk_ctx *ctx, const u8 *blobs, size_t stride) {
                                     (unsigned long long)b.cap, (unsigned long long)D.cap);
     u8 *base = nullptr;
     if (r == D.rank) {
-      base = (u8 *)D.arena;
+      base = (u8 *)D.arena.ptr();
     } else if (b.pid == (u64)getpid()) {
       base = (u8 *)(uintptr_t)b.ptr;
       if (b.device != ctx->device) {
@@ -638,35 +637,60 @@ static int dist_import(rk_ctx *ctx, const u8 *blobs, size_t stride) {
     }
     D.tr->peer_base[r] = base;
     // the arenas are carved identically (same capacity, same number of ranks): local offsets hold on every peer
-    D.pt.res[r] = (const u64 *)(base + ((const u8 *)D.res - (const u8 *)D.arena));
+    D.pt.res[r] = (const u64 *)(base + ((const u8 *)D.res - (const u8 *)D.arena.ptr()));
   }
-  D.tr->my_base = (const u8 *)D.arena;
+  D.tr->my_base = (const u8 *)D.arena.ptr();
   if (NcclTransport *nt = dynamic_cast<NcclTransport *>(D.tr)) nt->d_flag = D.flag, nt->d_flag_all = D.flag_all;
   D.pt.nr = D.world, D.pt.me = D.rank;
   D.peers_ready = true;
   return RK_OK;
 }
 
-// the count exchange with the matrix left on the device as well (d_small_all) and on the host (h_small); synchronises
-static int dist_gather_counts(rk_ctx *ctx) {
+// The count exchange: every rank publishes its row d_small (its error word W_ERR included; the caller has written the
+// rest) and gets everybody's rows, on the device in d_small_all and on the host in h_small.  A routed round passes
+// `push`: launched once the rows are on the device, it stores rows straight into their owners' buffers (peer memory),
+// and a barrier follows it, so the rows have landed everywhere when this returns.  Synchronises.
+static int dist_gather_counts(rk_ctx *ctx, const std::function<void()> &push = {}) {
   Dist &D = *ctx->dist;
   CK(cudaMemcpyAsync(D.d_small + W_ERR, &D.cnt->err, sizeof(u32), cudaMemcpyDeviceToDevice, ctx->stream));
   TR(D.tr->gather_small_begin(D.d_small, D.d_small_all, D.h_small, ctx->stream));
+  if (push) {
+    push();
+    TR(D.tr->barrier(ctx->stream));
+  }
   TR(D.tr->gather_small_end(D.d_small_all, D.h_small, ctx->stream));
   return RK_OK;
 }
 
-// error words of all ranks after a count exchange: every rank sees the same matrix, so every rank returns together
-static int dist_check_small(rk_ctx *ctx, bool range_errors) {
-  Dist &D = *ctx->dist;
+// error words of all ranks after a count exchange: every rank sees the same matrix, so every rank returns together.
+// With worklist_nomem, ERR_WORKLIST is a capacity error: RK_ERR_NOMEM with that message (it takes the capacity per rank).
+static int dist_check_small(rk_ctx *ctx, bool range_errors, const char *worklist_nomem = nullptr) {
+  const Dist &D = *ctx->dist;
   u32 e = 0;
   for (int r = 0; r < D.world; ++r) e |= D.h_small[(size_t)r * SMALL_WORDS + W_ERR];
   if (!e) return RK_OK;
+  if (worklist_nomem && (e & ERR_WORKLIST)) return fail(ctx, RK_ERR_NOMEM, worklist_nomem, (unsigned long long)D.cap);
   return fail(ctx, (range_errors && !(e & (ERR_WORKLIST | ERR_SPIN))) ? RK_ERR_RANGE : RK_ERR_INTERNAL, "%s", err_bits_text(e));
 }
 
-// every rank's copy of one of this rank's arena buffers (the rows of the big exchanges are stored there by the kernels)
-static void peer_rows(const Dist &D, uint4 *local, uint4 **outs);
+// after a count exchange: the rows every rank d receives (column word0 + d, summed over the senders) against bound.
+// fmt takes the rank, the rows and the capacity per rank; every rank sees the same matrix, so every rank returns together.
+static int check_inbound(rk_ctx *ctx, int word0, u64 bound, const char *fmt) {
+  const Dist &D = *ctx->dist;
+  for (int d = 0; d < D.world; ++d) {
+    const u64 in = column_sum(D.h_small, word0 + d, D.world);
+    if (in > bound) return fail(ctx, RK_ERR_NOMEM, fmt, d, (unsigned long long)in, (unsigned long long)D.cap);
+  }
+  return RK_OK;
+}
+
+// this rank's slice of a cut table, [cuts[me], cuts[me + 1]) with the end clamped to limit (the last rank's to limit):
+// sort keys taken relative to base need `bits` bits
+struct KeyRange { u32 base; u64 end; int bits; };
+static KeyRange rank_key_range(const u32 *cuts, int me, int nr, u64 limit) {
+  const u64 end = me + 1 < nr ? std::min<u64>(cuts[me + 1], limit) : limit;
+  return {cuts[me], end, key_bits(end > cuts[me] ? end - cuts[me] : 1)};
+}
 
 // block table of a per-pair exchange whose values the producing kernel stores straight into the peers' buffers:
 // forward = in send order (blocks by destination, landing where the rows of the load-time exchange landed),
@@ -680,9 +704,9 @@ static ScatterTable scatter_table(const Dist &D, const Exchange &ex, bool back, 
     t.start[d] = (u32)run;
     run += back ? ex.rcnt[d] : ex.scnt[d];
     t.dst_off[d] = (u32)(back ? ex.rpoff[d] : ex.poff[d]);
-    t.out[d] = d == D.rank ? (void *)local_buf : (void *)D.tr->on_peer(d, local_buf);
   }
   t.start[D.world] = (u32)run;
+  D.tr->peer_table(local_buf, t.out);
   return t;
 }
 
@@ -760,24 +784,20 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   // count per destination -> all ranks' counts on the device -> every tile stores its records straight into the owners'
   // receive buffers (peer memory over NVLink) -> barrier; the host reads the count matrix while the rows travel
   uint2 *outs[DIST_MAX_RANKS];
-  for (int d = 0; d < nr; ++d) outs[d] = d == me ? D.rec6_arr : D.tr->on_peer(d, D.rec6_arr);
+  D.tr->peer_table(D.rec6_arr, outs);
   launches += dist_count_plain(D.key0_loc, (u32)n_use, D.cuts0, nr, g.vsize - 1, D.tile_cnt, D.d_small + W_CNT_A, st);
-  CK(cudaMemcpyAsync(D.d_small + W_ERR, &D.cnt->err, sizeof(u32), cudaMemcpyDeviceToDevice, st));
   CK(cudaMemcpyAsync(D.d_small + W_CUTS, D.cuts0, (nr + 1) * sizeof(u32), cudaMemcpyDeviceToDevice, st));
   const u32 foff32 = (u32)file_off;
   CK(cudaMemcpyAsync(D.d_small + W_FOFF, &foff32, sizeof(u32), cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
-  TR(D.tr->gather_small_begin(D.d_small, D.d_small_all, D.h_small, st));
-  launches += dist_push_records(D.key0_loc, (u32)n_use, D.cuts0, nr, g.vsize - 1, D.rec4_loc, outs, (u32)D.cap, D.tile_cnt, D.d_small_all,
-                                SMALL_WORDS, me, st);
-  TR(D.tr->barrier(st));
-  TR(D.tr->gather_small_end(D.d_small_all, D.h_small, st));  // host sync 1
-  if (too_many || dist_check_small(ctx, true) != RK_OK) {
-    u32 e = 0;
-    for (int r = 0; r < nr; ++r) e |= D.h_small[(size_t)r * SMALL_WORDS + W_ERR];
-    if (e & ERR_WORKLIST) return fail(ctx, RK_ERR_NOMEM, "a rank holds more records than the capacity of %llu rows per rank given to rk_dist_init",
-                                      (unsigned long long)D.cap);
-    return dist_check_small(ctx, true);
-  }
+  if (const int rc = dist_gather_counts(ctx, [&] {  // host sync 1
+        launches += dist_push_records(D.key0_loc, (u32)n_use, D.cuts0, nr, g.vsize - 1, D.rec4_loc, outs, (u32)D.cap, D.tile_cnt,
+                                      D.d_small_all, SMALL_WORDS, me, st);
+      }))
+    return rc;
+  // (a rank whose slice exceeds the capacity loaded nothing and published ERR_WORKLIST)
+  if (const int rc = dist_check_small(ctx, true, "a rank holds more records than the capacity of %llu rows per rank given to rk_dist_init"))
+    return rc;
+  if (const int rc = check_inbound(ctx, W_CNT_A, D.cap, "rank %d would own %llu fragments, capacity is %llu rows per rank")) return rc;
   D.ex1.from_matrix(D.h_small, W_CNT_A, nr, me);
   // where every rank's slice starts (as its caller said) and, from the row sums of the count matrix (the dropped column
   // included), how long it is: the line records of RK_F_LINE_RECORDS find the rank that loaded a record by these starts,
@@ -790,34 +810,27 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
     if (s + 1 < nr && D.file_off[s] + n_s > D.h_small[(size_t)(s + 1) * SMALL_WORDS + W_FOFF]) D.slices_in_order = false;
   }
   D.tr->bytes_sent += (D.ex1.n_send - D.ex1.scnt[me]) * 24;  // (the rows this rank's kernels stored into peer memory)
-  u64 loaded_total = 0, m_of[DIST_MAX_RANKS] = {0};
+  u64 loaded_total = 0, off = 0;
   for (int d = 0; d <= nr; ++d) loaded_total += column_sum(D.h_small, W_CNT_A + d, nr);
-  u64 off = 0;
   for (int d = 0; d < nr; ++d) {
-    m_of[d] = column_sum(D.h_small, W_CNT_A + d, nr);
     D.pt.roff[d] = (u32)off;
-    if (d == me) D.rank_off = (u32)off;
-    off += m_of[d];
-    if (m_of[d] > D.cap) return fail(ctx, RK_ERR_NOMEM, "rank %d would own %llu fragments, capacity is %llu rows per rank", d,
-                                     (unsigned long long)m_of[d], (unsigned long long)D.cap);
+    off += column_sum(D.h_small, W_CNT_A + d, nr);
   }
+  D.rank_off = D.pt.roff[me];
   const u64 m_total = off;
   D.pt.roff[nr] = (u32)m_total;
   for (int d = nr + 1; d <= DIST_MAX_RANKS; ++d) D.pt.roff[d] = 0xFFFFFFFFu;
   CK(cudaMemcpyAsync(D.roff_dev, D.pt.roff, (nr + 1) * sizeof(u32), cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
   D.m_total = m_total, D.n_total_loaded = loaded_total;
-  const u32 m = (u32)m_of[me];
+  const u32 m = (u32)D.ex1.n_recv;
   D.m_loc = m;
 
   CK(cudaEventRecord(ev[2], st));
   // processing order: sources arrive in file order, so a stable sort by xStart/10 is the global order
   // the sort keys are taken relative to the rank's first xStart/10 bucket: log2(range of the rank) bits instead of log2(vsize)
-  const u32 *cuts0_h = D.h_small + (size_t)me * SMALL_WORDS + W_CUTS;
-  const u32 key0_base = cuts0_h[me];
-  const u64 key0_end = (me + 1 < nr && cuts0_h[me + 1] < g.vsize) ? cuts0_h[me + 1] : g.vsize;
-  const int bits_rank_l = ceil_log2(key0_end > key0_base ? key0_end - key0_base : 1) < 1 ? 1 : ceil_log2(key0_end - key0_base);
-  launches += dist_key0_of_rec(D.rec6_arr, m, key0_base, D.key0a, hist_of(0, bits_rank_l), st);
-  launches += launch_sort_pairs(D.key0a, nullptr, D.k0_r, D.aidx_r, D.tmp_k, D.tmp_v, m, bits_rank_l, D.sort_work, st, &D.cnt->err,
+  const KeyRange k0 = rank_key_range(D.h_small + (size_t)me * SMALL_WORDS + W_CUTS, me, nr, g.vsize);
+  launches += dist_key0_of_rec(D.rec6_arr, m, k0.base, D.key0a, hist_of(0, k0.bits), st);
+  launches += launch_sort_pairs(D.key0a, nullptr, D.k0_r, D.aidx_r, D.tmp_k, D.tmp_v, m, k0.bits, D.sort_work, st, &D.cnt->err,
                                 m ? D.prehist : nullptr);
   CK(cudaEventRecord(ev[3], st));
   launches += launch_keys(D.aidx_r, m, g, nullptr, linkx, linky, D.xl, D.yl_r, D.ys_r, D.kx2, D.ky, D.identity_r, st,
@@ -836,12 +849,8 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   launches += dist_split_axis(D.ky, D.yl_r, m, D.cuts_y, nr, D.rank_off, D.send_rows, D.perm_y, D.tile_cnt, D.d_small + W_CNT_B, st);
   CK(cudaMemcpyAsync(D.d_small + W_CUTS, D.cuts_y, (nr + 1) * sizeof(u32), cudaMemcpyDeviceToDevice, st));
   CK(cudaMemcpyAsync(D.d_small + W_CUTSX, D.cuts_x, 2 * nr * sizeof(u32), cudaMemcpyDeviceToDevice, st));
-  {
-    const int rc = dist_gather_counts(ctx);  // host sync 2
-    if (rc) return rc;
-    const int rc2 = dist_check_small(ctx, true);
-    if (rc2) return rc2;
-  }
+  if (const int rc = dist_gather_counts(ctx)) return rc;  // host sync 2
+  if (const int rc = dist_check_small(ctx, true)) return rc;
   D.exh.from_matrix(D.h_small, W_CNT_A, nr, me);
   D.exy.from_matrix(D.h_small, W_CNT_B, nr, me);
   for (int d = 0; d < nr; ++d) {
@@ -856,10 +865,7 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   }
   D.n_away = (u32)D.exh.n_send, D.n_halo = (u32)D.exh.n_recv, D.m_y = (u32)D.exy.n_recv;
   // Y sort keys relative to the first key of the rank's Y range
-  const u32 *cutsy_h = D.h_small + (size_t)me * SMALL_WORDS + W_CUTS;
-  const u32 ky_base = cutsy_h[me];
-  const u64 ky_end = (me + 1 < nr && cutsy_h[me + 1] < 2ull * g.nby) ? cutsy_h[me + 1] : 2ull * g.nby;
-  const int bits_y_l = ceil_log2(ky_end > ky_base ? ky_end - ky_base : 1) < 1 ? 1 : ceil_log2(ky_end - ky_base);
+  const KeyRange yr = rank_key_range(D.h_small + (size_t)me * SMALL_WORDS + W_CUTS, me, nr, 2ull * g.nby);
 
   // Both row exchanges come right after host sync 2: every rank's work queued before it is complete, so no rank still
   // reads its halo_recv / recv_rows (last read by the previous load and group) when the peers' pushes start.
@@ -883,8 +889,8 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
                                 (m + D.n_halo) ? D.prehist + 1024 : nullptr);
   CK(cudaEventRecord(ev[6], st));
   TR(D.tr->exchange_rows_end(st));
-  launches += dist_unpack_axis_rows(D.recv_rows, D.m_y, ky_base, D.ky_a, D.yl_a, D.grank_a, hist_of(2, bits_y_l), st);
-  launches += launch_sort_pairs(D.ky_a, nullptr, D.sky_a, D.ry_a, D.tmp_k, D.tmp_v, D.m_y, bits_y_l, D.sort_work, st, &D.cnt->err,
+  launches += dist_unpack_axis_rows(D.recv_rows, D.m_y, yr.base, D.ky_a, D.yl_a, D.grank_a, hist_of(2, yr.bits), st);
+  launches += launch_sort_pairs(D.ky_a, nullptr, D.sky_a, D.ry_a, D.tmp_k, D.tmp_v, D.m_y, yr.bits, D.sort_work, st, &D.cnt->err,
                                 D.m_y ? D.prehist + 2048 : nullptr);
   CK(cudaEventRecord(ev[7], st));
   D.loaded = true;
@@ -963,10 +969,8 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   launches += dist_root_scan(D.parent, m, D.gidscan, D.d_small + W_X0, D.scan_work, st);
   launches += dist_chase_local(D.parent, D.gidscan, m, D.rank_off, D.lroot, D.res, D.pend_idx[0], D.pend_key[0], D.n_pend, st);
   CK(cudaMemcpyAsync(D.d_small + W_X2, D.n_pend, sizeof(u32), cudaMemcpyDeviceToDevice, st));
-  {
-    const int rc = dist_gather_counts(ctx);  // host sync: roots and pending chains of every rank (also: every rank's res[] is final)
-    if (rc) return rc;
-  }
+  // host sync: roots and pending chains of every rank (also: every rank's res[] is final)
+  if (const int rc = dist_gather_counts(ctx)) return rc;
   // the root counts stay on the device as a column of the gathered matrix, in a copy that later gathers do not overwrite
   CK(cudaMemcpyAsync(D.nroots_mat, D.d_small_all, (size_t)nr * SMALL_WORDS * sizeof(u32), cudaMemcpyDeviceToDevice, st));
   const u32 *nroots = D.nroots_mat + W_X0;
@@ -980,21 +984,16 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
     const u32 bound = (u32)std::min<u64>(D.h_small[(size_t)me * SMALL_WORDS + W_X2], m);  // this rank's pending chains
     // ask: the ranks in question go to their owners
     uint4 *qouts[DIST_MAX_RANKS];
-    peer_rows(D, D.queries, qouts);
+    D.tr->peer_table(D.queries, qouts);
     launches += dist_chase_ask_count(D.pend_key[cur], bound, D.n_pend, D.roff_dev, nr, D.tile_cnt, D.d_small + W_CNT_A, st);
-    CK(cudaMemcpyAsync(D.d_small + W_ERR, &D.cnt->err, sizeof(u32), cudaMemcpyDeviceToDevice, st));
-    TR(D.tr->gather_small_begin(D.d_small, D.d_small_all, D.h_small, st));
-    launches += dist_chase_ask_push(D.pend_key[cur], bound, D.n_pend, D.roff_dev, nr, qouts, (u32)D.cap, D.apos, D.tile_cnt, D.d_small_all,
-                                    SMALL_WORDS, me, st);
-    TR(D.tr->barrier(st));
-    TR(D.tr->gather_small_end(D.d_small_all, D.h_small, st));
+    if (const int rc = dist_gather_counts(ctx, [&] {
+          launches += dist_chase_ask_push(D.pend_key[cur], bound, D.n_pend, D.roff_dev, nr, qouts, (u32)D.cap, D.apos, D.tile_cnt,
+                                          D.d_small_all, SMALL_WORDS, me, st);
+        }))
+      return rc;
+    if (const int rc = check_inbound(ctx, W_CNT_A, D.cap, "rank %d is asked about %llu chain ends, capacity is %llu rows per rank")) return rc;
     Exchange exq;
     exq.from_matrix(D.h_small, W_CNT_A, nr, me);
-    for (int d = 0; d < nr; ++d) {
-      const u64 in = column_sum(D.h_small, W_CNT_A + d, nr);
-      if (in > D.cap) return fail(ctx, RK_ERR_NOMEM, "rank %d is asked about %llu chain ends, capacity is %llu rows per rank", d,
-                                  (unsigned long long)in, (unsigned long long)D.cap);
-    }
     D.tr->bytes_sent += (exq.n_send - exq.scnt[me]) * 16 + (exq.n_recv - exq.rcnt[me]) * 8;
     // answer: every owner returns its res[] words, block by block, into the asking ranks' answer buffers
     launches += dist_chase_answer(D.queries, (u32)exq.n_recv, D.res, D.rank_off, scatter_table(D, exq, true, D.answers), st);
@@ -1005,8 +1004,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
     CK(cudaMemcpyAsync(D.n_pend, D.n_pend + 1, sizeof(u32), cudaMemcpyDeviceToDevice, st));
     cur ^= 1;
     CK(cudaMemcpyAsync(D.d_small + W_X2, D.n_pend, sizeof(u32), cudaMemcpyDeviceToDevice, st));
-    const int rc = dist_gather_counts(ctx);  // how many chains are still open, everywhere
-    if (rc) return rc;
+    if (const int rc = dist_gather_counts(ctx)) return rc;  // how many chains are still open, everywhere
   }
   launches += dist_chase_finish(D.pt, nroots, SMALL_WORDS, m, D.res, D.lroot, D.pend_idx[cur], D.pend_key[cur], D.n_pend, D.gid_l, D.gid_rank, st);
   // (no second barrier: the count exchange of the output stage below completes on a rank only after every rank has
@@ -1015,7 +1013,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   // output exchange: to the owner of the group-id range.  The ranges are cut for about equal sort_groups WORK: lines, with
   // the lines of groups with several members weighted up (groups founded early are the large ones: equal numbers of
   // groups gave rank 0 far more lines, equal numbers of lines still far more work — see k_cuts_from_hist).
-  const int bits_gid = ceil_log2(D.m_total) < 1 ? 1 : ceil_log2(D.m_total);  // group ids are < number of fragments
+  const int bits_gid = key_bits(D.m_total);  // group ids are < number of fragments
   const int shift_g = bits_gid > 12 ? bits_gid - 12 : 0;
   launches += dist_cuts_gid(nroots, SMALL_WORDS, nr, D.cuts_g, D.d_small + W_X1, st);  // (the total; the cuts are replaced below)
   launches += dist_coarse_hist(D.gid_rank, m, shift_g, 0, 0xFFFFFFFFu, D.hist, st);
@@ -1025,43 +1023,31 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   launches += dist_cuts_from_hist(D.hist_all, DIST_BINS, nr, shift_g, D.cuts_g, st, D.d_small + W_X1, line_cap);
   CK(cudaMemcpyAsync(D.d_small + W_CNT_B, D.cuts_g, (nr + 1) * sizeof(u32), cudaMemcpyDeviceToDevice, st));
   uint4 *outs[DIST_MAX_RANKS];
-  peer_rows(D, D.recv_rows, outs);
+  D.tr->peer_table(D.recv_rows, outs);
   launches += dist_count_plain(D.gid_rank, m, D.cuts_g, nr, 0xFFFFFFFFu, D.tile_cnt, D.d_small + W_CNT_A, st);
-  CK(cudaMemcpyAsync(D.d_small + W_ERR, &D.cnt->err, sizeof(u32), cudaMemcpyDeviceToDevice, st));
-  TR(D.tr->gather_small_begin(D.d_small, D.d_small_all, D.h_small, st));
-  launches += dist_push_gid(D.gid_rank, D.hfi_r, m, D.cuts_g, nr, outs, (u32)D.cap, D.tile_cnt, D.d_small_all, SMALL_WORDS, me, st);
-  TR(D.tr->barrier(st));
-  TR(D.tr->gather_small_end(D.d_small_all, D.h_small, st));  // host sync 3
-  {
-    const int rc2 = dist_check_small(ctx, false);
-    if (rc2) return rc2;
-  }
+  if (const int rc = dist_gather_counts(ctx, [&] {  // host sync 3
+        launches += dist_push_gid(D.gid_rank, D.hfi_r, m, D.cuts_g, nr, outs, (u32)D.cap, D.tile_cnt, D.d_small_all, SMALL_WORDS, me, st);
+      }))
+    return rc;
+  if (const int rc = dist_check_small(ctx, false)) return rc;
+  if (const int rc = check_inbound(ctx, W_CNT_A, D.cap, "rank %d would own %llu output lines, capacity is %llu rows per rank")) return rc;
   Exchange exg;
   exg.from_matrix(D.h_small, W_CNT_A, nr, me);
   D.tr->bytes_sent += (exg.n_send - exg.scnt[me]) * 16;
   const u64 total_groups = D.h_small[(size_t)me * SMALL_WORDS + W_X1];
   u64 line_off = 0;
-  for (int d = 0; d < nr; ++d) {
-    const u64 in = column_sum(D.h_small, W_CNT_A + d, nr);
-    if (in > D.cap) return fail(ctx, RK_ERR_NOMEM, "rank %d would own %llu output lines, capacity is %llu rows per rank", d,
-                                (unsigned long long)in, (unsigned long long)D.cap);
-    if (d < me) line_off += in;
-  }
+  for (int d = 0; d < me; ++d) line_off += column_sum(D.h_small, W_CNT_A + d, nr);
   const u32 mg = (u32)exg.n_recv;
-  const u32 *cuts_h = D.h_small + (size_t)me * SMALL_WORDS + W_CNT_B;
-  const u32 gid_base = cuts_h[me];
-  const u64 gid_end = (u64)cuts_h[me + 1] < total_groups ? (u64)cuts_h[me + 1] : total_groups;
-  const u64 local_groups = gid_end > gid_base ? gid_end - gid_base : 1;
-  const int bits_g = ceil_log2(local_groups) < 1 ? 1 : ceil_log2(local_groups);
+  const KeyRange gr = rank_key_range(D.h_small + (size_t)me * SMALL_WORDS + W_CNT_B, me, nr, total_groups);
   CK(cudaMemsetAsync(D.prehist + 3072, 0, 4 * 256 * 4, st));
-  launches += dist_gid_keys(D.recv_rows, mg, gid_base, D.gid_a, HistOut{D.prehist + 3072, (bits_g + 7) / 8, bits_g}, st);
+  launches += dist_gid_keys(D.recv_rows, mg, gr.base, D.gid_a, HistOut{D.prehist + 3072, (gr.bits + 7) / 8, gr.bits}, st);
   CK(cudaEventRecord(ev[4], st));
   // members arrive in processing order (sources in rank order): a stable sort by group id is push_back order
-  launches += launch_sort_pairs(D.gid_a, nullptr, D.sgid, D.srank_g, D.tmp_k, D.tmp_v, mg, bits_g, D.sort_work, st, &D.cnt->err,
+  launches += launch_sort_pairs(D.gid_a, nullptr, D.sgid, D.srank_g, D.tmp_k, D.tmp_v, mg, gr.bits, D.sort_work, st, &D.cnt->err,
                                 mg ? D.prehist + 3072 : nullptr);
   OrderArgs oa{};
   oa.sgid = D.sgid, oa.srank = D.srank_g, oa.hfi_r = D.recv_rows;
-  oa.m = mg, oa.do_sort = (flags & RK_F_NO_SORT) ? 0 : 1, oa.gid_base = gid_base;
+  oa.m = mg, oa.do_sort = (flags & RK_F_NO_SORT) ? 0 : 1, oa.gid_base = gr.base;
   order_carve(oa, D.order_scratch, D.cap);
   oa.work_count = D.cnt->work_g;
   oa.out_order = D.out_order, oa.out_gid = D.out_gid, oa.out_repval = D.out_repval, oa.out_identity = D.out_identity;
@@ -1075,20 +1061,15 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   if (line_records) {
     CK(cudaMemcpyAsync(D.cuts_g, D.file_off, nr * sizeof(u32), cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
     uint4 *qouts[DIST_MAX_RANKS];
-    peer_rows(D, D.queries, qouts);
+    D.tr->peer_table(D.queries, qouts);
     launches += dist_count_plain(D.out_order, mg, D.cuts_g, nr, 0xFFFFFFFFu, D.tile_cnt, D.d_small + W_CNT_A, st);
-    CK(cudaMemcpyAsync(D.d_small + W_ERR, &D.cnt->err, sizeof(u32), cudaMemcpyDeviceToDevice, st));
-    TR(D.tr->gather_small_begin(D.d_small, D.d_small_all, D.h_small, st));
-    launches += dist_line_ask_push(D.out_order, mg, D.cuts_g, nr, qouts, (u32)D.cap, D.tile_cnt, D.d_small_all, SMALL_WORDS, me, st);
-    TR(D.tr->barrier(st));
-    TR(D.tr->gather_small_end(D.d_small_all, D.h_small, st));  // host sync 4
-    const int rc2 = dist_check_small(ctx, false);
-    if (rc2) return rc2;
-    for (int d = 0; d < nr; ++d) {  // (a rank is asked only about the records of its slice, which fits its rows)
-      const u64 in = column_sum(D.h_small, W_CNT_A + d, nr);
-      if (in > D.cap) return fail(ctx, RK_ERR_NOMEM, "rank %d is asked for %llu line records, capacity is %llu rows per rank", d,
-                                  (unsigned long long)in, (unsigned long long)D.cap);
-    }
+    if (const int rc = dist_gather_counts(ctx, [&] {  // host sync 4
+          launches += dist_line_ask_push(D.out_order, mg, D.cuts_g, nr, qouts, (u32)D.cap, D.tile_cnt, D.d_small_all, SMALL_WORDS, me, st);
+        }))
+      return rc;
+    if (const int rc = dist_check_small(ctx, false)) return rc;
+    // (a rank is asked only about the records of its slice, which fits its rows)
+    if (const int rc = check_inbound(ctx, W_CNT_A, D.cap, "rank %d is asked for %llu line records, capacity is %llu rows per rank")) return rc;
     Exchange exl;
     exl.from_matrix(D.h_small, W_CNT_A, nr, me);
     D.tr->bytes_sent += (exl.n_send - exl.scnt[me]) * 16 + (exl.n_recv - exl.rcnt[me]) * sizeof(LineRow);
@@ -1123,8 +1104,8 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
     D.trace.dump(me, cb);
   }
   D.n_lines = mg, D.line_off = line_off;
-  D.gid_base = (u32)std::min<u64>(gid_base, total_groups);
-  D.n_groups_rank = (u32)(gid_end > D.gid_base ? gid_end - D.gid_base : 0);
+  D.gid_base = (u32)std::min<u64>(gr.base, total_groups);
+  D.n_groups_rank = (u32)(gr.end > D.gid_base ? gr.end - D.gid_base : 0);
   D.have_rows = line_records;
 
   out->n_kept = mg;
@@ -1157,10 +1138,6 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
     info->bytes_sent = D.tr->bytes_sent - sent0;
   }
   return RK_OK;
-}
-
-static void peer_rows(const Dist &D, uint4 *local, uint4 **outs) {
-  for (int d = 0; d < D.world; ++d) outs[d] = d == D.rank ? local : D.tr->on_peer(d, local);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -1201,7 +1178,6 @@ void dist_destroy(rk_ctx *c) {
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->stream);
   dist_release_buffers(*D);
-  if (D->h_small) cudaFreeHost(D->h_small);
   if (D->side) cudaStreamSynchronize(D->side), cudaStreamDestroy(D->side);
   delete D->tr;
   delete D;
@@ -1278,7 +1254,7 @@ int rk_dist_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_
   u64 nbytes = 0;
   char *buf = nullptr;
   int rc = dist_format_device(ctx, first_line, n_lines, &nbytes);
-  if (!rc) rc = format_text_buffer(ctx, nbytes, &buf);
+  if (!rc) rc = ctx->h_text.next(nbytes, &buf, ctx->err);
   if (!rc) rc = format_to_host(ctx, nbytes, buf, &out->ms_device);
   if (rc) return rc;
   out->text = buf;
@@ -1320,10 +1296,8 @@ struct rk_multi {
   // merged host result of the last rk_multi_group
   GrowBuffer h_res{cudaHostAllocDefault};
   std::vector<rk_dist_info> infos;
-  // rk_multi_format_lines: two alternating pinned text buffers; rk_multi_group_statistics: all groups (pinned, portable:
-  // copied into by every GPU)
-  GrowBuffer h_text[2] = {GrowBuffer(cudaHostAllocPortable), GrowBuffer(cudaHostAllocPortable)};
-  int h_text_next = 0;
+  // rk_multi_format_lines' text and rk_multi_group_statistics' groups (pinned, portable: copied into by every GPU)
+  TextBuffers h_text{cudaHostAllocPortable};
   GrowBuffer h_stats{cudaHostAllocPortable};
 };
 
@@ -1526,11 +1500,9 @@ int rk_multi_format_lines(rk_multi *mg, uint64_t first_line, uint64_t n_lines, r
   // ... and copies it to its place in one buffer: the parts in rank order are the lines in order
   for (int r = 0; r < mg->n; ++r) pos[r + 1] = pos[r] + nb[r];
   const u64 nbytes = pos[mg->n];
-  GrowBuffer &hb = mg->h_text[mg->h_text_next];
-  mg->h_text_next ^= 1;
-  rc = hb.reserve(nbytes + 1 > hb.cap() ? align_up(nbytes + nbytes / 8 + 4096, 4096) : nbytes + 1, nullptr, mg->err);
+  char *buf = nullptr;
+  rc = mg->h_text.next(nbytes, &buf, mg->err);
   if (rc) return rc;
-  char *buf = (char *)hb.ptr();
   rc = run_ranks(mg, [&](int r) { return format_to_host(mg->ctx[r], nb[r], buf + pos[r], &ms[r]); });
   if (rc) return rc;
   out->text = buf;

@@ -22,28 +22,37 @@ inline int ceil_log2(u64 x) {  // bits needed to represent values 0 .. x-1
   return b;
 }
 
+// radix bits of a sort key over `range` values: at least 1 (the sort makes at least one pass)
+inline int key_bits(u64 range) { return ceil_log2(range) < 1 ? 1 : ceil_log2(range); }
+
+// timing events, recycled: put() returns one for a later get()
+struct EventPool {
+  std::vector<cudaEvent_t> free;
+  cudaEvent_t get() {
+    if (!free.empty()) { cudaEvent_t e = free.back(); free.pop_back(); return e; }
+    cudaEvent_t e;
+    cudaEventCreate(&e);
+    return e;
+  }
+  void put(cudaEvent_t e) { free.push_back(e); }
+};
+
 // CUDA-event pair around every launch group; folded into per-kernel totals after each synchronisation
 struct Profiler {
   bool on = false;
   struct Rec { int kid; cudaEvent_t a, b; u64 units; };
   std::vector<Rec> open_recs;
-  std::vector<cudaEvent_t> pool;
+  EventPool pool;
   double ms[KID_COUNT] = {0};
   u64 launches[KID_COUNT] = {0};
   u64 units[KID_COUNT] = {0};
-  cudaEvent_t get() {
-    if (!pool.empty()) { cudaEvent_t e = pool.back(); pool.pop_back(); return e; }
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    return e;
-  }
   void fold() {  // call after the stream was synchronised
     for (auto &r : open_recs) {
       float t = 0.f;
       if (cudaEventElapsedTime(&t, r.a, r.b) == cudaSuccess) { ms[r.kid] += t; launches[r.kid] += 1; units[r.kid] += r.units; }
       else cudaGetLastError();
-      pool.push_back(r.a);
-      pool.push_back(r.b);
+      pool.put(r.a);
+      pool.put(r.b);
     }
     open_recs.clear();
   }
@@ -112,6 +121,24 @@ class GrowBuffer {
   unsigned flags_ = 0;
 };
 
+// Two pinned text buffers handed out in turn, so that a chunk of text stays valid while the next one is produced.
+// next() grows the other buffer to hold nbytes + 1, with headroom when it has to grow.
+class TextBuffers {
+ public:
+  explicit TextBuffers(unsigned host_flags) : b_{GrowBuffer(host_flags), GrowBuffer(host_flags)} {}
+  int next(u64 nbytes, char **buf, std::string &err) {
+    GrowBuffer &b = b_[next_];
+    next_ ^= 1;
+    const int rc = b.reserve(nbytes + 1 > b.cap() ? align_up(nbytes + nbytes / 8 + 4096, 4096) : nbytes + 1, nullptr, err);
+    *buf = (char *)b.ptr();
+    return rc;
+  }
+
+ private:
+  GrowBuffer b_[2];
+  int next_ = 0;
+};
+
 // The pinned host arrays of RK_F_HOST_RESULT for m lines, carved from one buffer of bytes(m) at 256-byte boundaries
 struct HostResult {
   static u64 bytes(u64 m) { return 3 * align_up(m * 4, 256) + align_up(m, 256); }
@@ -142,8 +169,8 @@ struct LinkWords { u64 x, y; };
 inline LinkWords link_map_words(const Geometry &g) { return {(2ull * g.nbx + 31) / 32 + 1, (2ull * g.nby + 31) / 32 + 1}; }
 struct SortBits { int rank, x, y; };
 inline SortBits sort_key_bits(const Geometry &g) {
-  return {ceil_log2(g.vsize) < 1 ? 1 : ceil_log2(g.vsize),  // (the sort clamps to >= 1 bit as well)
-          ceil_log2(2ull * g.nbx),                          // >= 2: nbx >= 2
+  return {key_bits(g.vsize),
+          ceil_log2(2ull * g.nbx),  // >= 2: nbx >= 2
           ceil_log2(2ull * g.nby)};
 }
 
@@ -221,9 +248,7 @@ struct rk_ctx {
 
   // K6 text output: device text + work area, pinned host mirror
   rk::GrowBuffer d_text;
-  // alternating: a chunk stays valid while the next one is produced
-  rk::GrowBuffer h_text[2] = {rk::GrowBuffer(cudaHostAllocDefault), rk::GrowBuffer(cudaHostAllocDefault)};
-  int h_text_next = 0;
+  rk::TextBuffers h_text{cudaHostAllocDefault};
 
   // K8 per-group statistics: device array + pinned host mirror
   rk::GrowBuffer d_stats, h_stats{cudaHostAllocDefault};
@@ -290,8 +315,6 @@ void dist_destroy(rk_ctx *c);  // multi.cu: releases c->dist (called by rk_destr
 // capi.cu: the work behind rk_format_lines / rk_group_statistics, shared with their partitioned forms (multi.cu).
 // K6 into the context's device text buffer (records ev[0]); *nbytes = the bytes formatted.  Synchronises.
 int format_on_device(rk_ctx *ctx, FormatArgs fa, u64 *nbytes);
-// the next of the context's two alternating pinned text buffers, grown to hold nbytes
-int format_text_buffer(rk_ctx *ctx, u64 nbytes, char **buf);
 // the formatted text to dst (pinned host memory); *ms_device = ev[0] .. the end of the copy.  Synchronises.
 int format_to_host(rk_ctx *ctx, u64 nbytes, char *dst, float *ms_device);
 // K8 into ctx->d_stats (and ctx->h_stats with RK_F_HOST_RESULT); see launch_group_stats.  Synchronises.
