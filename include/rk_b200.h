@@ -41,7 +41,7 @@ typedef enum {
                                 the line, for rk_dist_format_lines / rk_dist_group_statistics (rk_group ignores it) */
 
 enum { /* stage indices of ms_stage[] */
-  RK_ST_H2D = 0,     /* host -> device copy of the records (0 when the input was a device pointer) */
+  RK_ST_H2D = 0,     /* host -> device copy of the records or of rk_load_csv's text (0 for a device pointer) */
   RK_ST_DECODE,      /* K1  AoS -> SoA decode + validity + link bits                                  */
   RK_ST_RANKSORT,    /* K2a stable LSD radix sort by xStart/10                                        */
   RK_ST_KEYS,        /* K2  rank-order SoA gather + super-bucket keys                                  */
@@ -136,6 +136,28 @@ int rk_load_aos(rk_ctx *ctx, const void *frags, uint64_t n, uint64_t seqx_len, u
 int rk_load_packed(rk_ctx *ctx, const uint32_t *key4, const uint8_t *strand, const uint32_t *rest4, uint64_t n, uint64_t seqx_len,
                    uint64_t seqy_len, unsigned flags, rk_load_stats *stats);
 
+/* Replaces FragmentsDatabase::FragmentsDatabase from the text on (src/FragmentsDatabase.cpp:91-100): takes the body of a
+ * GECKO CSV (the bytes after its 16 header lines) in host memory of any kind or in device memory, splits it into rows on
+ * '\n' as std::getline does, applies readFragment's rules (src/FragmentsDatabase.cpp:17-50) to every row on the device, and
+ * loads the accepted rows in file order: the database rk_load_packed (or rk_load_aos, when a value needs 33 or more bits)
+ * builds from the host parser's records.  A row whose tokens leave the plain grammar (digits; digits[.digits] for the
+ * similarity: signs, blanks, exponents, 19+ digits, a float on a rounding midpoint, ...) is parsed by the host parser
+ * inside this call; only such rows' bytes come back from a device body.  seqx_len/seqy_len are the LOADED lengths
+ * (header value + 1); total_frags is the header's "Total fragments": more accepted rows than that return RK_ERR_RANGE
+ * ("Unexpected number of fragments", src/FragmentsDatabase.cpp:99) and leave nothing loaded.  The parsed arrays belong
+ * to the context's database, so body may be freed when the call returns.  A body larger than the device's free memory
+ * returns RK_ERR_NOMEM.  ms_stage[RK_ST_H2D] of stats is the text upload.  csv may be NULL.  Synchronous. */
+typedef struct {
+  uint64_t n_rows;       /* rows of the body, the empty one after a final '\n' included */
+  uint64_t n_accepted;   /* records loaded (= rk_load_stats.n_loaded) */
+  uint64_t n_host_rows;  /* rows outside the plain grammar, decided by the host parser */
+  int wide;              /* 1: a value needs 33 or more bits; the records were loaded as 109-byte records */
+  float ms_upload;       /* host -> device copy of the text (0 for a device body) */
+  float ms_parse;        /* row split, parse, host rows and compaction on the device */
+} rk_csv_stats;
+int rk_load_csv(rk_ctx *ctx, const char *body, uint64_t bytes, uint64_t seqx_len, uint64_t seqy_len, uint64_t total_frags,
+                unsigned flags, rk_load_stats *stats, rk_csv_stats *csv);
+
 /* Replaces generate_fragment_groups + generate_diagonal_func + sort_groups
  * (src/commonFunctions.cpp:41-80,161-177,148-159; call sites src/repkiller.cpp:84-91) for one
  * (len_ratio, pos_ratio) pair.  Both ratios must be > 0 (src/commonFunctions.cpp:26-27).  Synchronous. */
@@ -201,8 +223,9 @@ void rk_host_free(void *p);
 int rk_diagonal_func(rk_ctx *ctx, uint64_t *diag_func);
 
 /* Test/diagnostic access to intermediate device arrays of the last load/group, copied to `host` (capacity
- * `bytes`).  Names: "rank_fidx", "parent", "gid_rank", "hkey".  Returns the number of bytes the array has, or
- * a negative rk_status. */
+ * `bytes`).  Names: "rank_fidx", "parent", "gid_rank", "hkey", and the loaded compact arrays of a load that has them
+ * (rk_load_packed, rk_load_csv without wide values): "key4" (n_loaded x 4 uint32), "strand" (n_loaded bytes), "rest4"
+ * (n_loaded x 4 uint32).  Returns the number of bytes the array has, or a negative rk_status. */
 int64_t rk_debug_fetch(rk_ctx *ctx, const char *name, void *host, uint64_t bytes);
 
 /* Per-kernel device time: when enabled, every kernel launch of later calls on this context is bracketed by a

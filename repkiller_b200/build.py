@@ -60,7 +60,7 @@ def build_host(force: bool = False) -> str | None:
     mains = sorted(glob.glob(os.path.join(CSRC, "host", "main", "*.cpp")))
     if not mains:
         return None
-    deps = common + mains + glob.glob(os.path.join(CSRC, "host", "*.h")) + [LIB]
+    deps = common + mains + glob.glob(os.path.join(CSRC, "host", "*.h")) + [os.path.join(CSRC, "rk_csv_row.cuh"), LIB]  # (the row rules)
     os.makedirs(os.path.dirname(CLI), exist_ok=True)
     for m in mains:
         exe = os.path.join(os.path.dirname(CLI), os.path.basename(m)[:-4])

@@ -21,7 +21,7 @@ STAGES = ["h2d", "decode", "ranksort", "keys", "xsort", "ysort", "xmatch", "ymat
 NSTAGES = len(STAGES)
 
 # every symbol include/rk_b200.h declares
-SYMBOLS = ["rk_create", "rk_create_view", "rk_create_error", "rk_destroy", "rk_last_error", "rk_set_stream", "rk_load_aos", "rk_load_packed", "rk_group", "rk_sort_groups", "rk_host_alloc", "rk_host_free",
+SYMBOLS = ["rk_create", "rk_create_view", "rk_create_error", "rk_destroy", "rk_last_error", "rk_set_stream", "rk_load_aos", "rk_load_packed", "rk_load_csv", "rk_group", "rk_sort_groups", "rk_host_alloc", "rk_host_free",
            "rk_diagonal_func", "rk_format_lines", "rk_debug_fetch", "rk_profile_enable", "rk_profile_read", "rk_sort_pairs_work_bytes", "rk_sort_pairs", "rk_version",
            "rk_gen_workload", "rk_sort_members", "rk_group_statistics", "rk_sol_create", "rk_sol_destroy", "rk_sol_insert", "rk_sol_get_associated", "rk_sol_last_error",
            # one comparison over several GPUs
@@ -43,6 +43,11 @@ class RkError(RuntimeError):
 class _LoadStats(C.Structure):
     _fields_ = [("n_loaded", C.c_uint64), ("n_kept", C.c_uint64), ("vsize", C.c_uint64),
                 ("ms_stage", C.c_float * NSTAGES), ("ms_device", C.c_float), ("n_launches", C.c_uint64)]
+
+
+class _CsvStats(C.Structure):
+    _fields_ = [("n_rows", C.c_uint64), ("n_accepted", C.c_uint64), ("n_host_rows", C.c_uint64), ("wide", C.c_int),
+                ("ms_upload", C.c_float), ("ms_parse", C.c_float)]
 
 
 class _KernelTime(C.Structure):
@@ -89,6 +94,8 @@ def load_library():
     L.rk_set_stream.argtypes = [C.c_void_p, C.c_void_p]
     L.rk_load_aos.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint, C.POINTER(_LoadStats)]
     L.rk_load_packed.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint, C.POINTER(_LoadStats)]
+    L.rk_load_csv.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint, C.POINTER(_LoadStats),
+                              C.POINTER(_CsvStats)]
     L.rk_group.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_uint, C.POINTER(_Result)]
     L.rk_diagonal_func.argtypes = [C.c_void_p, C.c_void_p]
     L.rk_debug_fetch.argtypes = [C.c_void_p, C.c_char_p, C.c_void_p, C.c_uint64]
@@ -152,6 +159,18 @@ class LoadStats:
     ms_stage: dict
     ms_device: float
     n_launches: int = 0
+
+
+@dataclass
+class CsvStats:
+    """what rk_load_csv saw in the text: rows (the empty one after a final newline included), records loaded, rows left
+    to the host parser, whether the 109-byte route was taken, and the device times of the upload and the parse"""
+    n_rows: int
+    n_accepted: int
+    n_host_rows: int
+    wide: bool
+    ms_upload: float
+    ms_parse: float
 
 
 @dataclass
@@ -255,6 +274,30 @@ class Context:
         return LoadStats(st.n_loaded, st.n_kept, st.vsize, {STAGES[i]: st.ms_stage[i] for i in range(NSTAGES)}, st.ms_device,
                          st.n_launches)
 
+    def load_csv(self, body, seqx_len: int, seqy_len: int, total_frags: int, timing: bool = True):
+        """The body of a GECKO CSV (the bytes after its 16 header lines) parsed and loaded on the device (rk_load_csv):
+        bytes, a uint8 numpy array, or a uint8 torch tensor on the CPU or on this context's GPU.  seqx_len/seqy_len are the
+        LOADED lengths (header value + 1), total_frags the header's "Total fragments".  Returns (LoadStats, CsvStats)."""
+        if isinstance(body, (bytes, bytearray)):
+            arr = np.frombuffer(bytes(body), dtype=np.uint8)
+            ptr, n = arr.ctypes.data, arr.nbytes
+        elif isinstance(body, np.ndarray):
+            arr = np.ascontiguousarray(body).view(np.uint8)
+            ptr, n = arr.ctypes.data, arr.nbytes
+        elif type(body).__module__.startswith("torch"):
+            arr = body.contiguous()
+            assert arr.element_size() == 1
+            ptr, n = arr.data_ptr(), arr.numel()
+        else:
+            raise TypeError("load_csv takes bytes, a uint8 numpy array or a uint8 torch tensor")
+        st, cs = _LoadStats(), _CsvStats()
+        self._check(self._L.rk_load_csv(self._h, C.c_void_p(ptr) if n else None, n, seqx_len, seqy_len, total_frags,
+                                        F_TIMING if timing else 0, C.byref(st), C.byref(cs)))
+        self._keep = None  # the parsed rows are the database's own: the text may go
+        return (LoadStats(st.n_loaded, st.n_kept, st.vsize, {STAGES[i]: st.ms_stage[i] for i in range(NSTAGES)}, st.ms_device,
+                          st.n_launches),
+                CsvStats(cs.n_rows, cs.n_accepted, cs.n_host_rows, bool(cs.wide), cs.ms_upload, cs.ms_parse))
+
     def group(self, len_ratio: float, pos_ratio: float, host_result: bool = True, sort: bool = True, timing: bool = True,
               copy: bool = True) -> Groups:
         """copy=False: the host arrays are views of the library-owned pinned result buffers (what a C caller gets);
@@ -308,11 +351,13 @@ class Context:
             self._check(self._L.rk_diagonal_func(self._h, C.c_void_p(out.ctypes.data)))
         return out
 
-    def debug_fetch(self, name: str) -> np.ndarray:
+    def debug_fetch(self, name: str, dtype=np.uint32) -> np.ndarray:
+        """a device array of the last load/group (rk_debug_fetch); "strand" is bytes (dtype=np.uint8), "key4" and "rest4"
+        four uint32 per record"""
         sz = self._L.rk_debug_fetch(self._h, name.encode(), None, 0)
         if sz < 0:
             self._check(int(sz))
-        out = np.zeros(sz // 4, dtype=np.uint32)
+        out = np.zeros(sz // np.dtype(dtype).itemsize, dtype=dtype)
         if sz:
             got = self._L.rk_debug_fetch(self._h, name.encode(), C.c_void_p(out.ctypes.data), out.nbytes)
             if got < 0:

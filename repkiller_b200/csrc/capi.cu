@@ -1,10 +1,13 @@
 // C ABI of librk_b200.so (include/rk_b200.h): context, device workspace, and the launch sequences that stand
 // in for FragmentsDatabase's constructor (rk_load_aos) and for generate_fragment_groups +
 // generate_diagonal_func + sort_groups (rk_group).  Reference call sites: /root/reference/src/repkiller.cpp:52,84-91.
+#include <algorithm>
+#include <atomic>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "rk_ctx.cuh"
@@ -24,7 +27,7 @@ void set_create_error(const std::string &s) {
 const char *const kKernelNames[KID_COUNT] = {"k_decode", "k_radix_hist", "k_scan", "k_radix_scatter", "k_keys", "k_match_small",
                                              "k_match_long", "k_chase", "k_hkey", "k_pack", "k_order_tile",
                                              "k_groupsort_large", "k_finalize", "k_diag_table", "k_groupsort_warp", "k_format", "k_dist_rows",
-                                             "k_group_stats", "k_chase_exits"};
+                                             "k_group_stats", "k_chase_exits", "k_csv_lines", "k_csv_rows"};
 
 thread_local Profiler *tl_prof = nullptr;
 
@@ -337,8 +340,8 @@ struct LoadSource {
 
 // FragmentsDatabase's constructor after parsing (src/FragmentsDatabase.cpp:84-100) on the device: K1, the processing
 // order (K2a), the occupation-list buckets of both axes (K2 keys, K2b/c) and generate_diagonal_func per fragment (K5a).
-int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_len, uint64_t seqy_len, unsigned flags, rk_load_stats *stats) {
-  if (n >= 0xFFFFFFF0ull) return fail(ctx, RK_ERR_ARG, "more than 2^32-16 records per context; partition the input");
+// the refusals of every load, before it touches the context
+int load_refusal(rk_ctx *ctx, uint64_t seqx_len, uint64_t seqy_len) {
   if (seqx_len >= (1ull << 32) || seqy_len >= (1ull << 32))
     return fail(ctx, RK_ERR_RANGE, "sequence length does not fit in 32 bits");
   if (ctx->is_view) return fail(ctx, RK_ERR_STATE, "a view groups the database of the context it was made from; load that context instead");
@@ -346,6 +349,12 @@ int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_le
   if (const int views = ctx->db->refs - 1)
     return fail(ctx, RK_ERR_STATE, "%d view%s of this context %s live: destroy %s before loading another database", views,
                 views == 1 ? "" : "s", views == 1 ? "is" : "are", views == 1 ? "it" : "them");
+  return RK_OK;
+}
+
+int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_len, uint64_t seqy_len, unsigned flags, rk_load_stats *stats) {
+  if (n >= 0xFFFFFFF0ull) return fail(ctx, RK_ERR_ARG, "more than 2^32-16 records per context; partition the input");
+  if (const int rc = load_refusal(ctx, seqx_len, seqy_len)) return rc;
   CK(cudaSetDevice(ctx->device));
   ProfGuard pg(ctx);
   ctx->loaded = false;
@@ -466,7 +475,213 @@ int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_le
   return RK_OK;
 }
 
+// rk_load_csv's events on ctx->ev, after the ones load_common records (0..7)
+enum { EV_CSV_UP0 = 8, EV_CSV_UP1, EV_CSV_PARSED };
+
+// The host text to the device through the context's pinned ring, CSV_CHUNK bytes at a time: up to CSV_RING_SLOTS / 2
+// threads each copy their chunks into their own two slots and queue the upload and the newline count of each chunk on
+// the context's stream, so that a chunk's host copy overlaps the uploads and counts queued before it.
+int csv_upload(rk_ctx *ctx, const char *body, u64 bytes, u8 *dst, u32 *tile_cnt) {
+  CsvScratch &cs = ctx->csv;
+  const u64 chunks = (bytes + CSV_CHUNK - 1) / CSV_CHUNK;
+  const u64 cores = std::max(1u, std::thread::hardware_concurrency() / 2);
+  const int workers = (int)std::min<u64>(std::min<u64>(CSV_RING_SLOTS / 2, cores), chunks);
+  const int rc = cs.ring.reserve((u64)2 * workers * CSV_CHUNK, ctx->stream, ctx->err);
+  if (rc) return rc;
+  for (cudaEvent_t &e : cs.slot_done)
+    if (!e) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  u8 *ring = (u8 *)cs.ring.ptr();
+  std::mutex mu;
+  cudaError_t first = cudaSuccess;
+  std::atomic<bool> failed{false};
+  auto work = [&](int w) {
+    cudaError_t e = cudaSetDevice(ctx->device);
+    for (u64 c = w, k = 0; c < chunks && e == cudaSuccess && !failed; c += workers, ++k) {
+      const int slot = 2 * w + (int)(k & 1);
+      const u64 off = c * CSV_CHUNK, len = std::min(CSV_CHUNK, bytes - off);
+      if (k >= 2) e = cudaEventSynchronize(cs.slot_done[slot]);  // the slot's previous upload is done
+      if (e != cudaSuccess) break;
+      memcpy(ring + slot * CSV_CHUNK, body + off, len);
+      e = cudaMemcpyAsync(dst + off, ring + slot * CSV_CHUNK, len, cudaMemcpyHostToDevice, ctx->stream);
+      if (e == cudaSuccess) e = cudaEventRecord(cs.slot_done[slot], ctx->stream);
+      if (e == cudaSuccess) launch_csv_count(dst, bytes, off / CSV_COUNT_TILE, csv_count_tiles(len), tile_cnt, ctx->stream);
+    }
+    if (e != cudaSuccess) {
+      std::lock_guard<std::mutex> lk(mu);
+      if (first == cudaSuccess) first = e;
+      failed = true;
+    }
+  };
+  std::vector<std::thread> pool;
+  for (int w = 1; w < workers; ++w) pool.emplace_back(work, w);
+  work(0);
+  for (auto &t : pool) t.join();
+  if (first != cudaSuccess) return fail(ctx, RK_ERR_CUDA, "rk_load_csv: text upload: %s", cudaGetErrorString(first));
+  return RK_OK;
+}
+
+// The rows the device left to the host parser: their bytes (from the caller's host text, or copied back from the device
+// text), readFragment on each, and the accepted ones as (row, 109-byte record).  Raises *wide for a wide record.
+int csv_host_rows(rk_ctx *ctx, const char *body, bool on_device, const u8 *text, const u32 *d_list, u32 n_host, const u64 *start,
+                  std::vector<u32> &rows, std::vector<u8> &recs, bool *wide) {
+  CsvScratch &cs = ctx->csv;
+  cudaStream_t st = ctx->stream;
+  std::vector<u32> list(n_host);
+  std::vector<ulonglong2> spans(n_host);
+  int rc = cs.host.reserve(align_up((u64)n_host * 16, 256) + align_up((u64)n_host * 8, 256), st, ctx->err);
+  if (rc) return rc;
+  ulonglong2 *d_spans = (ulonglong2 *)cs.host.ptr();
+  launch_csv_host_spans(d_list, n_host, start, d_spans, st);
+  CK(cudaMemcpyAsync(list.data(), d_list, (u64)n_host * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(spans.data(), d_spans, (u64)n_host * 16, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  std::vector<u64> off(n_host + 1, 0);
+  for (u32 i = 0; i < n_host; ++i) off[i + 1] = off[i] + (spans[i].y - spans[i].x);
+  std::vector<char> copied;
+  if (on_device) {  // only these rows' bytes come back
+    const u64 a = align_up((u64)n_host * 16, 256), b = align_up((u64)n_host * 8, 256);
+    rc = cs.host.reserve(a + b + off[n_host] + 16, st, ctx->err);
+    if (rc) return rc;
+    u8 *h = (u8 *)cs.host.ptr();
+    CK(cudaMemcpyAsync(h, spans.data(), (u64)n_host * 16, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h + a, off.data(), (u64)n_host * 8, cudaMemcpyHostToDevice, st));
+    launch_csv_gather(text, (const ulonglong2 *)h, (const u64 *)(h + a), n_host, h + a + b, st);
+    copied.resize(off[n_host] + 1);
+    CK(cudaMemcpyAsync(copied.data(), h + a + b, off[n_host], cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+  }
+  static const int kWideFields[7] = {OFF_XSTART, OFF_YSTART, OFF_LENGTH, OFF_IDENT, OFF_XEND, OFF_YEND, OFF_SCORE};
+  u8 rec[RK_FRAG_BYTES];
+  for (u32 i = 0; i < n_host; ++i) {
+    const char *line = on_device ? copied.data() + off[i] : body + spans[i].x;
+    if (!csv_read_row_host(line, spans[i].y - spans[i].x, rec)) continue;
+    rows.push_back(list[i]);
+    recs.insert(recs.end(), rec, rec + RK_FRAG_BYTES);
+    u64 any = 0;
+    for (int f : kWideFields) {
+      u64 v;
+      memcpy(&v, rec + f, 8);
+      any |= v;
+    }
+    if (any >> 32) *wide = true;  // the host route's test for the 109-byte load
+  }
+  return RK_OK;
+}
+
 }  // namespace
+
+extern "C" {
+
+int rk_load_csv(rk_ctx *ctx, const char *body, uint64_t bytes, uint64_t seqx_len, uint64_t seqy_len, uint64_t total_frags, unsigned flags,
+                rk_load_stats *stats, rk_csv_stats *csv) {
+  if (!ctx) return RK_ERR_ARG;
+  if (!body && bytes) return fail(ctx, RK_ERR_ARG, "null text pointer");
+  if (const int rc = load_refusal(ctx, seqx_len, seqy_len)) return rc;
+  CK(cudaSetDevice(ctx->device));
+  ctx->loaded = false;
+  ctx->have_group = false;
+  CsvScratch &cs = ctx->csv;
+  cudaStream_t st = ctx->stream;
+  cudaEvent_t *ev = ctx->ev;
+  const bool on_device = bytes && is_device_pointer(body);
+  const bool copy_text = !on_device || ((uintptr_t)body & 15);  // the kernels read the text 16 bytes at a time
+  u64 n_rows = 0, n_host = 0, n_acc = 0;
+  bool wide = false;
+  LoadSource src;
+  {
+    ProfGuard pg(ctx);
+    // the text scratch: [text][tile counts][their scan words][counters]
+    const u64 tiles = csv_count_tiles(bytes);
+    const u64 text_b = copy_text ? align_up(bytes + 16, 256) : 0, cnt_b = align_up((tiles + 1) * 4, 256),
+              scan_b = align_up(csv_scan_words(tiles) * 4, 256);
+    int rc = cs.text.reserve(text_b + cnt_b + scan_b + 256, st, ctx->err);
+    if (rc) {
+      const std::string e = ctx->err;
+      return fail(ctx, rc, "rk_load_csv: %llu bytes of text: %s", (unsigned long long)bytes, e.c_str());
+    }
+    u8 *tb = (u8 *)cs.text.ptr();
+    const u8 *text = copy_text ? tb : (const u8 *)body;
+    u32 *tile_cnt = (u32 *)(tb + text_b), *tile_bsum = (u32 *)(tb + text_b + cnt_b);
+    CsvCounters *cnt = (CsvCounters *)(tb + text_b + cnt_b + scan_b);
+    CsvCounters h{};
+    CK(cudaMemsetAsync(cnt, 0, sizeof(CsvCounters), st));
+    CK(cudaMemsetAsync(tile_cnt, 0, 4, st));
+    CK(cudaEventRecord(ev[EV_CSV_UP0], st));
+    if (!on_device) {
+      if (bytes && (rc = csv_upload(ctx, body, bytes, tb, tile_cnt))) return rc;
+    } else {
+      if (copy_text) CK(cudaMemcpyAsync(tb, body, bytes, cudaMemcpyDeviceToDevice, st));
+      launch_csv_count(text, bytes, 0, tiles, tile_cnt, st);
+    }
+    CK(cudaEventRecord(ev[EV_CSV_UP1], st));
+    launch_csv_tile_scan(tile_cnt, tiles, tile_bsum, cnt, st);
+    CK(cudaMemcpyAsync(&h, cnt, sizeof h, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+    n_rows = (u64)h.n_lines + 1;  // the segment after the last '\n' is a row too (empty after a final '\n')
+    if (n_rows >= 0xFFFFFFF0ull) return fail(ctx, RK_ERR_ARG, "more than 2^32-16 rows per context; partition the input");
+
+    // the row arrays: [start (n_rows + 1)][slot / host list (n_rows)][scan words][status (n_rows)]
+    const u64 start_b = align_up((n_rows + 1) * 8, 256), slot_b = align_up(n_rows * 4, 256), rscan_b = align_up(csv_scan_words(n_rows) * 4, 256);
+    rc = cs.rows.reserve(start_b + slot_b + rscan_b + align_up(n_rows, 256), st, ctx->err);
+    if (rc) return rc;
+    u8 *rb = (u8 *)cs.rows.ptr();
+    u64 *start = (u64 *)rb;
+    u32 *slot = (u32 *)(rb + start_b), *row_bsum = (u32 *)(rb + start_b + slot_b);
+    u8 *status = rb + start_b + slot_b + rscan_b;
+    launch_csv_starts(text, bytes, tile_cnt, start, n_rows, st);
+    launch_csv_classify(text, bytes, start, n_rows, status, slot, cnt, st);
+    CK(cudaMemcpyAsync(&h, cnt, sizeof h, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+    n_host = h.n_host;
+    wide = h.wide != 0;
+
+    std::vector<u32> host_rows;
+    std::vector<u8> host_recs;
+    if (n_host && (rc = csv_host_rows(ctx, body, on_device, text, slot, (u32)n_host, start, host_rows, host_recs, &wide))) return rc;
+    n_acc = (u64)h.n_accepted + host_rows.size();
+    if (n_acc > total_frags) return fail(ctx, RK_ERR_RANGE, "Unexpected number of fragments");  // FragmentsDatabase.cpp:99
+
+    // the host-accepted records, then the parsed rows at their slots in the database's own buffer
+    const u64 nh = host_rows.size(), hrows_b = align_up(nh * 4, 256);
+    if (nh) {
+      rc = cs.host.reserve(hrows_b + nh * RK_FRAG_BYTES, st, ctx->err);
+      if (rc) return rc;
+      CK(cudaMemcpyAsync(cs.host.ptr(), host_rows.data(), nh * 4, cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync((u8 *)cs.host.ptr() + hrows_b, host_recs.data(), nh * RK_FRAG_BYTES, cudaMemcpyHostToDevice, st));
+    }
+    const u64 key_b = align_up(n_acc * 16, 256);
+    rc = ctx->db->csv_out.reserve(wide ? align_up(n_acc * RK_FRAG_BYTES + 16, 256) : 2 * key_b + align_up(n_acc, 256), st, ctx->err);
+    if (rc) return rc;
+    u8 *ob = (u8 *)ctx->db->csv_out.ptr();
+    CsvOut o{};
+    if (wide) {
+      o.aos = ob;
+      src.aos = ob;
+    } else {
+      o.key4 = (uint4 *)ob, o.rest4 = (uint4 *)(ob + key_b), o.strand = ob + 2 * key_b;
+      src.key4 = o.key4, src.rest4 = o.rest4, src.strand = o.strand;
+    }
+    launch_csv_emit(text, bytes, start, n_rows, status, nh ? (const u32 *)cs.host.ptr() : nullptr, (u32)nh,
+                    nh ? (const u8 *)cs.host.ptr() + hrows_b : nullptr, slot, row_bsum, o, st);
+    CK(cudaEventRecord(ev[EV_CSV_PARSED], st));
+  }
+  const int rc = load_common(ctx, src, n_acc, seqx_len, seqy_len, flags, stats);
+  if (rc) return rc;
+  const float ms_up = ev_ms(ev[EV_CSV_UP0], ev[EV_CSV_UP1]), ms_parse = ev_ms(ev[EV_CSV_UP1], ev[EV_CSV_PARSED]);
+  if (stats && (flags & RK_F_TIMING)) stats->ms_stage[RK_ST_H2D] = on_device ? 0.f : ms_up;
+  if (csv) {
+    memset(csv, 0, sizeof *csv);
+    csv->n_rows = n_rows, csv->n_accepted = n_acc, csv->n_host_rows = n_host, csv->wide = wide;
+    csv->ms_upload = on_device ? 0.f : ms_up;
+    csv->ms_parse = ms_parse;
+  }
+  return RK_OK;
+}
+
+}  // extern "C"
 
 extern "C" {
 
@@ -669,7 +884,12 @@ int64_t rk_debug_fetch(rk_ctx *ctx, const char *name, void *host, uint64_t bytes
   const Database &db = *ctx->db;
   const void *src = nullptr;
   u64 sz = (u64)db.m * 4;
-  if (!strcmp(name, "rank_fidx")) src = db.fidx_r;
+  if (!strcmp(name, "key4") || !strcmp(name, "strand") || !strcmp(name, "rest4")) {  // the loaded compact arrays, file order
+    src = name[0] == 'k' ? (const void *)db.pk_key : name[0] == 'r' ? (const void *)db.pk_rest : (const void *)db.pk_strand;
+    if (!src) return fail(ctx, RK_ERR_STATE, "the load has no %s array (109-byte records, or rk_load_packed without rest4)", name);
+    sz = db.n * (name[0] == 's' ? 1 : 16);
+    if (name[0] == 'r' && db.side_copy) CK(cudaStreamWaitEvent(ctx->stream, db.copy_done, 0));
+  } else if (!strcmp(name, "rank_fidx")) src = db.fidx_r;
   else if (!strcmp(name, "k0_r")) src = db.k0_r;
   else if (!strcmp(name, "skx")) src = db.skx;
   else if (!strcmp(name, "rx")) src = db.rx;

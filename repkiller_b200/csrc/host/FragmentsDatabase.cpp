@@ -5,7 +5,6 @@
 #include <algorithm>
 #include <atomic>
 
-#include <cerrno>
 #include <chrono>
 #include <cstdlib>
 #include <cstring>
@@ -15,119 +14,7 @@
 #include <thread>
 #include <vector>
 
-// One CSV row -> record.  Semantics of the reference's readFragment (FragmentsDatabase.cpp:17-50), which
-// tokenises with 14 x getline(stream, buf, ','):
-//  * a token ends at ',' or at the end of the row; an EMPTY token rejects the row (:25);
-//  * once the row is exhausted the extraction fails and buf keeps the previous token, so a short row is
-//    padded with its last field ("Frag,5" loads with every numeric field 5 and strand '5');
-//  * a trailing ',' produces one empty token (row rejected);
-//  * field 0 must be "Frag" (:29); numeric fields through atoll; similarity AND ident from stof(field 10)
-//    (:39-40; field 9 is ignored); a row whose similarity does not parse is rejected (:46-48).
-namespace {
-// atoll / strtof are what the reference calls; the two helpers below return the same values for the plain tokens a GECKO
-// file is made of (all digits; digits[.digits]) without the copy, the locale machinery and the errno round trip, and
-// say "no" for everything else (signs, blanks, exponents, overlong tokens), which then takes the library call.
-inline bool plain_u64(const char *p, size_t n, uint64_t &v) {  // 1..18 digits: below 2^63, atoll returns the same
-  if (n == 0 || n > 18) return false;
-  uint64_t x = 0;
-  for (size_t i = 0; i < n; ++i) {
-    const unsigned c = (unsigned char)p[i] - '0';
-    if (c > 9) return false;
-    x = x * 10 + c;
-  }
-  v = x;
-  return true;
-}
-// digits[.digits] with an integer mantissa below 2^53 and at most 22 fraction digits: mantissa and power of ten are
-// exact doubles, their quotient is the correctly rounded double, and narrowing it gives the correctly rounded float
-// (what strtof returns) unless the double sits on the midpoint of two floats — then the library decides.
-inline bool plain_float(const char *p, size_t n, float &out) {
-  static const double P10[23] = {1e0,  1e1,  1e2,  1e3,  1e4,  1e5,  1e6,  1e7,  1e8,  1e9,  1e10, 1e11,
-                                 1e12, 1e13, 1e14, 1e15, 1e16, 1e17, 1e18, 1e19, 1e20, 1e21, 1e22};
-  uint64_t m = 0;
-  int digits = 0, frac = 0;
-  bool dot = false;
-  for (size_t i = 0; i < n; ++i) {
-    const unsigned c = (unsigned char)p[i] - '0';
-    if (c <= 9) {
-      if (++digits > 18) return false;
-      m = m * 10 + c;
-      frac += dot;
-    } else if (p[i] == '.' && !dot) {
-      dot = true;
-    } else {
-      return false;
-    }
-  }
-  if (digits == 0 || frac > 22 || m >= (1ull << 53)) return false;
-  const double d = (double)m / P10[frac];
-  uint64_t bits;
-  memcpy(&bits, &d, sizeof bits);
-  const uint32_t low = (uint32_t)(bits & 0x1FFFFFFFu);  // the 29 bits a float drops
-  if (low >= 0x0FFFFFFFu && low <= 0x10000001u) return false;
-  out = (float)d;
-  return true;
-}
-}  // namespace
-
-bool parse_plain_float(const char *p, size_t n, float *out) { return plain_float(p, n, *out); }
-
-bool readFragment(FragFile *frag, const char *line, size_t len) {
-  const char *tok[14];
-  size_t tlen[14];
-  size_t pos = 0;
-  bool exhausted = false;
-  const char *cur = nullptr;
-  size_t curlen = 0;
-  for (int i = 0; i < 14; ++i) {
-    if (!exhausted) {
-      const size_t s = pos;
-      while (pos < len && line[pos] != ',') ++pos;
-      cur = line + s;
-      curlen = pos - s;
-      if (pos < len) ++pos;
-      else exhausted = true;
-    }
-    if (curlen == 0) return false;
-    tok[i] = cur;
-    tlen[i] = curlen;
-  }
-  if (!(tlen[0] == 4 && memcmp(tok[0], "Frag", 4) == 0)) return false;
-  char buf[72];
-  auto cstr = [&](int i) -> const char * {
-    const size_t l = tlen[i] < 71 ? tlen[i] : 71;
-    memcpy(buf, tok[i], l);
-    buf[l] = 0;
-    return buf;
-  };
-  auto num = [&](int i) -> long long {
-    uint64_t v;
-    return plain_u64(tok[i], tlen[i], v) ? (long long)v : atoll(cstr(i));
-  };
-  frag->xStart = (uint64_t)num(1);
-  frag->yStart = (uint64_t)num(2);
-  frag->diag = (int64_t)frag->xStart - (int64_t)frag->yStart;
-  frag->xEnd = (uint64_t)num(3);
-  frag->yEnd = (uint64_t)num(4);
-  frag->strand = tok[5][0];
-  frag->block = num(6);
-  frag->length = (uint64_t)num(7);
-  frag->score = (uint64_t)num(8);
-  float sim;
-  if (!plain_float(tok[10], tlen[10], sim)) {
-    const char *s = cstr(10);
-    char *endp = nullptr;
-    errno = 0;
-    sim = strtof(s, &endp);  // std::stof: invalid_argument when nothing converts, out_of_range on ERANGE
-    if (endp == s || errno == ERANGE) return false;
-  }
-  frag->ident = (uint64_t)sim;
-  frag->similarity = sim;
-  frag->seqX = 0;
-  frag->seqY = 1;
-  memset(frag->evalue, 0, sizeof frag->evalue);
-  return true;
-}
+bool parse_plain_float(const char *p, size_t n, float *out) { return rk_csv::plain_float(p, n, *out); }
 
 namespace {
 long long value_after_colon(const std::string &line) {  // atoll(line.substr(line.find(':') + 1)), :62,65,72
@@ -284,6 +171,25 @@ FragsInput detect_frags_input(const std::string &path, std::ifstream &stream) {
   return (gecko_frags_layout_ok((size_t)(fin - here)) && first == 0) ? FragsInput::gecko_binary : FragsInput::csv;
 }
 
+void read_stream_rest(std::ifstream &in, FragsText &out) {
+  const std::streampos here = in.tellg();
+  in.seekg(0, std::ios::end);
+  const std::streampos fin = in.tellg();
+  if (here != std::streampos(-1) && fin != std::streampos(-1) && fin >= here) {
+    in.seekg(here);
+    const size_t want = (size_t)(fin - here);
+    out.raw.reset(new char[want + 1]);
+    in.read(out.raw.get(), (std::streamsize)want);
+    out.size = (size_t)in.gcount();
+    out.data = out.raw.get();
+  } else {  // not seekable
+    in.clear();
+    out.fallback.assign((std::istreambuf_iterator<char>(in)), std::istreambuf_iterator<char>());
+    out.data = out.fallback.data();
+    out.size = out.fallback.size();
+  }
+}
+
 FragmentsDatabase::FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, const std::vector<int> &devices,
                                      FragsInput input) {
   using clk = std::chrono::steady_clock;
@@ -298,28 +204,10 @@ FragmentsDatabase::FragmentsDatabase(std::ifstream &frags_file, sequence_manager
     ~Joiner() { if (t.joinable()) t.join(); }
   } create_joiner{create_thread};
   // slurp the rest of the stream in one read; lines are split on '\n' like std::getline
-  std::unique_ptr<char[]> raw;  // (not a std::string: resize() would zero-fill ~1 GB first)
-  std::string fallback;
-  const char *data = nullptr;
-  size_t size = 0;
-  {
-    const std::streampos here = frags_file.tellg();
-    frags_file.seekg(0, std::ios::end);
-    const std::streampos fin = frags_file.tellg();
-    if (here != std::streampos(-1) && fin != std::streampos(-1) && fin >= here) {
-      frags_file.seekg(here);
-      const size_t want = (size_t)(fin - here);
-      raw.reset(new char[want + 1]);
-      frags_file.read(raw.get(), (std::streamsize)want);
-      size = (size_t)frags_file.gcount();
-      data = raw.get();
-    } else {  // not seekable
-      frags_file.clear();
-      fallback.assign((std::istreambuf_iterator<char>(frags_file)), std::istreambuf_iterator<char>());
-      data = fallback.data();
-      size = fallback.size();
-    }
-  }
+  FragsText text;
+  read_stream_rest(frags_file, text);
+  const char *data = text.data;
+  const size_t size = text.size;
   const auto t1 = clk::now();
   const FragsHead head = read_frags_head(data, size, input);
   header = head.header;
@@ -404,6 +292,7 @@ FragmentsDatabase::FragmentsDatabase(std::ifstream &frags_file, sequence_manager
 // so iterating begin()..end() visits exactly the fragments, in exactly the order, that rk_group processes.
 void FragmentsDatabase::build_buckets() const {
   std::unique_ptr<std::vector<FragFile>[]> b(new std::vector<FragFile>[vsize]);
+  const FragFile *recs = records();
   const uint64_t kept = load_stats_.n_kept;
   std::vector<uint32_t> rank_fidx(kept ? kept : 1);
   if (kept) {
@@ -411,13 +300,36 @@ void FragmentsDatabase::build_buckets() const {
     if (got < 0) throw std::runtime_error(std::string("repkiller-b200: ") + rk_last_error(ctx_));
   }
   for (uint64_t i = 0; i < kept; ++i) {
-    const FragFile &f = records_[rank_fidx[i]];
+    const FragFile &f = recs[rank_fidx[i]];
     b[f.xStart / 10].push_back(f);
   }
   if (kept < count_)  // fragments of bucket getA()-1: loaded by the reference, never visited (FragmentsDatabase.h:29-31)
     for (uint64_t i = 0; i < count_; ++i)
-      if (records_[i].xStart / 10 == vsize - 1) b[vsize - 1].push_back(records_[i]);
+      if (recs[i].xStart / 10 == vsize - 1) b[vsize - 1].push_back(recs[i]);
   buckets_ = std::move(b);
+}
+
+// After rk_load_csv the host records come from the kept text, parsed by the host parser: the same records the device
+// loaded (both apply readFragment's rules), and the same bytes the host route's constructor holds.
+const FragFile *FragmentsDatabase::records() const {
+  std::call_once(records_once_, [this] {
+    if (!text_) return;
+    FragsHead head;
+    head.body_pos = body_pos_;
+    std::vector<std::vector<FragFile>> chunks = read_frags_records(text_->data, text_->size, head, 0);  // all cores
+    uint64_t accepted = 0;
+    for (const auto &c : chunks) accepted += c.size();
+    if (accepted != count_) throw std::runtime_error("repkiller-b200: the host parser accepted a different number of rows than the device");
+    records_ = (FragFile *)malloc((accepted ? accepted : 1) * sizeof(FragFile));
+    if (!records_) throw std::runtime_error("Could not allocate memory for fragments!");
+    uint64_t off = 0;
+    for (const auto &c : chunks) {
+      if (!c.empty()) memcpy(records_ + off, c.data(), c.size() * sizeof(FragFile));
+      off += c.size();
+    }
+    text_.reset();
+  });
+  return records_;
 }
 
 const std::vector<FragFile> *FragmentsDatabase::begin() const {

@@ -1,6 +1,7 @@
 // Drop-in for the reference's FragmentsDatabase (/root/reference/src/FragmentsDatabase.h:15-35): same
 // constructor and accessors, but the per-bucket vector<FragFile>[] is replaced by the records in file order
-// (pinned host memory) plus the device-side processing order built by rk_load_aos.
+// plus the device-side processing order built by the load (rk_load_packed / rk_load_aos after the host parser, or
+// rk_load_csv, which parses the rows on the device).
 #pragma once
 
 #include <cstdint>
@@ -10,10 +11,10 @@
 #include <string>
 #include <vector>
 
+#include "../rk_csv_row.cuh"  // readFragment (reference: FragmentsDatabase.cpp:17-50) and the number rules the device shares
 #include "rk_b200.h"
 #include "structs.h"
 
-bool readFragment(FragFile *frag, const char *line, size_t len);  // reference: FragmentsDatabase.cpp:17-50
 // the strtof fast path of readFragment (digits[.digits]): true and the correctly rounded float, or false = ask strtof
 bool parse_plain_float(const char *p, size_t n, float *out);
 // data rows of text[pos, size) parsed by nthreads threads; the accepted records of consecutive ranges, in file order
@@ -37,9 +38,20 @@ struct FragsHead {
 };
 FragsHead read_frags_head(const char *data, size_t size, FragsInput input);
 std::vector<std::vector<FragFile>> read_frags_records(const char *data, size_t size, const FragsHead &head, unsigned nthreads);
+// The rest of a stream in one buffer (not a std::string when the stream can seek: resize() would zero-fill ~1 GB first).
+struct FragsText {
+  std::unique_ptr<char[]> raw;
+  std::string fallback;  // a stream that cannot seek
+  const char *data = nullptr;
+  size_t size = 0;
+};
+void read_stream_rest(std::ifstream &in, FragsText &out);
+
+// Tag of the constructor that parses the CSV rows on the device (host/FragmentsDatabaseDeviceCsv.cpp, rk_load_csv).
+struct CsvOnDevice {};
 
 class FragmentsDatabase {
-  FragFile *records_ = nullptr;  // file order
+  mutable FragFile *records_ = nullptr;  // file order (built by records() on first use after rk_load_csv)
   unsigned char *packed_ = nullptr;  // pinned: the compact arrays handed to rk_load_packed
   uint64_t count_ = 0, cap_ = 0;
   size_t vsize = 0;
@@ -48,6 +60,12 @@ class FragmentsDatabase {
   std::string header;
   rk_load_stats load_stats_{};
   double ms_read_ = 0, ms_parse_ = 0, ms_device_load_ = 0;  // host wall clock of the three ingest phases
+  // rk_load_csv: the file, kept so that records() can parse it on the host when a caller asks for host records
+  mutable std::unique_ptr<FragsText> text_;
+  size_t body_pos_ = 0;
+  mutable std::once_flag records_once_;
+  bool device_parser_ = false;
+  rk_csv_stats csv_stats_{};
   // the reference's bucket array, built on first use from the processing order the device computed (K2a)
   mutable std::unique_ptr<std::vector<FragFile>[]> buckets_;
   mutable std::once_flag buckets_once_;
@@ -80,6 +98,10 @@ class FragmentsDatabase {
   // input = gecko_binary: the stream is a .frags file; every record loads as readFragment would load its CSV row
   FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, const std::vector<int> &devices,
                     FragsInput input = FragsInput::csv);
+  // One device, CSV input: the rows are parsed on the device (rk_load_csv) into the same database the host parser plus
+  // rk_load_packed / rk_load_aos builds.  The file text is kept; records(), begin() and the facades that read host
+  // records parse it on first use with the host parser (parse_rows_parallel), so they hand out the same records.
+  FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, int device, CsvOnDevice);
   ~FragmentsDatabase();
   FragmentsDatabase(const FragmentsDatabase &) = delete;
   FragmentsDatabase &operator=(const FragmentsDatabase &) = delete;
@@ -91,11 +113,13 @@ class FragmentsDatabase {
   // processing order; the grouping functions of this repo do not need it.
   const std::vector<FragFile> *begin() const;
   const std::vector<FragFile> *end() const { return begin() + vsize - 1; }
-  const FragFile *records() const { return records_; }   // the records in file order
+  const FragFile *records() const;                      // the records in file order
   rk_ctx *ctx() const { return ctx_; }
   rk_multi *multi() const { return multi_; }
   const rk_load_stats &load_stats() const { return load_stats_; }
   double ms_read() const { return ms_read_; }
   double ms_parse() const { return ms_parse_; }
   double ms_device_load() const { return ms_device_load_; }
+  bool device_parser() const { return device_parser_; }  // built by the CsvOnDevice constructor
+  const rk_csv_stats &csv_stats() const { return csv_stats_; }
 };

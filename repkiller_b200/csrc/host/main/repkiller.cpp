@@ -4,7 +4,8 @@
 // Parameter pairs are processed in argv order on one device context while the writer thread saves the previous
 // result; every pair writes the same path (as in the reference, repkiller.cpp:95-96), so the last pair's file
 // remains ([survey choice]: the reference's 3-thread pool makes the survivor timing dependent).
-// RK_TIMING=1 prints per-stage device times on stderr (writer=device|host: which writer made the file); RK_DEVICE selects
+// RK_TIMING=1 prints per-stage device times on stderr (parser=device|host: which parser read the CSV rows, with the parse
+// milliseconds; writer=device|host: which writer made the file); RK_DEVICE selects
 // the GPU; RK_LEGACY_WRITER=1 formats the output on the host through FGList + SaverQueue instead of on the device (K6).
 // RK_DEVICES=0,1,... partitions the comparison over several GPUs (rk_create_multi; NCCL between distinct devices); every
 // GPU formats its own range of output lines (RK_F_LINE_RECORDS, rk_multi_format_lines), or the host writer does it
@@ -13,6 +14,7 @@
 #include <cstdlib>
 #include <fstream>
 #include <iostream>
+#include <memory>
 #include <queue>
 #include <stdexcept>
 #include <string>
@@ -90,13 +92,23 @@ int main(int argc, char *argv[]) {
   const bool legacy_writer = getenv("RK_LEGACY_WRITER") != nullptr;
 
   sequence_manager seq_manager;
-  // (beside the reference's CSV: GECKO's binary .frags container, see FragmentsDatabase.h)
-  FragmentsDatabase frag_db(frags_file, seq_manager, devices, detect_frags_input(multifrags_path, frags_file));
+  // (beside the reference's CSV: GECKO's binary .frags container, see FragmentsDatabase.h).  One device and CSV input: the
+  // rows are parsed on the device; several devices and .frags input take the host parser.
+  const FragsInput input = detect_frags_input(multifrags_path, frags_file);
+  std::unique_ptr<FragmentsDatabase> db_owner(devices.size() == 1 && input == FragsInput::csv
+                                                  ? new FragmentsDatabase(frags_file, seq_manager, devices[0], CsvOnDevice{})
+                                                  : new FragmentsDatabase(frags_file, seq_manager, devices, input));
+  const FragmentsDatabase &frag_db = *db_owner;
   frags_file.close();
   if (timing) {
     const rk_load_stats &ls = frag_db.load_stats();
     std::cerr << "[rk] loaded=" << ls.n_loaded << " kept=" << ls.n_kept << " device_ms=" << ls.ms_device << " host: read_ms=" << frag_db.ms_read()
-              << " parse_ms=" << frag_db.ms_parse() << " load_call_ms=" << frag_db.ms_device_load() << "\n";
+              << " parse_ms=" << frag_db.ms_parse() << " load_call_ms=" << frag_db.ms_device_load();
+    if (frag_db.device_parser())
+      std::cerr << " parser=device upload_ms=" << frag_db.csv_stats().ms_upload << " device_parse_ms=" << frag_db.csv_stats().ms_parse
+                << " host_rows=" << frag_db.csv_stats().n_host_rows << "\n";
+    else
+      std::cerr << " parser=host\n";
   }
 
   SaverQueue sq(seq_manager);

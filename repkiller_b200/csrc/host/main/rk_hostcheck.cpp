@@ -9,6 +9,9 @@
 //                                             the reference's call sequence (repkiller.cpp:83-96):
 //                                             generate_fragment_groups -> generate_diagonal_func -> sort_groups ->
 //                                             save_all_frag_pairs, each through its own facade (GPU)
+//   rk_hostcheck steps_device <in.csv> <out.csv> <len_ratio> <pos_ratio>
+//                                             the same on a database whose CSV rows were parsed on the device (the
+//                                             CsvOnDevice constructor, rk_load_csv) (GPU)
 //   rk_hostcheck pool <in.csv> <out_prefix> <threads> <len_ratio> <pos_ratio> [<len_ratio> <pos_ratio>]...
 //                                             the body of the reference's execWithParams (the four calls of steps) for
 //                                             every pair, run by <threads> threads that share one FragmentsDatabase, as
@@ -39,6 +42,7 @@
 #include <fstream>
 #include <iostream>
 #include <iterator>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -200,10 +204,12 @@ int main(int argc, char **argv) {
     sq.stop();
     return 0;
   }
-  if (mode == "steps" && argc >= 6) {
+  if ((mode == "steps" || mode == "steps_device") && argc >= 6) {
     std::ifstream in(argv[2], std::ifstream::in | std::ifstream::binary);
     sequence_manager sm;
-    FragmentsDatabase db(in, sm, 0, detect_frags_input(argv[2], in));
+    std::unique_ptr<FragmentsDatabase> owner(mode == "steps" ? new FragmentsDatabase(in, sm, 0, detect_frags_input(argv[2], in))
+                                                             : new FragmentsDatabase(in, sm, 0, CsvOnDevice{}));
+    const FragmentsDatabase &db = *owner;
     FGList groups;
     generate_fragment_groups(db, groups, sm, std::stod(argv[4]), std::stod(argv[5]));
     std::vector<size_t> diag(db.getA());

@@ -134,7 +134,7 @@ __device__ __forceinline__ void hist_flush(u32 (*h)[HIST_RADIX], const HistOut &
 enum KernelId {
   KID_DECODE = 0, KID_RADIX_HIST, KID_SCAN, KID_RADIX_SCATTER, KID_KEYS, KID_MATCH_SMALL, KID_MATCH_LONG, KID_CHASE,
   KID_HKEY, KID_PACK, KID_GSORT_SMALL, KID_GSORT_LARGE, KID_FINALIZE, KID_DIAG, KID_GSORT_WARP, KID_FORMAT, KID_DIST_ROWS, KID_STATS, KID_CHASE_EXITS,
-  KID_COUNT
+  KID_CSV_LINES, KID_CSV_ROWS, KID_COUNT
 };
 void prof_begin(int kid, cudaStream_t st, unsigned long long units);
 void prof_end(cudaStream_t st);
@@ -362,6 +362,43 @@ struct rk_group_stats_dev {
 // comparison, whose groups gid_base .. gid_base+n_groups-1 are all on the rank and whose line j is line line_off + j).
 int launch_group_stats(const u32 *out_order, const u32 *out_gid, const float *out_identity, const uint4 *rec4, const LineRow *rows,
                        u32 m, u32 n_groups, u32 gid_base, u32 line_off, rk_group_stats_dev *st, cudaStream_t stream);
+
+// K9 (k9_csv.cu): CSV rows parsed on the device (rk_load_csv).  Row status bytes:
+constexpr u8 CSV_REJECT = 0, CSV_ACCEPT = 1, CSV_HOST = 2, CSV_HOST_ACCEPT = 3;  // host: readFragment decides
+constexpr u8 CSV_WIDE = 4;  // an accepted row with a value of 33 or more bits
+constexpr u32 CSV_COUNT_TILE = 4096;  // bytes per CTA of the newline count (256 threads x 16 bytes)
+inline u64 csv_count_tiles(u64 bytes) { return (bytes + CSV_COUNT_TILE - 1) / CSV_COUNT_TILE; }
+struct CsvCounters {
+  u32 n_lines;     // '\n' in the text (the scan total of the tile counts)
+  u32 n_host;      // rows appended to the host list
+  u32 n_accepted;  // rows accepted on the device
+  u32 wide;        // an accepted row is wide
+};
+struct CsvOut {  // where the accepted rows go: the compact arrays, or the 109-byte records when aos is set
+  uint4 *key4, *rest4;
+  u8 *strand;
+  u8 *aos;
+};
+// '\n' counts of count tiles tile0 .. tile0 + n_tiles (the text up to the end of them must be on the device)
+int launch_csv_count(const u8 *text, u64 bytes, u64 tile0, u64 n_tiles, u32 *tile_cnt, cudaStream_t st);
+u64 csv_scan_words(u64 n);  // the scan's work words for n elements (rk_scan.cuh: scan_work_words)
+// exclusive scan of the tile counts in place (bsum: csv_scan_words(tiles) words); the total to cnt->n_lines
+int launch_csv_tile_scan(u32 *tile_cnt, u64 n_tiles, u32 *bsum, CsvCounters *cnt, cudaStream_t st);
+// the start offset of every row from the scanned tile counts, start[n_rows] = bytes + 1
+int launch_csv_starts(const u8 *text, u64 bytes, const u32 *tile_base, u64 *start, u64 n_rows, cudaStream_t st);
+// status of every row; host rows appended to host_list (cnt->n_host), rows accepted here counted (cnt->n_accepted),
+// cnt->wide raised by a wide accepted row
+int launch_csv_classify(const u8 *text, u64 bytes, const u64 *start, u64 n_rows, u8 *status, u32 *host_list, CsvCounters *cnt,
+                        cudaStream_t st);
+// {start, end} of the listed rows; their bytes back to back from dst + off[i]
+int launch_csv_host_spans(const u32 *rows, u32 n, const u64 *start, ulonglong2 *spans, cudaStream_t st);
+int launch_csv_gather(const u8 *text, const ulonglong2 *spans, const u64 *off, u32 n, u8 *dst, cudaStream_t st);
+// the accepted rows at their file-order slots: host_rows / host_recs are the rows readFragment accepted on the host
+// (row index, 109-byte record); slot: n_rows words, bsum: csv_scan_words(n_rows)
+int launch_csv_emit(const u8 *text, u64 bytes, const u64 *start, u64 n_rows, u8 *status, const u32 *host_rows, u32 n_host_acc,
+                    const u8 *host_recs, u32 *slot, u32 *bsum, CsvOut o, cudaStream_t st);
+// host side: readFragment (the host parser's rule for one row) into a 109-byte record; false = the row is rejected
+bool csv_read_row_host(const char *line, u64 len, void *record);
 
 u64 order_scratch_bytes(u64 m);
 void order_carve(OrderArgs &a, void *scratch, u64 m);  // sets packed .. worklist, work_cap

@@ -183,6 +183,24 @@ inline bool is_device_pointer(const void *p) {
 
 struct Dist;  // multi.cu: this context's part in a comparison partitioned over several GPUs
 
+// rk_load_csv's scratch on the loading context: the text on the device with its tile counts, the row arrays, the host
+// rows' spans and records, and the pinned ring the text is uploaded through (CSV_RING_SLOTS slots of CSV_CHUNK bytes;
+// two per upload thread, each with the event of its last copy).
+constexpr int CSV_RING_SLOTS = 8;
+constexpr u64 CSV_CHUNK = 4ull << 20;
+struct CsvScratch {
+  GrowBuffer text, rows, host;
+  GrowBuffer ring{cudaHostAllocDefault};
+  cudaEvent_t slot_done[CSV_RING_SLOTS] = {};
+  CsvScratch() = default;
+  CsvScratch(const CsvScratch &) = delete;
+  CsvScratch &operator=(const CsvScratch &) = delete;
+  ~CsvScratch() {
+    for (cudaEvent_t e : slot_done)
+      if (e) cudaEventDestroy(e);
+  }
+};
+
 // What a load writes and a grouping only reads: the load's sizes, the records (staged, or the caller's device pointer),
 // the processing order, the bucket sorts of both axes and h (carve_load), plus the side copy of a compact load.  A
 // context owns one; its views (rk_create_view) hold a reference to it instead of a copy, and the last context to be
@@ -197,6 +215,8 @@ struct Database {
   u64 n = 0;  // records loaded
   u32 m = 0;  // records kept
   Geometry g{};
+
+  GrowBuffer csv_out;  // rk_load_csv: the parsed rows (compact arrays, or 109-byte records when a value is wide)
 
   const u8 *aos_dev = nullptr;  // the loaded records on the device (own copy, or the caller's device pointer)
   const uint4 *pk_key = nullptr, *pk_rest = nullptr;  // ... or the compact arrays of rk_load_packed (aos_dev == nullptr)
@@ -255,6 +275,8 @@ struct rk_ctx {
   rk::u64 n_groups_last = 0;
 
   rk::GrowBuffer d_diag;  // rk_diagonal_func's table
+
+  rk::CsvScratch csv;  // rk_load_csv
 
   bool loaded = false;
   bool have_group = false;
