@@ -287,6 +287,22 @@ int rk_dist_import(rk_ctx *ctx, const void *blobs /* nranks x RK_DIST_BLOB_BYTES
  * record; slices in rank order make up the file.  Replaces FragmentsDatabase::FragmentsDatabase like rk_load_aos. */
 int rk_dist_load_aos(rk_ctx *ctx, const void *frags, uint64_t n_local, uint64_t file_offset, uint64_t seqx_len, uint64_t seqy_len,
                      unsigned flags, rk_load_stats *stats);
+/* rk_load_csv over the ranks.  slice: this rank's part of a GECKO CSV body (the bytes after the 16 header lines), in host
+ * memory of any kind or in device memory; the slices in rank order make up the body.  Every non-empty slice before the
+ * last non-empty one must end with '\n', so that every cut falls at the start of a row; a slice may be empty.  A row
+ * belongs to the rank whose slice holds its first byte; the empty row after a final '\n' to the last rank.  The library
+ * counts the rows of every rank and gives each record its index among the accepted rows of the whole body (no file
+ * offset to pass).  Groups, text and statistics are bit-identical to rk_load_csv + rk_group on one GPU and to
+ * rk_dist_load_aos on the same records.  The parsed rows belong to the rank (compact rows, or 109-byte records when a
+ * value of its slice needs 33 or more bits), so the slice may be freed when the call returns.  csv: this rank's counts
+ * (n_rows: the rows that start in its slice; their sum over the ranks is rk_load_csv's n_rows).  stats as
+ * rk_dist_load_aos reports them, ms_stage[RK_ST_H2D] = the text upload.  Refusals reach every rank with the same code
+ * and message, and leave nothing loaded: a slice that does not end a row (RK_ERR_ARG), more accepted rows over the ranks
+ * than total_frags (RK_ERR_RANGE, "Unexpected number of fragments"), 2^32-16 or more of them (RK_ERR_ARG), a rank with
+ * more than its capacity (RK_ERR_NOMEM), and a rank whose own parse failed (its text allocation, more than 2^32-16 rows
+ * in its slice).  Collective. */
+int rk_dist_load_csv(rk_ctx *ctx, const char *slice, uint64_t bytes, uint64_t seqx_len, uint64_t seqy_len, uint64_t total_frags,
+                     unsigned flags, rk_load_stats *stats, rk_csv_stats *csv);
 /* out: THIS RANK's range of output lines (order = file indices of the whole file, gid = global group ids); n_groups is
  * the global count.  info may be NULL. */
 int rk_dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flags, rk_result *out, rk_dist_info *info);
@@ -315,6 +331,14 @@ const char *rk_multi_transport(const rk_multi *m); /* "nccl" or "local" */
 /* frags: the whole file in HOST memory; the ranks take consecutive slices. */
 int rk_multi_load_aos(rk_multi *m, const void *frags, uint64_t n, uint64_t seqx_len, uint64_t seqy_len, unsigned flags,
                       rk_load_stats *stats);
+/* body: a whole GECKO CSV body in HOST memory (a device pointer returns RK_ERR_ARG).  Cut r of N is one byte past the first
+ * '\n' at or after byte bytes*r/N (the end of the body when there is none), and each rank parses its slice as
+ * rk_dist_load_csv does.  The capacity per rank is sized after the rows are counted: 1.5 x the most rows one rank may
+ * load + 65536.  csv: sums over the ranks; wide = 1 when any rank is wide; ms_upload / ms_parse = the largest of the
+ * ranks'.  The text is copied by at most max(N, T) host threads in all, T = the copy threads of one rk_load_csv
+ * (at most 4): each rank copies on its own thread, and helpers only while the ranks are fewer than T. */
+int rk_multi_load_csv(rk_multi *m, const char *body, uint64_t bytes, uint64_t seqx_len, uint64_t seqy_len, uint64_t total_frags,
+                      unsigned flags, rk_load_stats *stats, rk_csv_stats *csv);
 /* out: the whole result in pinned host memory owned by m (device pointers are NULL), valid until the next call. */
 int rk_multi_group(rk_multi *m, double len_ratio, double pos_ratio, unsigned flags, rk_result *out);
 int rk_multi_info(const rk_multi *m, int rank, rk_dist_info *info);

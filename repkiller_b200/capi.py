@@ -25,10 +25,10 @@ SYMBOLS = ["rk_create", "rk_create_view", "rk_create_error", "rk_destroy", "rk_l
            "rk_diagonal_func", "rk_format_lines", "rk_debug_fetch", "rk_profile_enable", "rk_profile_read", "rk_sort_pairs_work_bytes", "rk_sort_pairs", "rk_version",
            "rk_gen_workload", "rk_sort_members", "rk_group_statistics", "rk_sol_create", "rk_sol_destroy", "rk_sol_insert", "rk_sol_get_associated", "rk_sol_last_error",
            # one comparison over several GPUs
-           "rk_dist_unique_id", "rk_dist_init", "rk_dist_export", "rk_dist_import", "rk_dist_load_aos", "rk_dist_group",
+           "rk_dist_unique_id", "rk_dist_init", "rk_dist_export", "rk_dist_import", "rk_dist_load_aos", "rk_dist_load_csv", "rk_dist_group",
            "rk_dist_format_lines", "rk_dist_group_statistics",
            "rk_create_multi", "rk_destroy_multi", "rk_multi_last_error", "rk_multi_ranks", "rk_multi_ctx", "rk_multi_transport",
-           "rk_multi_load_aos", "rk_multi_group", "rk_multi_info", "rk_multi_format_lines", "rk_multi_group_statistics"]
+           "rk_multi_load_aos", "rk_multi_load_csv", "rk_multi_group", "rk_multi_info", "rk_multi_format_lines", "rk_multi_group_statistics"]
 DIST_ID_BYTES, DIST_BLOB_BYTES = 128, 128
 GROUP_STATS_DTYPE = np.dtype([("count", "<u4"), ("x_lo", "<u4"), ("x_hi", "<u4"), ("y_lo", "<u4"), ("y_hi", "<u4"), ("first_line", "<u4"),
                               ("mean_identity", "<f8"), ("multiplicity", "<f8")])
@@ -114,6 +114,7 @@ def load_library():
     L.rk_dist_export.argtypes = [C.c_void_p, C.c_void_p]
     L.rk_dist_import.argtypes = [C.c_void_p, C.c_void_p]
     L.rk_dist_load_aos.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint, C.POINTER(_LoadStats)]
+    L.rk_dist_load_csv.argtypes = L.rk_load_csv.argtypes
     L.rk_dist_group.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_uint, C.POINTER(_Result), C.POINTER(_DistInfo)]
     L.rk_dist_format_lines.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(_Text)]
     L.rk_dist_group_statistics.argtypes = [C.c_void_p, C.c_uint, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_uint64),
@@ -129,6 +130,7 @@ def load_library():
     L.rk_multi_transport.argtypes = [C.c_void_p]
     L.rk_multi_transport.restype = C.c_char_p
     L.rk_multi_load_aos.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint, C.POINTER(_LoadStats)]
+    L.rk_multi_load_csv.argtypes = L.rk_load_csv.argtypes
     L.rk_multi_group.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_uint, C.POINTER(_Result)]
     L.rk_multi_info.argtypes = [C.c_void_p, C.c_int, C.POINTER(_DistInfo)]
     L.rk_multi_format_lines.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(_Text)]
@@ -278,25 +280,12 @@ class Context:
         """The body of a GECKO CSV (the bytes after its 16 header lines) parsed and loaded on the device (rk_load_csv):
         bytes, a uint8 numpy array, or a uint8 torch tensor on the CPU or on this context's GPU.  seqx_len/seqy_len are the
         LOADED lengths (header value + 1), total_frags the header's "Total fragments".  Returns (LoadStats, CsvStats)."""
-        if isinstance(body, (bytes, bytearray)):
-            arr = np.frombuffer(bytes(body), dtype=np.uint8)
-            ptr, n = arr.ctypes.data, arr.nbytes
-        elif isinstance(body, np.ndarray):
-            arr = np.ascontiguousarray(body).view(np.uint8)
-            ptr, n = arr.ctypes.data, arr.nbytes
-        elif type(body).__module__.startswith("torch"):
-            arr = body.contiguous()
-            assert arr.element_size() == 1
-            ptr, n = arr.data_ptr(), arr.numel()
-        else:
-            raise TypeError("load_csv takes bytes, a uint8 numpy array or a uint8 torch tensor")
+        arr, ptr, n = _text_arg(body, "load_csv")
         st, cs = _LoadStats(), _CsvStats()
         self._check(self._L.rk_load_csv(self._h, C.c_void_p(ptr) if n else None, n, seqx_len, seqy_len, total_frags,
                                         F_TIMING if timing else 0, C.byref(st), C.byref(cs)))
         self._keep = None  # the parsed rows are the database's own: the text may go
-        return (LoadStats(st.n_loaded, st.n_kept, st.vsize, {STAGES[i]: st.ms_stage[i] for i in range(NSTAGES)}, st.ms_device,
-                          st.n_launches),
-                CsvStats(cs.n_rows, cs.n_accepted, cs.n_host_rows, bool(cs.wide), cs.ms_upload, cs.ms_parse))
+        return _csv_result(st, cs)
 
     def group(self, len_ratio: float, pos_ratio: float, host_result: bool = True, sort: bool = True, timing: bool = True,
               copy: bool = True) -> Groups:
@@ -408,6 +397,16 @@ class Context:
                                              F_TIMING if timing else 0, C.byref(st)))
         return LoadStats(st.n_loaded, st.n_kept, st.vsize, {STAGES[i]: st.ms_stage[i] for i in range(NSTAGES)}, st.ms_device,
                          st.n_launches)
+
+    def dist_load_csv(self, body, seqx_len: int, seqy_len: int, total_frags: int, timing: bool = False):
+        """This rank's slice of a GECKO CSV body (rk_dist_load_csv; collective): the body types of load_csv.  Every slice
+        before the last non-empty one ends with a newline; the library works out the file offsets.  Returns (LoadStats,
+        CsvStats) with this rank's counts."""
+        arr, ptr, n = _text_arg(body, "dist_load_csv")
+        st, cs = _LoadStats(), _CsvStats()
+        self._check(self._L.rk_dist_load_csv(self._h, C.c_void_p(ptr) if n else None, n, seqx_len, seqy_len, total_frags,
+                                             F_TIMING if timing else 0, C.byref(st), C.byref(cs)))
+        return _csv_result(st, cs)
 
     def dist_group(self, len_ratio: float, pos_ratio: float, host_result: bool = True, sort: bool = True, timing: bool = False,
                    copy: bool = True, line_records: bool = False):
@@ -532,6 +531,27 @@ def dist_unique_id() -> bytes:
     return buf.raw
 
 
+def _text_arg(body, what: str):
+    """(object to keep alive, address, bytes) of a text argument: bytes, a uint8 numpy array or a uint8 torch tensor"""
+    if isinstance(body, (bytes, bytearray)):
+        arr = np.frombuffer(bytes(body), dtype=np.uint8)
+        return arr, arr.ctypes.data, arr.nbytes
+    if isinstance(body, np.ndarray):
+        arr = np.ascontiguousarray(body).view(np.uint8)
+        return arr, arr.ctypes.data, arr.nbytes
+    if type(body).__module__.startswith("torch"):
+        arr = body.contiguous()
+        assert arr.element_size() == 1
+        return arr, arr.data_ptr(), arr.numel()
+    raise TypeError(f"{what} takes bytes, a uint8 numpy array or a uint8 torch tensor")
+
+
+def _csv_result(st: "_LoadStats", cs: "_CsvStats"):
+    return (LoadStats(st.n_loaded, st.n_kept, st.vsize, {STAGES[i]: st.ms_stage[i] for i in range(NSTAGES)}, st.ms_device,
+                      st.n_launches),
+            CsvStats(cs.n_rows, cs.n_accepted, cs.n_host_rows, bool(cs.wide), cs.ms_upload, cs.ms_parse))
+
+
 class Multi:
     """One comparison over several GPUs of one process (rk_create_multi): the library runs one host thread per GPU."""
 
@@ -574,6 +594,16 @@ class Multi:
         st = _LoadStats()
         self._check(self._L.rk_multi_load_aos(self._h, C.c_void_p(rec.ctypes.data), rec.nbytes // 109, seqx_len, seqy_len, 0, C.byref(st)))
         return LoadStats(st.n_loaded, st.n_kept, st.vsize, {}, st.ms_device, st.n_launches)
+
+    def load_csv(self, body, seqx_len: int, seqy_len: int, total_frags: int, timing: bool = False):
+        """A whole GECKO CSV body in host memory (bytes or a uint8 numpy array), cut into one slice per rank at row starts
+        and parsed by every rank on its GPU (rk_multi_load_csv).  Returns (LoadStats, CsvStats): the counts summed over
+        the ranks, the upload and parse times the largest of the ranks'."""
+        arr, ptr, n = _text_arg(body, "Multi.load_csv")
+        st, cs = _LoadStats(), _CsvStats()
+        self._check(self._L.rk_multi_load_csv(self._h, C.c_void_p(ptr) if n else None, n, seqx_len, seqy_len, total_frags,
+                                              F_TIMING if timing else 0, C.byref(st), C.byref(cs)))
+        return _csv_result(st, cs)
 
     def group(self, len_ratio: float, pos_ratio: float, sort: bool = True, line_records: bool = False) -> Groups:
         """line_records: every rank also gets the records of its output lines, for format_lines / group_statistics"""

@@ -475,17 +475,13 @@ int load_common(rk_ctx *ctx, const LoadSource &src, uint64_t n, uint64_t seqx_le
   return RK_OK;
 }
 
-// rk_load_csv's events on ctx->ev, after the ones load_common records (0..7)
-enum { EV_CSV_UP0 = 8, EV_CSV_UP1, EV_CSV_PARSED };
-
-// The host text to the device through the context's pinned ring, CSV_CHUNK bytes at a time: up to CSV_RING_SLOTS / 2
-// threads each copy their chunks into their own two slots and queue the upload and the newline count of each chunk on
-// the context's stream, so that a chunk's host copy overlaps the uploads and counts queued before it.
-int csv_upload(rk_ctx *ctx, const char *body, u64 bytes, u8 *dst, u32 *tile_cnt) {
+// The host text to the device through the context's pinned ring, CSV_CHUNK bytes at a time: up to `threads` threads
+// (at most CSV_RING_SLOTS / 2) each copy their chunks into their own two slots and queue the upload and the newline count
+// of each chunk on the context's stream, so that a chunk's host copy overlaps the uploads and counts queued before it.
+int csv_upload(rk_ctx *ctx, const char *body, u64 bytes, u8 *dst, u32 *tile_cnt, int threads) {
   CsvScratch &cs = ctx->csv;
   const u64 chunks = (bytes + CSV_CHUNK - 1) / CSV_CHUNK;
-  const u64 cores = std::max(1u, std::thread::hardware_concurrency() / 2);
-  const int workers = (int)std::min<u64>(std::min<u64>(CSV_RING_SLOTS / 2, cores), chunks);
+  const int workers = (int)std::min<u64>(std::max(1, std::min(threads, CSV_RING_SLOTS / 2)), chunks);
   const int rc = cs.ring.reserve((u64)2 * workers * CSV_CHUNK, ctx->stream, ctx->err);
   if (rc) return rc;
   for (cudaEvent_t &e : cs.slot_done)
@@ -571,6 +567,107 @@ int csv_host_rows(rk_ctx *ctx, const char *body, bool on_device, const u8 *text,
 
 }  // namespace
 
+namespace rk {
+
+int csv_upload_threads() {
+  const u64 cores = std::max(1u, std::thread::hardware_concurrency() / 2);
+  return (int)std::min<u64>(CSV_RING_SLOTS / 2, cores);
+}
+
+int csv_parse_local(rk_ctx *ctx, const char *body, u64 bytes, int threads, CsvParse &p) {
+  CsvScratch &cs = ctx->csv;
+  cudaStream_t st = ctx->stream;
+  cudaEvent_t *ev = ctx->ev;
+  p.bytes = bytes;
+  p.on_device = bytes && is_device_pointer(body);
+  const bool copy_text = !p.on_device || ((uintptr_t)body & 15);  // the kernels read the text 16 bytes at a time
+  // the text scratch: [text][tile counts][their scan words][counters]
+  const u64 tiles = csv_count_tiles(bytes);
+  const u64 text_b = copy_text ? align_up(bytes + 16, 256) : 0, cnt_b = align_up((tiles + 1) * 4, 256),
+            scan_b = align_up(csv_scan_words(tiles) * 4, 256);
+  int rc = cs.text.reserve(text_b + cnt_b + scan_b + 256, st, ctx->err);
+  if (rc) {
+    const std::string e = ctx->err;
+    return fail(ctx, rc, "rk_load_csv: %llu bytes of text: %s", (unsigned long long)bytes, e.c_str());
+  }
+  u8 *tb = (u8 *)cs.text.ptr();
+  const u8 *text = copy_text ? tb : (const u8 *)body;
+  p.text = text;
+  u32 *tile_cnt = (u32 *)(tb + text_b), *tile_bsum = (u32 *)(tb + text_b + cnt_b);
+  CsvCounters *cnt = (CsvCounters *)(tb + text_b + cnt_b + scan_b);
+  CsvCounters h{};
+  CK(cudaMemsetAsync(cnt, 0, sizeof(CsvCounters), st));
+  CK(cudaMemsetAsync(tile_cnt, 0, 4, st));
+  CK(cudaEventRecord(ev[EV_CSV_UP0], st));
+  if (!p.on_device) {
+    if (bytes && (rc = csv_upload(ctx, body, bytes, tb, tile_cnt, threads))) return rc;
+  } else {
+    if (copy_text) CK(cudaMemcpyAsync(tb, body, bytes, cudaMemcpyDeviceToDevice, st));
+    launch_csv_count(text, bytes, 0, tiles, tile_cnt, st);
+  }
+  CK(cudaEventRecord(ev[EV_CSV_UP1], st));
+  launch_csv_tile_scan(tile_cnt, tiles, tile_bsum, cnt, st);
+  CK(cudaMemcpyAsync(&h, cnt, sizeof h, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  CK(cudaGetLastError());
+  const u64 n_rows = (u64)h.n_lines + 1;  // the segment after the last '\n' is a row too (empty after a final '\n')
+  p.n_rows = n_rows;
+  if (n_rows >= 0xFFFFFFF0ull) return fail(ctx, RK_ERR_ARG, "more than 2^32-16 rows per context; partition the input");
+
+  // the row arrays: [start (n_rows + 1)][slot / host list (n_rows)][scan words][status (n_rows)]
+  const u64 start_b = align_up((n_rows + 1) * 8, 256), slot_b = align_up(n_rows * 4, 256), rscan_b = align_up(csv_scan_words(n_rows) * 4, 256);
+  rc = cs.rows.reserve(start_b + slot_b + rscan_b + align_up(n_rows, 256), st, ctx->err);
+  if (rc) return rc;
+  u8 *rb = (u8 *)cs.rows.ptr();
+  p.start = (u64 *)rb;
+  p.slot = (u32 *)(rb + start_b), p.row_bsum = (u32 *)(rb + start_b + slot_b);
+  p.status = rb + start_b + slot_b + rscan_b;
+  launch_csv_starts(text, bytes, tile_cnt, p.start, n_rows, st);
+  launch_csv_classify(text, bytes, p.start, n_rows, p.status, p.slot, cnt, st);
+  CK(cudaMemcpyAsync(&h, cnt, sizeof h, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  CK(cudaGetLastError());
+  p.n_host = h.n_host;
+  p.n_dev_acc = h.n_accepted;
+  p.wide = h.wide != 0;
+  p.host_rows.clear();
+  p.host_recs.clear();
+  if (p.n_host && (rc = csv_host_rows(ctx, body, p.on_device, text, p.slot, (u32)p.n_host, p.start, p.host_rows, p.host_recs, &p.wide)))
+    return rc;
+  return RK_OK;
+}
+
+u64 csv_out_bytes(u64 n, bool wide) {
+  return wide ? align_up(n * RK_FRAG_BYTES + 16, 256) : 2 * align_up(n * 16, 256) + align_up(n, 256);
+}
+
+int csv_emit(rk_ctx *ctx, const CsvParse &p, GrowBuffer &out, CsvOut *o) {
+  CsvScratch &cs = ctx->csv;
+  cudaStream_t st = ctx->stream;
+  const u64 n_acc = p.n_accepted();
+  // the host-accepted records, then the parsed rows at their slots in `out`
+  const u64 nh = p.host_rows.size(), hrows_b = align_up(nh * 4, 256);
+  if (nh) {
+    const int rc = cs.host.reserve(hrows_b + nh * RK_FRAG_BYTES, st, ctx->err);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(cs.host.ptr(), p.host_rows.data(), nh * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync((u8 *)cs.host.ptr() + hrows_b, p.host_recs.data(), nh * RK_FRAG_BYTES, cudaMemcpyHostToDevice, st));
+  }
+  const u64 key_b = align_up(n_acc * 16, 256);
+  const int rc = out.reserve(csv_out_bytes(n_acc, p.wide), st, ctx->err);
+  if (rc) return rc;
+  u8 *ob = (u8 *)out.ptr();
+  *o = CsvOut{};
+  if (p.wide) o->aos = ob;
+  else o->key4 = (uint4 *)ob, o->rest4 = (uint4 *)(ob + key_b), o->strand = ob + 2 * key_b;
+  launch_csv_emit(p.text, p.bytes, p.start, p.n_rows, p.status, nh ? (const u32 *)cs.host.ptr() : nullptr, (u32)nh,
+                  nh ? (const u8 *)cs.host.ptr() + hrows_b : nullptr, p.slot, p.row_bsum, *o, st);
+  CK(cudaEventRecord(ctx->ev[EV_CSV_PARSED], st));
+  return RK_OK;
+}
+
+}  // namespace rk
+
 extern "C" {
 
 int rk_load_csv(rk_ctx *ctx, const char *body, uint64_t bytes, uint64_t seqx_len, uint64_t seqy_len, uint64_t total_frags, unsigned flags,
@@ -581,101 +678,28 @@ int rk_load_csv(rk_ctx *ctx, const char *body, uint64_t bytes, uint64_t seqx_len
   CK(cudaSetDevice(ctx->device));
   ctx->loaded = false;
   ctx->have_group = false;
-  CsvScratch &cs = ctx->csv;
-  cudaStream_t st = ctx->stream;
   cudaEvent_t *ev = ctx->ev;
-  const bool on_device = bytes && is_device_pointer(body);
-  const bool copy_text = !on_device || ((uintptr_t)body & 15);  // the kernels read the text 16 bytes at a time
-  u64 n_rows = 0, n_host = 0, n_acc = 0;
-  bool wide = false;
+  CsvParse p;
   LoadSource src;
   {
     ProfGuard pg(ctx);
-    // the text scratch: [text][tile counts][their scan words][counters]
-    const u64 tiles = csv_count_tiles(bytes);
-    const u64 text_b = copy_text ? align_up(bytes + 16, 256) : 0, cnt_b = align_up((tiles + 1) * 4, 256),
-              scan_b = align_up(csv_scan_words(tiles) * 4, 256);
-    int rc = cs.text.reserve(text_b + cnt_b + scan_b + 256, st, ctx->err);
-    if (rc) {
-      const std::string e = ctx->err;
-      return fail(ctx, rc, "rk_load_csv: %llu bytes of text: %s", (unsigned long long)bytes, e.c_str());
-    }
-    u8 *tb = (u8 *)cs.text.ptr();
-    const u8 *text = copy_text ? tb : (const u8 *)body;
-    u32 *tile_cnt = (u32 *)(tb + text_b), *tile_bsum = (u32 *)(tb + text_b + cnt_b);
-    CsvCounters *cnt = (CsvCounters *)(tb + text_b + cnt_b + scan_b);
-    CsvCounters h{};
-    CK(cudaMemsetAsync(cnt, 0, sizeof(CsvCounters), st));
-    CK(cudaMemsetAsync(tile_cnt, 0, 4, st));
-    CK(cudaEventRecord(ev[EV_CSV_UP0], st));
-    if (!on_device) {
-      if (bytes && (rc = csv_upload(ctx, body, bytes, tb, tile_cnt))) return rc;
-    } else {
-      if (copy_text) CK(cudaMemcpyAsync(tb, body, bytes, cudaMemcpyDeviceToDevice, st));
-      launch_csv_count(text, bytes, 0, tiles, tile_cnt, st);
-    }
-    CK(cudaEventRecord(ev[EV_CSV_UP1], st));
-    launch_csv_tile_scan(tile_cnt, tiles, tile_bsum, cnt, st);
-    CK(cudaMemcpyAsync(&h, cnt, sizeof h, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    CK(cudaGetLastError());
-    n_rows = (u64)h.n_lines + 1;  // the segment after the last '\n' is a row too (empty after a final '\n')
-    if (n_rows >= 0xFFFFFFF0ull) return fail(ctx, RK_ERR_ARG, "more than 2^32-16 rows per context; partition the input");
-
-    // the row arrays: [start (n_rows + 1)][slot / host list (n_rows)][scan words][status (n_rows)]
-    const u64 start_b = align_up((n_rows + 1) * 8, 256), slot_b = align_up(n_rows * 4, 256), rscan_b = align_up(csv_scan_words(n_rows) * 4, 256);
-    rc = cs.rows.reserve(start_b + slot_b + rscan_b + align_up(n_rows, 256), st, ctx->err);
+    int rc = csv_parse_local(ctx, body, bytes, csv_upload_threads(), p);
     if (rc) return rc;
-    u8 *rb = (u8 *)cs.rows.ptr();
-    u64 *start = (u64 *)rb;
-    u32 *slot = (u32 *)(rb + start_b), *row_bsum = (u32 *)(rb + start_b + slot_b);
-    u8 *status = rb + start_b + slot_b + rscan_b;
-    launch_csv_starts(text, bytes, tile_cnt, start, n_rows, st);
-    launch_csv_classify(text, bytes, start, n_rows, status, slot, cnt, st);
-    CK(cudaMemcpyAsync(&h, cnt, sizeof h, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    CK(cudaGetLastError());
-    n_host = h.n_host;
-    wide = h.wide != 0;
-
-    std::vector<u32> host_rows;
-    std::vector<u8> host_recs;
-    if (n_host && (rc = csv_host_rows(ctx, body, on_device, text, slot, (u32)n_host, start, host_rows, host_recs, &wide))) return rc;
-    n_acc = (u64)h.n_accepted + host_rows.size();
-    if (n_acc > total_frags) return fail(ctx, RK_ERR_RANGE, "Unexpected number of fragments");  // FragmentsDatabase.cpp:99
-
-    // the host-accepted records, then the parsed rows at their slots in the database's own buffer
-    const u64 nh = host_rows.size(), hrows_b = align_up(nh * 4, 256);
-    if (nh) {
-      rc = cs.host.reserve(hrows_b + nh * RK_FRAG_BYTES, st, ctx->err);
-      if (rc) return rc;
-      CK(cudaMemcpyAsync(cs.host.ptr(), host_rows.data(), nh * 4, cudaMemcpyHostToDevice, st));
-      CK(cudaMemcpyAsync((u8 *)cs.host.ptr() + hrows_b, host_recs.data(), nh * RK_FRAG_BYTES, cudaMemcpyHostToDevice, st));
-    }
-    const u64 key_b = align_up(n_acc * 16, 256);
-    rc = ctx->db->csv_out.reserve(wide ? align_up(n_acc * RK_FRAG_BYTES + 16, 256) : 2 * key_b + align_up(n_acc, 256), st, ctx->err);
-    if (rc) return rc;
-    u8 *ob = (u8 *)ctx->db->csv_out.ptr();
-    CsvOut o{};
-    if (wide) {
-      o.aos = ob;
-      src.aos = ob;
-    } else {
-      o.key4 = (uint4 *)ob, o.rest4 = (uint4 *)(ob + key_b), o.strand = ob + 2 * key_b;
-      src.key4 = o.key4, src.rest4 = o.rest4, src.strand = o.strand;
-    }
-    launch_csv_emit(text, bytes, start, n_rows, status, nh ? (const u32 *)cs.host.ptr() : nullptr, (u32)nh,
-                    nh ? (const u8 *)cs.host.ptr() + hrows_b : nullptr, slot, row_bsum, o, st);
-    CK(cudaEventRecord(ev[EV_CSV_PARSED], st));
+    if (p.n_accepted() > total_frags) return fail(ctx, RK_ERR_RANGE, "Unexpected number of fragments");  // FragmentsDatabase.cpp:99
+    CsvOut o;
+    if ((rc = csv_emit(ctx, p, ctx->db->csv_out, &o))) return rc;
+    if (o.aos) src.aos = o.aos;
+    else src.key4 = o.key4, src.rest4 = o.rest4, src.strand = o.strand;
   }
+  const u64 n_acc = p.n_accepted();
   const int rc = load_common(ctx, src, n_acc, seqx_len, seqy_len, flags, stats);
   if (rc) return rc;
   const float ms_up = ev_ms(ev[EV_CSV_UP0], ev[EV_CSV_UP1]), ms_parse = ev_ms(ev[EV_CSV_UP1], ev[EV_CSV_PARSED]);
-  if (stats && (flags & RK_F_TIMING)) stats->ms_stage[RK_ST_H2D] = on_device ? 0.f : ms_up;
+  if (stats && (flags & RK_F_TIMING)) stats->ms_stage[RK_ST_H2D] = p.on_device ? 0.f : ms_up;
   if (csv) {
     memset(csv, 0, sizeof *csv);
-    csv->n_rows = n_rows, csv->n_accepted = n_acc, csv->n_host_rows = n_host, csv->wide = wide;
-    csv->ms_upload = on_device ? 0.f : ms_up;
+    csv->n_rows = p.n_rows, csv->n_accepted = n_acc, csv->n_host_rows = p.n_host, csv->wide = p.wide;
+    csv->ms_upload = p.on_device ? 0.f : ms_up;
     csv->ms_parse = ms_parse;
   }
   return RK_OK;

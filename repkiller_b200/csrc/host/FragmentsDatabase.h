@@ -47,7 +47,8 @@ struct FragsText {
 };
 void read_stream_rest(std::ifstream &in, FragsText &out);
 
-// Tag of the constructor that parses the CSV rows on the device (host/FragmentsDatabaseDeviceCsv.cpp, rk_load_csv).
+// Tag of the constructors that parse the CSV rows on the device (host/FragmentsDatabaseDeviceCsv.cpp, rk_load_csv; over
+// several devices host/FragmentsDatabaseMultiCsv.cpp, rk_multi_load_csv).
 struct CsvOnDevice {};
 
 class FragmentsDatabase {
@@ -102,6 +103,9 @@ class FragmentsDatabase {
   // rk_load_packed / rk_load_aos builds.  The file text is kept; records(), begin() and the facades that read host
   // records parse it on first use with the host parser (parse_rows_parallel), so they hand out the same records.
   FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, int device, CsvOnDevice);
+  // Several devices, CSV input: every device parses its slice of the rows (rk_multi_load_csv); ctx() is null and multi()
+  // set, as with the host parser's constructor for several devices.  The text is kept for records() as above.
+  FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, const std::vector<int> &devices, CsvOnDevice);
   ~FragmentsDatabase();
   FragmentsDatabase(const FragmentsDatabase &) = delete;
   FragmentsDatabase &operator=(const FragmentsDatabase &) = delete;
@@ -120,6 +124,6 @@ class FragmentsDatabase {
   double ms_read() const { return ms_read_; }
   double ms_parse() const { return ms_parse_; }
   double ms_device_load() const { return ms_device_load_; }
-  bool device_parser() const { return device_parser_; }  // built by the CsvOnDevice constructor
+  bool device_parser() const { return device_parser_; }  // built by a CsvOnDevice constructor
   const rk_csv_stats &csv_stats() const { return csv_stats_; }
 };

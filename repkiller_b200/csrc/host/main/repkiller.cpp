@@ -5,7 +5,8 @@
 // result; every pair writes the same path (as in the reference, repkiller.cpp:95-96), so the last pair's file
 // remains ([survey choice]: the reference's 3-thread pool makes the survivor timing dependent).
 // RK_TIMING=1 prints per-stage device times on stderr (parser=device|host: which parser read the CSV rows, with the parse
-// milliseconds; writer=device|host: which writer made the file); RK_DEVICE selects
+// milliseconds, over several GPUs the largest rank's, and the rows left to the host parser summed over the ranks;
+// writer=device|host: which writer made the file); RK_DEVICE selects
 // the GPU; RK_LEGACY_WRITER=1 formats the output on the host through FGList + SaverQueue instead of on the device (K6).
 // RK_DEVICES=0,1,... partitions the comparison over several GPUs (rk_create_multi; NCCL between distinct devices); every
 // GPU formats its own range of output lines (RK_F_LINE_RECORDS, rk_multi_format_lines), or the host writer does it
@@ -92,12 +93,13 @@ int main(int argc, char *argv[]) {
   const bool legacy_writer = getenv("RK_LEGACY_WRITER") != nullptr;
 
   sequence_manager seq_manager;
-  // (beside the reference's CSV: GECKO's binary .frags container, see FragmentsDatabase.h).  One device and CSV input: the
-  // rows are parsed on the device; several devices and .frags input take the host parser.
+  // (beside the reference's CSV: GECKO's binary .frags container, see FragmentsDatabase.h).  CSV input: the rows are parsed
+  // on the device, over several devices each parsing its slice; .frags input takes the host parser.
   const FragsInput input = detect_frags_input(multifrags_path, frags_file);
-  std::unique_ptr<FragmentsDatabase> db_owner(devices.size() == 1 && input == FragsInput::csv
-                                                  ? new FragmentsDatabase(frags_file, seq_manager, devices[0], CsvOnDevice{})
-                                                  : new FragmentsDatabase(frags_file, seq_manager, devices, input));
+  std::unique_ptr<FragmentsDatabase> db_owner(
+      input != FragsInput::csv ? new FragmentsDatabase(frags_file, seq_manager, devices, input)
+      : devices.size() == 1    ? new FragmentsDatabase(frags_file, seq_manager, devices[0], CsvOnDevice{})
+                               : new FragmentsDatabase(frags_file, seq_manager, devices, CsvOnDevice{}));
   const FragmentsDatabase &frag_db = *db_owner;
   frags_file.close();
   if (timing) {

@@ -257,14 +257,14 @@ __global__ void __launch_bounds__(256) k_decode_packed(const uint4 *__restrict__
 }
 
 int launch_decode_packed(const uint4 *key4, const u8 *strand, u64 n, Geometry g, u32 *key0, u32 *link_x, u32 *link_y, u32 *n_dropped,
-                         u32 *err, cudaStream_t st, uint4 *rec4, HistOut hist) {
+                         u32 *err, cudaStream_t st, uint4 *rec4, HistOut hist, u32 fidx_base) {
   if (n == 0) return 0;
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   u64 grid = (n + 255) / 256;
   if (grid > (u64)sms * 8) grid = (u64)sms * 8;
-  DecodeOut o{nullptr, nullptr, nullptr, rec4, nullptr, nullptr, key0, link_x, link_y, n_dropped, err, hist, 0u};
+  DecodeOut o{nullptr, nullptr, nullptr, rec4, nullptr, nullptr, key0, link_x, link_y, n_dropped, err, hist, fidx_base};
   KScope ks(KID_DECODE, st, n);
   k_decode_packed<<<(unsigned)grid, 256, 0, st>>>(key4, strand, n, g, o);
   return 1;

@@ -24,12 +24,7 @@ __device__ __forceinline__ LineRow load_fields(const FormatArgs &a, u32 j) {
   if (a.rows) return a.rows[j];
   const u32 fidx = a.order[j];
   if (a.aos) return line_row_of_record(a.aos + (u64)fidx * FRAG_BYTES);
-  LineRow f;  // compact ingest: two 16-byte words and a byte
-  const uint4 k = a.pk_key[fidx], r = a.pk_rest[fidx];
-  f.xs = k.x, f.ys = k.y, f.len = k.z, f.ident = k.w;
-  f.xe = r.x, f.ye = r.y, f.score = r.z, f.sim_bits = r.w;
-  f.strand = a.pk_strand[fidx];
-  return f;
+  return line_row_of_packed(a.pk_key, a.pk_rest, a.pk_strand, fidx);  // compact ingest
 }
 
 template <class Sink>

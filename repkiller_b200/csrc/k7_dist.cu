@@ -771,14 +771,17 @@ __global__ void __launch_bounds__(256) k_chase_map(const u64 *__restrict__ res, 
 // ---- line records ----------------------------------------------------------------------------------------------------
 // The rank that loaded a record answers every request for it with the line row, stored straight into the asking rank's
 // rows[line] (requests arrive in blocks by source rank: the block gives the asking rank, the request its line).
+// PACKED: the rank holds compact rows (pk) instead of 109-byte records (aos).
+template <bool PACKED>
 __global__ void __launch_bounds__(256) k_line_answer(const uint4 *__restrict__ requests, u32 n, const u8 *__restrict__ aos, u32 file_lo,
-                                                     ScatterTable back) {
+                                                     ScatterTable back, PackedRows pk) {
   const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= n) return;
   const uint4 q = requests[t];
   int s = 0;
   for (int r = 1; r < back.nr; ++r) s = back.start[r] <= t ? r : s;
-  const LineRow row = line_row_of_record(aos + (u64)(q.x - file_lo) * FRAG_BYTES);
+  const LineRow row = PACKED ? line_row_of_packed(pk.key, pk.rest, pk.strand, q.x - file_lo)
+                             : line_row_of_record(aos + (u64)(q.x - file_lo) * FRAG_BYTES);
   uint4 *dst = reinterpret_cast<uint4 *>(reinterpret_cast<LineRow *>(back.out[s]) + q.y);
   const uint4 *src = reinterpret_cast<const uint4 *>(&row);
 #pragma unroll
@@ -1034,10 +1037,12 @@ int dist_line_ask_push(const u32 *order, u32 n, const u32 *file_cuts, int nr, ui
   return push_rows(RouteArgs{order, n, file_cuts, nr, me, 0xFFFFFFFFu, 0, out_cap, nullptr}, tile_cnt, counts_all, row_stride, me,
                    PayLineReq{order, row_outs<uint4>(outs, nr)}, st);
 }
-int dist_line_answer(const uint4 *requests, u32 n, const u8 *aos, u32 file_lo, const ScatterTable &back, cudaStream_t st) {
+int dist_line_answer(const uint4 *requests, u32 n, const u8 *aos, const PackedRows &pk, u32 file_lo, const ScatterTable &back,
+                     cudaStream_t st) {
   if (n == 0) return 0;
   KScope ks(KID_DIST_ROWS, st, n);
-  k_line_answer<<<blocks_for(n), 256, 0, st>>>(requests, n, aos, file_lo, back);
+  if (aos) k_line_answer<false><<<blocks_for(n), 256, 0, st>>>(requests, n, aos, file_lo, back, pk);
+  else k_line_answer<true><<<blocks_for(n), 256, 0, st>>>(requests, n, aos, file_lo, back, pk);
   return 1;
 }
 int dist_or_rows(const u32 *all, u64 row_stride, int nr, u64 words, u32 *out, cudaStream_t st) {

@@ -389,7 +389,7 @@ struct Dist {
   Trace trace;
   cudaStream_t side = nullptr;  // rows that travel while kernels run (the Y exchange beside the X sort)
   // grow-only side buffers whose size depends on the input, not on cap
-  GrowBuffer aos_buf;
+  GrowBuffer aos_buf;  // this rank's records: a host slice staged (109 B per row), or its parsed CSV rows (compact or 109 B)
   GrowBuffer link_buf;  // u32 [hist0][linkx_loc][linky_loc] (one all-gather) [linkx][linky][gather: world * the first three]
   GrowBuffer h_res{cudaHostAllocDefault};
 
@@ -401,6 +401,7 @@ struct Dist {
   u64 m_total = 0, n_total_loaded = 0;
   Exchange ex1, exh, exy;
   const u8 *aos_src = nullptr;          // this rank's slice of the records on the device (aos_buf or the caller's pointer)
+  PackedRows pk_src{};                  // ... or its compact rows (rk_dist_load_csv without a wide value; aos_src == nullptr)
   u32 file_off[DIST_MAX_RANKS] = {0};  // first file index of every rank's slice
   bool slices_in_order = false;         // every slice ends at or before the next rank's starts: file_off[] routes a file index
 
@@ -713,12 +714,13 @@ static ScatterTable scatter_table(const Dist &D, const Exchange &ex, bool back, 
 // ---------------------------------------------------------------------------------------------------------------------
 // load: FragmentsDatabase's constructor over the ranks (src/FragmentsDatabase.cpp:84-100)
 // ---------------------------------------------------------------------------------------------------------------------
+// pk: the slice as compact rows on the device (rk_dist_load_csv) instead of 109-byte records at frags
 static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u64 seqx_len, u64 seqy_len, unsigned flags,
-                     rk_load_stats *stats) {
+                     rk_load_stats *stats, const PackedRows *pk = nullptr) {
   Dist &D = *ctx->dist;
   const int nr = D.world, me = D.rank;
   if (!D.peers_ready) return fail(ctx, RK_ERR_STATE, "rk_dist_load_aos before rk_dist_import");
-  if (!frags && n_loc) return fail(ctx, RK_ERR_ARG, "null record pointer");
+  if (!frags && !pk && n_loc) return fail(ctx, RK_ERR_ARG, "null record pointer");
   if (seqx_len >= (1ull << 32) || seqy_len >= (1ull << 32)) return fail(ctx, RK_ERR_RANGE, "sequence length does not fit in 32 bits");
   if (file_off + n_loc >= 0xFFFFFFF0ull) return fail(ctx, RK_ERR_ARG, "more than 2^32-16 records in one comparison");
   CK(cudaSetDevice(ctx->device));
@@ -745,18 +747,19 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   u32 *hist0 = (u32 *)D.link_buf.ptr(), *linkx_loc = hist0 + DIST_BINS, *linky_loc = linkx_loc + lxw, *linkx = linky_loc + lyw, *linky = linkx + lxw,
       *pub_all = linky + lyw;
 
-  const bool on_device = n_use && is_device_pointer(frags);
+  const bool on_device = n_use && !pk && is_device_pointer(frags);
   if (on_device && ((uintptr_t)frags & 15)) return fail(ctx, RK_ERR_ARG, "device record pointer must be 16-byte aligned");
   const u8 *aos = (const u8 *)frags;
   cudaEvent_t *ev = ctx->ev;
   CK(cudaEventRecord(ev[0], st));
-  if (!on_device && n_use) {
+  if (!on_device && !pk && n_use) {
     const int rc2 = D.aos_buf.reserve(align_up(n_use * RK_FRAG_BYTES, 16) + 16, st, ctx->err);
     if (rc2) return rc2;
     CK(cudaMemcpyAsync(D.aos_buf.ptr(), frags, n_use * RK_FRAG_BYTES, cudaMemcpyHostToDevice, st));
     aos = (const u8 *)D.aos_buf.ptr();
   }
-  D.aos_src = aos;
+  D.aos_src = pk ? nullptr : aos;
+  D.pk_src = pk ? *pk : PackedRows{};
   CK(cudaEventRecord(ev[1], st));
   u64 launches = 0;
 
@@ -770,8 +773,12 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
     const u32 e = ERR_WORKLIST;  // reported below as a capacity error
     CK(cudaMemcpyAsync(&D.cnt->err, &e, 4, cudaMemcpyHostToDevice, st));
   }
-  launches += launch_decode(aos, n_use, g, nullptr, nullptr, nullptr, nullptr, nullptr, D.key0_loc, linkx_loc, linky_loc,
-                            &D.cnt->n_dropped, &D.cnt->err, st, D.rec4_loc, HistOut{nullptr, 0, 0}, (u32)file_off);
+  if (pk)
+    launches += launch_decode_packed(pk->key, pk->strand, n_use, g, D.key0_loc, linkx_loc, linky_loc, &D.cnt->n_dropped, &D.cnt->err, st,
+                                     D.rec4_loc, HistOut{nullptr, 0, 0}, (u32)file_off);
+  else
+    launches += launch_decode(aos, n_use, g, nullptr, nullptr, nullptr, nullptr, nullptr, D.key0_loc, linkx_loc, linky_loc,
+                              &D.cnt->n_dropped, &D.cnt->err, st, D.rec4_loc, HistOut{nullptr, 0, 0}, (u32)file_off);
   // exchange 1: to the owner of the xStart/10 range
   const int shift0 = D.bits_rank > 12 ? D.bits_rank - 12 : 0;
   launches += dist_coarse_hist(D.key0_loc, (u32)n_use, shift0, 0, g.vsize - 1, hist0, st);
@@ -911,6 +918,120 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
       stats->ms_stage[RK_ST_YSORT] = ev_ms(ev[6], ev[7]);   // Y exchange + Y sort
       stats->ms_device = ev_ms(ev[1], ev[7]);
     }
+  }
+  return RK_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// load from text: FragmentsDatabase's row loop (src/FragmentsDatabase.cpp:91-100) over the ranks, each rank parsing its slice
+// ---------------------------------------------------------------------------------------------------------------------
+// The local half of rk_dist_load_csv: rk_load_csv's parse of this rank's slice, up to the host rows.  Needs no other
+// rank and no partition buffers (rk_multi_load_csv sizes them from its result).  A failure is kept in the state, not
+// returned: it travels to every rank in the count exchange of the collective half.
+struct DistCsv {
+  CsvParse p;
+  int rc = RK_OK;
+  std::string err;
+  bool nl_end = false;  // the slice ends with '\n'
+};
+static void dist_csv_local(rk_ctx *ctx, const char *slice, u64 bytes, int threads, DistCsv &L) {
+  L = DistCsv{};
+  ctx->loaded = ctx->have_group = false;
+  if (ctx->dist) ctx->dist->loaded = ctx->dist->have_rows = false;
+  auto run = [&]() -> int {
+    if (!slice && bytes) return fail(ctx, RK_ERR_ARG, "null text pointer");
+    CK(cudaSetDevice(ctx->device));
+    ProfGuard pg(ctx);
+    if (const int rc = csv_parse_local(ctx, slice, bytes, threads, L.p)) return rc;
+    if (bytes) {
+      char last = 0;
+      if (L.p.on_device) CK(cudaMemcpy(&last, slice + bytes - 1, 1, cudaMemcpyDeviceToHost));
+      else last = slice[bytes - 1];
+      L.nl_end = last == '\n';
+    }
+    return RK_OK;
+  };
+  L.rc = run();
+  if (L.rc) L.err = ctx->err;
+}
+
+// the count exchange of rk_dist_load_csv: one row of CW_WORDS per rank; a rank whose local half failed sends the start of
+// its error message in the CW_MSG words, so that every rank returns the same text
+enum { CW_ACC, CW_NL, CW_FLAGS, CW_RC, CW_MSG, CW_WORDS = CW_MSG + 28 };
+static_assert(CW_WORDS <= SMALL_WORDS, "the count row fits the rows of d_small");
+constexpr u32 CWF_WIDE = 1, CWF_BYTES = 2, CWF_NL_END = 4, CWF_ROWS = 8;  // CWF_ROWS: more than 2^32-16 rows in the slice
+
+// The collective half: the counts of every rank, the verdicts every rank reaches from them, this rank's file offset,
+// the emit into Dist::aos_buf and dist_load on it.
+static int dist_csv_finish(rk_ctx *ctx, DistCsv &L, u64 seqx_len, u64 seqy_len, u64 total_frags, unsigned flags, rk_load_stats *stats,
+                           rk_csv_stats *csv) {
+  Dist &D = *ctx->dist;
+  const int nr = D.world, me = D.rank;
+  if (!D.peers_ready) return fail(ctx, RK_ERR_STATE, "rk_dist_load_csv before rk_dist_import");
+  CK(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  const CsvParse &p = L.p;
+  u32 row[CW_WORDS] = {0, 0, 0, (u32)L.rc};
+  if (L.rc) {
+    if (L.rc == RK_ERR_ARG && p.n_rows >= 0xFFFFFFF0ull) row[CW_FLAGS] |= CWF_ROWS;
+    memcpy(&row[CW_MSG], L.err.c_str(), std::min<size_t>(L.err.size(), (CW_WORDS - CW_MSG) * 4 - 1));  // (row is zeroed: terminated)
+  } else {
+    row[CW_ACC] = (u32)p.n_accepted();
+    row[CW_NL] = (u32)(p.n_rows - 1);
+    row[CW_FLAGS] = (p.wide ? CWF_WIDE : 0) | (p.bytes ? CWF_BYTES : 0) | (L.nl_end ? CWF_NL_END : 0);
+  }
+  CK(cudaMemcpyAsync(D.d_small, row, sizeof row, cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
+  TR(D.tr->all_gather(D.d_small, D.d_small_all, sizeof row, st));
+  std::vector<u32> all((size_t)nr * CW_WORDS);
+  CK(cudaMemcpyAsync(all.data(), D.d_small_all, all.size() * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  auto W = [&](int r, int w) { return all[(size_t)r * CW_WORDS + w]; };
+  // every rank sees the same words, so every rank reaches the same verdict
+  int last = -1;  // the last rank with a non-empty slice
+  for (int r = 0; r < nr; ++r)
+    if (W(r, CW_FLAGS) & CWF_BYTES) last = r;
+  for (int r = 0; r < nr; ++r) {
+    if (!W(r, CW_RC)) continue;
+    if (W(r, CW_FLAGS) & CWF_ROWS) return fail(ctx, RK_ERR_ARG, "rank %d: more than 2^32-16 rows in its slice of the text", r);
+    return fail(ctx, (int)W(r, CW_RC), "rank %d could not parse its slice of the text: %s", r,
+                (const char *)&all[(size_t)r * CW_WORDS + CW_MSG]);
+  }
+  for (int r = 0; r < last; ++r)
+    if ((W(r, CW_FLAGS) & CWF_BYTES) && !(W(r, CW_FLAGS) & CWF_NL_END))
+      return fail(ctx, RK_ERR_ARG, "rank %d: its slice of the text does not end with '\\n' (every slice before the last must end a row)", r);
+  u64 total = 0, file_off = 0;
+  for (int r = 0; r < nr; ++r) {
+    if (r == me) file_off = total;
+    total += W(r, CW_ACC);
+  }
+  if (total > total_frags) return fail(ctx, RK_ERR_RANGE, "Unexpected number of fragments");  // FragmentsDatabase.cpp:99
+  if (total >= 0xFFFFFFF0ull) return fail(ctx, RK_ERR_ARG, "more than 2^32-16 records in one comparison");
+  for (int r = 0; r < nr; ++r)
+    if (W(r, CW_ACC) > D.cap)
+      return fail(ctx, RK_ERR_NOMEM, "a rank holds more records than the capacity of %llu rows per rank given to rk_dist_init",
+                  (unsigned long long)D.cap);
+  // the final row of the text (the empty one after a final '\n') is the last slice's; every other slice ends with '\n',
+  // and the empty segment after it is no row
+  const int holder = (last >= 0 && !(W(last, CW_FLAGS) & CWF_NL_END)) ? last : nr - 1;
+  const u64 n_rows = (u64)W(me, CW_NL) + (holder == me ? 1 : 0);
+
+  CsvOut o;
+  {
+    ProfGuard pg(ctx);
+    if (const int rc = csv_emit(ctx, p, D.aos_buf, &o)) return rc;
+  }
+  const PackedRows pk{o.key4, o.rest4, o.strand};
+  const u64 n_acc = p.n_accepted();
+  if (const int rc = dist_load(ctx, o.aos, n_acc, file_off, seqx_len, seqy_len, flags, stats, o.aos ? nullptr : &pk)) return rc;
+  CK(cudaStreamSynchronize(st));
+  cudaEvent_t *ev = ctx->ev;
+  const float ms_up = p.on_device ? 0.f : ev_ms(ev[EV_CSV_UP0], ev[EV_CSV_UP1]), ms_parse = ev_ms(ev[EV_CSV_UP1], ev[EV_CSV_PARSED]);
+  if (stats && (flags & RK_F_TIMING)) stats->ms_stage[RK_ST_H2D] = ms_up;
+  if (csv) {
+    memset(csv, 0, sizeof *csv);
+    csv->n_rows = n_rows, csv->n_accepted = n_acc, csv->n_host_rows = p.n_host, csv->wide = p.wide;
+    csv->ms_upload = ms_up;
+    csv->ms_parse = ms_parse;
   }
   return RK_OK;
 }
@@ -1073,7 +1194,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
     Exchange exl;
     exl.from_matrix(D.h_small, W_CNT_A, nr, me);
     D.tr->bytes_sent += (exl.n_send - exl.scnt[me]) * 16 + (exl.n_recv - exl.rcnt[me]) * sizeof(LineRow);
-    launches += dist_line_answer(D.queries, (u32)exl.n_recv, D.aos_src, D.file_off[me], scatter_table(D, exl, true, D.line_rows), st);
+    launches += dist_line_answer(D.queries, (u32)exl.n_recv, D.aos_src, D.pk_src, D.file_off[me], scatter_table(D, exl, true, D.line_rows), st);
     TR(D.tr->barrier(st));
     CK(cudaEventRecord(ev[8], st));
   }
@@ -1238,6 +1359,15 @@ int rk_dist_load_aos(rk_ctx *ctx, const void *frags, uint64_t n_local, uint64_t 
   if (!ctx) return RK_ERR_ARG;
   if (!ctx->dist) return fail(ctx, RK_ERR_STATE, "rk_dist_load_aos before rk_dist_init");
   return dist_load(ctx, frags, n_local, file_offset, seqx_len, seqy_len, flags, stats);
+}
+
+int rk_dist_load_csv(rk_ctx *ctx, const char *slice, uint64_t bytes, uint64_t seqx_len, uint64_t seqy_len, uint64_t total_frags,
+                     unsigned flags, rk_load_stats *stats, rk_csv_stats *csv) {
+  if (!ctx) return RK_ERR_ARG;
+  if (!ctx->dist) return fail(ctx, RK_ERR_STATE, "rk_dist_load_csv before rk_dist_init");
+  DistCsv L;
+  dist_csv_local(ctx, slice, bytes, csv_upload_threads(), L);
+  return dist_csv_finish(ctx, L, seqx_len, seqy_len, total_frags, flags, stats, csv);
 }
 
 int rk_dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flags, rk_result *out, rk_dist_info *info) {
@@ -1418,6 +1548,63 @@ int rk_multi_load_aos(rk_multi *mg, const void *frags, uint64_t n, uint64_t seqx
   if (stats) {
     *stats = st[0];
     for (int r = 1; r < mg->n; ++r) stats->n_launches += st[r].n_launches;
+  }
+  mg->have_load = true;
+  return RK_OK;
+}
+
+int rk_multi_load_csv(rk_multi *mg, const char *body, uint64_t bytes, uint64_t seqx_len, uint64_t seqy_len, uint64_t total_frags,
+                      unsigned flags, rk_load_stats *stats, rk_csv_stats *csv) {
+  if (!mg || (!body && bytes)) return RK_ERR_ARG;
+  mg->have_load = false;
+  if (bytes && is_device_pointer(body)) {
+    mg->err = "rk_multi_load_csv takes the text in host memory";
+    return RK_ERR_ARG;
+  }
+  // cut r: one byte past the first '\n' at or after bytes * r / N (the end of the text when there is none)
+  const int n = mg->n;
+  std::vector<u64> lo(n + 1, bytes);
+  lo[0] = 0;
+  for (int r = 1; r < n; ++r) {
+    const u64 a = bytes * (u64)r / (u64)n;
+    const void *nl = a < bytes ? memchr(body + a, '\n', bytes - a) : nullptr;
+    lo[r] = nl ? (u64)((const char *)nl - body) + 1 : bytes;
+  }
+  // step 1, the local half on every rank; the capacity follows from the rows each rank may load: the device's accepted
+  // rows plus the rows left to the host (the rule of rk_multi_load_aos: the largest slice x 1.5 + 65536)
+  // the copy threads of all ranks together: those of one rk_load_csv, or one per rank (its own thread) when there are more ranks
+  const int threads = std::max(1, csv_upload_threads() / n);
+  std::vector<DistCsv> loc(n);
+  int rc = run_ranks(mg, [&](int r) {
+    dist_csv_local(mg->ctx[r], body + lo[r], lo[r + 1] - lo[r], threads, loc[r]);
+    return RK_OK;
+  });
+  if (rc) return rc;
+  u64 biggest = 0;
+  for (int r = 0; r < n; ++r)
+    if (!loc[r].rc) biggest = std::max(biggest, loc[r].p.n_dev_acc + loc[r].p.n_host);
+  const u64 want = biggest + biggest / 2 + (1u << 16);
+  if (want > mg->cap && (rc = multi_set_capacity(mg, want))) return rc;
+  // step 2, the collective half
+  std::vector<rk_load_stats> st(n);
+  std::vector<rk_csv_stats> cs(n);
+  rc = run_ranks(mg, [&](int r) { return dist_csv_finish(mg->ctx[r], loc[r], seqx_len, seqy_len, total_frags, flags, &st[r], &cs[r]); });
+  if (rc) return rc;
+  if (stats) {
+    *stats = st[0];
+    for (int r = 1; r < n; ++r) {
+      stats->n_launches += st[r].n_launches;
+      stats->ms_stage[RK_ST_H2D] = std::max(stats->ms_stage[RK_ST_H2D], st[r].ms_stage[RK_ST_H2D]);
+    }
+  }
+  if (csv) {
+    memset(csv, 0, sizeof *csv);
+    for (int r = 0; r < n; ++r) {
+      csv->n_rows += cs[r].n_rows, csv->n_accepted += cs[r].n_accepted, csv->n_host_rows += cs[r].n_host_rows;
+      csv->wide |= cs[r].wide;
+      csv->ms_upload = std::max(csv->ms_upload, cs[r].ms_upload);
+      csv->ms_parse = std::max(csv->ms_parse, cs[r].ms_parse);
+    }
   }
   mg->have_load = true;
   return RK_OK;

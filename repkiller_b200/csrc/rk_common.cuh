@@ -163,7 +163,7 @@ int launch_decode(const u8 *aos, u64 n, Geometry g, u32 *xs, u32 *ys, u32 *len, 
 
 // K1 for the compact ingest: {xStart, yStart, length, ident} words + strand bytes instead of 109-byte records
 int launch_decode_packed(const uint4 *key4, const u8 *strand, u64 n, Geometry g, u32 *key0, u32 *link_x, u32 *link_y, u32 *n_dropped,
-                         u32 *err, cudaStream_t st, uint4 *rec4, HistOut hist);
+                         u32 *err, cudaStream_t st, uint4 *rec4, HistOut hist, u32 fidx_base = 0);
 
 // K2: stable LSD radix sort of (key,value) pairs; result in keys_out/vals_out.
 u64 sort_work_bytes(u64 n);
@@ -268,6 +268,20 @@ __device__ __forceinline__ LineRow line_row_of_record(const u8 *rec) {
   f.strand = rec[OFF_STRAND];
   return f;
 }
+// the compact rows of rk_load_packed / rk_load_csv: {xStart, yStart, length, ident} {xEnd, yEnd, score, similarity bits}, strand
+struct PackedRows {
+  const uint4 *key, *rest;
+  const u8 *strand;
+};
+// the same fields from the compact rows: two 16-byte words and a byte per row
+__device__ __forceinline__ LineRow line_row_of_packed(const uint4 *pk_key, const uint4 *pk_rest, const u8 *pk_strand, u32 fidx) {
+  LineRow f;
+  const uint4 k = pk_key[fidx], r = pk_rest[fidx];
+  f.xs = k.x, f.ys = k.y, f.len = k.z, f.ident = k.w;
+  f.xe = r.x, f.ye = r.y, f.score = r.z, f.sim_bits = r.w;
+  f.strand = pk_strand[fidx];
+  return f;
+}
 // K6: the text of output lines first_line .. first_line+n_lines (commonFunctions.cpp:101-115) from the loaded records and
 // the result arrays of the last grouping.
 struct FormatArgs {
@@ -348,7 +362,9 @@ int dist_or_rows(const u32 *all, u64 row_stride, int nr, u64 words, u32 *out, cu
 // cuts = the ranks' first file indices); the owner answers with the line row, stored at the asking rank's rows[line]
 int dist_line_ask_push(const u32 *order, u32 n, const u32 *file_cuts, int nr, uint4 *const *outs, u32 out_cap, u32 *tile_cnt,
                        const u32 *counts_all, u32 row_stride, int me, cudaStream_t st);
-int dist_line_answer(const uint4 *requests, u32 n, const u8 *aos, u32 file_lo, const ScatterTable &back, cudaStream_t st);
+// (the owner's rows: its 109-byte records aos, or its compact rows pk when aos is null)
+int dist_line_answer(const uint4 *requests, u32 n, const u8 *aos, const PackedRows &pk, u32 file_lo, const ScatterTable &back,
+                     cudaStream_t st);
 
 // sort_groups as a function of (groups, diag_func): h = |y - d| per member, member index, zero identity (sol.cu)
 int launch_member_keys(const u64 *y, const u64 *d, u32 m, u32 *h, u32 *idx, float *zero, u32 *err, cudaStream_t st);

@@ -200,6 +200,8 @@ struct CsvScratch {
       if (e) cudaEventDestroy(e);
   }
 };
+// the parse's events on ctx->ev, after the ones a load records (0..7)
+enum { EV_CSV_UP0 = 8, EV_CSV_UP1, EV_CSV_PARSED };
 
 // What a load writes and a grouping only reads: the load's sizes, the records (staged, or the caller's device pointer),
 // the processing order, the bucket sorts of both axes and h (carve_load), plus the side copy of a compact load.  A
@@ -342,5 +344,33 @@ int format_to_host(rk_ctx *ctx, u64 nbytes, char *dst, float *ms_device);
 // K8 into ctx->d_stats (and ctx->h_stats with RK_F_HOST_RESULT); see launch_group_stats.  Synchronises.
 int group_stats_run(rk_ctx *ctx, unsigned flags, const u32 *order, const u32 *gid, const float *identity, const uint4 *rec4,
                     const LineRow *rows, u32 m, u64 ng, u32 gid_base, u32 line_off);
+
+// capi.cu: rk_load_csv's parse in two halves, shared with rk_dist_load_csv (multi.cu), which exchanges the counts of
+// the first half over the ranks before it runs the second.
+struct CsvParse {
+  bool on_device = false;    // the caller's text is in device memory
+  const u8 *text = nullptr;  // the text on the device: the caller's, or the context's copy
+  u64 bytes = 0;
+  u64 n_rows = 0;            // '\n' + 1: the segment after the last '\n' is a row too
+  u64 n_host = 0;            // rows left to the host parser
+  u64 n_dev_acc = 0;         // rows accepted on the device
+  bool wide = false;         // an accepted row has a value of 33 or more bits
+  u64 *start = nullptr;      // the row arrays in CsvScratch::rows
+  u32 *slot = nullptr, *row_bsum = nullptr;
+  u8 *status = nullptr;
+  std::vector<u32> host_rows;  // the host rows readFragment accepted, and their 109-byte records
+  std::vector<u8> host_recs;
+  u64 n_accepted() const { return n_dev_acc + host_rows.size(); }
+};
+// copy threads of one text upload
+int csv_upload_threads();
+// The local half: text scratch, upload with the newline counts (at most `threads` copy threads), tile scan, row starts,
+// classify and the host rows.  Records ev[EV_CSV_UP0] and ev[EV_CSV_UP1].  Synchronises.
+int csv_parse_local(rk_ctx *ctx, const char *body, u64 bytes, int threads, CsvParse &p);
+// bytes of the parsed rows of n accepted rows: three compact arrays, or 109-byte records when wide
+u64 csv_out_bytes(u64 n, bool wide);
+// The emit: the host-accepted records to the device, `out` grown to csv_out_bytes, and every accepted row at its
+// file-order slot in it; *o says where the rows are.  Records ev[EV_CSV_PARSED].
+int csv_emit(rk_ctx *ctx, const CsvParse &p, GrowBuffer &out, CsvOut *o);
 
 }  // namespace rk

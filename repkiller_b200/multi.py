@@ -22,6 +22,34 @@ def slice_bounds(n: int, rank: int, world: int) -> tuple[int, int]:
     return cut(rank), cut(rank + 1)
 
 
+def csv_slice_bounds(path: str, body_pos: int, rank: int, world: int, window: int = 1 << 16) -> tuple[int, int]:
+    """[lo, hi) of rank's slice of a GECKO CSV file whose body (the bytes after the 16 header lines) starts at byte
+    body_pos, for rk_dist_load_csv: cut r is one byte past the first newline at or after body byte bytes * r / world, or
+    the end of the file when there is none (rk_multi_load_csv's rule).  Only a window after each of the two cuts is read,
+    so each process reads just the bytes around its own slice."""
+    import os
+    size = os.path.getsize(path)
+    n = size - body_pos
+
+    def cut(r: int, f) -> int:
+        if r <= 0:
+            return body_pos
+        if r >= world:
+            return size
+        pos = body_pos + n * r // world
+        while pos < size:
+            f.seek(pos)
+            chunk = f.read(window)
+            k = chunk.find(b"\n")
+            if k >= 0:
+                return pos + k + 1
+            pos += len(chunk)
+        return size
+
+    with open(path, "rb") as f:
+        return cut(rank, f), cut(rank + 1, f)
+
+
 def default_capacity(n_per_rank: int) -> int:
     """workspace rows per rank: room for an uneven partition (the cuts of the output exchange balance sort_groups work, not
     lines: a rank whose groups are small gets more lines)"""
