@@ -190,11 +190,25 @@ void read_stream_rest(std::ifstream &in, FragsText &out) {
   }
 }
 
+// Both public constructors delegate to the empty one first, so that the destructor releases the contexts and buffers when
+// ingest() throws.
 FragmentsDatabase::FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, const std::vector<int> &devices,
-                                     FragsInput input) {
+                                     FragsInput input)
+    : FragmentsDatabase() {
+  ingest(frags_file, seq_manager, devices, input, false);
+}
+
+FragmentsDatabase::FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, const std::vector<int> &devices,
+                                     CsvOnDevice)
+    : FragmentsDatabase() {
+  ingest(frags_file, seq_manager, devices, FragsInput::csv, true);
+}
+
+void FragmentsDatabase::ingest(std::ifstream &frags_file, sequence_manager &seq_manager, const std::vector<int> &devices,
+                               FragsInput input, bool csv_on_device) {
   using clk = std::chrono::steady_clock;
   const auto t0 = clk::now();
-  // CUDA start-up (a few hundred ms) runs beside the file read and the parse
+  // CUDA start-up (a few hundred ms, every device's) runs beside the file read and the host parse
   std::thread create_thread([this, &devices] {
     if (devices.size() > 1) multi_ = rk_create_multi(devices.data(), (int)devices.size());
     else ctx_ = rk_create(devices.empty() ? 0 : devices[0]);
@@ -204,10 +218,10 @@ FragmentsDatabase::FragmentsDatabase(std::ifstream &frags_file, sequence_manager
     ~Joiner() { if (t.joinable()) t.join(); }
   } create_joiner{create_thread};
   // slurp the rest of the stream in one read; lines are split on '\n' like std::getline
-  FragsText text;
-  read_stream_rest(frags_file, text);
-  const char *data = text.data;
-  const size_t size = text.size;
+  std::unique_ptr<FragsText> text(new FragsText);
+  read_stream_rest(frags_file, *text);
+  const char *data = text->data;
+  const size_t size = text->size;
   const auto t1 = clk::now();
   const FragsHead head = read_frags_head(data, size, input);
   header = head.header;
@@ -216,74 +230,90 @@ FragmentsDatabase::FragmentsDatabase(std::ifstream &frags_file, sequence_manager
   const uint64_t total_frags = head.total_frags;
   seq_manager.read_header(header);
   vsize = 1 + seq_manager.get_sequence_by_label(0).len / 10;  // :84
-
-  // The device gets the compact form (rk_load_packed: 33 B per fragment over PCIe instead of the 109-byte record): pinned
-  // memory for it is allocated beside the parse, for min(T, bytes / 28) records — a full GECKO row has 14 non-empty
-  // fields and 13 commas, i.e. at least 30 bytes with its line end.  This is only a guess: readFragment's short-row
-  // padding also accepts rows like "Frag,5" (7 bytes), so the count is checked after the parse and the buffers are
-  // re-allocated for exactly `accepted` records when the guess was too small.  (A binary file states its count.)
-  const uint64_t rows_upper = head.binary ? total_frags : (size - head.body_pos) / 28 + 1;
-  cap_ = (rows_upper < total_frags ? rows_upper : total_frags) + 2;
   create_thread.join();
   if (!ctx_ && !multi_) throw std::runtime_error(std::string("repkiller-b200: ") + rk_create_error());
-  auto packed_bytes = [](uint64_t cap) { return cap * 33 + 64; };
-  std::thread alloc_thread([this, &packed_bytes] { packed_ = (unsigned char *)rk_host_alloc(packed_bytes(cap_)); });
-  Joiner alloc_joiner{alloc_thread};
-  std::vector<std::vector<FragFile>> chunks = read_frags_records(data, size, head, 0);
-  uint64_t accepted = 0;
-  for (const auto &c : chunks) accepted += c.size();
-  alloc_thread.join();
-  if (accepted > total_frags) throw std::runtime_error("Unexpected number of fragments");  // :99
-  if (accepted > cap_) {  // short rows: more records than bytes / 28
-    if (packed_) rk_host_free(packed_);
-    cap_ = accepted;
-    packed_ = (unsigned char *)rk_host_alloc(packed_bytes(cap_));
-  }
-  records_ = (FragFile *)malloc((accepted ? accepted : 1) * sizeof(FragFile));
-  if (!records_ || !packed_) throw std::runtime_error("Could not allocate memory for fragments!");  // :86
-  // records in file order (the facades hand out pointers into them) and, beside them, the compact arrays for the device:
-  // key4 = {xStart, yStart, length, ident}, rest4 = {xEnd, yEnd, score, similarity bits}, one strand byte
-  uint32_t *key4 = (uint32_t *)packed_, *rest4 = key4 + 4 * cap_;
-  unsigned char *strand = (unsigned char *)(rest4 + 4 * cap_);
-  std::atomic<bool> wide{false};  // a value beyond 32 bits: the device then takes the 109-byte records (rk_load_aos)
-  {
-    std::vector<std::thread> pool;
-    uint64_t off = 0;
-    for (auto &c : chunks) {
-      if (!c.empty())
-        pool.emplace_back([this, off, &c, key4, rest4, strand, &wide] {
-          memcpy(records_ + off, c.data(), c.size() * sizeof(FragFile));
-          bool w = false;
-          for (size_t k = 0; k < c.size(); ++k) {
-            const FragFile &f = c[k];
-            const uint64_t i = off + k;
-            w = w || ((f.xStart | f.yStart | f.length | f.ident | f.xEnd | f.yEnd | f.score) >> 32) != 0;
-            key4[4 * i] = (uint32_t)f.xStart, key4[4 * i + 1] = (uint32_t)f.yStart, key4[4 * i + 2] = (uint32_t)f.length, key4[4 * i + 3] = (uint32_t)f.ident;
-            rest4[4 * i] = (uint32_t)f.xEnd, rest4[4 * i + 1] = (uint32_t)f.yEnd, rest4[4 * i + 2] = (uint32_t)f.score;
-            memcpy(&rest4[4 * i + 3], &f.similarity, 4);
-            strand[i] = (unsigned char)f.strand;
-          }
-          if (w) wide = true;
-        });
-      off += c.size();
-    }
-    for (auto &th : pool) th.join();
-  }
-  count_ = accepted;
-  const auto t2 = clk::now();
 
-  const uint64_t lx1 = seq_manager.get_sequence_by_label(0).len, ly1 = seq_manager.get_sequence_by_label(1).len;
-  if (multi_) {  // the ranks take consecutive slices of the records
-    if (rk_multi_load_aos(multi_, records_, count_, lx1, ly1, RK_F_TIMING, &load_stats_) != RK_OK)
-      throw std::runtime_error(std::string("repkiller-b200: ") + rk_multi_last_error(multi_));
+  int rc;
+  uint64_t accepted = 0;
+  auto t2 = clk::now();
+  if (csv_on_device) {  // the device splits and parses the rows; over several devices every one parses its slice
+    const char *body = data + head.body_pos;
+    const uint64_t bytes = size - head.body_pos;
+    rc = multi_ ? rk_multi_load_csv(multi_, body, bytes, head.seqx_len, head.seqy_len, total_frags, RK_F_TIMING, &load_stats_, &csv_stats_)
+                : rk_load_csv(ctx_, body, bytes, head.seqx_len, head.seqy_len, total_frags, RK_F_TIMING, &load_stats_, &csv_stats_);
   } else {
-    const int rc = wide ? rk_load_aos(ctx_, records_, count_, lx1, ly1, RK_F_TIMING, &load_stats_)
-                        : rk_load_packed(ctx_, key4, strand, rest4, count_, lx1, ly1, RK_F_TIMING, &load_stats_);
-    if (rc != RK_OK) throw std::runtime_error(std::string("repkiller-b200: ") + rk_last_error(ctx_));
+    // The device gets the compact form (rk_load_packed: 33 B per fragment over PCIe instead of the 109-byte record):
+    // pinned memory for it is allocated beside the parse, for min(T, bytes / 28) records — a full GECKO row has 14
+    // non-empty fields and 13 commas, i.e. at least 30 bytes with its line end.  This is only a guess: readFragment's
+    // short-row padding also accepts rows like "Frag,5" (7 bytes), so the count is checked after the parse and the buffers
+    // are re-allocated for exactly `accepted` records when the guess was too small.  (A binary file states its count.)
+    const uint64_t rows_upper = head.binary ? total_frags : (size - head.body_pos) / 28 + 1;
+    uint64_t cap = (rows_upper < total_frags ? rows_upper : total_frags) + 2;
+    auto packed_bytes = [](uint64_t records) { return records * 33 + 64; };
+    std::thread alloc_thread([this, cap, &packed_bytes] { packed_ = (unsigned char *)rk_host_alloc(packed_bytes(cap)); });
+    Joiner alloc_joiner{alloc_thread};
+    std::vector<std::vector<FragFile>> chunks = read_frags_records(data, size, head, 0);
+    for (const auto &c : chunks) accepted += c.size();
+    alloc_thread.join();
+    if (accepted > total_frags) throw std::runtime_error("Unexpected number of fragments");  // :99
+    if (accepted > cap) {  // short rows: more records than bytes / 28
+      if (packed_) rk_host_free(packed_);
+      cap = accepted;
+      packed_ = (unsigned char *)rk_host_alloc(packed_bytes(cap));
+    }
+    records_ = (FragFile *)malloc((accepted ? accepted : 1) * sizeof(FragFile));
+    if (!records_ || !packed_) throw std::runtime_error("Could not allocate memory for fragments!");  // :86
+    // records in file order (the facades hand out pointers into them) and, beside them, the compact arrays for the device:
+    // key4 = {xStart, yStart, length, ident}, rest4 = {xEnd, yEnd, score, similarity bits}, one strand byte
+    uint32_t *key4 = (uint32_t *)packed_, *rest4 = key4 + 4 * cap;
+    unsigned char *strand = (unsigned char *)(rest4 + 4 * cap);
+    std::atomic<bool> wide{false};  // a value beyond 32 bits: the device then takes the 109-byte records (rk_load_aos)
+    {
+      std::vector<std::thread> pool;
+      uint64_t off = 0;
+      for (auto &c : chunks) {
+        if (!c.empty())
+          pool.emplace_back([this, off, &c, key4, rest4, strand, &wide] {
+            memcpy(records_ + off, c.data(), c.size() * sizeof(FragFile));
+            bool w = false;
+            for (size_t k = 0; k < c.size(); ++k) {
+              const FragFile &f = c[k];
+              const uint64_t i = off + k;
+              w = w || ((f.xStart | f.yStart | f.length | f.ident | f.xEnd | f.yEnd | f.score) >> 32) != 0;
+              key4[4 * i] = (uint32_t)f.xStart, key4[4 * i + 1] = (uint32_t)f.yStart, key4[4 * i + 2] = (uint32_t)f.length, key4[4 * i + 3] = (uint32_t)f.ident;
+              rest4[4 * i] = (uint32_t)f.xEnd, rest4[4 * i + 1] = (uint32_t)f.yEnd, rest4[4 * i + 2] = (uint32_t)f.score;
+              memcpy(&rest4[4 * i + 3], &f.similarity, 4);
+              strand[i] = (unsigned char)f.strand;
+            }
+            if (w) wide = true;
+          });
+        off += c.size();
+      }
+      for (auto &th : pool) th.join();
+    }
+    t2 = clk::now();
+    const uint64_t lx1 = seq_manager.get_sequence_by_label(0).len, ly1 = seq_manager.get_sequence_by_label(1).len;
+    rc = multi_  ? rk_multi_load_aos(multi_, records_, accepted, lx1, ly1, RK_F_TIMING, &load_stats_)  // consecutive slices per rank
+         : wide  ? rk_load_aos(ctx_, records_, accepted, lx1, ly1, RK_F_TIMING, &load_stats_)
+                 : rk_load_packed(ctx_, key4, strand, rest4, accepted, lx1, ly1, RK_F_TIMING, &load_stats_);
+  }
+  if (rc != RK_OK) {
+    const std::string err = multi_ ? rk_multi_last_error(multi_) : rk_last_error(ctx_);
+    // the device parser's count refusal, as the host route throws it (:99); over several devices it carries a "rank r: " prefix
+    if (rc == RK_ERR_RANGE && err.find("Unexpected number of fragments") != std::string::npos)
+      throw std::runtime_error("Unexpected number of fragments");
+    throw std::runtime_error("repkiller-b200: " + err);
   }
   const auto t3 = clk::now();
+  count_ = csv_on_device ? load_stats_.n_loaded : accepted;
+  device_parser_ = csv_on_device;
+  if (csv_on_device) {  // the text is kept for records(), which parses it with the host parser on first use
+    body_pos_ = head.body_pos;
+    text_ = std::move(text);
+  }
   ms_read_ = std::chrono::duration<double, std::milli>(t1 - t0).count();
-  ms_parse_ = std::chrono::duration<double, std::milli>(t2 - t1).count();
+  // host route: the host parse; device route: the device's text upload and row parse (over several devices the largest rank's)
+  ms_parse_ = csv_on_device ? csv_stats_.ms_upload + csv_stats_.ms_parse : std::chrono::duration<double, std::milli>(t2 - t1).count();
   ms_device_load_ = std::chrono::duration<double, std::milli>(t3 - t2).count();
 }
 
@@ -309,7 +339,7 @@ void FragmentsDatabase::build_buckets() const {
   buckets_ = std::move(b);
 }
 
-// After rk_load_csv the host records come from the kept text, parsed by the host parser: the same records the device
+// After a device parse the host records come from the kept text, parsed by the host parser: the same records the device
 // loaded (both apply readFragment's rules), and the same bytes the host route's constructor holds.
 const FragFile *FragmentsDatabase::records() const {
   std::call_once(records_once_, [this] {

@@ -1,7 +1,8 @@
 // Drop-in for the reference's FragmentsDatabase (/root/reference/src/FragmentsDatabase.h:15-35): same
 // constructor and accessors, but the per-bucket vector<FragFile>[] is replaced by the records in file order
-// plus the device-side processing order built by the load (rk_load_packed / rk_load_aos after the host parser, or
-// rk_load_csv, which parses the rows on the device).
+// plus the device-side processing order built by the load.  Every constructor runs one routine (ingest): the file read
+// beside the CUDA start-up, the 16 header lines, then one load call — the host parser's records to rk_load_packed /
+// rk_load_aos / rk_multi_load_aos, or the CSV body to rk_load_csv / rk_multi_load_csv, which parse the rows on the devices.
 #pragma once
 
 #include <cstdint>
@@ -47,21 +48,20 @@ struct FragsText {
 };
 void read_stream_rest(std::ifstream &in, FragsText &out);
 
-// Tag of the constructors that parse the CSV rows on the device (host/FragmentsDatabaseDeviceCsv.cpp, rk_load_csv; over
-// several devices host/FragmentsDatabaseMultiCsv.cpp, rk_multi_load_csv).
+// Tag of the constructors that parse the CSV rows on the device (rk_load_csv; over several devices rk_multi_load_csv).
 struct CsvOnDevice {};
 
 class FragmentsDatabase {
-  mutable FragFile *records_ = nullptr;  // file order (built by records() on first use after rk_load_csv)
+  mutable FragFile *records_ = nullptr;  // file order (built by records() on first use after a device parse)
   unsigned char *packed_ = nullptr;  // pinned: the compact arrays handed to rk_load_packed
-  uint64_t count_ = 0, cap_ = 0;
+  uint64_t count_ = 0;
   size_t vsize = 0;
   rk_ctx *ctx_ = nullptr;
   rk_multi *multi_ = nullptr;  // several GPUs: one comparison partitioned over them (rk_create_multi)
   std::string header;
   rk_load_stats load_stats_{};
   double ms_read_ = 0, ms_parse_ = 0, ms_device_load_ = 0;  // host wall clock of the three ingest phases
-  // rk_load_csv: the file, kept so that records() can parse it on the host when a caller asks for host records
+  // device parse: the file, kept so that records() can parse it on the host when a caller asks for host records
   mutable std::unique_ptr<FragsText> text_;
   size_t body_pos_ = 0;
   mutable std::once_flag records_once_;
@@ -71,6 +71,10 @@ class FragmentsDatabase {
   mutable std::unique_ptr<std::vector<FragFile>[]> buckets_;
   mutable std::once_flag buckets_once_;
   void build_buckets() const;
+  FragmentsDatabase() = default;
+  // the body of every constructor; devices.size() > 1 partitions the comparison over them
+  void ingest(std::ifstream &frags_file, sequence_manager &seq_manager, const std::vector<int> &devices, FragsInput input,
+              bool csv_on_device);
 
  public:
   // The grouping contexts of the facades (generate_fragment_groups, generate_diagonal_func, group_and_sort), so that they
@@ -92,19 +96,20 @@ class FragmentsDatabase {
  public:
   // Parses the GECKO CSV exactly like the reference (16 header lines, Frag rows, readFragment's accept/pad
   // rules), fills seq_manager, then hands the records to the GPU.  Throws std::runtime_error like the
-  // reference on "Unexpected number of fragments"; also on device errors (message from rk_last_error).
+  // reference on "Unexpected number of fragments"; also on device errors (message from rk_last_error).  Every
+  // constructor that throws has released the contexts and buffers it made.
   FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, int device = 0, FragsInput input = FragsInput::csv)
       : FragmentsDatabase(frags_file, seq_manager, std::vector<int>{device}, input) {}
   // several devices: the comparison is partitioned over them (rk_multi_*); ctx() is then null and multi() is set
   // input = gecko_binary: the stream is a .frags file; every record loads as readFragment would load its CSV row
   FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, const std::vector<int> &devices,
                     FragsInput input = FragsInput::csv);
-  // One device, CSV input: the rows are parsed on the device (rk_load_csv) into the same database the host parser plus
-  // rk_load_packed / rk_load_aos builds.  The file text is kept; records(), begin() and the facades that read host
-  // records parse it on first use with the host parser (parse_rows_parallel), so they hand out the same records.
-  FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, int device, CsvOnDevice);
-  // Several devices, CSV input: every device parses its slice of the rows (rk_multi_load_csv); ctx() is null and multi()
-  // set, as with the host parser's constructor for several devices.  The text is kept for records() as above.
+  // CSV input with the rows parsed on the device (rk_load_csv; over several devices every one parses its slice,
+  // rk_multi_load_csv) into the same database the host parser's constructor builds.  The file text is kept; records(),
+  // begin() and the facades that read host records parse it on first use with the host parser (parse_rows_parallel), so
+  // they hand out the same records.
+  FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, int device, CsvOnDevice)
+      : FragmentsDatabase(frags_file, seq_manager, std::vector<int>{device}, CsvOnDevice{}) {}
   FragmentsDatabase(std::ifstream &frags_file, sequence_manager &seq_manager, const std::vector<int> &devices, CsvOnDevice);
   ~FragmentsDatabase();
   FragmentsDatabase(const FragmentsDatabase &) = delete;

@@ -96,10 +96,8 @@ int main(int argc, char *argv[]) {
   // (beside the reference's CSV: GECKO's binary .frags container, see FragmentsDatabase.h).  CSV input: the rows are parsed
   // on the device, over several devices each parsing its slice; .frags input takes the host parser.
   const FragsInput input = detect_frags_input(multifrags_path, frags_file);
-  std::unique_ptr<FragmentsDatabase> db_owner(
-      input != FragsInput::csv ? new FragmentsDatabase(frags_file, seq_manager, devices, input)
-      : devices.size() == 1    ? new FragmentsDatabase(frags_file, seq_manager, devices[0], CsvOnDevice{})
-                               : new FragmentsDatabase(frags_file, seq_manager, devices, CsvOnDevice{}));
+  std::unique_ptr<FragmentsDatabase> db_owner(input == FragsInput::csv ? new FragmentsDatabase(frags_file, seq_manager, devices, CsvOnDevice{})
+                                                                       : new FragmentsDatabase(frags_file, seq_manager, devices, input));
   const FragmentsDatabase &frag_db = *db_owner;
   frags_file.close();
   if (timing) {

@@ -217,58 +217,3 @@ def test_input_format_detection(tmp_path):
     rc, got, _, info = _ingest(tmp_path / "a.frags", tmp_path, env={"RK_INPUT_FORMAT": "csv"})
     assert rc == 0 and info[3] == 0
 
-
-def _fnv(b: bytes) -> str:
-    h = 1469598103934665603
-    for chunk in (b[i:i + (1 << 16)] for i in range(0, len(b), 1 << 16)):
-        for v in chunk:
-            h = ((h ^ v) * 1099511628211) & ((1 << 64) - 1)
-    return f"{h:016x}"
-
-
-def test_constructor_hands_the_same_arrays_to_the_library_for_both_containers(tmp_path):
-    """tests/native/ingest_glue_check.cpp: the FragmentsDatabase constructor linked against a recording stand-in for the
-    library (no GPU, nothing computed).  CSV and .frags input must lead to the same load call — count, sequence lengths,
-    compact arrays — and to the same records and accessors; wide values take the 109-byte route; several devices the
-    partitioned one."""
-    host = os.path.join(ROOT, "repkiller_b200", "csrc", "host")
-    exe = tmp_path / "glue"
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-pthread", "-I", os.path.join(ROOT, "include"), "-o", str(exe),
-                           os.path.join(ROOT, "tests", "native", "ingest_glue_check.cpp"),
-                           os.path.join(host, "FragmentsDatabase.cpp"), os.path.join(host, "GeckoFrags.cpp")])
-    w, rec = _binary_case(n=4_000, seed=11)
-    csv_path, bin_path = tmp_path / "in.csv", tmp_path / "in.frags"
-    frags.write_csv(str(csv_path), rec, w.lx, w.ly)
-    frags.write_gecko_binary(str(bin_path), rec, w.lx, w.ly)
-    want, _, _ = frags.gecko_binary_as_loaded(bin_path.read_bytes())
-
-    def run(path, *extra):
-        p = subprocess.run([str(exe), str(path), *extra], capture_output=True, text=True)
-        assert p.returncode == 0, p.stdout + p.stderr
-        return p.stdout.strip().split("\n")
-
-    a, b = run(csv_path), run(bin_path)
-    assert a[:3] == b[:3] and a[4] == b[4]             # load call, accessors, records, live objects; only the header text differs
-    key4 = np.stack([want["xStart"], want["yStart"], want["length"], want["ident"]], axis=1).astype(np.uint32)
-    rest4 = np.stack([want["xEnd"].astype(np.uint32), want["yEnd"].astype(np.uint32), want["score"].astype(np.uint32),
-                      want["similarity"].view(np.uint32)], axis=1)
-    assert a[0] == (f"call rk_load_packed n={w.n} seqx_len={w.lx + 1} seqy_len={w.ly + 1} key4={_fnv(key4.tobytes())} "
-                    f"strand={_fnv(want['strand'].tobytes())} rest4={_fnv(rest4.tobytes())}")
-    assert a[1] == f"getA={1 + (w.lx + 1) // 10} total={w.n} seqs=2 len0={w.lx + 1} len1={w.ly + 1} max={max(w.lx, w.ly) + 1}"
-    assert a[2] == f"records={_fnv(want.tobytes())}"
-    assert a[3].startswith("header_lines=16 ") and b[3].startswith("header_lines=16 ")
-    assert a[4] == "live ctx=0 multi=0 host=0"
-    # several devices: the records go to the partitioned load
-    m = run(bin_path, "3")
-    assert m[0] == f"call rk_multi_load_aos ranks=3 n={w.n} seqx_len={w.lx + 1} seqy_len={w.ly + 1} records={_fnv(want.tobytes())}"
-    # a value beyond 32 bits: the 109-byte records instead of the compact arrays
-    rec["score"][7] = 2**40
-    frags.write_gecko_binary(str(bin_path), rec, w.lx, w.ly)
-    frags.write_csv(str(csv_path), rec, w.lx, w.ly)
-    want, _, _ = frags.gecko_binary_as_loaded(bin_path.read_bytes())
-    a, b = run(csv_path), run(bin_path)
-    assert a[0] == b[0] == f"call rk_load_aos n={w.n} seqx_len={w.lx + 1} seqy_len={w.ly + 1} records={_fnv(want.tobytes())}"
-    # "Total fragments" smaller than the accepted rows: the reference's exception (FragmentsDatabase.cpp:99)
-    frags.write_csv(str(csv_path), rec, w.lx, w.ly, total_frags=w.n - 1)
-    p = subprocess.run([str(exe), str(csv_path)], capture_output=True, text=True)
-    assert p.returncode == 1 and "Unexpected number of fragments" in p.stdout
