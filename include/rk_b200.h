@@ -317,6 +317,22 @@ int rk_dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flag
 int rk_dist_format_lines(rk_ctx *ctx, uint64_t first_line, uint64_t n_lines, rk_text *out);
 int rk_dist_group_statistics(rk_ctx *ctx, unsigned flags, const rk_group_stats **stats, const rk_group_stats **d_stats,
                              uint64_t *first_gid, uint64_t *n_groups);
+/* Views of a partitioned comparison: a second grouping context per rank over the partition database the ranks loaded,
+ * so that several ratio pairs group one load at the same time.  A rank's view shares its load read-only (the records,
+ * the processing order and the bucket sorts of both passes) and has its own stream, transport, grouping workspace
+ * (mapped into the peers' views) and result, text and statistics buffers.
+ *  - rk_dist_group / rk_dist_format_lines / rk_dist_group_statistics / rk_set_stream work on a view as on its base and
+ *    give bit-identical results for the same pair.  Calls on different contexts of one partitioned load may run at the
+ *    same time from different host threads (on one context they are still serialised by the caller).
+ *  - The partition database is reference-counted per rank: it is freed with the last of the base and its views.
+ *  - rk_dist_load_* (rk_multi_load_*) on a view, or on a base with live views (the message names how many; nothing
+ *    changes), and rk_dist_init on either return RK_ERR_STATE.  rk_create_view refuses rank contexts and views alike.
+ *  - A view of a view shares the same database.
+ * rk_dist_create_view: the process-per-GPU form, collective like rk_dist_init.  Rank 0 calls rk_dist_unique_id and
+ * broadcasts the id; every rank calls rk_dist_create_view on its base, then rk_dist_export and rk_dist_import on the
+ * view.  The view has its own NCCL communicator.  NULL (rk_create_error) when base holds no partitioned load, which
+ * every rank sees alike, or when this rank's workspace cannot be allocated: the other ranks must then destroy theirs. */
+rk_ctx *rk_dist_create_view(rk_ctx *base, const void *id128);
 
 typedef struct rk_multi rk_multi;
 /* One context per listed device.  The ranks push their rows into each other's device memory.  Distinct devices exchange
@@ -348,6 +364,13 @@ int rk_multi_info(const rk_multi *m, int rank, rk_dist_info *info);
  * rk_multi_group_statistics: all groups in gid order, in host memory owned by m (valid until the next call). */
 int rk_multi_format_lines(rk_multi *m, uint64_t first_line, uint64_t n_lines, rk_text *out);
 int rk_multi_group_statistics(rk_multi *m, const rk_group_stats **stats, uint64_t *n_groups);
+/* A view of base's partitioned load (see rk_dist_create_view for what a view shares and the rules): the same devices,
+ * one view context per rank, mapped into each other, with a new NCCL communicator over the devices when base uses NCCL
+ * and its own host-memory group otherwise.  rk_multi_group, rk_multi_format_lines, rk_multi_group_statistics and
+ * rk_multi_info work on it as on base, with its own result buffers; rk_multi_ctx gives its rank contexts.  Destroy it
+ * with rk_destroy_multi, before or after base.  NULL (rk_create_error) before a successful load of base, or when an
+ * allocation fails. */
+rk_multi *rk_multi_create_view(rk_multi *base);
 
 /* Tooling: records start .. start+count of the synthetic workload of repkiller_b200/gen.py, generated on the device
  * (lx, ly are the header values, i.e. loaded length - 1). */

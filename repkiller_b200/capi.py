@@ -26,9 +26,10 @@ SYMBOLS = ["rk_create", "rk_create_view", "rk_create_error", "rk_destroy", "rk_l
            "rk_gen_workload", "rk_sort_members", "rk_group_statistics", "rk_sol_create", "rk_sol_destroy", "rk_sol_insert", "rk_sol_get_associated", "rk_sol_last_error",
            # one comparison over several GPUs
            "rk_dist_unique_id", "rk_dist_init", "rk_dist_export", "rk_dist_import", "rk_dist_load_aos", "rk_dist_load_csv", "rk_dist_group",
-           "rk_dist_format_lines", "rk_dist_group_statistics",
+           "rk_dist_format_lines", "rk_dist_group_statistics", "rk_dist_create_view",
            "rk_create_multi", "rk_destroy_multi", "rk_multi_last_error", "rk_multi_ranks", "rk_multi_ctx", "rk_multi_transport",
-           "rk_multi_load_aos", "rk_multi_load_csv", "rk_multi_group", "rk_multi_info", "rk_multi_format_lines", "rk_multi_group_statistics"]
+           "rk_multi_load_aos", "rk_multi_load_csv", "rk_multi_group", "rk_multi_info", "rk_multi_format_lines", "rk_multi_group_statistics",
+           "rk_multi_create_view"]
 DIST_ID_BYTES, DIST_BLOB_BYTES = 128, 128
 GROUP_STATS_DTYPE = np.dtype([("count", "<u4"), ("x_lo", "<u4"), ("x_hi", "<u4"), ("y_lo", "<u4"), ("y_hi", "<u4"), ("first_line", "<u4"),
                               ("mean_identity", "<f8"), ("multiplicity", "<f8")])
@@ -119,6 +120,8 @@ def load_library():
     L.rk_dist_format_lines.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(_Text)]
     L.rk_dist_group_statistics.argtypes = [C.c_void_p, C.c_uint, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_uint64),
                                            C.POINTER(C.c_uint64)]
+    L.rk_dist_create_view.argtypes = [C.c_void_p, C.c_void_p]
+    L.rk_dist_create_view.restype = C.c_void_p
     L.rk_create_multi.argtypes = [C.POINTER(C.c_int), C.c_int]
     L.rk_create_multi.restype = C.c_void_p
     L.rk_destroy_multi.argtypes = [C.c_void_p]
@@ -135,6 +138,8 @@ def load_library():
     L.rk_multi_info.argtypes = [C.c_void_p, C.c_int, C.POINTER(_DistInfo)]
     L.rk_multi_format_lines.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(_Text)]
     L.rk_multi_group_statistics.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]
+    L.rk_multi_create_view.argtypes = [C.c_void_p]
+    L.rk_multi_create_view.restype = C.c_void_p
     L.rk_sol_create.argtypes = [C.c_int, C.c_double, C.c_double, C.c_uint64]
     L.rk_sol_create.restype = C.c_void_p
     L.rk_sol_destroy.argtypes = [C.c_void_p]
@@ -383,6 +388,18 @@ class Context:
         assert len(unique_id) == DIST_ID_BYTES
         self._check(self._L.rk_dist_init(self._h, rank, world, C.c_char_p(unique_id), cap_per_rank))
 
+    def dist_view(self, unique_id: bytes) -> "Context":
+        """A view of this rank's partitioned load (rk_dist_create_view; collective): a second grouping context with its
+        own stream, NCCL communicator and workspace.  unique_id: a fresh dist_unique_id() of rank 0, broadcast; then
+        every rank calls dist_export / dist_import on the view, as after dist_init."""
+        assert len(unique_id) == DIST_ID_BYTES
+        h = self._L.rk_dist_create_view(self._h, C.c_char_p(unique_id))
+        if not h:
+            raise RkError(-1, self._L.rk_create_error().decode())
+        v = Context._wrap(h, self.device)
+        v._keep = getattr(self, "_keep", None)
+        return v
+
     def dist_export(self) -> bytes:
         buf = C.create_string_buffer(DIST_BLOB_BYTES)
         self._check(self._L.rk_dist_export(self._h, buf))
@@ -566,6 +583,22 @@ class Multi:
     @property
     def transport(self) -> str:
         return self._L.rk_multi_transport(self._h).decode()
+
+    def view(self) -> "Multi":
+        """A second grouping context per rank over this comparison's load (rk_multi_create_view): its own streams,
+        transport, workspace and result buffers.  Different Multi objects of one load may group at the same time from
+        different threads; the load lives until the last of them is closed."""
+        h = self._L.rk_multi_create_view(self._h)
+        if not h:
+            raise RkError(-1, self._L.rk_create_error().decode())
+        v = Multi.__new__(Multi)
+        v._L, v._h, v.n = self._L, h, self.n
+        v._keep = getattr(self, "_keep", None)
+        return v
+
+    def ctx(self, rank: int) -> int:
+        """the handle of rank's context (rk_multi_ctx), for calls on one rank"""
+        return self._L.rk_multi_ctx(self._h, rank)
 
     def close(self):
         if getattr(self, "_h", None):

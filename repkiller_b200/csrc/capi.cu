@@ -15,14 +15,17 @@
 using namespace rk;
 
 namespace {
-
 std::mutex g_create_mu;        // rk_create may run on several threads (one context per GPU)
 std::string g_create_error;   // guarded by g_create_mu; rk_create_error() returns a per-thread copy
 thread_local std::string tl_create_error;
-void set_create_error(const std::string &s) {
+}  // namespace
+
+void rk::set_create_error(const std::string &s) {
   std::lock_guard<std::mutex> lk(g_create_mu);
   g_create_error = s;
 }
+
+namespace {
 
 const char *const kKernelNames[KID_COUNT] = {"k_decode", "k_radix_hist", "k_scan", "k_radix_scatter", "k_keys", "k_match_small",
                                              "k_match_long", "k_chase", "k_hkey", "k_pack", "k_order_tile",

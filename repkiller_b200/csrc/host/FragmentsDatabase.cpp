@@ -369,6 +369,7 @@ const std::vector<FragFile> *FragmentsDatabase::begin() const {
 
 FragmentsDatabase::~FragmentsDatabase() {
   for (rk_ctx *v : pool_.views) rk_destroy(v);
+  for (rk_multi *v : pool_.multi_views) rk_destroy_multi(v);
   if (ctx_) rk_destroy(ctx_);
   if (multi_) rk_destroy_multi(multi_);
   free(records_);

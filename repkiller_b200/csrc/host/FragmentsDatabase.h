@@ -80,13 +80,13 @@ class FragmentsDatabase {
   // The grouping contexts of the facades (generate_fragment_groups, generate_diagonal_func, group_and_sort), so that they
   // may run on several threads at once like the reference's: a call checks out ctx() when it is free, else an idle view
   // of it (rk_create_view, made by commonFunctions.cpp when every pooled context is busy), and checks it back in.  Over
-  // several GPUs the calls take multi_mu instead, one comparison at a time.
+  // several GPUs the same holds for multi() and its views (rk_multi_create_view).
   struct ContextPool {
     std::mutex mu;
-    bool base_busy = false;              // ctx() is checked out
+    bool base_busy = false;              // ctx() (several GPUs: multi()) is checked out
     std::vector<rk_ctx *> views;         // every view made for the pool; destroyed with the database
     std::vector<rk_ctx *> idle_views;    // the ones not checked out
-    std::mutex multi_mu;
+    std::vector<rk_multi *> multi_views, idle_multi_views;  // the same over several GPUs
   };
   ContextPool &pool() const { return pool_; }
 

@@ -59,39 +59,54 @@ void build_groups(const FragmentsDatabase &db, const rk_result &r, FGList &out) 
 [[noreturn]] void device_error(rk_ctx *ctx) { throw std::runtime_error(std::string("repkiller-b200: ") + rk_last_error(ctx)); }
 
 // One grouping context of the database's pool (FragmentsDatabase::ContextPool) for the duration of one facade call:
-// ctx() when it is free, so that one thread makes exactly the calls it always made; else an idle view, or a new one.
-class PooledContext {
+// the base (ctx(), or multi() over several GPUs) when it is free, so that one thread makes exactly the calls it always
+// made; else an idle view, or a new one.  H is rk_ctx or rk_multi.
+template <class H>
+class Pooled {
   const FragmentsDatabase &db_;
-  rk_ctx *ctx_ = nullptr;
+  H *h_ = nullptr;
+  static H *base(const FragmentsDatabase &db);
+  static std::vector<H *> &views(FragmentsDatabase::ContextPool &p);
+  static std::vector<H *> &idle(FragmentsDatabase::ContextPool &p);
+  static H *create_view(H *base);
 
  public:
-  explicit PooledContext(const FragmentsDatabase &db) : db_(db) {
-    if (!db.ctx()) return;  // several GPUs: no single-GPU context (the calls below then report the error)
+  explicit Pooled(const FragmentsDatabase &db) : db_(db) {
+    if (!base(db)) return;  // the other device count: no such context (the calls below then report the error)
     FragmentsDatabase::ContextPool &p = db.pool();
     std::lock_guard<std::mutex> lk(p.mu);
     if (!p.base_busy) {
       p.base_busy = true;
-      ctx_ = db.ctx();
-    } else if (!p.idle_views.empty()) {
-      ctx_ = p.idle_views.back();
-      p.idle_views.pop_back();
-    } else {  // reads only the load of ctx(), which may be grouping on another thread meanwhile
-      ctx_ = rk_create_view(db.ctx());
-      if (!ctx_) throw std::runtime_error(std::string("repkiller-b200: ") + rk_create_error());
-      p.views.push_back(ctx_);
+      h_ = base(db);
+    } else if (!idle(p).empty()) {
+      h_ = idle(p).back();
+      idle(p).pop_back();
+    } else {  // reads only the load of the base, which may be grouping on another thread meanwhile
+      h_ = create_view(base(db));
+      if (!h_) throw std::runtime_error(std::string("repkiller-b200: ") + rk_create_error());
+      views(p).push_back(h_);
     }
   }
-  ~PooledContext() {
-    if (!ctx_) return;
+  ~Pooled() {
+    if (!h_) return;
     FragmentsDatabase::ContextPool &p = db_.pool();
     std::lock_guard<std::mutex> lk(p.mu);
-    if (ctx_ == db_.ctx()) p.base_busy = false;
-    else p.idle_views.push_back(ctx_);
+    if (h_ == base(db_)) p.base_busy = false;
+    else idle(p).push_back(h_);
   }
-  PooledContext(const PooledContext &) = delete;
-  PooledContext &operator=(const PooledContext &) = delete;
-  rk_ctx *get() const { return ctx_; }
+  Pooled(const Pooled &) = delete;
+  Pooled &operator=(const Pooled &) = delete;
+  H *get() const { return h_; }
 };
+template <> rk_ctx *Pooled<rk_ctx>::base(const FragmentsDatabase &db) { return db.ctx(); }
+template <> std::vector<rk_ctx *> &Pooled<rk_ctx>::views(FragmentsDatabase::ContextPool &p) { return p.views; }
+template <> std::vector<rk_ctx *> &Pooled<rk_ctx>::idle(FragmentsDatabase::ContextPool &p) { return p.idle_views; }
+template <> rk_ctx *Pooled<rk_ctx>::create_view(rk_ctx *b) { return rk_create_view(b); }
+template <> rk_multi *Pooled<rk_multi>::base(const FragmentsDatabase &db) { return db.multi(); }
+template <> std::vector<rk_multi *> &Pooled<rk_multi>::views(FragmentsDatabase::ContextPool &p) { return p.multi_views; }
+template <> std::vector<rk_multi *> &Pooled<rk_multi>::idle(FragmentsDatabase::ContextPool &p) { return p.idle_multi_views; }
+template <> rk_multi *Pooled<rk_multi>::create_view(rk_multi *b) { return rk_multi_create_view(b); }
+using PooledContext = Pooled<rk_ctx>;
 
 }  // namespace
 
@@ -162,10 +177,10 @@ FGList *group_and_sort(const FragmentsDatabase &frags_db, double len_ratio, doub
   rk_result r;
   FGList *fgl = new FGList;
   if (frags_db.multi()) {  // one comparison over several GPUs: the ranks' ranges of lines come back concatenated
-    std::lock_guard<std::mutex> lk(frags_db.pool().multi_mu);
-    if (rk_multi_group(frags_db.multi(), len_ratio, pos_ratio, RK_F_TIMING, &r) != RK_OK) {
+    Pooled<rk_multi> pm(frags_db);
+    if (rk_multi_group(pm.get(), len_ratio, pos_ratio, RK_F_TIMING, &r) != RK_OK) {
       delete fgl;
-      throw std::runtime_error(std::string("repkiller-b200: ") + rk_multi_last_error(frags_db.multi()));
+      throw std::runtime_error(std::string("repkiller-b200: ") + rk_multi_last_error(pm.get()));
     }
     build_groups(frags_db, r, *fgl);
   } else {

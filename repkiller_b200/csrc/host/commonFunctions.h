@@ -29,7 +29,7 @@ void generate_diagonal_func(const FragmentsDatabase &fdb, size_t *diag_func);
 // every group are computed on the device (rk_sort_members, K5b) on a context of its own (GPU RK_DEVICE, default 0).
 void sort_groups(FGList &fgl, const size_t *diag_func);
 // One call for the three above (what the CLI uses: no intermediate host lists).  stats' host arrays belong to the
-// context that grouped; over several GPUs the calls are serialised.
+// context that grouped (over several GPUs: its rk_multi), valid until that context's next grouping.
 FGList *group_and_sort(const FragmentsDatabase &frags_db, double len_ratio, double pos_ratio, rk_result *stats = nullptr);
 
 // reference: commonFunctions.cpp:101-146 (the writer; byte-identical output)

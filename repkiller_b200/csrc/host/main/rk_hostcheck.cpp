@@ -17,6 +17,12 @@
 //                                             every pair, run by <threads> threads that share one FragmentsDatabase, as
 //                                             the reference's thread pool does (repkiller.cpp:60-72); pair k writes
 //                                             <out_prefix>-<k>.csv.  Prints how many grouping contexts the facades used (GPU)
+//   rk_hostcheck group_pool <in.csv> <devices> <threads> <len_ratio> <pos_ratio> [<len_ratio> <pos_ratio>]...
+//                                             group_and_sort of every pair on one database over <devices> (a comma list,
+//                                             as RK_DEVICES; "0,0,0" is three ranks on device 0), run by <threads> threads
+//                                             that share it.  Prints "pair <k> groups=<n> lines=<m> hash=<h>" per pair in
+//                                             pair order (h: FNV-1a over the file indices of the members, group by group),
+//                                             then how many grouping contexts the pool used (GPU)
 //   rk_hostcheck steps_pure <in.csv> <out.csv> <len_ratio> <pos_ratio> <len_ratio2> <pos_ratio2>
 //                                             sort_groups is a pure function: a second grouping with other ratios is
 //                                             made BEFORE the first list is sorted; the output is the first one's (GPU)
@@ -253,6 +259,53 @@ int main(int argc, char **argv) {
       return 4;
     }
     printf("%zu pairs on %d threads, %zu grouping contexts\n", pairs.size(), nthreads, 1 + db.pool().views.size());
+    return 0;
+  }
+  if (mode == "group_pool" && argc >= 7) {
+    std::ifstream in(argv[2], std::ifstream::in | std::ifstream::binary);
+    sequence_manager sm;
+    std::vector<int> devices;
+    for (const char *p = argv[3]; *p;) {
+      devices.push_back(atoi(p));
+      while (*p && *p != ',') ++p;
+      if (*p == ',') ++p;
+    }
+    FragmentsDatabase db(in, sm, devices, detect_frags_input(argv[2], in));
+    const int nthreads = std::max(1, atoi(argv[4]));
+    std::vector<std::pair<double, double>> pairs;
+    for (int i = 5; i + 1 < argc; i += 2) pairs.emplace_back(std::stod(argv[i]), std::stod(argv[i + 1]));
+    std::vector<std::string> lines(pairs.size());
+    std::atomic<size_t> next{0};
+    std::mutex err_mu;
+    std::string err;
+    auto worker = [&] {
+      for (size_t k; (k = next++) < pairs.size();) {
+        try {
+          FGList *fgl = group_and_sort(db, pairs[k].first, pairs[k].second);
+          uint64_t h = 1469598103934665603ull, m = 0;
+          auto mix = [&](uint64_t v) { h = (h ^ v) * 1099511628211ull; };
+          for (const FragsGroup *g : *fgl) {
+            for (const FragFile *f : *g) mix((uint64_t)(f - db.records())), ++m;
+            mix(~0ull);
+          }
+          lines[k] = "pair " + std::to_string(k) + " groups=" + std::to_string(fgl->size()) + " lines=" + std::to_string(m) +
+                     " hash=" + std::to_string(h);
+          free_groups(fgl);
+        } catch (const std::exception &e) {
+          std::lock_guard<std::mutex> lk(err_mu);
+          err = e.what();
+        }
+      }
+    };
+    std::vector<std::thread> pool;
+    for (int t = 0; t < nthreads; ++t) pool.emplace_back(worker);
+    for (auto &th : pool) th.join();
+    if (!err.empty()) {
+      fprintf(stderr, "%s\n", err.c_str());
+      return 4;
+    }
+    for (const std::string &l : lines) printf("%s\n", l.c_str());
+    printf("%zu grouping contexts\n", 1 + (db.multi() ? db.pool().multi_views.size() : db.pool().views.size()));
     return 0;
   }
   if (mode == "steps_pure" && argc >= 8) {

@@ -371,27 +371,23 @@ struct Trace {
 
 struct DistBlob {  // what a rank publishes so that its peers can read its parent / root-scan arrays
   u64 pid, ptr, cap;
-  int device, pad;
+  int device, view;  // view: the mapped memory is a view's workspace, not a partition arena
   cudaIpcMemHandle_t handle;
 };
 static_assert(sizeof(DistBlob) <= RK_DIST_BLOB_BYTES, "blob size");
 
-struct Dist {
-  int rank = 0, world = 1;
-  Transport *tr = nullptr;
+// The partition database of a rank: what a load writes and a grouping only reads.  The sizes and exchange tables of the
+// load, the rank's slice of the records, the rank-order and bucket-sorted arrays of both passes, and the load-time
+// regions (rec4_loc, send_rows, rec6_arr, the halo rows) that only the load uses.  The rank's base context and its views
+// (rk_multi_create_view, rk_dist_create_view) hold a reference to it; the last context to be destroyed frees it.  It
+// does not change while views are live: loading is refused then.
+struct DistDb {
+  std::atomic<int> refs{1};
+  GrowBuffer arena;  // carved by dist_carve: this database, then the workspace of the loading context
   u64 cap = 0, hcap = 0;
-  GrowBuffer arena;  // carved by dist_carve for cap rows per rank; grows only (rk_dist_init makes a new Dist)
-  void *peer_open[DIST_MAX_RANKS] = {nullptr};
-  bool peers_ready = false;
-  GrowBuffer small_host{cudaHostAllocDefault};
-  u32 *h_small = nullptr;  // [world][SMALL_WORDS] in small_host
-  PeerTable pt{};
-  Trace trace;
-  cudaStream_t side = nullptr;  // rows that travel while kernels run (the Y exchange beside the X sort)
   // grow-only side buffers whose size depends on the input, not on cap
   GrowBuffer aos_buf;  // this rank's records: a host slice staged (109 B per row), or its parsed CSV rows (compact or 109 B)
   GrowBuffer link_buf;  // u32 [hist0][linkx_loc][linky_loc] (one all-gather) [linkx][linky][gather: world * the first three]
-  GrowBuffer h_res{cudaHostAllocDefault};
 
   // state of the last load
   bool loaded = false;
@@ -404,37 +400,66 @@ struct Dist {
   PackedRows pk_src{};                  // ... or its compact rows (rk_dist_load_csv without a wide value; aos_src == nullptr)
   u32 file_off[DIST_MAX_RANKS] = {0};  // first file index of every rank's slice
   bool slices_in_order = false;         // every slice ends at or before the next rank's starts: file_off[] routes a file index
+  u32 roff[DIST_MAX_RANKS + 1] = {0};   // first rank-order index of every rank, then the total (PeerTable::roff)
+
+  // carved device pointers
+  u32 *cuts0 = nullptr, *cuts_y = nullptr, *cuts_x = nullptr;
+  uint4 *rec4_loc = nullptr, *send_rows = nullptr;
+  uint2 *rec6_arr = nullptr;  // the records this rank owns, in arrival order: 24-byte rows stored by the peers' push kernels
+  u32 *key0_loc = nullptr, *perm_x = nullptr, *perm_y = nullptr;
+  u32 *key0a = nullptr, *k0_r = nullptr, *aidx_r = nullptr;
+  uint2 *xl = nullptr, *yl_r = nullptr, *yl_a = nullptr;
+  u32 *ys_r = nullptr, *kx2 = nullptr, *ky = nullptr, *gfidx_r = nullptr;
+  float *identity_r = nullptr;
+  uint4 *hfi_r = nullptr;
+  uint4 *halo_send = nullptr, *halo_recv = nullptr;
+  u32 *halo_grank = nullptr;
+  u32 *skx = nullptr, *rx = nullptr, *ky_a = nullptr, *grank_a = nullptr, *sky_a = nullptr, *ry_a = nullptr;
+  u32 *roff_dev = nullptr;
+};
+
+// One context's part in a partitioned comparison: its transport, its peers' mappings and its grouping workspace, i.e.
+// everything rk_dist_group, rk_dist_format_lines and rk_dist_group_statistics write.  The load runs on the base context
+// and uses its workspace as scratch too (counters, count rows, sort scratch, recv_rows for the Y rows).
+struct Dist {
+  int rank = 0, world = 1;
+  Transport *tr = nullptr;
+  DistDb *db = nullptr;
+  bool is_view = false;  // groups on another context's database (db is shared), never loads
+  GrowBuffer arena;      // a view's workspace (dist_carve_work); the base's lies in db->arena
+  void *peer_open[DIST_MAX_RANKS] = {nullptr};
+  bool peers_ready = false;
+  GrowBuffer small_host{cudaHostAllocDefault};
+  u32 *h_small = nullptr;  // [world][SMALL_WORDS] in small_host
+  PeerTable pt{};
+  Trace trace;
+  cudaStream_t side = nullptr;  // rows that travel while kernels run (the Y exchange beside the X sort)
+  GrowBuffer h_res{cudaHostAllocDefault};
+  // the memory the peers map: the base's whole partition arena, or a view's workspace (every peer carves it identically)
+  u8 *map_base() const { return (u8 *)(is_view ? arena.ptr() : db->arena.ptr()); }
 
   // state of the last group: this rank's output lines and groups; line rows (RK_F_LINE_RECORDS) valid
   bool have_rows = false;
   u32 n_lines = 0, gid_base = 0, n_groups_rank = 0;
   u64 line_off = 0;
 
-  // carved device pointers
+  // carved device pointers (the workspace)
   Counters *cnt = nullptr;
   u32 *d_small = nullptr, *d_small_all = nullptr, *nroots_mat = nullptr;
   u32 *prehist = nullptr;  // 4 x [4][256]: digit counts of the rank / X / Y / gid sort keys, gathered by their producers
-  u32 *hist = nullptr, *hist_all = nullptr, *cuts0 = nullptr, *cuts_y = nullptr, *cuts_x = nullptr, *cuts_g = nullptr;
-  uint4 *rec4_loc = nullptr, *send_rows = nullptr, *recv_rows = nullptr;
-  uint2 *rec6_arr = nullptr;  // the records this rank owns, in arrival order: 24-byte rows stored by the peers' push kernels
-  LineRow *line_rows = nullptr;  // RK_F_LINE_RECORDS: one row per output line, over rec4_loc ++ send_rows ++ rec6_arr
-  u32 *key0_loc = nullptr, *tile_cnt = nullptr, *perm_x = nullptr, *perm_y = nullptr;
-  u32 *key0a = nullptr, *k0_r = nullptr, *aidx_r = nullptr, *tmp_k = nullptr, *tmp_v = nullptr;
+  u32 *hist = nullptr, *hist_all = nullptr, *cuts_g = nullptr;
+  uint4 *recv_rows = nullptr;
+  LineRow *line_rows = nullptr;  // RK_F_LINE_RECORDS: one row per output line
+  u32 *tile_cnt = nullptr, *tmp_k = nullptr, *tmp_v = nullptr;
   void *sort_work = nullptr;
-  uint2 *xl = nullptr, *yl_r = nullptr, *yl_a = nullptr;
-  u32 *ys_r = nullptr, *kx2 = nullptr, *ky = nullptr, *gfidx_r = nullptr;
-  float *identity_r = nullptr;
-  uint4 *hfi_r = nullptr;
-  uint4 *halo_send = nullptr, *halo_recv = nullptr;
-  u32 *halo_grank = nullptr, *away_res = nullptr;
-  u32 *skx = nullptr, *rx = nullptr, *ky_a = nullptr, *grank_a = nullptr, *sky_a = nullptr, *ry_a = nullptr;
+  u32 *away_res = nullptr;
   u32 *parent_x = nullptr, *xm_bits = nullptr, *parent = nullptr, *gidscan = nullptr, *parent_y = nullptr, *yo_s = nullptr;
   u8 *xm_a = nullptr;
   u32 *ent_rank = nullptr, *ent_c = nullptr, *ent_len = nullptr, *worklist = nullptr;
   u32 work_cap = 0;
   u32 *gid_rank = nullptr, *flag = nullptr, *flag_all = nullptr, *lroot = nullptr, *gid_l = nullptr;
   u32 *pend_idx[2] = {nullptr, nullptr}, *pend_key[2] = {nullptr, nullptr}, *n_pend = nullptr;  // forest: pending lists (double buffered)
-  u32 *apos = nullptr, *roff_dev = nullptr;
+  u32 *apos = nullptr;
   uint4 *queries = nullptr;  // forest bulk rounds: the ranks other GPUs ask this one about (stored by their push kernels)
   u64 *answers = nullptr;    // ... and the answers to this rank's questions, in the order it sent them (stored by the owners)
   u64 *res = nullptr;  // per fragment: what a walker from another GPU needs (k_chase_local); the peers read it
@@ -446,126 +471,147 @@ struct Dist {
   float *out_identity = nullptr;
 };
 
-static u64 dist_carve(Dist &D, u8 *base) {
+// bump allocation of one arena at 256-byte boundaries; base == nullptr only counts the bytes
+struct Carve {
+  u8 *base;
   u64 off = 0;
-  auto take = [&](u64 bytes) -> u8 * {
+  u8 *take(u64 bytes) {
     u8 *p = base ? base + off : nullptr;
     off += align_up(bytes ? bytes : 16, 256);
     return p;
-  };
-  const u64 M = D.cap, H = D.hcap, MC = M + H;
-  const int nr = D.world;
-  D.cnt = (Counters *)take(sizeof(Counters));
-  D.d_small = (u32 *)take(SMALL_WORDS * 4);
-  D.d_small_all = (u32 *)take((u64)nr * SMALL_WORDS * 4);
-  D.nroots_mat = (u32 *)take((u64)nr * SMALL_WORDS * 4);
-  D.prehist = (u32 *)take(4 * 4 * 256 * 4);
-  D.hist = (u32 *)take(DIST_BINS * 4);
-  D.hist_all = (u32 *)take((u64)nr * DIST_BINS * 4);
-  D.cuts0 = (u32 *)take((DIST_MAX_RANKS + 1) * 4);
-  D.cuts_y = (u32 *)take((DIST_MAX_RANKS + 1) * 4);
-  D.cuts_x = (u32 *)take(2 * DIST_MAX_RANKS * 4);
-  D.cuts_g = (u32 *)take((DIST_MAX_RANKS + 1) * 4);
-  D.rec4_loc = (uint4 *)take(M * 32);
-  D.send_rows = (uint4 *)take(M * 16);
-  D.rec6_arr = (uint2 *)take(M * 24);
-  // Only the load reads or writes the three regions above, so after it they hold the line rows of rk_dist_group with
-  // RK_F_LINE_RECORDS: 72 B per row of capacity, back to back, for 64 B per line (a rank never holds more lines than rows).
-  D.line_rows = (LineRow *)D.rec4_loc;
-  static_assert(sizeof(LineRow) <= 32 + 16 + 24, "line rows fit in the load-time regions");
-  D.recv_rows = (uint4 *)take(M * 16);
-  D.key0_loc = (u32 *)take(M * 4);
-  D.tile_cnt = (u32 *)take(dist_split_work_bytes(M));
-  D.perm_x = (u32 *)take(H * 4);
-  D.perm_y = (u32 *)take(M * 4);
-  D.key0a = (u32 *)take(M * 4);
-  D.k0_r = (u32 *)take(M * 4);
-  D.aidx_r = (u32 *)take(M * 4);
-  D.tmp_k = (u32 *)take(MC * 4);
-  D.tmp_v = (u32 *)take(MC * 4);
-  D.sort_work = take(sort_work_bytes(MC));
-  D.xl = (uint2 *)take(MC * 8);
-  D.yl_r = (uint2 *)take(M * 8);
-  D.yl_a = (uint2 *)take(M * 8);
-  D.ys_r = (u32 *)take(M * 4);
-  D.kx2 = (u32 *)take(MC * 4);
-  D.ky = (u32 *)take(M * 4);
-  D.gfidx_r = (u32 *)take(M * 4);
-  D.identity_r = (float *)take(M * 4);
-  D.hfi_r = (uint4 *)take(M * 16);
-  D.halo_send = (uint4 *)take(H * 16);
-  D.halo_recv = (uint4 *)take(H * 16);
-  D.halo_grank = (u32 *)take(H * 4);
-  D.away_res = (u32 *)take(H * 4);
-  D.skx = (u32 *)take(MC * 4);
-  D.rx = (u32 *)take(MC * 4);
-  D.ky_a = (u32 *)take(M * 4);
-  D.grank_a = (u32 *)take(M * 4);
-  D.sky_a = (u32 *)take(M * 4);
-  D.ry_a = (u32 *)take(M * 4);
-  D.parent_x = (u32 *)take(MC * 4);
-  D.xm_bits = (u32 *)take((MC + 31) / 32 * 4);
-  D.parent = (u32 *)take(M * 4);
-  D.gidscan = (u32 *)take(M * 4);
-  D.lroot = (u32 *)take(M * 4);
-  D.gid_l = (u32 *)take(M * 4);
-  for (int b = 0; b < 2; ++b) D.pend_idx[b] = (u32 *)take(M * 4), D.pend_key[b] = (u32 *)take(M * 4);
-  D.n_pend = (u32 *)take(16);
-  D.apos = (u32 *)take(M * 4);
-  D.roff_dev = (u32 *)take((DIST_MAX_RANKS + 1) * 4);
-  D.queries = (uint4 *)take(M * 16);
-  D.answers = (u64 *)take(M * 8);
-  D.res = (u64 *)take(M * 8);
-  D.flag = (u32 *)take(16);
-  D.flag_all = (u32 *)take(DIST_MAX_RANKS * 4);
-  D.parent_y = (u32 *)take(M * 4);
-  D.yo_s = (u32 *)take(M * 4);
-  D.xm_a = take(M);
-  D.ent_rank = (u32 *)take(MC * 4);
-  D.ent_c = (u32 *)take(MC * 4);
-  D.ent_len = (u32 *)take(MC * 4);
-  D.work_cap = (u32)(MC / 32 + 2);
-  D.worklist = (u32 *)take((u64)D.work_cap * 4);
-  D.gid_rank = (u32 *)take(M * 4);
-  D.scan_work = take(dist_scan_work_bytes((u32)M));
-  D.gid_a = (u32 *)take(M * 4);
-  D.sgid = (u32 *)take(M * 4);
-  D.srank_g = (u32 *)take(M * 4);
-  D.order_scratch = take(order_scratch_bytes(M));
-  D.out_order = (u32 *)take(M * 4);
-  D.out_gid = (u32 *)take(M * 4);
-  D.out_repval = take(M);
-  D.out_identity = (float *)take(M * 4);
-  return off;
+  }
+};
+
+// the partition database for B.cap rows per rank (B.hcap halo rows)
+static void dist_carve_db(DistDb &B, Carve &c) {
+  const u64 M = B.cap, H = B.hcap, MC = M + H;
+  B.cuts0 = (u32 *)c.take((DIST_MAX_RANKS + 1) * 4);
+  B.cuts_y = (u32 *)c.take((DIST_MAX_RANKS + 1) * 4);
+  B.cuts_x = (u32 *)c.take(2 * DIST_MAX_RANKS * 4);
+  B.rec4_loc = (uint4 *)c.take(M * 32);
+  B.send_rows = (uint4 *)c.take(M * 16);
+  B.rec6_arr = (uint2 *)c.take(M * 24);
+  B.key0_loc = (u32 *)c.take(M * 4);
+  B.perm_x = (u32 *)c.take(H * 4);
+  B.perm_y = (u32 *)c.take(M * 4);
+  B.key0a = (u32 *)c.take(M * 4);
+  B.k0_r = (u32 *)c.take(M * 4);
+  B.aidx_r = (u32 *)c.take(M * 4);
+  B.xl = (uint2 *)c.take(MC * 8);
+  B.yl_r = (uint2 *)c.take(M * 8);
+  B.yl_a = (uint2 *)c.take(M * 8);
+  B.ys_r = (u32 *)c.take(M * 4);
+  B.kx2 = (u32 *)c.take(MC * 4);
+  B.ky = (u32 *)c.take(M * 4);
+  B.gfidx_r = (u32 *)c.take(M * 4);
+  B.identity_r = (float *)c.take(M * 4);
+  B.hfi_r = (uint4 *)c.take(M * 16);
+  B.halo_send = (uint4 *)c.take(H * 16);
+  B.halo_recv = (uint4 *)c.take(H * 16);
+  B.halo_grank = (u32 *)c.take(H * 4);
+  B.skx = (u32 *)c.take(MC * 4);
+  B.rx = (u32 *)c.take(MC * 4);
+  B.ky_a = (u32 *)c.take(M * 4);
+  B.grank_a = (u32 *)c.take(M * 4);
+  B.sky_a = (u32 *)c.take(M * 4);
+  B.ry_a = (u32 *)c.take(M * 4);
+  B.roff_dev = (u32 *)c.take((DIST_MAX_RANKS + 1) * 4);
 }
 
-static void dist_release_buffers(Dist &D) {
+// a grouping workspace for cap rows per rank (hcap halo rows) over D.world ranks.  A view carries its own line rows,
+// 64 B per row of capacity; the base's overlay the load-time regions of its database (dist_carve).
+static void dist_carve_work(Dist &D, u64 cap, u64 hcap, Carve &c) {
+  const u64 M = cap, H = hcap, MC = M + H;
+  const int nr = D.world;
+  D.cnt = (Counters *)c.take(sizeof(Counters));
+  D.d_small = (u32 *)c.take(SMALL_WORDS * 4);
+  D.d_small_all = (u32 *)c.take((u64)nr * SMALL_WORDS * 4);
+  D.nroots_mat = (u32 *)c.take((u64)nr * SMALL_WORDS * 4);
+  D.prehist = (u32 *)c.take(4 * 4 * 256 * 4);
+  D.hist = (u32 *)c.take(DIST_BINS * 4);
+  D.hist_all = (u32 *)c.take((u64)nr * DIST_BINS * 4);
+  D.cuts_g = (u32 *)c.take((DIST_MAX_RANKS + 1) * 4);
+  D.line_rows = D.is_view ? (LineRow *)c.take(M * sizeof(LineRow)) : (LineRow *)D.db->rec4_loc;
+  D.recv_rows = (uint4 *)c.take(M * 16);
+  D.tile_cnt = (u32 *)c.take(dist_split_work_bytes(M));
+  D.tmp_k = (u32 *)c.take(MC * 4);
+  D.tmp_v = (u32 *)c.take(MC * 4);
+  D.sort_work = c.take(sort_work_bytes(MC));
+  D.away_res = (u32 *)c.take(H * 4);
+  D.parent_x = (u32 *)c.take(MC * 4);
+  D.xm_bits = (u32 *)c.take((MC + 31) / 32 * 4);
+  D.parent = (u32 *)c.take(M * 4);
+  D.gidscan = (u32 *)c.take(M * 4);
+  D.lroot = (u32 *)c.take(M * 4);
+  D.gid_l = (u32 *)c.take(M * 4);
+  for (int b = 0; b < 2; ++b) D.pend_idx[b] = (u32 *)c.take(M * 4), D.pend_key[b] = (u32 *)c.take(M * 4);
+  D.n_pend = (u32 *)c.take(16);
+  D.apos = (u32 *)c.take(M * 4);
+  D.queries = (uint4 *)c.take(M * 16);
+  D.answers = (u64 *)c.take(M * 8);
+  D.res = (u64 *)c.take(M * 8);
+  D.flag = (u32 *)c.take(16);
+  D.flag_all = (u32 *)c.take(DIST_MAX_RANKS * 4);
+  D.parent_y = (u32 *)c.take(M * 4);
+  D.yo_s = (u32 *)c.take(M * 4);
+  D.xm_a = c.take(M);
+  D.ent_rank = (u32 *)c.take(MC * 4);
+  D.ent_c = (u32 *)c.take(MC * 4);
+  D.ent_len = (u32 *)c.take(MC * 4);
+  D.work_cap = (u32)(MC / 32 + 2);
+  D.worklist = (u32 *)c.take((u64)D.work_cap * 4);
+  D.gid_rank = (u32 *)c.take(M * 4);
+  D.scan_work = c.take(dist_scan_work_bytes((u32)M));
+  D.gid_a = (u32 *)c.take(M * 4);
+  D.sgid = (u32 *)c.take(M * 4);
+  D.srank_g = (u32 *)c.take(M * 4);
+  D.order_scratch = c.take(order_scratch_bytes(M));
+  D.out_order = (u32 *)c.take(M * 4);
+  D.out_gid = (u32 *)c.take(M * 4);
+  D.out_repval = c.take(M);
+  D.out_identity = (float *)c.take(M * 4);
+}
+
+// the base's partition arena: the database, then its workspace, whose line rows overlay rec4_loc ++ send_rows ++
+// rec6_arr.  Only the load reads or writes those three regions, so after it they hold the line rows of rk_dist_group
+// with RK_F_LINE_RECORDS: 72 B per row of capacity, back to back, for 64 B per line (a rank never holds more lines than
+// rows).  A view cannot share them (two contexts would write the same rows) and carries its own.
+static u64 dist_carve(Dist &D, u8 *base) {
+  static_assert(sizeof(LineRow) <= 32 + 16 + 24, "line rows fit in the load-time regions");
+  Carve c{base};
+  dist_carve_db(*D.db, c);
+  dist_carve_work(D, D.db->cap, D.db->hcap, c);
+  return c.off;
+}
+
+static void dist_release_peers(Dist &D) {
   for (int r = 0; r < DIST_MAX_RANKS; ++r) {
     if (D.peer_open[r]) cudaIpcCloseMemHandle(D.peer_open[r]);
     D.peer_open[r] = nullptr;
   }
   D.peers_ready = false;
-  D.cap = D.hcap = 0;
-  D.loaded = false;
 }
 
-// grows the partition buffers to cap rows per rank; the peers must import again afterwards
+// grows the partition arena of a base context to cap rows per rank; the peers must import again afterwards
 static int dist_allocate(rk_ctx *ctx, u64 cap) {
   Dist &D = *ctx->dist;
+  DistDb &B = *D.db;
   CK(cudaSetDevice(ctx->device));
   CK(cudaStreamSynchronize(ctx->stream));
-  dist_release_buffers(D);
+  dist_release_peers(D);
+  B.cap = B.hcap = 0;
+  B.loaded = false;
   if (cap < 1024) cap = 1024;
   if (cap >= 0xFFFFFF00ull) return fail(ctx, RK_ERR_ARG, "capacity per rank must stay below 2^32");
-  D.cap = cap;
-  D.hcap = cap / 8 + 65536;
+  B.cap = cap;
+  B.hcap = cap / 8 + 65536;
   std::string err;
-  const int rc = D.arena.reserve(dist_carve(D, nullptr), nullptr, err);
+  const int rc = B.arena.reserve(dist_carve(D, nullptr), nullptr, err);
   if (rc) {
-    dist_release_buffers(D);
+    B.cap = B.hcap = 0;
     return fail(ctx, rc, "%llu rows per rank: %s", (unsigned long long)cap, err.c_str());
   }
-  dist_carve(D, (u8 *)D.arena.ptr());
+  dist_carve(D, (u8 *)B.arena.ptr());
   return RK_OK;
 }
 
@@ -578,19 +624,42 @@ static int tr_fail(rk_ctx *ctx, int rc) { return fail(ctx, rc, "%s", ctx->dist->
     if (rc_ != RK_OK) return tr_fail(ctx, rc_);   \
   } while (0)
 
+// views that share ctx's load: of a single-GPU load (rk_create_view) or of its partition database
+static int live_views(const rk_ctx *ctx) {
+  if (ctx->dist) return ctx->dist->is_view ? 0 : ctx->dist->db->refs - 1;
+  return ctx->db ? ctx->db->refs - 1 : 0;
+}
+
+// the refusals of a load on a rank context, before it touches anything: a view, or a base with live views
+static int dist_load_refusal(rk_ctx *ctx) {
+  if (ctx->dist->is_view)
+    return fail(ctx, RK_ERR_STATE, "a view groups the partition database of the context it was made from; load that context instead");
+  if (const int views = live_views(ctx))
+    return fail(ctx, RK_ERR_STATE, "%d view%s of this context %s live: destroy %s before loading another database", views,
+                views == 1 ? "" : "s", views == 1 ? "is" : "are", views == 1 ? "it" : "them");
+  return RK_OK;
+}
+
+// rk_dist_init on a view, or on a context with live views
+static int dist_init_refusal(rk_ctx *ctx) {
+  if (ctx->is_view) return fail(ctx, RK_ERR_STATE, "a view cannot take part in a partitioned comparison");
+  if (live_views(ctx)) return fail(ctx, RK_ERR_STATE, "views of this context are live: destroy them before rk_dist_init");
+  return RK_OK;
+}
+
 static int dist_init_common(rk_ctx *ctx, int rank, int world, Transport *tr, u64 cap) {
   if (world < 1 || world > DIST_MAX_RANKS || rank < 0 || rank >= world) {
     delete tr;
     return fail(ctx, RK_ERR_ARG, "rank %d of %d: at most %d ranks", rank, world, DIST_MAX_RANKS);
   }
-  if (ctx->is_view || (ctx->db && ctx->db->refs > 1)) {  // partitioned comparisons have no views (rk_create_view)
+  if (const int rc = dist_init_refusal(ctx)) {
     delete tr;
-    return fail(ctx, RK_ERR_STATE, "%s", ctx->is_view ? "a view cannot take part in a partitioned comparison"
-                                                      : "views of this context are live: destroy them before rk_dist_init");
+    return rc;
   }
   dist_destroy(ctx);
   Dist *D = new Dist;
   D->rank = rank, D->world = world, D->tr = tr;
+  D->db = new DistDb;
   tr->rank = rank, tr->world = world;
   ctx->dist = D;
   D->trace.on = getenv("RK_DIST_TRACE") != nullptr;
@@ -602,12 +671,68 @@ static int dist_init_common(rk_ctx *ctx, int rank, int world, Transport *tr, u64
   return dist_allocate(ctx, cap);
 }
 
+// the reason no view can be made of `base`, or nullptr
+static const char *dist_view_refusal(const rk_ctx *base) {
+  if (!base || !base->dist) return "the context is not part of a comparison partitioned over several GPUs (rk_dist_init / rk_multi)";
+  if (!base->dist->db->loaded)
+    return "the context holds no partition database (it needs a successful rk_dist_load_aos, rk_dist_load_csv or rk_multi_load_*)";
+  return nullptr;
+}
+
+// A view of the rank context `base` (which holds a load): a new context on its device that shares base's partition
+// database and has its own transport `tr` (taken over, deleted on failure) and grouping workspace.  The peers' views
+// are mapped by dist_export / dist_import afterwards.  NULL on failure, with err set.
+static rk_ctx *dist_view_create(rk_ctx *base, Transport *tr, std::string &err) {
+  if (const char *why = dist_view_refusal(base)) {
+    delete tr;
+    err = why;
+    return nullptr;
+  }
+  const Dist &S = *base->dist;
+  DistDb &B = *S.db;
+  rk_ctx *c = rk_create(base->device);
+  if (!c) {
+    delete tr;
+    err = rk_create_error();
+    return nullptr;
+  }
+  c->is_view = true;
+  Dist *V = new Dist;
+  V->rank = S.rank, V->world = S.world, V->tr = tr;
+  tr->rank = S.rank, tr->world = S.world;
+  V->db = &B;
+  ++B.refs;
+  V->is_view = true;
+  c->dist = V;
+  V->trace.on = S.trace.on;
+  // all of the workspace now, sized by the database's capacity: no later call of a view allocates it
+  Carve count{nullptr};
+  dist_carve_work(*V, B.cap, B.hcap, count);
+  Carve carve{nullptr};
+  int rc = V->small_host.reserve((u64)V->world * SMALL_WORDS * sizeof(u32), nullptr, c->err);
+  if (!rc) rc = V->arena.reserve(count.off, nullptr, c->err);
+  if (!rc) {
+    V->h_small = (u32 *)V->small_host.ptr();
+    carve.base = (u8 *)V->arena.ptr();
+    dist_carve_work(*V, B.cap, B.hcap, carve);
+    cudaError_t e = cudaMemsetAsync(V->cnt, 0, sizeof(Counters), c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess) rc = fail(c, RK_ERR_CUDA, "%s", cudaGetErrorString(e));
+  }
+  if (rc) {
+    err = c->err;
+    rk_destroy(c);
+    return nullptr;
+  }
+  return c;
+}
+
 static int dist_export(rk_ctx *ctx, DistBlob *b) {
   Dist &D = *ctx->dist;
   memset(b, 0, sizeof *b);
-  b->pid = (u64)getpid(), b->ptr = (u64)(uintptr_t)D.arena.ptr(), b->cap = D.cap, b->device = ctx->device;
+  b->pid = (u64)getpid(), b->ptr = (u64)(uintptr_t)D.map_base(), b->cap = D.db->cap, b->device = ctx->device, b->view = D.is_view;
   CK(cudaSetDevice(ctx->device));
-  CK(cudaIpcGetMemHandle(&b->handle, D.arena.ptr()));
+  CK(cudaIpcGetMemHandle(&b->handle, D.map_base()));
   return RK_OK;
 }
 
@@ -617,11 +742,13 @@ static int dist_import(rk_ctx *ctx, const u8 *blobs, size_t stride) {
   for (int r = 0; r < D.world; ++r) {
     DistBlob b;
     memcpy(&b, blobs + (size_t)r * stride, sizeof b);
-    if (b.cap != D.cap) return fail(ctx, RK_ERR_ARG, "rank %d was initialised with capacity %llu, this rank with %llu", r,
-                                    (unsigned long long)b.cap, (unsigned long long)D.cap);
+    if (b.cap != D.db->cap) return fail(ctx, RK_ERR_ARG, "rank %d was initialised with capacity %llu, this rank with %llu", r,
+                                        (unsigned long long)b.cap, (unsigned long long)D.db->cap);
+    if (b.view != (int)D.is_view)
+      return fail(ctx, RK_ERR_ARG, "rank %d exported a %s, this rank is a %s", r, b.view ? "view" : "base context", D.is_view ? "view" : "base context");
     u8 *base = nullptr;
     if (r == D.rank) {
-      base = (u8 *)D.arena.ptr();
+      base = D.map_base();
     } else if (b.pid == (u64)getpid()) {
       base = (u8 *)(uintptr_t)b.ptr;
       if (b.device != ctx->device) {
@@ -638,9 +765,9 @@ static int dist_import(rk_ctx *ctx, const u8 *blobs, size_t stride) {
     }
     D.tr->peer_base[r] = base;
     // the arenas are carved identically (same capacity, same number of ranks): local offsets hold on every peer
-    D.pt.res[r] = (const u64 *)(base + ((const u8 *)D.res - (const u8 *)D.arena.ptr()));
+    D.pt.res[r] = (const u64 *)(base + ((const u8 *)D.res - D.map_base()));
   }
-  D.tr->my_base = (const u8 *)D.arena.ptr();
+  D.tr->my_base = D.map_base();
   if (NcclTransport *nt = dynamic_cast<NcclTransport *>(D.tr)) nt->d_flag = D.flag, nt->d_flag_all = D.flag_all;
   D.pt.nr = D.world, D.pt.me = D.rank;
   D.peers_ready = true;
@@ -670,7 +797,7 @@ static int dist_check_small(rk_ctx *ctx, bool range_errors, const char *worklist
   u32 e = 0;
   for (int r = 0; r < D.world; ++r) e |= D.h_small[(size_t)r * SMALL_WORDS + W_ERR];
   if (!e) return RK_OK;
-  if (worklist_nomem && (e & ERR_WORKLIST)) return fail(ctx, RK_ERR_NOMEM, worklist_nomem, (unsigned long long)D.cap);
+  if (worklist_nomem && (e & ERR_WORKLIST)) return fail(ctx, RK_ERR_NOMEM, worklist_nomem, (unsigned long long)D.db->cap);
   return fail(ctx, (range_errors && !(e & (ERR_WORKLIST | ERR_SPIN))) ? RK_ERR_RANGE : RK_ERR_INTERNAL, "%s", err_bits_text(e));
 }
 
@@ -680,7 +807,7 @@ static int check_inbound(rk_ctx *ctx, int word0, u64 bound, const char *fmt) {
   const Dist &D = *ctx->dist;
   for (int d = 0; d < D.world; ++d) {
     const u64 in = column_sum(D.h_small, word0 + d, D.world);
-    if (in > bound) return fail(ctx, RK_ERR_NOMEM, fmt, d, (unsigned long long)in, (unsigned long long)D.cap);
+    if (in > bound) return fail(ctx, RK_ERR_NOMEM, fmt, d, (unsigned long long)in, (unsigned long long)D.db->cap);
   }
   return RK_OK;
 }
@@ -718,6 +845,7 @@ static ScatterTable scatter_table(const Dist &D, const Exchange &ex, bool back, 
 static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u64 seqx_len, u64 seqy_len, unsigned flags,
                      rk_load_stats *stats, const PackedRows *pk = nullptr) {
   Dist &D = *ctx->dist;
+  DistDb &B = *D.db;
   const int nr = D.world, me = D.rank;
   if (!D.peers_ready) return fail(ctx, RK_ERR_STATE, "rk_dist_load_aos before rk_dist_import");
   if (!frags && !pk && n_loc) return fail(ctx, RK_ERR_ARG, "null record pointer");
@@ -726,25 +854,25 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   CK(cudaSetDevice(ctx->device));
   ProfGuard pg(ctx);
   cudaStream_t st = ctx->stream;
-  D.loaded = false;
+  B.loaded = false;
   D.have_rows = false;
   ctx->have_group = false;
   // NOTE: argument errors that only ONE rank can see (n_loc > cap) are turned into an error word all ranks receive with
   // the first count exchange, so that no rank is left waiting in a collective.
-  const bool too_many = n_loc > D.cap;
+  const bool too_many = n_loc > B.cap;
   const u64 n_use = too_many ? 0 : n_loc;
 
   const Geometry g = make_geometry(seqx_len, seqy_len);
-  D.g = g;
+  B.g = g;
   const SortBits bits = sort_key_bits(g);
-  D.bits_rank = bits.rank, D.bits_y = bits.y;
+  B.bits_rank = bits.rank, B.bits_y = bits.y;
   const LinkWords lw = link_map_words(g);
   const u64 lxw = lw.x, lyw = lw.y;
   const u64 pub_words = DIST_BINS + lxw + lyw;  // what a rank publishes after K1: its xStart/10 histogram and its link maps
   const u64 link_need = pub_words + lxw + lyw + (u64)nr * pub_words + 64;
-  const int rc = D.link_buf.reserve(link_need * 4, st, ctx->err);
+  const int rc = B.link_buf.reserve(link_need * 4, st, ctx->err);
   if (rc) return rc;
-  u32 *hist0 = (u32 *)D.link_buf.ptr(), *linkx_loc = hist0 + DIST_BINS, *linky_loc = linkx_loc + lxw, *linkx = linky_loc + lyw, *linky = linkx + lxw,
+  u32 *hist0 = (u32 *)B.link_buf.ptr(), *linkx_loc = hist0 + DIST_BINS, *linky_loc = linkx_loc + lxw, *linkx = linky_loc + lyw, *linky = linkx + lxw,
       *pub_all = linky + lyw;
 
   const bool on_device = n_use && !pk && is_device_pointer(frags);
@@ -753,13 +881,13 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   cudaEvent_t *ev = ctx->ev;
   CK(cudaEventRecord(ev[0], st));
   if (!on_device && !pk && n_use) {
-    const int rc2 = D.aos_buf.reserve(align_up(n_use * RK_FRAG_BYTES, 16) + 16, st, ctx->err);
+    const int rc2 = B.aos_buf.reserve(align_up(n_use * RK_FRAG_BYTES, 16) + 16, st, ctx->err);
     if (rc2) return rc2;
-    CK(cudaMemcpyAsync(D.aos_buf.ptr(), frags, n_use * RK_FRAG_BYTES, cudaMemcpyHostToDevice, st));
-    aos = (const u8 *)D.aos_buf.ptr();
+    CK(cudaMemcpyAsync(B.aos_buf.ptr(), frags, n_use * RK_FRAG_BYTES, cudaMemcpyHostToDevice, st));
+    aos = (const u8 *)B.aos_buf.ptr();
   }
-  D.aos_src = pk ? nullptr : aos;
-  D.pk_src = pk ? *pk : PackedRows{};
+  B.aos_src = pk ? nullptr : aos;
+  B.pk_src = pk ? *pk : PackedRows{};
   CK(cudaEventRecord(ev[1], st));
   u64 launches = 0;
 
@@ -774,111 +902,111 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
     CK(cudaMemcpyAsync(&D.cnt->err, &e, 4, cudaMemcpyHostToDevice, st));
   }
   if (pk)
-    launches += launch_decode_packed(pk->key, pk->strand, n_use, g, D.key0_loc, linkx_loc, linky_loc, &D.cnt->n_dropped, &D.cnt->err, st,
-                                     D.rec4_loc, HistOut{nullptr, 0, 0}, (u32)file_off);
+    launches += launch_decode_packed(pk->key, pk->strand, n_use, g, B.key0_loc, linkx_loc, linky_loc, &D.cnt->n_dropped, &D.cnt->err, st,
+                                     B.rec4_loc, HistOut{nullptr, 0, 0}, (u32)file_off);
   else
-    launches += launch_decode(aos, n_use, g, nullptr, nullptr, nullptr, nullptr, nullptr, D.key0_loc, linkx_loc, linky_loc,
-                              &D.cnt->n_dropped, &D.cnt->err, st, D.rec4_loc, HistOut{nullptr, 0, 0}, (u32)file_off);
+    launches += launch_decode(aos, n_use, g, nullptr, nullptr, nullptr, nullptr, nullptr, B.key0_loc, linkx_loc, linky_loc,
+                              &D.cnt->n_dropped, &D.cnt->err, st, B.rec4_loc, HistOut{nullptr, 0, 0}, (u32)file_off);
   // exchange 1: to the owner of the xStart/10 range
-  const int shift0 = D.bits_rank > 12 ? D.bits_rank - 12 : 0;
-  launches += dist_coarse_hist(D.key0_loc, (u32)n_use, shift0, 0, g.vsize - 1, hist0, st);
+  const int shift0 = B.bits_rank > 12 ? B.bits_rank - 12 : 0;
+  launches += dist_coarse_hist(B.key0_loc, (u32)n_use, shift0, 0, g.vsize - 1, hist0, st);
   // one all-gather for everything K1 produced that the other ranks need: the histogram the cuts are made from and the link
   // maps (OR-ed over the ranks below, so that a run of linked buckets has one key everywhere)
   TR(D.tr->all_gather(hist0, pub_all, pub_words * 4, st));
-  launches += dist_cuts_from_hist(pub_all, pub_words, nr, shift0, D.cuts0, st);
+  launches += dist_cuts_from_hist(pub_all, pub_words, nr, shift0, B.cuts0, st);
   launches += dist_or_rows(pub_all + DIST_BINS, pub_words, nr, lxw, linkx, st);
   launches += dist_or_rows(pub_all + DIST_BINS + lxw, pub_words, nr, lyw, linky, st);
   // count per destination -> all ranks' counts on the device -> every tile stores its records straight into the owners'
   // receive buffers (peer memory over NVLink) -> barrier; the host reads the count matrix while the rows travel
   uint2 *outs[DIST_MAX_RANKS];
-  D.tr->peer_table(D.rec6_arr, outs);
-  launches += dist_count_plain(D.key0_loc, (u32)n_use, D.cuts0, nr, g.vsize - 1, D.tile_cnt, D.d_small + W_CNT_A, st);
-  CK(cudaMemcpyAsync(D.d_small + W_CUTS, D.cuts0, (nr + 1) * sizeof(u32), cudaMemcpyDeviceToDevice, st));
+  D.tr->peer_table(B.rec6_arr, outs);
+  launches += dist_count_plain(B.key0_loc, (u32)n_use, B.cuts0, nr, g.vsize - 1, D.tile_cnt, D.d_small + W_CNT_A, st);
+  CK(cudaMemcpyAsync(D.d_small + W_CUTS, B.cuts0, (nr + 1) * sizeof(u32), cudaMemcpyDeviceToDevice, st));
   const u32 foff32 = (u32)file_off;
   CK(cudaMemcpyAsync(D.d_small + W_FOFF, &foff32, sizeof(u32), cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
   if (const int rc = dist_gather_counts(ctx, [&] {  // host sync 1
-        launches += dist_push_records(D.key0_loc, (u32)n_use, D.cuts0, nr, g.vsize - 1, D.rec4_loc, outs, (u32)D.cap, D.tile_cnt,
+        launches += dist_push_records(B.key0_loc, (u32)n_use, B.cuts0, nr, g.vsize - 1, B.rec4_loc, outs, (u32)B.cap, D.tile_cnt,
                                       D.d_small_all, SMALL_WORDS, me, st);
       }))
     return rc;
   // (a rank whose slice exceeds the capacity loaded nothing and published ERR_WORKLIST)
   if (const int rc = dist_check_small(ctx, true, "a rank holds more records than the capacity of %llu rows per rank given to rk_dist_init"))
     return rc;
-  if (const int rc = check_inbound(ctx, W_CNT_A, D.cap, "rank %d would own %llu fragments, capacity is %llu rows per rank")) return rc;
-  D.ex1.from_matrix(D.h_small, W_CNT_A, nr, me);
+  if (const int rc = check_inbound(ctx, W_CNT_A, B.cap, "rank %d would own %llu fragments, capacity is %llu rows per rank")) return rc;
+  B.ex1.from_matrix(D.h_small, W_CNT_A, nr, me);
   // where every rank's slice starts (as its caller said) and, from the row sums of the count matrix (the dropped column
   // included), how long it is: the line records of RK_F_LINE_RECORDS find the rank that loaded a record by these starts,
   // which needs the slices in rank order without overlap.  Every rank sees the same matrix, so all agree on the verdict.
-  D.slices_in_order = true;
+  B.slices_in_order = true;
   for (int s = 0; s < nr; ++s) {
     u64 n_s = 0;
     for (int d = 0; d <= nr; ++d) n_s += D.h_small[(size_t)s * SMALL_WORDS + W_CNT_A + d];
-    D.file_off[s] = D.h_small[(size_t)s * SMALL_WORDS + W_FOFF];
-    if (s + 1 < nr && D.file_off[s] + n_s > D.h_small[(size_t)(s + 1) * SMALL_WORDS + W_FOFF]) D.slices_in_order = false;
+    B.file_off[s] = D.h_small[(size_t)s * SMALL_WORDS + W_FOFF];
+    if (s + 1 < nr && B.file_off[s] + n_s > D.h_small[(size_t)(s + 1) * SMALL_WORDS + W_FOFF]) B.slices_in_order = false;
   }
-  D.tr->bytes_sent += (D.ex1.n_send - D.ex1.scnt[me]) * 24;  // (the rows this rank's kernels stored into peer memory)
+  D.tr->bytes_sent += (B.ex1.n_send - B.ex1.scnt[me]) * 24;  // (the rows this rank's kernels stored into peer memory)
   u64 loaded_total = 0, off = 0;
   for (int d = 0; d <= nr; ++d) loaded_total += column_sum(D.h_small, W_CNT_A + d, nr);
   for (int d = 0; d < nr; ++d) {
-    D.pt.roff[d] = (u32)off;
+    B.roff[d] = (u32)off;
     off += column_sum(D.h_small, W_CNT_A + d, nr);
   }
-  D.rank_off = D.pt.roff[me];
+  B.rank_off = B.roff[me];
   const u64 m_total = off;
-  D.pt.roff[nr] = (u32)m_total;
-  for (int d = nr + 1; d <= DIST_MAX_RANKS; ++d) D.pt.roff[d] = 0xFFFFFFFFu;
-  CK(cudaMemcpyAsync(D.roff_dev, D.pt.roff, (nr + 1) * sizeof(u32), cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
-  D.m_total = m_total, D.n_total_loaded = loaded_total;
-  const u32 m = (u32)D.ex1.n_recv;
-  D.m_loc = m;
+  B.roff[nr] = (u32)m_total;
+  for (int d = nr + 1; d <= DIST_MAX_RANKS; ++d) B.roff[d] = 0xFFFFFFFFu;
+  CK(cudaMemcpyAsync(B.roff_dev, B.roff, (nr + 1) * sizeof(u32), cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
+  B.m_total = m_total, B.n_total_loaded = loaded_total;
+  const u32 m = (u32)B.ex1.n_recv;
+  B.m_loc = m;
 
   CK(cudaEventRecord(ev[2], st));
   // processing order: sources arrive in file order, so a stable sort by xStart/10 is the global order
   // the sort keys are taken relative to the rank's first xStart/10 bucket: log2(range of the rank) bits instead of log2(vsize)
   const KeyRange k0 = rank_key_range(D.h_small + (size_t)me * SMALL_WORDS + W_CUTS, me, nr, g.vsize);
-  launches += dist_key0_of_rec(D.rec6_arr, m, k0.base, D.key0a, hist_of(0, k0.bits), st);
-  launches += launch_sort_pairs(D.key0a, nullptr, D.k0_r, D.aidx_r, D.tmp_k, D.tmp_v, m, k0.bits, D.sort_work, st, &D.cnt->err,
+  launches += dist_key0_of_rec(B.rec6_arr, m, k0.base, B.key0a, hist_of(0, k0.bits), st);
+  launches += launch_sort_pairs(B.key0a, nullptr, B.k0_r, B.aidx_r, D.tmp_k, D.tmp_v, m, k0.bits, D.sort_work, st, &D.cnt->err,
                                 m ? D.prehist : nullptr);
   CK(cudaEventRecord(ev[3], st));
-  launches += launch_keys(D.aidx_r, m, g, nullptr, linkx, linky, D.xl, D.yl_r, D.ys_r, D.kx2, D.ky, D.identity_r, st,
-                          HistOut{nullptr, 0, 0}, HistOut{nullptr, 0, 0}, D.gfidx_r, 1u, D.rec6_arr);
-  launches += launch_hkey(D.k0_r, D.ys_r, m, nullptr, st, D.gfidx_r, D.identity_r, D.hfi_r);
+  launches += launch_keys(B.aidx_r, m, g, nullptr, linkx, linky, B.xl, B.yl_r, B.ys_r, B.kx2, B.ky, B.identity_r, st,
+                          HistOut{nullptr, 0, 0}, HistOut{nullptr, 0, 0}, B.gfidx_r, 1u, B.rec6_arr);
+  launches += launch_hkey(B.k0_r, B.ys_r, m, nullptr, st, B.gfidx_r, B.identity_r, B.hfi_r);
   CK(cudaEventRecord(ev[4], st));
   // X halo: fragments whose X super-bucket belongs to a higher rank
-  launches += dist_cuts_x(D.cuts0, nr, g, linkx, D.cuts_x, st);
-  launches += dist_split_halo(D.kx2, D.xl, m, D.cuts_x, nr, g.nbx, me, D.rank_off, D.halo_send, (u32)D.hcap, D.perm_x, D.tile_cnt,
+  launches += dist_cuts_x(B.cuts0, nr, g, linkx, B.cuts_x, st);
+  launches += dist_split_halo(B.kx2, B.xl, m, B.cuts_x, nr, g.nbx, me, B.rank_off, B.halo_send, (u32)B.hcap, B.perm_x, D.tile_cnt,
                               D.d_small + W_CNT_A, st);
   // Y: to the owner of the Y super-bucket range
-  const int shift_y = D.bits_y > 12 ? D.bits_y - 12 : 0;
-  launches += dist_coarse_hist(D.ky, m, shift_y, 0, 0xFFFFFFFFu, D.hist, st);
+  const int shift_y = B.bits_y > 12 ? B.bits_y - 12 : 0;
+  launches += dist_coarse_hist(B.ky, m, shift_y, 0, 0xFFFFFFFFu, D.hist, st);
   TR(D.tr->all_gather(D.hist, D.hist_all, DIST_BINS * 4, st));
-  launches += dist_cuts_from_hist(D.hist_all, DIST_BINS, nr, shift_y, D.cuts_y, st);
-  launches += dist_split_axis(D.ky, D.yl_r, m, D.cuts_y, nr, D.rank_off, D.send_rows, D.perm_y, D.tile_cnt, D.d_small + W_CNT_B, st);
-  CK(cudaMemcpyAsync(D.d_small + W_CUTS, D.cuts_y, (nr + 1) * sizeof(u32), cudaMemcpyDeviceToDevice, st));
-  CK(cudaMemcpyAsync(D.d_small + W_CUTSX, D.cuts_x, 2 * nr * sizeof(u32), cudaMemcpyDeviceToDevice, st));
+  launches += dist_cuts_from_hist(D.hist_all, DIST_BINS, nr, shift_y, B.cuts_y, st);
+  launches += dist_split_axis(B.ky, B.yl_r, m, B.cuts_y, nr, B.rank_off, B.send_rows, B.perm_y, D.tile_cnt, D.d_small + W_CNT_B, st);
+  CK(cudaMemcpyAsync(D.d_small + W_CUTS, B.cuts_y, (nr + 1) * sizeof(u32), cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(D.d_small + W_CUTSX, B.cuts_x, 2 * nr * sizeof(u32), cudaMemcpyDeviceToDevice, st));
   if (const int rc = dist_gather_counts(ctx)) return rc;  // host sync 2
   if (const int rc = dist_check_small(ctx, true)) return rc;
-  D.exh.from_matrix(D.h_small, W_CNT_A, nr, me);
-  D.exy.from_matrix(D.h_small, W_CNT_B, nr, me);
+  B.exh.from_matrix(D.h_small, W_CNT_A, nr, me);
+  B.exy.from_matrix(D.h_small, W_CNT_B, nr, me);
   for (int d = 0; d < nr; ++d) {
     const u64 halo_in = column_sum(D.h_small, W_CNT_A + d, nr), y_in = column_sum(D.h_small, W_CNT_B + d, nr);
     u64 halo_out = 0;
     for (int t = 0; t < nr; ++t) halo_out += D.h_small[(size_t)d * SMALL_WORDS + W_CNT_A + t];
-    if (halo_in > D.hcap || halo_out > D.hcap)
+    if (halo_in > B.hcap || halo_out > B.hcap)
       return fail(ctx, RK_ERR_NOMEM, "rank %d: %llu halo fragments in / %llu out, the halo capacity is %llu", d,
-                  (unsigned long long)halo_in, (unsigned long long)halo_out, (unsigned long long)D.hcap);
-    if (y_in > D.cap) return fail(ctx, RK_ERR_NOMEM, "rank %d would own %llu fragments in the Y pass, capacity is %llu rows per rank", d,
-                                  (unsigned long long)y_in, (unsigned long long)D.cap);
+                  (unsigned long long)halo_in, (unsigned long long)halo_out, (unsigned long long)B.hcap);
+    if (y_in > B.cap) return fail(ctx, RK_ERR_NOMEM, "rank %d would own %llu fragments in the Y pass, capacity is %llu rows per rank", d,
+                                  (unsigned long long)y_in, (unsigned long long)B.cap);
   }
-  D.n_away = (u32)D.exh.n_send, D.n_halo = (u32)D.exh.n_recv, D.m_y = (u32)D.exy.n_recv;
+  B.n_away = (u32)B.exh.n_send, B.n_halo = (u32)B.exh.n_recv, B.m_y = (u32)B.exy.n_recv;
   // Y sort keys relative to the first key of the rank's Y range
   const KeyRange yr = rank_key_range(D.h_small + (size_t)me * SMALL_WORDS + W_CUTS, me, nr, 2ull * g.nby);
 
   // Both row exchanges come right after host sync 2: every rank's work queued before it is complete, so no rank still
   // reads its halo_recv / recv_rows (last read by the previous load and group) when the peers' pushes start.
-  TR(D.tr->exchange_rows(D.halo_send, D.exh, D.halo_recv, 16, st));
+  TR(D.tr->exchange_rows(B.halo_send, B.exh, B.halo_recv, 16, st));
   // the Y rows travel (copy engines, NVLink) while this GPU unpacks its halo and sorts its X buckets
-  TR(D.tr->exchange_rows_begin(D.send_rows, D.exy, D.recv_rows, 16, st, D.side));
+  TR(D.tr->exchange_rows_begin(B.send_rows, B.exy, D.recv_rows, 16, st, D.side));
   // X sort keys relative to the first super-bucket of the rank's range (per strand class)
   const u32 *cutsx_h = D.h_small + (size_t)me * SMALL_WORDS + W_CUTSX;
   u32 x_base[2], x_range[2];
@@ -889,18 +1017,18 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   }
   const u32 x_R = std::max(x_range[0], x_range[1]);
   const int bits_x_l = ceil_log2(4ull * ((u64)x_R + 1));
-  launches += dist_x_local_keys(D.kx2, m, g.nbx, x_base, x_range, hist_of(1, bits_x_l), st);
-  launches += dist_unpack_halo_rows(D.halo_recv, D.n_halo, g.nbx, x_base, x_range, D.kx2 + m, D.xl + m, D.halo_grank, hist_of(1, bits_x_l), st);
+  launches += dist_x_local_keys(B.kx2, m, g.nbx, x_base, x_range, hist_of(1, bits_x_l), st);
+  launches += dist_unpack_halo_rows(B.halo_recv, B.n_halo, g.nbx, x_base, x_range, B.kx2 + m, B.xl + m, B.halo_grank, hist_of(1, bits_x_l), st);
   CK(cudaEventRecord(ev[5], st));
-  launches += launch_sort_pairs(D.kx2, nullptr, D.skx, D.rx, D.tmp_k, D.tmp_v, (u64)m + D.n_halo, bits_x_l, D.sort_work, st, &D.cnt->err,
-                                (m + D.n_halo) ? D.prehist + 1024 : nullptr);
+  launches += launch_sort_pairs(B.kx2, nullptr, B.skx, B.rx, D.tmp_k, D.tmp_v, (u64)m + B.n_halo, bits_x_l, D.sort_work, st, &D.cnt->err,
+                                (m + B.n_halo) ? D.prehist + 1024 : nullptr);
   CK(cudaEventRecord(ev[6], st));
   TR(D.tr->exchange_rows_end(st));
-  launches += dist_unpack_axis_rows(D.recv_rows, D.m_y, yr.base, D.ky_a, D.yl_a, D.grank_a, hist_of(2, yr.bits), st);
-  launches += launch_sort_pairs(D.ky_a, nullptr, D.sky_a, D.ry_a, D.tmp_k, D.tmp_v, D.m_y, yr.bits, D.sort_work, st, &D.cnt->err,
-                                D.m_y ? D.prehist + 2048 : nullptr);
+  launches += dist_unpack_axis_rows(D.recv_rows, B.m_y, yr.base, B.ky_a, B.yl_a, B.grank_a, hist_of(2, yr.bits), st);
+  launches += launch_sort_pairs(B.ky_a, nullptr, B.sky_a, B.ry_a, D.tmp_k, D.tmp_v, B.m_y, yr.bits, D.sort_work, st, &D.cnt->err,
+                                B.m_y ? D.prehist + 2048 : nullptr);
   CK(cudaEventRecord(ev[7], st));
-  D.loaded = true;
+  B.loaded = true;
 
   if (stats) {
     memset(stats, 0, sizeof *stats);
@@ -937,7 +1065,7 @@ struct DistCsv {
 static void dist_csv_local(rk_ctx *ctx, const char *slice, u64 bytes, int threads, DistCsv &L) {
   L = DistCsv{};
   ctx->loaded = ctx->have_group = false;
-  if (ctx->dist) ctx->dist->loaded = ctx->dist->have_rows = false;
+  if (ctx->dist) ctx->dist->db->loaded = ctx->dist->have_rows = false;
   auto run = [&]() -> int {
     if (!slice && bytes) return fail(ctx, RK_ERR_ARG, "null text pointer");
     CK(cudaSetDevice(ctx->device));
@@ -966,6 +1094,7 @@ constexpr u32 CWF_WIDE = 1, CWF_BYTES = 2, CWF_NL_END = 4, CWF_ROWS = 8;  // CWF
 static int dist_csv_finish(rk_ctx *ctx, DistCsv &L, u64 seqx_len, u64 seqy_len, u64 total_frags, unsigned flags, rk_load_stats *stats,
                            rk_csv_stats *csv) {
   Dist &D = *ctx->dist;
+  DistDb &B = *D.db;
   const int nr = D.world, me = D.rank;
   if (!D.peers_ready) return fail(ctx, RK_ERR_STATE, "rk_dist_load_csv before rk_dist_import");
   CK(cudaSetDevice(ctx->device));
@@ -1007,9 +1136,9 @@ static int dist_csv_finish(rk_ctx *ctx, DistCsv &L, u64 seqx_len, u64 seqy_len, 
   if (total > total_frags) return fail(ctx, RK_ERR_RANGE, "Unexpected number of fragments");  // FragmentsDatabase.cpp:99
   if (total >= 0xFFFFFFF0ull) return fail(ctx, RK_ERR_ARG, "more than 2^32-16 records in one comparison");
   for (int r = 0; r < nr; ++r)
-    if (W(r, CW_ACC) > D.cap)
+    if (W(r, CW_ACC) > B.cap)
       return fail(ctx, RK_ERR_NOMEM, "a rank holds more records than the capacity of %llu rows per rank given to rk_dist_init",
-                  (unsigned long long)D.cap);
+                  (unsigned long long)B.cap);
   // the final row of the text (the empty one after a final '\n') is the last slice's; every other slice ends with '\n',
   // and the empty segment after it is no row
   const int holder = (last >= 0 && !(W(last, CW_FLAGS) & CWF_NL_END)) ? last : nr - 1;
@@ -1018,7 +1147,7 @@ static int dist_csv_finish(rk_ctx *ctx, DistCsv &L, u64 seqx_len, u64 seqy_len, 
   CsvOut o;
   {
     ProfGuard pg(ctx);
-    if (const int rc = csv_emit(ctx, p, D.aos_buf, &o)) return rc;
+    if (const int rc = csv_emit(ctx, p, B.aos_buf, &o)) return rc;
   }
   const PackedRows pk{o.key4, o.rest4, o.strand};
   const u64 n_acc = p.n_accepted();
@@ -1041,18 +1170,21 @@ static int dist_csv_finish(rk_ctx *ctx, DistCsv &L, u64 seqx_len, u64 seqy_len, 
 // ---------------------------------------------------------------------------------------------------------------------
 static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flags, rk_result *out, rk_dist_info *info) {
   Dist &D = *ctx->dist;
+  DistDb &B = *D.db;
   const int nr = D.world, me = D.rank;
-  if (!D.loaded) return fail(ctx, RK_ERR_STATE, "rk_dist_group before a successful rk_dist_load_aos");
+  if (!B.loaded) return fail(ctx, RK_ERR_STATE, "rk_dist_group before a successful rk_dist_load_aos");
+  if (!D.peers_ready) return fail(ctx, RK_ERR_STATE, "rk_dist_group before rk_dist_import");
   if (!(len_ratio > 0)) return fail(ctx, RK_ERR_ARG, "Ratio between length and position must be greater than zero");
   if (!(pos_ratio > 0)) return fail(ctx, RK_ERR_ARG, "Position proximity must be greater than zero");
-  if ((flags & RK_F_LINE_RECORDS) && !D.slices_in_order)
+  if ((flags & RK_F_LINE_RECORDS) && !B.slices_in_order)
     return fail(ctx, RK_ERR_ARG, "RK_F_LINE_RECORDS needs the ranks' slices of the file in rank order (file_offset of rk_dist_load_aos)");
   CK(cudaSetDevice(ctx->device));
   ProfGuard pg(ctx);
   memset(out, 0, sizeof *out);
   cudaStream_t st = ctx->stream;
   cudaEvent_t *ev = ctx->ev;
-  const u32 m = D.m_loc, nh = D.n_halo, mc = m + nh;
+  const u32 m = B.m_loc, nh = B.n_halo, mc = m + nh;
+  memcpy(D.pt.roff, B.roff, sizeof B.roff);
   u64 launches = 0;
   const u64 sent0 = D.tr->bytes_sent;
   const bool line_records = (flags & RK_F_LINE_RECORDS) != 0;
@@ -1062,33 +1194,33 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   CK(cudaEventRecord(ev[0], st));
   // X pass at home over [own fragments ++ halo]
   MatchArgs mx{};
-  mx.skey = D.skx, mx.srank = D.rx, mx.cl_r = D.xl, mx.parent = D.parent_x, mx.xm_bits = D.xm_bits;
-  mx.m = mc, mx.max_index = D.g.mx, mx.len_ratio = len_ratio, mx.pos_ratio = pos_ratio, mx.is_y = 0;
+  mx.skey = B.skx, mx.srank = B.rx, mx.cl_r = B.xl, mx.parent = D.parent_x, mx.xm_bits = D.xm_bits;
+  mx.m = mc, mx.max_index = B.g.mx, mx.len_ratio = len_ratio, mx.pos_ratio = pos_ratio, mx.is_y = 0;
   mx.worklist = D.worklist, mx.work_count = D.cnt->work_x, mx.work_cap = D.work_cap;
   mx.ent_rank = D.ent_rank, mx.ent_c = D.ent_c, mx.ent_len = D.ent_len, mx.err = &D.cnt->err;
   mx.key_shift = 1;
   launches += launch_match(mx, st);
-  launches += dist_x_owners(D.parent_x, m, nh, D.rank_off, D.halo_grank, D.parent, scatter_table(D, D.exh, true, D.away_res), st);
+  launches += dist_x_owners(D.parent_x, m, nh, B.rank_off, B.halo_grank, D.parent, scatter_table(D, B.exh, true, D.away_res), st);
   TR(D.tr->barrier(st));  // the halo owners are stored by the kernel above straight into their home ranks' away_res
-  launches += dist_apply_away(D.away_res, D.perm_x, D.n_away, D.parent, st);
+  launches += dist_apply_away(D.away_res, B.perm_x, B.n_away, D.parent, st);
   CK(cudaEventRecord(ev[1], st));
   // Y pass on the owners of the Y ranges: X-matched fragments insert without a query (commonFunctions.cpp:59)
-  launches += dist_pack_xm(D.parent, D.perm_y, m, scatter_table(D, D.exy, false, D.xm_a), st);
+  launches += dist_pack_xm(D.parent, B.perm_y, m, scatter_table(D, B.exy, false, D.xm_a), st);
   if (m) CK(cudaMemsetAsync(D.yo_s, 0xFF, (size_t)m * 4, st));  // "no Y owner" until a peer stores one (after the barrier)
   TR(D.tr->barrier(st));
-  if (D.m_y) CK(cudaMemsetAsync(D.parent_y, 0xFF, (size_t)D.m_y * 4, st));
+  if (B.m_y) CK(cudaMemsetAsync(D.parent_y, 0xFF, (size_t)B.m_y * 4, st));
   MatchArgs my = mx;
-  my.skey = D.sky_a, my.srank = D.ry_a, my.cl_r = D.yl_a, my.parent = D.parent_y, my.m = D.m_y, my.max_index = D.g.my, my.is_y = 1;
+  my.skey = B.sky_a, my.srank = B.ry_a, my.cl_r = B.yl_a, my.parent = D.parent_y, my.m = B.m_y, my.max_index = B.g.my, my.is_y = 1;
   my.work_count = D.cnt->work_y, my.key_shift = 0, my.xm_bytes = D.xm_a;
   launches += launch_match(my, st);
-  launches += dist_y_owners(D.parent_y, D.grank_a, D.m_y, scatter_table(D, D.exy, true, D.yo_s), st);
+  launches += dist_y_owners(D.parent_y, B.grank_a, B.m_y, scatter_table(D, B.exy, true, D.yo_s), st);
   TR(D.tr->barrier(st));
-  launches += dist_merge_y(D.yo_s, D.perm_y, m, D.parent, st);
+  launches += dist_merge_y(D.yo_s, B.perm_y, m, D.parent, st);
   CK(cudaEventRecord(ev[2], st));
   // forest: roots per rank; local chains; the chains that leave the GPU are resolved in bulk rounds while there are many
   // of them anywhere, the rest by walking through the peers' memory (k7_dist.cu)
   launches += dist_root_scan(D.parent, m, D.gidscan, D.d_small + W_X0, D.scan_work, st);
-  launches += dist_chase_local(D.parent, D.gidscan, m, D.rank_off, D.lroot, D.res, D.pend_idx[0], D.pend_key[0], D.n_pend, st);
+  launches += dist_chase_local(D.parent, D.gidscan, m, B.rank_off, D.lroot, D.res, D.pend_idx[0], D.pend_key[0], D.n_pend, st);
   CK(cudaMemcpyAsync(D.d_small + W_X2, D.n_pend, sizeof(u32), cudaMemcpyDeviceToDevice, st));
   // host sync: roots and pending chains of every rank (also: every rank's res[] is final)
   if (const int rc = dist_gather_counts(ctx)) return rc;
@@ -1106,18 +1238,18 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
     // ask: the ranks in question go to their owners
     uint4 *qouts[DIST_MAX_RANKS];
     D.tr->peer_table(D.queries, qouts);
-    launches += dist_chase_ask_count(D.pend_key[cur], bound, D.n_pend, D.roff_dev, nr, D.tile_cnt, D.d_small + W_CNT_A, st);
+    launches += dist_chase_ask_count(D.pend_key[cur], bound, D.n_pend, B.roff_dev, nr, D.tile_cnt, D.d_small + W_CNT_A, st);
     if (const int rc = dist_gather_counts(ctx, [&] {
-          launches += dist_chase_ask_push(D.pend_key[cur], bound, D.n_pend, D.roff_dev, nr, qouts, (u32)D.cap, D.apos, D.tile_cnt,
+          launches += dist_chase_ask_push(D.pend_key[cur], bound, D.n_pend, B.roff_dev, nr, qouts, (u32)B.cap, D.apos, D.tile_cnt,
                                           D.d_small_all, SMALL_WORDS, me, st);
         }))
       return rc;
-    if (const int rc = check_inbound(ctx, W_CNT_A, D.cap, "rank %d is asked about %llu chain ends, capacity is %llu rows per rank")) return rc;
+    if (const int rc = check_inbound(ctx, W_CNT_A, B.cap, "rank %d is asked about %llu chain ends, capacity is %llu rows per rank")) return rc;
     Exchange exq;
     exq.from_matrix(D.h_small, W_CNT_A, nr, me);
     D.tr->bytes_sent += (exq.n_send - exq.scnt[me]) * 16 + (exq.n_recv - exq.rcnt[me]) * 8;
     // answer: every owner returns its res[] words, block by block, into the asking ranks' answer buffers
-    launches += dist_chase_answer(D.queries, (u32)exq.n_recv, D.res, D.rank_off, scatter_table(D, exq, true, D.answers), st);
+    launches += dist_chase_answer(D.queries, (u32)exq.n_recv, D.res, B.rank_off, scatter_table(D, exq, true, D.answers), st);
     TR(D.tr->barrier(st));
     // apply: roots end a chain, anything else is asked about in the next round
     launches += dist_chase_apply(D.pt, nroots, SMALL_WORDS, bound, D.pend_idx[cur], D.pend_key[cur], D.apos, D.answers, D.n_pend, D.gid_l,
@@ -1134,24 +1266,24 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   // output exchange: to the owner of the group-id range.  The ranges are cut for about equal sort_groups WORK: lines, with
   // the lines of groups with several members weighted up (groups founded early are the large ones: equal numbers of
   // groups gave rank 0 far more lines, equal numbers of lines still far more work — see k_cuts_from_hist).
-  const int bits_gid = key_bits(D.m_total);  // group ids are < number of fragments
+  const int bits_gid = key_bits(B.m_total);  // group ids are < number of fragments
   const int shift_g = bits_gid > 12 ? bits_gid - 12 : 0;
   launches += dist_cuts_gid(nroots, SMALL_WORDS, nr, D.cuts_g, D.d_small + W_X1, st);  // (the total; the cuts are replaced below)
   launches += dist_coarse_hist(D.gid_rank, m, shift_g, 0, 0xFFFFFFFFu, D.hist, st);
   TR(D.tr->all_gather(D.hist, D.hist_all, DIST_BINS * 4, st));
   // no range may hold more lines than a rank has rows (RK_DIST_LINE_CAP: tests — a tighter bound than the capacity)
-  const u64 line_cap = getenv("RK_DIST_LINE_CAP") ? std::min<u64>(D.cap, strtoull(getenv("RK_DIST_LINE_CAP"), nullptr, 10)) : D.cap;
+  const u64 line_cap = getenv("RK_DIST_LINE_CAP") ? std::min<u64>(B.cap, strtoull(getenv("RK_DIST_LINE_CAP"), nullptr, 10)) : B.cap;
   launches += dist_cuts_from_hist(D.hist_all, DIST_BINS, nr, shift_g, D.cuts_g, st, D.d_small + W_X1, line_cap);
   CK(cudaMemcpyAsync(D.d_small + W_CNT_B, D.cuts_g, (nr + 1) * sizeof(u32), cudaMemcpyDeviceToDevice, st));
   uint4 *outs[DIST_MAX_RANKS];
   D.tr->peer_table(D.recv_rows, outs);
   launches += dist_count_plain(D.gid_rank, m, D.cuts_g, nr, 0xFFFFFFFFu, D.tile_cnt, D.d_small + W_CNT_A, st);
   if (const int rc = dist_gather_counts(ctx, [&] {  // host sync 3
-        launches += dist_push_gid(D.gid_rank, D.hfi_r, m, D.cuts_g, nr, outs, (u32)D.cap, D.tile_cnt, D.d_small_all, SMALL_WORDS, me, st);
+        launches += dist_push_gid(D.gid_rank, B.hfi_r, m, D.cuts_g, nr, outs, (u32)B.cap, D.tile_cnt, D.d_small_all, SMALL_WORDS, me, st);
       }))
     return rc;
   if (const int rc = dist_check_small(ctx, false)) return rc;
-  if (const int rc = check_inbound(ctx, W_CNT_A, D.cap, "rank %d would own %llu output lines, capacity is %llu rows per rank")) return rc;
+  if (const int rc = check_inbound(ctx, W_CNT_A, B.cap, "rank %d would own %llu output lines, capacity is %llu rows per rank")) return rc;
   Exchange exg;
   exg.from_matrix(D.h_small, W_CNT_A, nr, me);
   D.tr->bytes_sent += (exg.n_send - exg.scnt[me]) * 16;
@@ -1169,7 +1301,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   OrderArgs oa{};
   oa.sgid = D.sgid, oa.srank = D.srank_g, oa.hfi_r = D.recv_rows;
   oa.m = mg, oa.do_sort = (flags & RK_F_NO_SORT) ? 0 : 1, oa.gid_base = gr.base;
-  order_carve(oa, D.order_scratch, D.cap);
+  order_carve(oa, D.order_scratch, B.cap);
   oa.work_count = D.cnt->work_g;
   oa.out_order = D.out_order, oa.out_gid = D.out_gid, oa.out_repval = D.out_repval, oa.out_identity = D.out_identity;
   oa.err = &D.cnt->err;
@@ -1180,21 +1312,21 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   // pushed into the owners' `queries` (free again: the forest is done), the answers stored back by the owners' kernel,
   // a barrier.  The gid cuts are spent, so cuts_g carries the slice starts.
   if (line_records) {
-    CK(cudaMemcpyAsync(D.cuts_g, D.file_off, nr * sizeof(u32), cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
+    CK(cudaMemcpyAsync(D.cuts_g, B.file_off, nr * sizeof(u32), cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
     uint4 *qouts[DIST_MAX_RANKS];
     D.tr->peer_table(D.queries, qouts);
     launches += dist_count_plain(D.out_order, mg, D.cuts_g, nr, 0xFFFFFFFFu, D.tile_cnt, D.d_small + W_CNT_A, st);
     if (const int rc = dist_gather_counts(ctx, [&] {  // host sync 4
-          launches += dist_line_ask_push(D.out_order, mg, D.cuts_g, nr, qouts, (u32)D.cap, D.tile_cnt, D.d_small_all, SMALL_WORDS, me, st);
+          launches += dist_line_ask_push(D.out_order, mg, D.cuts_g, nr, qouts, (u32)B.cap, D.tile_cnt, D.d_small_all, SMALL_WORDS, me, st);
         }))
       return rc;
     if (const int rc = dist_check_small(ctx, false)) return rc;
     // (a rank is asked only about the records of its slice, which fits its rows)
-    if (const int rc = check_inbound(ctx, W_CNT_A, D.cap, "rank %d is asked for %llu line records, capacity is %llu rows per rank")) return rc;
+    if (const int rc = check_inbound(ctx, W_CNT_A, B.cap, "rank %d is asked for %llu line records, capacity is %llu rows per rank")) return rc;
     Exchange exl;
     exl.from_matrix(D.h_small, W_CNT_A, nr, me);
     D.tr->bytes_sent += (exl.n_send - exl.scnt[me]) * 16 + (exl.n_recv - exl.rcnt[me]) * sizeof(LineRow);
-    launches += dist_line_answer(D.queries, (u32)exl.n_recv, D.aos_src, D.pk_src, D.file_off[me], scatter_table(D, exl, true, D.line_rows), st);
+    launches += dist_line_answer(D.queries, (u32)exl.n_recv, B.aos_src, B.pk_src, B.file_off[me], scatter_table(D, exl, true, D.line_rows), st);
     TR(D.tr->barrier(st));
     CK(cudaEventRecord(ev[8], st));
   }
@@ -1216,7 +1348,7 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   if (D.trace.on) {
     char cb[240];
     snprintf(cb, sizeof cb, "ranked=%u halo_in=%u halo_out=%u y=%u lines=%u groups=%llu stages x=%.3f y=%.3f forest=%.3f exch=%.3f order=%.3f |", m, nh,
-             D.n_away, D.m_y, mg, (unsigned long long)total_groups, ev_ms(ev[0], ev[1]), ev_ms(ev[1], ev[2]), ev_ms(ev[2], ev[3]),
+             B.n_away, B.m_y, mg, (unsigned long long)total_groups, ev_ms(ev[0], ev[1]), ev_ms(ev[1], ev[2]), ev_ms(ev[2], ev[3]),
              ev_ms(ev[3], ev[4]), ev_ms(ev[4], ev[5]));
     if (line_records) {
       const size_t k = strlen(cb) - 2;  // before the closing " |"
@@ -1246,16 +1378,16 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   if (info) {
     memset(info, 0, sizeof *info);
     info->rank = me, info->world = nr;
-    info->total_loaded = D.n_total_loaded;
-    info->total_kept = D.m_total;
+    info->total_loaded = B.n_total_loaded;
+    info->total_kept = B.m_total;
     info->total_groups = total_groups;
     info->line_offset = line_off;
     info->n_lines = mg;
-    info->rank_offset = D.rank_off;
+    info->rank_offset = B.rank_off;
     info->n_ranked = m;
     info->n_halo_in = nh;
-    info->n_halo_out = D.n_away;
-    info->n_y = D.m_y;
+    info->n_halo_out = B.n_away;
+    info->n_y = B.m_y;
     info->bytes_sent = D.tr->bytes_sent - sent0;
   }
   return RK_OK;
@@ -1298,9 +1430,10 @@ void dist_destroy(rk_ctx *c) {
   Dist *D = c->dist;
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->stream);
-  dist_release_buffers(*D);
+  dist_release_peers(*D);
   if (D->side) cudaStreamSynchronize(D->side), cudaStreamDestroy(D->side);
   delete D->tr;
+  if (--D->db->refs == 0) delete D->db;  // the partition database stays while other contexts of it are live
   delete D;
   c->dist = nullptr;
 }
@@ -1325,6 +1458,7 @@ int rk_dist_unique_id(void *id128) {
 
 int rk_dist_init(rk_ctx *ctx, int rank, int nranks, const void *id128, uint64_t cap_per_rank) {
   if (!ctx || !id128) return RK_ERR_ARG;
+  if (const int rc = dist_init_refusal(ctx)) return rc;  // (before the communicator: every rank refuses alike)
   NcclApi &N = nccl_api();
   if (!N.ok()) return fail(ctx, RK_ERR_CUDA, "NCCL is not available: %s", N.err.c_str());
   CK(cudaSetDevice(ctx->device));
@@ -1339,6 +1473,46 @@ int rk_dist_init(rk_ctx *ctx, int rank, int nranks, const void *id128, uint64_t 
     return rc;
   }
   return dist_init_common(ctx, rank, nranks, tr, cap_per_rank);
+}
+
+rk_ctx *rk_dist_create_view(rk_ctx *base, const void *id128) {
+  if (!id128) {
+    set_create_error("rk_dist_create_view: null unique id");
+    return nullptr;
+  }
+  // the refusals before the communicator starts: every rank's base is in the same state, so every rank refuses alike
+  if (const char *why = dist_view_refusal(base)) {
+    set_create_error(std::string("rk_dist_create_view: ") + why);
+    return nullptr;
+  }
+  NcclApi &N = nccl_api();
+  if (!N.ok()) {
+    set_create_error("rk_dist_create_view: NCCL is not available: " + N.err);
+    return nullptr;
+  }
+  const Dist &S = *base->dist;
+  if (cudaSetDevice(base->device) != cudaSuccess) {
+    cudaGetLastError();
+    set_create_error("rk_dist_create_view: cudaSetDevice failed");
+    return nullptr;
+  }
+  ncclUniqueId id;
+  memcpy(&id, id128, sizeof id);
+  NcclTransport *tr = new NcclTransport;
+  const ncclResult_t r = N.CommInitRank(&tr->comm, S.world, id, S.rank);
+  if (r != ncclSuccess) {
+    tr->comm = nullptr;
+    delete tr;
+    set_create_error(std::string("rk_dist_create_view: ncclCommInitRank: ") + N.GetErrorString(r));
+    return nullptr;
+  }
+  std::string err;
+  rk_ctx *v = dist_view_create(base, tr, err);
+  if (!v) {
+    set_create_error("rk_dist_create_view: " + err);
+    return nullptr;
+  }
+  return v;
 }
 
 int rk_dist_export(rk_ctx *ctx, void *blob) {
@@ -1358,6 +1532,7 @@ int rk_dist_load_aos(rk_ctx *ctx, const void *frags, uint64_t n_local, uint64_t 
                      unsigned flags, rk_load_stats *stats) {
   if (!ctx) return RK_ERR_ARG;
   if (!ctx->dist) return fail(ctx, RK_ERR_STATE, "rk_dist_load_aos before rk_dist_init");
+  if (const int rc = dist_load_refusal(ctx)) return rc;
   return dist_load(ctx, frags, n_local, file_offset, seqx_len, seqy_len, flags, stats);
 }
 
@@ -1365,6 +1540,7 @@ int rk_dist_load_csv(rk_ctx *ctx, const char *slice, uint64_t bytes, uint64_t se
                      unsigned flags, rk_load_stats *stats, rk_csv_stats *csv) {
   if (!ctx) return RK_ERR_ARG;
   if (!ctx->dist) return fail(ctx, RK_ERR_STATE, "rk_dist_load_csv before rk_dist_init");
+  if (const int rc = dist_load_refusal(ctx)) return rc;
   DistCsv L;
   dist_csv_local(ctx, slice, bytes, csv_upload_threads(), L);
   return dist_csv_finish(ctx, L, seqx_len, seqy_len, total_frags, flags, stats, csv);
@@ -1433,6 +1609,31 @@ struct rk_multi {
 
 namespace {
 
+// the transport of rank r: over mg's communicators, or through its LocalGroup
+Transport *multi_transport(rk_multi *mg, int r) {
+  if (mg->use_nccl) {
+    NcclTransport *t = new NcclTransport;
+    t->comm = mg->comms[r];
+    t->own_comm = false;
+    return t;
+  }
+  LocalTransport *t = new LocalTransport;
+  t->g = &mg->local;
+  return t;
+}
+
+// one communicator per device when the devices are distinct (NCCL); else, or when NCCL fails to start, the ranks are
+// threads of this process and the local transport always works
+void multi_init_comms(rk_multi *mg) {
+  if (!mg->use_nccl) return;
+  NcclApi &N = nccl_api();
+  mg->comms.resize(mg->n);
+  if (!N.ok() || N.CommInitAll(mg->comms.data(), mg->n, mg->devices.data()) != ncclSuccess) {
+    mg->comms.clear();
+    mg->use_nccl = false;
+  }
+}
+
 template <class F>
 int run_ranks(rk_multi *mg, F fn) {  // fn(rank) on one thread per rank; first failing rank's code and message
   std::vector<int> rc(mg->n, RK_OK);
@@ -1447,33 +1648,32 @@ int run_ranks(rk_multi *mg, F fn) {  // fn(rank) on one thread per rank; first f
   return RK_OK;
 }
 
+// every rank's partition arena (a view: its workspace) mapped into every other rank
+int multi_map_peers(rk_multi *mg) {
+  std::vector<u8> blobs((size_t)mg->n * RK_DIST_BLOB_BYTES, 0);
+  const int rc = run_ranks(mg, [&](int r) { return dist_export(mg->ctx[r], (DistBlob *)(blobs.data() + (size_t)r * RK_DIST_BLOB_BYTES)); });
+  return rc ? rc : run_ranks(mg, [&](int r) { return dist_import(mg->ctx[r], blobs.data(), RK_DIST_BLOB_BYTES); });
+}
+
 int multi_set_capacity(rk_multi *mg, u64 cap) {
   int rc = run_ranks(mg, [&](int r) {
     rk_ctx *c = mg->ctx[r];
-    if (!c->dist) {
-      Transport *tr;
-      if (mg->use_nccl) {
-        NcclTransport *t = new NcclTransport;
-        t->comm = mg->comms[r];
-        t->own_comm = false;
-        tr = t;
-      } else {
-        LocalTransport *t = new LocalTransport;
-        t->g = &mg->local;
-        tr = t;
-      }
-      return dist_init_common(c, r, mg->n, tr, cap);
-    }
+    if (!c->dist) return dist_init_common(c, r, mg->n, multi_transport(mg, r), cap);
     return dist_allocate(c, cap);
   });
   if (rc) return rc;
-  std::vector<u8> blobs((size_t)mg->n * RK_DIST_BLOB_BYTES, 0);
-  rc = run_ranks(mg, [&](int r) { return dist_export(mg->ctx[r], (DistBlob *)(blobs.data() + (size_t)r * RK_DIST_BLOB_BYTES)); });
-  if (rc) return rc;
-  rc = run_ranks(mg, [&](int r) { return dist_import(mg->ctx[r], blobs.data(), RK_DIST_BLOB_BYTES); });
-  if (rc) return rc;
+  if ((rc = multi_map_peers(mg))) return rc;
   mg->cap = cap;
   return RK_OK;
+}
+
+// the load refusals of rk_multi_load_*: a view, or a base with live views (rank 0 speaks for all: they are made together)
+int multi_load_refusal(rk_multi *mg) {
+  rk_ctx *c = mg->ctx[0];
+  if (!c->dist) return RK_OK;
+  const int rc = dist_load_refusal(c);
+  if (rc) mg->err = c->err;
+  return rc;
 }
 
 }  // namespace
@@ -1499,15 +1699,43 @@ rk_multi *rk_create_multi(const int *devices, int ndev) {
     }
     mg->ctx.push_back(c);
   }
-  if (mg->use_nccl) {
-    NcclApi &N = nccl_api();
-    mg->comms.resize(ndev);
-    if (!N.ok() || N.CommInitAll(mg->comms.data(), ndev, devices) != ncclSuccess) {
-      mg->comms.clear();
-      mg->use_nccl = false;  // ranks are threads of this process: the local transport always works
-    }
-  }
+  multi_init_comms(mg);
   return mg;
+}
+
+rk_multi *rk_multi_create_view(rk_multi *base) {
+  if (!base) {
+    set_create_error("rk_multi_create_view: null rk_multi");
+    return nullptr;
+  }
+  if (!base->have_load) {
+    set_create_error("rk_multi_create_view: no partition database (it needs a successful rk_multi_load_aos or rk_multi_load_csv)");
+    return nullptr;
+  }
+  rk_multi *v = new rk_multi;
+  v->n = base->n;
+  v->local.n = base->n;
+  v->devices = base->devices;
+  v->use_nccl = base->use_nccl;
+  multi_init_comms(v);
+  for (int r = 0; r < v->n; ++r) {
+    std::string err;
+    rk_ctx *c = dist_view_create(base->ctx[r], multi_transport(v, r), err);
+    if (!c) {
+      set_create_error("rk_multi_create_view: rank " + std::to_string(r) + ": " + err);
+      rk_destroy_multi(v);
+      return nullptr;
+    }
+    v->ctx.push_back(c);
+  }
+  if (multi_map_peers(v)) {
+    set_create_error("rk_multi_create_view: " + v->err);
+    rk_destroy_multi(v);
+    return nullptr;
+  }
+  v->cap = base->cap;
+  v->have_load = true;
+  return v;
 }
 
 void rk_destroy_multi(rk_multi *mg) {
@@ -1525,6 +1753,7 @@ const char *rk_multi_transport(const rk_multi *mg) { return !mg ? "" : (mg->use_
 int rk_multi_load_aos(rk_multi *mg, const void *frags, uint64_t n, uint64_t seqx_len, uint64_t seqy_len, unsigned flags,
                       rk_load_stats *stats) {
   if (!mg || (!frags && n)) return RK_ERR_ARG;
+  if (const int rc = multi_load_refusal(mg)) return rc;
   mg->have_load = false;
   // every rank starts with a contiguous slice of the file (slices start on a 16-record boundary: 16-byte aligned records)
   std::vector<u64> lo(mg->n + 1);
@@ -1556,6 +1785,7 @@ int rk_multi_load_aos(rk_multi *mg, const void *frags, uint64_t n, uint64_t seqx
 int rk_multi_load_csv(rk_multi *mg, const char *body, uint64_t bytes, uint64_t seqx_len, uint64_t seqy_len, uint64_t total_frags,
                       unsigned flags, rk_load_stats *stats, rk_csv_stats *csv) {
   if (!mg || (!body && bytes)) return RK_ERR_ARG;
+  if (const int rc = multi_load_refusal(mg)) return rc;
   mg->have_load = false;
   if (bytes && is_device_pointer(body)) {
     mg->err = "rk_multi_load_csv takes the text in host memory";

@@ -335,6 +335,7 @@ struct ProfGuard {  // routes the launchers' KScope events to this context for t
 const char *err_bits_text(u32 e);
 float ev_ms(cudaEvent_t a, cudaEvent_t b);
 void dist_destroy(rk_ctx *c);  // multi.cu: releases c->dist (called by rk_destroy)
+void set_create_error(const std::string &s);  // capi.cu: the text rk_create_error() returns
 
 // capi.cu: the work behind rk_format_lines / rk_group_statistics, shared with their partitioned forms (multi.cu).
 // K6 into the context's device text buffer (records ev[0]); *nbytes = the bytes formatted.  Synchronises.
