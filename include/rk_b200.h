@@ -303,6 +303,22 @@ int rk_dist_load_aos(rk_ctx *ctx, const void *frags, uint64_t n_local, uint64_t 
  * in its slice).  Collective. */
 int rk_dist_load_csv(rk_ctx *ctx, const char *slice, uint64_t bytes, uint64_t seqx_len, uint64_t seqy_len, uint64_t total_frags,
                      unsigned flags, rk_load_stats *stats, rk_csv_stats *csv);
+/* rk_load_packed over the ranks: this rank's contiguous slice of the file in the compact form of rk_load_packed (key4,
+ * strand, rest4 or NULL; 33 B per fragment instead of 109 B), n_local fragments, file_offset = index of its first one, as
+ * rk_dist_load_aos takes them.  Groups, text and statistics are bit-identical to rk_dist_load_aos on the same records.
+ *  - Host arrays, pinned or pageable, are copied into the rank's buffers (rest4 beside the load's kernels), and every copy
+ *    has finished when the call returns: the caller may overwrite or free all three arrays then.
+ *  - Device arrays must be on the rank's device, key4 and rest4 16-byte aligned; they are used in place and must stay where
+ *    they are for rk_dist_group with RK_F_LINE_RECORDS, as device records of rk_dist_load_aos must.
+ *  - rest4 == NULL: grouping works; a later rk_dist_group with RK_F_LINE_RECORDS returns RK_ERR_ARG on every rank when any
+ *    rank loaded fragments without rest4.
+ *  - Refusals reach every rank with the same code and message (prefixed by the rank that refused) and leave nothing
+ *    loaded: a null key4 or strand with n_local > 0, arrays partly in host and partly in device memory, a misaligned device
+ *    array or one on another device (RK_ERR_ARG), n_local over the capacity or a failed staging allocation
+ *    (RK_ERR_NOMEM), a sequence length of 2^32 or more (RK_ERR_RANGE), 2^32-16 or more records (RK_ERR_ARG); then the
+ *    refusals of rk_dist_load_aos (a coordinate beyond the sequence: RK_ERR_RANGE).  Collective. */
+int rk_dist_load_packed(rk_ctx *ctx, const uint32_t *key4, const uint8_t *strand, const uint32_t *rest4, uint64_t n_local,
+                        uint64_t file_offset, uint64_t seqx_len, uint64_t seqy_len, unsigned flags, rk_load_stats *stats);
 /* out: THIS RANK's range of output lines (order = file indices of the whole file, gid = global group ids); n_groups is
  * the global count.  info may be NULL. */
 int rk_dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flags, rk_result *out, rk_dist_info *info);
@@ -355,6 +371,12 @@ int rk_multi_load_aos(rk_multi *m, const void *frags, uint64_t n, uint64_t seqx_
  * (at most 4): each rank copies on its own thread, and helpers only while the ranks are fewer than T. */
 int rk_multi_load_csv(rk_multi *m, const char *body, uint64_t bytes, uint64_t seqx_len, uint64_t seqy_len, uint64_t total_frags,
                       unsigned flags, rk_load_stats *stats, rk_csv_stats *csv);
+/* key4, strand, rest4 (or NULL): the whole file in the compact form of rk_load_packed, in HOST memory (a device array
+ * returns RK_ERR_ARG); the ranks take the slices of rk_multi_load_aos, and the capacity per rank is sized as there, so
+ * rk_multi_info reports the same partition for both loads.  Every rank loads its slice as rk_dist_load_packed does; the
+ * arrays may be freed when the call returns.  ms_stage[RK_ST_H2D] of stats = the largest of the ranks' copies. */
+int rk_multi_load_packed(rk_multi *m, const uint32_t *key4, const uint8_t *strand, const uint32_t *rest4, uint64_t n, uint64_t seqx_len,
+                         uint64_t seqy_len, unsigned flags, rk_load_stats *stats);
 /* out: the whole result in pinned host memory owned by m (device pointers are NULL), valid until the next call. */
 int rk_multi_group(rk_multi *m, double len_ratio, double pos_ratio, unsigned flags, rk_result *out);
 int rk_multi_info(const rk_multi *m, int rank, rk_dist_info *info);

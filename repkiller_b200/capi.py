@@ -25,10 +25,10 @@ SYMBOLS = ["rk_create", "rk_create_view", "rk_create_error", "rk_destroy", "rk_l
            "rk_diagonal_func", "rk_format_lines", "rk_debug_fetch", "rk_profile_enable", "rk_profile_read", "rk_sort_pairs_work_bytes", "rk_sort_pairs", "rk_version",
            "rk_gen_workload", "rk_sort_members", "rk_group_statistics", "rk_sol_create", "rk_sol_destroy", "rk_sol_insert", "rk_sol_get_associated", "rk_sol_last_error",
            # one comparison over several GPUs
-           "rk_dist_unique_id", "rk_dist_init", "rk_dist_export", "rk_dist_import", "rk_dist_load_aos", "rk_dist_load_csv", "rk_dist_group",
-           "rk_dist_format_lines", "rk_dist_group_statistics", "rk_dist_create_view",
+           "rk_dist_unique_id", "rk_dist_init", "rk_dist_export", "rk_dist_import", "rk_dist_load_aos", "rk_dist_load_csv", "rk_dist_load_packed",
+           "rk_dist_group", "rk_dist_format_lines", "rk_dist_group_statistics", "rk_dist_create_view",
            "rk_create_multi", "rk_destroy_multi", "rk_multi_last_error", "rk_multi_ranks", "rk_multi_ctx", "rk_multi_transport",
-           "rk_multi_load_aos", "rk_multi_load_csv", "rk_multi_group", "rk_multi_info", "rk_multi_format_lines", "rk_multi_group_statistics",
+           "rk_multi_load_aos", "rk_multi_load_csv", "rk_multi_load_packed", "rk_multi_group", "rk_multi_info", "rk_multi_format_lines", "rk_multi_group_statistics",
            "rk_multi_create_view"]
 DIST_ID_BYTES, DIST_BLOB_BYTES = 128, 128
 GROUP_STATS_DTYPE = np.dtype([("count", "<u4"), ("x_lo", "<u4"), ("x_hi", "<u4"), ("y_lo", "<u4"), ("y_hi", "<u4"), ("first_line", "<u4"),
@@ -116,6 +116,7 @@ def load_library():
     L.rk_dist_import.argtypes = [C.c_void_p, C.c_void_p]
     L.rk_dist_load_aos.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint, C.POINTER(_LoadStats)]
     L.rk_dist_load_csv.argtypes = L.rk_load_csv.argtypes
+    L.rk_dist_load_packed.argtypes = [C.c_void_p] * 4 + [C.c_uint64] * 4 + [C.c_uint, C.POINTER(_LoadStats)]
     L.rk_dist_group.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_uint, C.POINTER(_Result), C.POINTER(_DistInfo)]
     L.rk_dist_format_lines.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(_Text)]
     L.rk_dist_group_statistics.argtypes = [C.c_void_p, C.c_uint, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_uint64),
@@ -134,6 +135,7 @@ def load_library():
     L.rk_multi_transport.restype = C.c_char_p
     L.rk_multi_load_aos.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint, C.POINTER(_LoadStats)]
     L.rk_multi_load_csv.argtypes = L.rk_load_csv.argtypes
+    L.rk_multi_load_packed.argtypes = L.rk_load_packed.argtypes
     L.rk_multi_group.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_uint, C.POINTER(_Result)]
     L.rk_multi_info.argtypes = [C.c_void_p, C.c_int, C.POINTER(_DistInfo)]
     L.rk_multi_format_lines.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(_Text)]
@@ -266,15 +268,9 @@ class Context:
     def load_packed(self, key4, strand, rest4, seqx_len: int, seqy_len: int, n: int | None = None, timing: bool = True) -> LoadStats:
         """The compact ingest (rk_load_packed): numpy arrays key4 [n,4] u32, strand [n] u8, rest4 [n,4] u32 or None — or int
         pointers (host or device) with n given."""
-        if isinstance(key4, np.ndarray):
-            k, s_ = np.ascontiguousarray(key4, dtype=np.uint32), np.ascontiguousarray(strand, dtype=np.uint8)
-            r = np.ascontiguousarray(rest4, dtype=np.uint32) if rest4 is not None else None
-            n = s_.shape[0]
-            self._keep = (k, s_, r)
-            pk, ps, pr = k.ctypes.data, s_.ctypes.data, (r.ctypes.data if r is not None else None)
-        else:
-            pk, ps, pr = int(key4), int(strand), (int(rest4) if rest4 else None)
-            assert n is not None
+        keep, pk, ps, pr, n = _packed_args(key4, strand, rest4, n)
+        if keep is not None:
+            self._keep = keep
         st = _LoadStats()
         self._check(self._L.rk_load_packed(self._h, C.c_void_p(pk), C.c_void_p(ps), C.c_void_p(pr) if pr else None, n, seqx_len, seqy_len,
                                            F_TIMING if timing else 0, C.byref(st)))
@@ -425,6 +421,19 @@ class Context:
                                              F_TIMING if timing else 0, C.byref(st), C.byref(cs)))
         return _csv_result(st, cs)
 
+    def dist_load_packed(self, key4, strand, rest4, file_offset: int, seqx_len: int, seqy_len: int, n: int | None = None,
+                         timing: bool = False) -> LoadStats:
+        """This rank's slice of the file in the compact form (rk_dist_load_packed; collective): the arguments of load_packed,
+        file_offset = the file index of the slice's first fragment.  Host arrays are copied before the call returns;
+        device arrays (int pointers on this rank's device, key4 and rest4 16-byte aligned) are used in place."""
+        _, pk, ps, pr, n = _packed_args(key4, strand, rest4, n)
+        st = _LoadStats()
+        self._check(self._L.rk_dist_load_packed(self._h, C.c_void_p(pk) if pk else None, C.c_void_p(ps) if ps else None,
+                                                C.c_void_p(pr) if pr else None, n, file_offset, seqx_len, seqy_len,
+                                                F_TIMING if timing else 0, C.byref(st)))
+        return LoadStats(st.n_loaded, st.n_kept, st.vsize, {STAGES[i]: st.ms_stage[i] for i in range(NSTAGES)}, st.ms_device,
+                         st.n_launches)
+
     def dist_group(self, len_ratio: float, pos_ratio: float, host_result: bool = True, sort: bool = True, timing: bool = False,
                    copy: bool = True, line_records: bool = False):
         """(Groups of THIS rank's range of output lines, info dict); line_records: for dist_format_lines /
@@ -484,6 +493,17 @@ def _groups_of(r: "_Result", host_result: bool, copy: bool) -> Groups:
     return Groups(m, r.n_groups, arr(r.order, np.uint32), arr(r.gid, np.uint32), arr(r.repval, np.uint8), arr(r.identity, np.float32),
                   {"order": r.d_order, "gid": r.d_gid, "repval": r.d_repval, "identity": r.d_identity},
                   {STAGES[i]: r.ms_stage[i] for i in range(NSTAGES)}, r.ms_device, r.n_launches)
+
+
+def _packed_args(key4, strand, rest4, n):
+    """(arrays to keep alive or None, key4, strand, rest4 addresses (rest4 None when absent), n) of the compact arrays:
+    numpy arrays key4 [n,4] u32, strand [n] u8, rest4 [n,4] u32 or None — or int pointers with n given"""
+    if isinstance(key4, np.ndarray):
+        k, s_ = np.ascontiguousarray(key4, dtype=np.uint32), np.ascontiguousarray(strand, dtype=np.uint8)
+        r = np.ascontiguousarray(rest4, dtype=np.uint32) if rest4 is not None else None
+        return (k, s_, r), k.ctypes.data, s_.ctypes.data, (r.ctypes.data if r is not None else None), s_.shape[0]
+    assert n is not None
+    return None, int(key4), int(strand), (int(rest4) if rest4 else None), n
 
 
 def pack_records(rec: np.ndarray):
@@ -637,6 +657,17 @@ class Multi:
         self._check(self._L.rk_multi_load_csv(self._h, C.c_void_p(ptr) if n else None, n, seqx_len, seqy_len, total_frags,
                                               F_TIMING if timing else 0, C.byref(st), C.byref(cs)))
         return _csv_result(st, cs)
+
+    def load_packed(self, key4, strand, rest4, seqx_len: int, seqy_len: int, n: int | None = None, timing: bool = False) -> LoadStats:
+        """The whole file in the compact form of Context.load_packed, in host memory (numpy arrays, or int host pointers with
+        n given), cut into load()'s slices (rk_multi_load_packed); the arrays may go when this returns."""
+        _, pk, ps, pr, n = _packed_args(key4, strand, rest4, n)
+        st = _LoadStats()
+        self._check(self._L.rk_multi_load_packed(self._h, C.c_void_p(pk) if pk else None, C.c_void_p(ps) if ps else None,
+                                                 C.c_void_p(pr) if pr else None, n, seqx_len, seqy_len, F_TIMING if timing else 0,
+                                                 C.byref(st)))
+        return LoadStats(st.n_loaded, st.n_kept, st.vsize, {STAGES[i]: st.ms_stage[i] for i in range(NSTAGES)}, st.ms_device,
+                         st.n_launches)
 
     def group(self, len_ratio: float, pos_ratio: float, sort: bool = True, line_records: bool = False) -> Groups:
         """line_records: every rank also gets the records of its output lines, for format_lines / group_statistics"""

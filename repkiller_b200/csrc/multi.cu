@@ -386,7 +386,8 @@ struct DistDb {
   GrowBuffer arena;  // carved by dist_carve: this database, then the workspace of the loading context
   u64 cap = 0, hcap = 0;
   // grow-only side buffers whose size depends on the input, not on cap
-  GrowBuffer aos_buf;  // this rank's records: a host slice staged (109 B per row), or its parsed CSV rows (compact or 109 B)
+  GrowBuffer aos_buf;  // this rank's records: a host slice staged (109 B per row), its parsed CSV rows (compact or 109 B), or
+                       // its host compact arrays staged (33 B per row, laid out as csv_emit lays out compact rows)
   GrowBuffer link_buf;  // u32 [hist0][linkx_loc][linky_loc] (one all-gather) [linkx][linky][gather: world * the first three]
 
   // state of the last load
@@ -397,7 +398,9 @@ struct DistDb {
   u64 m_total = 0, n_total_loaded = 0;
   Exchange ex1, exh, exy;
   const u8 *aos_src = nullptr;          // this rank's slice of the records on the device (aos_buf or the caller's pointer)
-  PackedRows pk_src{};                  // ... or its compact rows (rk_dist_load_csv without a wide value; aos_src == nullptr)
+  PackedRows pk_src{};                  // ... or its compact rows (rk_dist_load_csv without a wide value, rk_dist_load_packed;
+                                        // aos_src == nullptr)
+  int rest_missing = -1;                // rk_dist_load_packed: the first rank that loaded records without rest4, or -1
   u32 file_off[DIST_MAX_RANKS] = {0};  // first file index of every rank's slice
   bool slices_in_order = false;         // every slice ends at or before the next rank's starts: file_off[] routes a file index
   u32 roff[DIST_MAX_RANKS + 1] = {0};   // first rank-order index of every rank, then the total (PeerTable::roff)
@@ -675,7 +678,8 @@ static int dist_init_common(rk_ctx *ctx, int rank, int world, Transport *tr, u64
 static const char *dist_view_refusal(const rk_ctx *base) {
   if (!base || !base->dist) return "the context is not part of a comparison partitioned over several GPUs (rk_dist_init / rk_multi)";
   if (!base->dist->db->loaded)
-    return "the context holds no partition database (it needs a successful rk_dist_load_aos, rk_dist_load_csv or rk_multi_load_*)";
+    return "the context holds no partition database (it needs a successful rk_dist_load_aos, rk_dist_load_csv, rk_dist_load_packed or "
+           "rk_multi_load_*)";
   return nullptr;
 }
 
@@ -855,6 +859,7 @@ static int dist_load(rk_ctx *ctx, const void *frags, u64 n_loc, u64 file_off, u6
   ProfGuard pg(ctx);
   cudaStream_t st = ctx->stream;
   B.loaded = false;
+  B.rest_missing = -1;  // (rk_dist_load_packed sets it after this returns)
   D.have_rows = false;
   ctx->have_group = false;
   // NOTE: argument errors that only ONE rank can see (n_loc > cap) are turned into an error word all ranks receive with
@@ -1166,6 +1171,112 @@ static int dist_csv_finish(rk_ctx *ctx, DistCsv &L, u64 seqx_len, u64 seqy_len, 
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
+// load from compact arrays: rk_load_packed over the ranks
+// ---------------------------------------------------------------------------------------------------------------------
+// the device of a device pointer; -1 for host memory of any kind
+static int device_of(const void *p) {
+  cudaPointerAttributes pa;
+  if (cudaPointerGetAttributes(&pa, p) == cudaSuccess && pa.type == cudaMemoryTypeDevice) return pa.device;
+  cudaGetLastError();
+  return -1;
+}
+
+// the status row of rk_dist_load_packed, gathered before anything is copied or loaded: a rank whose own checks failed
+// sends its code and the start of its message, so that every rank returns the same code and text
+enum { PW_RC, PW_NO_REST, PW_MSG, PW_WORDS = PW_MSG + 28 };
+static_assert(PW_WORDS <= SMALL_WORDS, "the status row fits the rows of d_small");
+
+// The rank-local checks of rk_dist_load_packed and, for host arrays, the staging area in aos_buf (key4, rest4, strand as
+// csv_emit places them).  Touches no peer; the verdict travels in the status row.
+static int dist_packed_local(rk_ctx *ctx, const u32 *key4, const u8 *strand, const u32 *rest4, u64 n, u64 file_off, u64 seqx_len,
+                             u64 seqy_len, PackedRows *pk) {
+  Dist &D = *ctx->dist;
+  DistDb &B = *D.db;
+  if (!D.peers_ready) return fail(ctx, RK_ERR_STATE, "rk_dist_load_packed before rk_dist_import");
+  if (seqx_len >= (1ull << 32) || seqy_len >= (1ull << 32)) return fail(ctx, RK_ERR_RANGE, "sequence length does not fit in 32 bits");
+  if (file_off + n >= 0xFFFFFFF0ull) return fail(ctx, RK_ERR_ARG, "more than 2^32-16 records in one comparison");
+  if (n > B.cap)
+    return fail(ctx, RK_ERR_NOMEM, "a rank holds more records than the capacity of %llu rows per rank given to rk_dist_init",
+                (unsigned long long)B.cap);
+  *pk = PackedRows{};
+  if (!n) return RK_OK;
+  if (!key4 || !strand) return fail(ctx, RK_ERR_ARG, "null array");
+  const int dev = device_of(key4);
+  if (device_of(strand) != dev || (rest4 && device_of(rest4) != dev))
+    return fail(ctx, RK_ERR_ARG, "the arrays of rk_dist_load_packed must all be host or all be device memory");
+  if (dev >= 0) {
+    if (dev != ctx->device) return fail(ctx, RK_ERR_ARG, "the arrays are on device %d, this rank's context on device %d", dev, ctx->device);
+    if (((uintptr_t)key4 & 15) || ((uintptr_t)rest4 & 15)) return fail(ctx, RK_ERR_ARG, "device arrays key4 and rest4 must be 16-byte aligned");
+    *pk = PackedRows{(const uint4 *)key4, (const uint4 *)rest4, strand};
+    return RK_OK;
+  }
+  CK(cudaSetDevice(ctx->device));
+  if (const int rc = B.aos_buf.reserve(csv_out_bytes(n, false), ctx->stream, ctx->err)) {
+    const std::string e = ctx->err;
+    return fail(ctx, rc, "rk_dist_load_packed: %llu rows: %s", (unsigned long long)n, e.c_str());
+  }
+  const u64 key_b = align_up(n * 16, 256);
+  u8 *ob = (u8 *)B.aos_buf.ptr();
+  *pk = PackedRows{(const uint4 *)ob, rest4 ? (const uint4 *)(ob + key_b) : nullptr, ob + 2 * key_b};
+  return RK_OK;
+}
+
+// rk_dist_load_packed: the local checks, one status all-gather (every rank reaches the same verdict), then the copies of
+// host arrays — key4 and strand on the context's stream before K1, rest4 on the database's copy stream beside the load's
+// kernels — and dist_load on the compact rows.  Every copy has finished when this returns, whatever the outcome.
+static int dist_load_packed(rk_ctx *ctx, const u32 *key4, const u8 *strand, const u32 *rest4, u64 n, u64 file_off, u64 seqx_len,
+                            u64 seqy_len, unsigned flags, rk_load_stats *stats) {
+  Dist &D = *ctx->dist;
+  DistDb &B = *D.db;
+  B.loaded = false;
+  B.aos_src = nullptr, B.pk_src = PackedRows{};
+  D.have_rows = false;
+  ctx->loaded = ctx->have_group = false;
+  PackedRows pk;
+  const int lrc = dist_packed_local(ctx, key4, strand, rest4, n, file_off, seqx_len, seqy_len, &pk);
+  CK(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  u32 row[PW_WORDS] = {(u32)lrc, (u32)(n && !rest4)};
+  if (lrc) memcpy(&row[PW_MSG], ctx->err.c_str(), std::min<size_t>(ctx->err.size(), (PW_WORDS - PW_MSG) * 4 - 1));
+  CK(cudaMemcpyAsync(D.d_small, row, sizeof row, cudaMemcpyHostToDevice, st));  // (pageable source: staged at once)
+  TR(D.tr->all_gather(D.d_small, D.d_small_all, sizeof row, st));
+  std::vector<u32> all((size_t)D.world * PW_WORDS);
+  CK(cudaMemcpyAsync(all.data(), D.d_small_all, all.size() * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  int no_rest = -1;
+  for (int r = 0; r < D.world; ++r) {
+    const u32 *w = &all[(size_t)r * PW_WORDS];
+    if (w[PW_RC]) return fail(ctx, (int)w[PW_RC], "rank %d: %s", r, (const char *)&w[PW_MSG]);
+    if (w[PW_NO_REST] && no_rest < 0) no_rest = r;
+  }
+  const bool staged = n && pk.key != (const uint4 *)key4;
+  cudaEvent_t *ev = ctx->ev;
+  Database &db = *ctx->db;
+  if (staged) {
+    CK(cudaEventRecord(ev[EV_PK_UP0], st));
+    CK(cudaMemcpyAsync((void *)pk.key, key4, n * 16, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync((void *)pk.strand, strand, n, cudaMemcpyHostToDevice, st));
+    CK(cudaEventRecord(ev[EV_PK_UP1], st));
+    if (rest4) {  // only the line records read it: it travels while K1 and the exchanges run
+      CK(cudaStreamWaitEvent(db.copy_stream, ev[EV_PK_UP0], 0));  // (after the work queued on st is done with aos_buf)
+      CK(cudaMemcpyAsync((void *)pk.rest, rest4, n * 16, cudaMemcpyHostToDevice, db.copy_stream));
+      CK(cudaEventRecord(ev[EV_PK_REST], db.copy_stream));
+    }
+  }
+  const int rc = dist_load(ctx, nullptr, n, file_off, seqx_len, seqy_len, flags, stats, &pk);
+  // the caller may overwrite or free its arrays once this returns: wait for every copy, on success and failure alike
+  const cudaError_t e1 = staged ? cudaEventSynchronize(ev[EV_PK_UP1]) : cudaSuccess;
+  const cudaError_t e2 = staged && rest4 ? cudaEventSynchronize(ev[EV_PK_REST]) : cudaSuccess;
+  if (rc) return rc;
+  CK(e1);
+  CK(e2);
+  B.rest_missing = no_rest;
+  if (stats && (flags & RK_F_TIMING))
+    stats->ms_stage[RK_ST_H2D] = !staged ? 0.f : std::max(ev_ms(ev[EV_PK_UP0], ev[EV_PK_UP1]), rest4 ? ev_ms(ev[EV_PK_UP0], ev[EV_PK_REST]) : 0.f);
+  return RK_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
 // group: generate_fragment_groups + generate_diagonal_func + sort_groups over the ranks
 // ---------------------------------------------------------------------------------------------------------------------
 static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flags, rk_result *out, rk_dist_info *info) {
@@ -1178,6 +1289,9 @@ static int dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned 
   if (!(pos_ratio > 0)) return fail(ctx, RK_ERR_ARG, "Position proximity must be greater than zero");
   if ((flags & RK_F_LINE_RECORDS) && !B.slices_in_order)
     return fail(ctx, RK_ERR_ARG, "RK_F_LINE_RECORDS needs the ranks' slices of the file in rank order (file_offset of rk_dist_load_aos)");
+  if ((flags & RK_F_LINE_RECORDS) && B.rest_missing >= 0)
+    return fail(ctx, RK_ERR_ARG, "RK_F_LINE_RECORDS needs the xEnd/yEnd/score/similarity array: rank %d loaded its compact rows without rest4",
+                B.rest_missing);
   CK(cudaSetDevice(ctx->device));
   ProfGuard pg(ctx);
   memset(out, 0, sizeof *out);
@@ -1546,6 +1660,14 @@ int rk_dist_load_csv(rk_ctx *ctx, const char *slice, uint64_t bytes, uint64_t se
   return dist_csv_finish(ctx, L, seqx_len, seqy_len, total_frags, flags, stats, csv);
 }
 
+int rk_dist_load_packed(rk_ctx *ctx, const uint32_t *key4, const uint8_t *strand, const uint32_t *rest4, uint64_t n_local,
+                        uint64_t file_offset, uint64_t seqx_len, uint64_t seqy_len, unsigned flags, rk_load_stats *stats) {
+  if (!ctx) return RK_ERR_ARG;
+  if (!ctx->dist) return fail(ctx, RK_ERR_STATE, "rk_dist_load_packed before rk_dist_init");
+  if (const int rc = dist_load_refusal(ctx)) return rc;
+  return dist_load_packed(ctx, key4, strand, rest4, n_local, file_offset, seqx_len, seqy_len, flags, stats);
+}
+
 int rk_dist_group(rk_ctx *ctx, double len_ratio, double pos_ratio, unsigned flags, rk_result *out, rk_dist_info *info) {
   if (!ctx || !out) return RK_ERR_ARG;
   if (!ctx->dist) return fail(ctx, RK_ERR_STATE, "rk_dist_group before rk_dist_init");
@@ -1667,6 +1789,22 @@ int multi_set_capacity(rk_multi *mg, u64 cap) {
   return RK_OK;
 }
 
+// the slices of an n-record file, lo[r] .. lo[r + 1] for rank r (rk_multi_load_aos, rk_multi_load_packed): every rank starts
+// with a contiguous slice of the file (slices start on a 16-record boundary: 16-byte aligned records); the capacity grows
+// to 1.5 x the largest slice + 65536
+int multi_record_slices(rk_multi *mg, u64 n, std::vector<u64> &lo) {
+  lo.assign(mg->n + 1, 0);
+  for (int r = 0; r <= mg->n; ++r) {
+    u64 b = n * (u64)r / (u64)mg->n;
+    if (r < mg->n) b -= b % 16;
+    lo[r] = r == mg->n ? n : b;
+  }
+  u64 biggest = 0;
+  for (int r = 0; r < mg->n; ++r) biggest = std::max(biggest, lo[r + 1] - lo[r]);
+  const u64 want = biggest + biggest / 2 + (1u << 16);
+  return want > mg->cap ? multi_set_capacity(mg, want) : RK_OK;
+}
+
 // the load refusals of rk_multi_load_*: a view, or a base with live views (rank 0 speaks for all: they are made together)
 int multi_load_refusal(rk_multi *mg) {
   rk_ctx *c = mg->ctx[0];
@@ -1709,7 +1847,8 @@ rk_multi *rk_multi_create_view(rk_multi *base) {
     return nullptr;
   }
   if (!base->have_load) {
-    set_create_error("rk_multi_create_view: no partition database (it needs a successful rk_multi_load_aos or rk_multi_load_csv)");
+    set_create_error("rk_multi_create_view: no partition database (it needs a successful rk_multi_load_aos, rk_multi_load_csv or "
+                     "rk_multi_load_packed)");
     return nullptr;
   }
   rk_multi *v = new rk_multi;
@@ -1755,20 +1894,8 @@ int rk_multi_load_aos(rk_multi *mg, const void *frags, uint64_t n, uint64_t seqx
   if (!mg || (!frags && n)) return RK_ERR_ARG;
   if (const int rc = multi_load_refusal(mg)) return rc;
   mg->have_load = false;
-  // every rank starts with a contiguous slice of the file (slices start on a 16-record boundary: 16-byte aligned records)
-  std::vector<u64> lo(mg->n + 1);
-  for (int r = 0; r <= mg->n; ++r) {
-    u64 b = n * (u64)r / (u64)mg->n;
-    if (r < mg->n) b -= b % 16;
-    lo[r] = r == mg->n ? n : b;
-  }
-  u64 biggest = 0;
-  for (int r = 0; r < mg->n; ++r) biggest = std::max(biggest, lo[r + 1] - lo[r]);
-  const u64 want = biggest + biggest / 2 + (1u << 16);
-  if (want > mg->cap) {
-    const int rc = multi_set_capacity(mg, want);
-    if (rc) return rc;
-  }
+  std::vector<u64> lo;
+  if (const int rc = multi_record_slices(mg, n, lo)) return rc;
   std::vector<rk_load_stats> st(mg->n);
   const int rc = run_ranks(mg, [&](int r) {
     return dist_load(mg->ctx[r], (const u8 *)frags + lo[r] * RK_FRAG_BYTES, lo[r + 1] - lo[r], lo[r], seqx_len, seqy_len, flags, &st[r]);
@@ -1834,6 +1961,34 @@ int rk_multi_load_csv(rk_multi *mg, const char *body, uint64_t bytes, uint64_t s
       csv->wide |= cs[r].wide;
       csv->ms_upload = std::max(csv->ms_upload, cs[r].ms_upload);
       csv->ms_parse = std::max(csv->ms_parse, cs[r].ms_parse);
+    }
+  }
+  mg->have_load = true;
+  return RK_OK;
+}
+
+int rk_multi_load_packed(rk_multi *mg, const uint32_t *key4, const uint8_t *strand, const uint32_t *rest4, uint64_t n, uint64_t seqx_len,
+                         uint64_t seqy_len, unsigned flags, rk_load_stats *stats) {
+  if (!mg || (n && (!key4 || !strand))) return RK_ERR_ARG;
+  if (const int rc = multi_load_refusal(mg)) return rc;
+  mg->have_load = false;
+  if (n && (is_device_pointer(key4) || is_device_pointer(strand) || (rest4 && is_device_pointer(rest4)))) {
+    mg->err = "rk_multi_load_packed takes the arrays in host memory";
+    return RK_ERR_ARG;
+  }
+  std::vector<u64> lo;  // the slices and the capacity of rk_multi_load_aos: both loads partition a file alike
+  if (const int rc = multi_record_slices(mg, n, lo)) return rc;
+  std::vector<rk_load_stats> st(mg->n);
+  const int rc = run_ranks(mg, [&](int r) {
+    return dist_load_packed(mg->ctx[r], key4 ? key4 + lo[r] * 4 : nullptr, strand ? strand + lo[r] : nullptr,
+                            rest4 ? rest4 + lo[r] * 4 : nullptr, lo[r + 1] - lo[r], lo[r], seqx_len, seqy_len, flags, &st[r]);
+  });
+  if (rc) return rc;
+  if (stats) {
+    *stats = st[0];
+    for (int r = 1; r < mg->n; ++r) {
+      stats->n_launches += st[r].n_launches;
+      stats->ms_stage[RK_ST_H2D] = std::max(stats->ms_stage[RK_ST_H2D], st[r].ms_stage[RK_ST_H2D]);
     }
   }
   mg->have_load = true;

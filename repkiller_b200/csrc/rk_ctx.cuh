@@ -202,6 +202,9 @@ struct CsvScratch {
 };
 // the parse's events on ctx->ev, after the ones a load records (0..7)
 enum { EV_CSV_UP0 = 8, EV_CSV_UP1, EV_CSV_PARSED };
+// rk_dist_load_packed's copies of host arrays: key4 and strand on the context's stream, rest4 on the copy stream
+enum { EV_PK_UP0 = EV_CSV_PARSED + 1, EV_PK_UP1, EV_PK_REST };
+static_assert(EV_PK_REST < RK_NSTAGES + 2, "the events fit rk_ctx::ev");
 
 // What a load writes and a grouping only reads: the load's sizes, the records (staged, or the caller's device pointer),
 // the processing order, the bucket sorts of both axes and h (carve_load), plus the side copy of a compact load.  A
