@@ -169,11 +169,16 @@ int rk_sort_groups(rk_ctx *ctx, unsigned flags, rk_result *out);
 
 /* Per-group statistics of the last rk_group / rk_sort_groups (not part of the reference's output file; its groups are the
  * FragsGroups of src/commonFunctions.cpp:56-76 in creation order): one entry per group id.  x/y span = [min start,
- * max(start + length)); mean_identity = mean of the identity column; multiplicity = sum of lengths / X span (how many
- * copies cover the span).  Integers are exact; the two doubles agree with a sequential evaluation to ~1e-15 relative.
+ * max(start + length)), the ends 64-bit (they can pass 2^32).  multiplicity = (double)L / (double)(x_hi - x_lo), L the
+ * exact sum of the lengths (how many copies cover the span), 0 for an empty span.  mean_identity = RN(S) / (double)count,
+ * S the exact sum of the members' identity column and RN round to nearest even; NaN (bits 0xFFF8000000000000, the
+ * column's 0xFFC00000 widened) if a member is NaN, otherwise +inf if a member is +inf.  Every field is exact by that
+ * definition, so it is bit-identical in every run, on a view, and over any number of ranks.  An identity outside the
+ * range K1 produces returns RK_ERR_INTERNAL.
  * stats: pinned host array owned by the context (valid until the next call), d_stats: the same on the device. */
 typedef struct {
-  uint32_t count, x_lo, x_hi, y_lo, y_hi, first_line;
+  uint32_t count, x_lo, y_lo, first_line;
+  uint64_t x_hi, y_hi;
   double mean_identity, multiplicity;
 } rk_group_stats;
 int rk_group_statistics(rk_ctx *ctx, unsigned flags, const rk_group_stats **stats, const rk_group_stats **d_stats, uint64_t *n_groups);

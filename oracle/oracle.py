@@ -152,22 +152,60 @@ def write_input_csv(path: str, records: np.ndarray, lx_header: int, ly_header: i
         raise OSError(f"cannot write {path}")
 
 
-def group_statistics(records: np.ndarray, g: OracleGroups) -> np.ndarray:
-    """sequential per-group reduction over the oracle's groups (checker of rk_group_statistics)"""
+NAN_BITS = 0xFFF8000000000000   # the identity column's NaN (0xFFC00000) widened to binary64
+
+
+def _to_f64(v: np.ndarray) -> np.ndarray:
+    """uint64 -> float64 rounded to nearest even (Python's int -> float) for the values above 2^53"""
+    out = v.astype(np.float64)
+    big = np.flatnonzero(v >= np.uint64(1 << 53))
+    out[big] = [float(int(x)) for x in v[big]]
+    return out
+
+
+def group_statistics(records: np.ndarray, order, gid=None, identity=None) -> np.ndarray:
+    """rk_group_statistics by its definition (include/rk_b200.h), evaluated exactly: one row per group of the output lines
+    (order: file index of each line, gid: nondecreasing dense group ids, identity: the float32 identity column).
+    Integers from uint64 reductions; mean_identity = math.fsum of the members (the exactly rounded sum) / count, NaN
+    (NAN_BITS) if a member is NaN, else +inf if one is +inf; multiplicity = float(sum of lengths) / float(X span).
+    `order` may also be the OracleGroups of group(): its order, out_gid and identity are used."""
+    import math
     from repkiller_b200.capi import GROUP_STATS_DTYPE
-    L = lib()
-    L.rko_group_statistics.argtypes = [C.c_void_p, C.POINTER(_Result), C.c_void_p]
-    L.rko_group_statistics.restype = C.c_int
-    r = _Result()
-    r.n_kept, r.n_groups = g.n_kept, g.n_groups
-    keep = [np.ascontiguousarray(g.order), np.ascontiguousarray(g.out_gid), np.ascontiguousarray(g.identity)]
-    r.order = keep[0].ctypes.data_as(C.POINTER(C.c_uint32))
-    r.out_gid = keep[1].ctypes.data_as(C.POINTER(C.c_uint32))
-    r.identity = keep[2].ctypes.data_as(C.POINTER(C.c_float))
-    rec = np.ascontiguousarray(records)
-    out = np.zeros(g.n_groups, dtype=GROUP_STATS_DTYPE)
-    if L.rko_group_statistics(rec.ctypes.data, C.byref(r), out.ctypes.data):
-        raise ValueError("rko_group_statistics failed")
+    if isinstance(order, OracleGroups):
+        order, gid, identity = order.order, order.out_gid, order.identity
+    order = np.asarray(order, np.int64)
+    gid = np.asarray(gid, np.int64)
+    ident = np.asarray(identity, np.float32).astype(np.float64)
+    m = order.shape[0]
+    if m == 0:
+        return np.zeros(0, GROUP_STATS_DTYPE)
+    starts = np.r_[0, np.flatnonzero(gid[1:] != gid[:-1]) + 1]
+    n_groups = starts.shape[0]
+    if (gid[starts] != gid[0] + np.arange(n_groups)).any():
+        raise ValueError("group ids are not dense and nondecreasing")
+    count = np.diff(np.r_[starts, m])
+    xs, ys, ln = (np.asarray(records[f])[order].astype(np.uint64) for f in ("xStart", "yStart", "length"))
+    out = np.zeros(n_groups, GROUP_STATS_DTYPE)
+    out["count"], out["first_line"] = count, starts
+    out["x_lo"], out["y_lo"] = np.minimum.reduceat(xs, starts), np.minimum.reduceat(ys, starts)
+    out["x_hi"], out["y_hi"] = np.maximum.reduceat(xs + ln, starts), np.maximum.reduceat(ys + ln, starts)
+    span = out["x_hi"] - np.minimum.reduceat(xs, starts)
+    total = np.add.reduceat(ln, starts)
+    mult = np.zeros(n_groups)
+    nz = span > 0
+    mult[nz] = _to_f64(total[nz]) / _to_f64(span[nz])
+    out["multiplicity"] = mult
+    has_nan = np.add.reduceat(np.isnan(ident).astype(np.int64), starts) > 0
+    has_inf = np.add.reduceat(np.isposinf(ident).astype(np.int64), starts) > 0
+    s = ident[starts].copy()                      # singletons
+    vals = ident.tolist()
+    for k in np.flatnonzero((count > 1) & ~has_nan & ~has_inf).tolist():
+        a = int(starts[k])
+        s[k] = math.fsum(vals[a:a + int(count[k])])
+    s[has_inf] = math.inf
+    mean = s / count.astype(np.float64)
+    mean.view(np.uint64)[has_nan] = np.uint64(NAN_BITS)
+    out["mean_identity"] = mean
     return out
 
 

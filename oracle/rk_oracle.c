@@ -571,33 +571,3 @@ int rko_write_input_csv(const char *path, const rko_frag *recs, uint64_t n, uint
   }
   return fclose(f) ? -1 : 0;
 }
-
-/* rk_group_statistics checker: plain sequential sums over the output lines of every group (double accumulators). */
-int rko_group_statistics(const rko_frag *recs, const rko_result *r, rko_group_stats *out) {
-  uint64_t j = 0;
-  for (uint64_t g = 0; g < r->n_groups; ++g) {
-    rko_group_stats s;
-    memset(&s, 0, sizeof s);
-    s.x_lo = s.y_lo = 0xFFFFFFFFu;
-    s.first_line = (uint32_t)j;
-    double sum_len = 0.0, sum_ident = 0.0;
-    while (j < r->n_kept && r->out_gid[j] == g) {
-      const rko_frag *f = &recs[r->order[j]];
-      const uint32_t x0 = (uint32_t)f->xStart, x1 = (uint32_t)(f->xStart + f->length);
-      const uint32_t y0 = (uint32_t)f->yStart, y1 = (uint32_t)(f->yStart + f->length);
-      if (x0 < s.x_lo) s.x_lo = x0;
-      if (x1 > s.x_hi) s.x_hi = x1;
-      if (y0 < s.y_lo) s.y_lo = y0;
-      if (y1 > s.y_hi) s.y_hi = y1;
-      sum_len += (double)f->length;
-      sum_ident += (double)r->identity[j];
-      ++s.count;
-      ++j;
-    }
-    if (s.count == 0) return -1; /* group ids are dense */
-    s.mean_identity = sum_ident / (double)s.count;
-    s.multiplicity = (s.x_hi - s.x_lo) ? sum_len / (double)(s.x_hi - s.x_lo) : 0.0;
-    out[g] = s;
-  }
-  return j == r->n_kept ? 0 : -1;
-}

@@ -76,15 +76,6 @@ int rko_write_input_csv(const char *path, const rko_frag *recs, uint64_t n, uint
 /* libstdc++ std::sort order of idx[0..n) under comp(a,b) = h[a] < h[b] (sort_groups, commonFunctions.cpp:158) */
 void rko_std_sort_by_key(uint32_t *idx, uint64_t n, const uint64_t *h);
 
-/* Per-group statistics over the reference's groups (the FragsGroups of commonFunctions.cpp:56-76 as save_frag_pair
- * writes them, :117-129): a sequential reduction, one entry per group id.  Checker for rk_group_statistics (the
- * reference computes no such statistics; the definitions are in include/rk_b200.h). */
-typedef struct {
-  uint32_t count, x_lo, x_hi, y_lo, y_hi, first_line;
-  double mean_identity, multiplicity;
-} rko_group_stats;
-int rko_group_statistics(const rko_frag *recs, const rko_result *r, rko_group_stats *out /* r->n_groups entries */);
-
 /* One SequenceOcupationList (SequenceOcupationList.cpp:3-96) with a 64-bit tag per entry in place of the FragsGroup
  * pointer: the checker of rk_sol_*.  insert returns -1 when center/100 lies beyond the lists, -2 when memory runs out
  * (nothing inserted); get stores the tag of the winner (0: none) and returns -2 when a probe would read beyond the

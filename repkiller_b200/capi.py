@@ -31,7 +31,7 @@ SYMBOLS = ["rk_create", "rk_create_view", "rk_create_error", "rk_destroy", "rk_l
            "rk_multi_load_aos", "rk_multi_load_csv", "rk_multi_load_packed", "rk_multi_group", "rk_multi_info", "rk_multi_format_lines", "rk_multi_group_statistics",
            "rk_multi_create_view"]
 DIST_ID_BYTES, DIST_BLOB_BYTES = 128, 128
-GROUP_STATS_DTYPE = np.dtype([("count", "<u4"), ("x_lo", "<u4"), ("x_hi", "<u4"), ("y_lo", "<u4"), ("y_hi", "<u4"), ("first_line", "<u4"),
+GROUP_STATS_DTYPE = np.dtype([("count", "<u4"), ("x_lo", "<u4"), ("y_lo", "<u4"), ("first_line", "<u4"), ("x_hi", "<u8"), ("y_hi", "<u8"),
                               ("mean_identity", "<f8"), ("multiplicity", "<f8")])
 
 
@@ -98,6 +98,7 @@ def load_library():
     L.rk_load_csv.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint, C.POINTER(_LoadStats),
                               C.POINTER(_CsvStats)]
     L.rk_group.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_uint, C.POINTER(_Result)]
+    L.rk_sort_groups.argtypes = [C.c_void_p, C.c_uint, C.POINTER(_Result)]
     L.rk_diagonal_func.argtypes = [C.c_void_p, C.c_void_p]
     L.rk_debug_fetch.argtypes = [C.c_void_p, C.c_char_p, C.c_void_p, C.c_uint64]
     L.rk_debug_fetch.restype = C.c_int64
@@ -310,6 +311,12 @@ class Context:
                       arr(r.identity, np.float32),
                       {"order": r.d_order, "gid": r.d_gid, "repval": r.d_repval, "identity": r.d_identity},
                       {STAGES[i]: r.ms_stage[i] for i in range(NSTAGES)}, r.ms_device, r.n_launches)
+
+    def sort_groups(self, host_result: bool = True, copy: bool = True) -> Groups:
+        """rk_sort_groups: after group(..., sort=False), the members of every group ordered on the device (sort_groups)"""
+        r = _Result()
+        self._check(self._L.rk_sort_groups(self._h, F_HOST_RESULT if host_result else 0, C.byref(r)))
+        return _groups_of(r, host_result, copy)
 
     def format_lines(self, first_line: int = 0, n_lines: int | None = None) -> bytes:
         """Text of the output lines of the last group() (commonFunctions.cpp:101-115), formatted on the device; the

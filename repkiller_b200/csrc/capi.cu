@@ -792,17 +792,26 @@ int group_stats_run(rk_ctx *ctx, unsigned flags, const u32 *order, const u32 *gi
                     const LineRow *rows, u32 m, u64 ng, u32 gid_base, u32 line_off) {
   CK(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
+  // d_stats: the public array, then K8's error word and its accumulators (scratch)
   const u64 need = ng * sizeof(rk_group_stats), grown = (ng + ng / 8 + 1024) * sizeof(rk_group_stats);
-  int rc = ctx->d_stats.reserve(need > ctx->d_stats.cap() ? grown : need, st, ctx->err);
+  const u64 acc_off = align_up(need, 256) + 256;
+  const u64 d_need = acc_off + ng * sizeof(StatsAcc), d_grown = d_need + (ng / 8 + 1024) * (sizeof(rk_group_stats) + sizeof(StatsAcc));
+  int rc = ctx->d_stats.reserve(d_need > ctx->d_stats.cap() ? d_grown : d_need, st, ctx->err);
   if (rc) return rc;
-  launch_group_stats(order, gid, identity, rec4, rows, m, (u32)ng, gid_base, line_off, (rk_group_stats_dev *)ctx->d_stats.ptr(), st);
+  char *base = (char *)ctx->d_stats.ptr();
+  u32 *err = (u32 *)(base + acc_off - 256);
+  launch_group_stats(order, gid, identity, rec4, rows, m, (u32)ng, gid_base, line_off, (rk_group_stats_dev *)base,
+                     (StatsAcc *)(base + acc_off), err, st);
+  if (ng) CK(cudaMemcpyAsync(&ctx->h_cnt->pad, err, sizeof(u32), cudaMemcpyDeviceToHost, st));
   if ((flags & RK_F_HOST_RESULT) && ng) {
     rc = ctx->h_stats.reserve(need > ctx->h_stats.cap() ? grown : need, st, ctx->err);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(ctx->h_stats.ptr(), ctx->d_stats.ptr(), need, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(ctx->h_stats.ptr(), base, need, cudaMemcpyDeviceToHost, st));
   }
   CK(cudaStreamSynchronize(st));
   CK(cudaGetLastError());
+  if (ng && ctx->h_cnt->pad)
+    return fail(ctx, RK_ERR_INTERNAL, "an identity outside [100/2^32, 100*2^64] (nor 0, NaN or +inf): the exact sum cannot hold it");
   return RK_OK;
 }
 }  // namespace rk
@@ -810,7 +819,7 @@ int group_stats_run(rk_ctx *ctx, unsigned flags, const u32 *order, const u32 *gi
 extern "C" {
 
 int rk_group_statistics(rk_ctx *ctx, unsigned flags, const rk_group_stats **stats, const rk_group_stats **d_stats, uint64_t *n_groups) {
-  static_assert(sizeof(rk_group_stats) == sizeof(rk_group_stats_dev) && sizeof(rk_group_stats) == 40, "stats layout");
+  static_assert(sizeof(rk_group_stats) == sizeof(rk_group_stats_dev) && sizeof(rk_group_stats) == 48, "stats layout");
   if (!ctx) return RK_ERR_ARG;
   if (!ctx->loaded || !ctx->have_group) return fail(ctx, RK_ERR_STATE, "rk_group_statistics before rk_group");
   CK(cudaSetDevice(ctx->device));

@@ -371,13 +371,23 @@ int launch_member_keys(const u64 *y, const u64 *d, u32 m, u32 *h, u32 *idx, floa
 
 // K8: per-group statistics over the output arrays (same layout as rk_group_stats of include/rk_b200.h)
 struct rk_group_stats_dev {
-  u32 count, x_lo, x_hi, y_lo, y_hi, first_line;
+  u32 count, x_lo, y_lo, first_line;
+  u64 x_hi, y_hi;
   double mean_identity, multiplicity;
+};
+// K8's per-group accumulators: integers only, so their final values do not depend on the order of the atomics
+struct StatsAcc {
+  u32 count, x_lo, y_lo, first_line;
+  u64 x_hi, y_hi, len_sum;
+  u64 digit[4];    // identity * 2^49 in 32-bit digits, each column summed over the members
+  u64 n_nan_inf;   // NaN members in the low word, +inf members in the high word
 };
 // The span fields come from rec4[2 * order[j]] (one GPU) or from rows[j] (rows != nullptr: a rank of a partitioned
 // comparison, whose groups gid_base .. gid_base+n_groups-1 are all on the rank and whose line j is line line_off + j).
+// acc: n_groups accumulators of scratch; *err ends nonzero when an identity lies outside K1's bound (see k8_stats.cu).
 int launch_group_stats(const u32 *out_order, const u32 *out_gid, const float *out_identity, const uint4 *rec4, const LineRow *rows,
-                       u32 m, u32 n_groups, u32 gid_base, u32 line_off, rk_group_stats_dev *st, cudaStream_t stream);
+                       u32 m, u32 n_groups, u32 gid_base, u32 line_off, rk_group_stats_dev *st, StatsAcc *acc, u32 *err,
+                       cudaStream_t stream);
 
 // K9 (k9_csv.cu): CSV rows parsed on the device (rk_load_csv).  Row status bytes:
 constexpr u8 CSV_REJECT = 0, CSV_ACCEPT = 1, CSV_HOST = 2, CSV_HOST_ACCEPT = 3;  // host: readFragment decides
